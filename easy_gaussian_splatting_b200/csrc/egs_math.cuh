@@ -243,11 +243,18 @@ EGS_HD void pack_tile_rect(int32_t x0, int32_t y0, int32_t x1, int32_t y1, int32
   extent = empty ? 0 : (w | (h << 16));
 }
 
+// Camera gradient of one (camera, Gaussian) pair, 15 floats: v_R[9] (row major) and v_t[3] of the view matrix's
+// top 3x4 block, then v_campos[3], the gradient w.r.t. the camera centre the SH directions are taken from.
+constexpr int kCamGradFloats = 15;
+
 // VJP of project_fwd for a visible Gaussian (SURVEY.md A-8).  Accumulates (+=) into
 // v_mean[3], v_quat[4], v_scale[3].
+// v_cam (nullable, with the Gaussian's world-space mean): also accumulates v_R and v_t (entries 0..11 of the camera
+// gradient above) through mean_c = R m + t and cov_c = R Sigma R^T.  A literal nullptr compiles the block out.
 EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera& cam, float v_m2x, float v_m2y,
                         float v_depth, float v_ca, float v_cb, float v_cc, const ProjOut& o, float v_mean[3],
-                        float v_quat[4], float v_scale[3], float v_comp = 0.f, float eps2d = 0.f) {
+                        float v_quat[4], float v_scale[3], float v_comp = 0.f, float eps2d = 0.f,
+                        float* v_cam = nullptr, const float* mean = nullptr) {
   // conic = inverse(cov2d'):  V = -Q * G * Q with G = [[v_ca, v_cb/2],[v_cb/2, v_cc]]
   float q00 = o.ca, q01 = o.cb, q11 = o.cc;
   float g00 = v_ca, g01 = 0.5f * v_cb, g11 = v_cc;
@@ -301,6 +308,32 @@ EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera&
   v_mean[2] += W[2] * vx + W[5] * vy + W[8] * vz;
   // v_Sigma = W^T v_Sc W
   float vkm[9] = {vk00, vk01, vk02, vk10, vk11, vk12, vk20, vk21, vk22};
+  if (v_cam != nullptr) {
+    // mean_c = W m + t: v_W += v_mean_c m^T, v_t += v_mean_c
+    const float vc[3] = {vx, vy, vz};
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+#pragma unroll
+      for (int j = 0; j < 3; ++j) v_cam[i * 3 + j] += vc[i] * mean[j];
+      v_cam[9 + i] += vc[i];
+    }
+    // cov_c = W Sigma W^T: v_W += (v_Sc + v_Sc^T) W Sigma
+    const float* S = st.S;
+    const float Sm[9] = {S[0], S[1], S[2], S[1], S[3], S[4], S[2], S[4], S[5]};
+    float WS[9];
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int j = 0; j < 3; ++j)
+        WS[i * 3 + j] = W[i * 3 + 0] * Sm[0 * 3 + j] + W[i * 3 + 1] * Sm[1 * 3 + j] + W[i * 3 + 2] * Sm[2 * 3 + j];
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int j = 0; j < 3; ++j)
+        v_cam[i * 3 + j] += (vkm[i * 3 + 0] + vkm[0 * 3 + i]) * WS[0 * 3 + j] +
+                            (vkm[i * 3 + 1] + vkm[1 * 3 + i]) * WS[1 * 3 + j] +
+                            (vkm[i * 3 + 2] + vkm[2 * 3 + i]) * WS[2 * 3 + j];
+  }
   float Tm[9];  // Tm = vSc * W
 #pragma unroll
   for (int i = 0; i < 3; ++i)
@@ -431,9 +464,11 @@ EGS_HD void sh_color_fwd(int degree, const float mean[3], const Camera& cam, con
 }
 
 // VJP of sh_color_fwd.  rgb_stored is the forward output (gradient passes where it is > 0).
-// Accumulates (+=) into vco[48] and v_mean[3].
+// Accumulates (+=) into vco[48] and v_mean[3].  v_cam (nullable): dir = mean - campos, so the direction gradient is
+// also subtracted from v_campos (entries 12..14 of the camera gradient, see project_bwd).
 EGS_HD void sh_color_bwd(int degree, const float mean[3], const Camera& cam, const float (&co)[48],
-                         const float rgb_stored[3], const float v_rgb_in[3], float (&vco)[48], float v_mean[3]) {
+                         const float rgb_stored[3], const float v_rgb_in[3], float (&vco)[48], float v_mean[3],
+                         float* v_cam = nullptr) {
   const int nb = (degree + 1) * (degree + 1);
   float v_rgb[3];
   v_rgb[0] = (rgb_stored[0] > 0.f) ? v_rgb_in[0] : 0.f;
@@ -460,10 +495,50 @@ EGS_HD void sh_color_bwd(int degree, const float mean[3], const Camera& cam, con
     float vx, vy, vz;
     sh_basis_vjp(degree, x, y, z, g, vx, vy, vz);
     float dp = vx * x + vy * y + vz * z;
-    v_mean[0] += (vx - dp * x) * inorm;
-    v_mean[1] += (vy - dp * y) * inorm;
-    v_mean[2] += (vz - dp * z) * inorm;
+    const float d0 = (vx - dp * x) * inorm, d1 = (vy - dp * y) * inorm, d2 = (vz - dp * z) * inorm;
+    v_mean[0] += d0;
+    v_mean[1] += d1;
+    v_mean[2] += d2;
+    if (v_cam != nullptr) { v_cam[12] -= d0; v_cam[13] -= d1; v_cam[14] -= d2; }
   }
+}
+
+// The [4,4] gradient of one view matrix V from its camera gradient summed over the Gaussians (v_R, v_t, g = v_campos,
+// see project_bwd).  campos = inv(V)[:3,3] with inv(V) = [[A, c], [0, 1]] (A = R^-1 by the same adjugate as
+// load_camera, c = campos), and the VJP of a matrix inverse is -inv(V)^T G inv(V)^T with g in column 3 of G:
+//   v_V = [[v_R, v_t], [0, 0]] - [[(A^T g) c^T, A^T g], [(c.g) c^T, c.g]]
+// The bottom row is not zero when the SH directions carry a gradient, as in gsplat.
+EGS_HD void viewmat_grad_finalize(const float* V, const float vcam[kCamGradFloats], float out[16]) {
+  const float r[9] = {V[0], V[1], V[2], V[4], V[5], V[6], V[8], V[9], V[10]};
+  const float t[3] = {V[3], V[7], V[11]};
+  float a[9];
+  a[0] = r[4] * r[8] - r[5] * r[7];
+  a[1] = r[2] * r[7] - r[1] * r[8];
+  a[2] = r[1] * r[5] - r[2] * r[4];
+  a[3] = r[5] * r[6] - r[3] * r[8];
+  a[4] = r[0] * r[8] - r[2] * r[6];
+  a[5] = r[2] * r[3] - r[0] * r[5];
+  a[6] = r[3] * r[7] - r[4] * r[6];
+  a[7] = r[1] * r[6] - r[0] * r[7];
+  a[8] = r[0] * r[4] - r[1] * r[3];
+  const float det = r[0] * a[0] + r[1] * a[3] + r[2] * a[6];
+  const float id = 1.0f / det;
+  float c[3];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) c[i] = -(a[i * 3 + 0] * t[0] + a[i * 3 + 1] * t[1] + a[i * 3 + 2] * t[2]) * id;
+  const float* g = vcam + 12;
+  float Atg[3];  // A^T g, A = a * id
+#pragma unroll
+  for (int i = 0; i < 3; ++i) Atg[i] = (a[0 * 3 + i] * g[0] + a[1 * 3 + i] * g[1] + a[2 * 3 + i] * g[2]) * id;
+  const float cg = c[0] * g[0] + c[1] * g[1] + c[2] * g[2];
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+#pragma unroll
+    for (int j = 0; j < 3; ++j) out[i * 4 + j] = vcam[i * 3 + j] - Atg[i] * c[j];
+    out[i * 4 + 3] = vcam[9 + i] - Atg[i];
+    out[12 + i] = -(cg * c[i]);
+  }
+  out[15] = -cg;
 }
 
 }  // namespace egs

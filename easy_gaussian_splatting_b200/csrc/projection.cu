@@ -335,22 +335,136 @@ struct ProjBwdParams {
   float2* absgrad;  // nullable [C,N]: sum over pixels of |d L / d means2d|, copied out of the gradient records
   int n_begin, n_end;  // projection_bwd_sh16_kernel: the Gaussians of this launch (chunked launches let the gradient
                        // exchange of one chunk overlap the backward pass of the next, egs_projection_bwd_range)
+  // viewmat gradients (the VG instantiations only): per camera, one 16-float partial of the camera gradient
+  // (egs_math.cuh kCamGradFloats, padded) per warp of the launch, camera-major: [C][gridDim.x * 4][16]; the counters
+  // [C] of viewmat_grad_finalize_kernel are cleared by block 0
+  float* cam_partials;
+  int* cam_counters;
 };
 
 constexpr int kProjBwdThreads = 128;
 constexpr int kMaxCamerasSmem = 64;
 
+// ---- gradients w.r.t. the view matrices -------------------------------------------------------------------------------
+// The camera gradient is a sum over all Gaussians per camera.  Each warp sums its 32 lanes' contributions to one camera
+// with a fixed shuffle tree and lane 0 stores the warp's partial; viewmat_grad_finalize_kernel then sums the partials
+// in a fixed order.  No float atomics anywhere: the same gradient records give bit-identical v_viewmats.
+constexpr int kCamPartialFloats = 16;
+constexpr int kVgFinalizeThreads = 256;
+constexpr int kVgMaxSlices = 32;
+
+// Warp partials of a launch of the backward kernels (both run 4 warps per block).
+inline int64_t vg_partial_slots(int64_t n_gauss) { return ceil_div(n_gauss, 128) * 4; }
+// Blocks per camera of the finalize kernel: each sums one contiguous slice of the partials.
+inline int vg_slices(int64_t slots) {
+  const int64_t s = ceil_div(slots, 4 * kVgFinalizeThreads);
+  return (int)(s < 1 ? 1 : s > kVgMaxSlices ? kVgMaxSlices : s);
+}
+
+// Warp-uniform `any`: false = no lane of the warp sees this camera, the partial is zero (no shuffles).
+__device__ __forceinline__ void store_cam_partial(float (&v)[kCamGradFloats], bool any, float* __restrict__ dst, int lane) {
+  if (any) {
+#pragma unroll
+    for (int k = 0; k < kCamGradFloats; ++k)
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) v[k] += __shfl_down_sync(0xffffffffu, v[k], off);
+  }
+  if (lane == 0) {
+    float4* d = reinterpret_cast<float4*>(dst);
+    if (any) {
+      d[0] = make_float4(v[0], v[1], v[2], v[3]);
+      d[1] = make_float4(v[4], v[5], v[6], v[7]);
+      d[2] = make_float4(v[8], v[9], v[10], v[11]);
+      d[3] = make_float4(v[12], v[13], v[14], 0.f);
+    } else {
+      const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+      d[0] = z; d[1] = z; d[2] = z; d[3] = z;
+    }
+  }
+}
+
+__device__ __forceinline__ float* cam_partial(const ProjBwdParams& p, int c, int warp) {
+  const size_t slots = (size_t)gridDim.x * 4;
+  return p.cam_partials + ((size_t)c * slots + (size_t)blockIdx.x * 4 + warp) * kCamPartialFloats;
+}
+
+__device__ __forceinline__ void clear_cam_counters(const ProjBwdParams& p) {
+  if (blockIdx.x == 0)
+    for (int c = threadIdx.x; c < p.C; c += blockDim.x) p.cam_counters[c] = 0;
+}
+
+// grid (slices, C): block (s, c) sums slice s of camera c's warp partials (strided per thread, then a fixed tree) into
+// slices[c][s]; the last block of a camera to finish sums the slices in order and writes v_viewmats[c] (16 floats).
+__global__ void __launch_bounds__(kVgFinalizeThreads) viewmat_grad_finalize_kernel(
+    int n_slots, const float* __restrict__ partials, float* __restrict__ slices, int* __restrict__ counters,
+    const float* __restrict__ viewmats, float* __restrict__ v_viewmats) {
+  __shared__ float red[kCamGradFloats][kVgFinalizeThreads];
+  __shared__ bool last;
+  const int s = blockIdx.x, S = gridDim.x, c = blockIdx.y, tid = threadIdx.x;
+  const int per = (n_slots + S - 1) / S;
+  const int begin = s * per, end = min(n_slots, begin + per);
+  float acc[kCamGradFloats];
+#pragma unroll
+  for (int k = 0; k < kCamGradFloats; ++k) acc[k] = 0.f;
+  const float4* src = reinterpret_cast<const float4*>(partials + (size_t)c * n_slots * kCamPartialFloats);
+  for (int i = begin + tid; i < end; i += kVgFinalizeThreads) {
+    const float4 a = src[(size_t)i * 4 + 0], b = src[(size_t)i * 4 + 1], d = src[(size_t)i * 4 + 2], e = src[(size_t)i * 4 + 3];
+    acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
+    acc[4] += b.x; acc[5] += b.y; acc[6] += b.z; acc[7] += b.w;
+    acc[8] += d.x; acc[9] += d.y; acc[10] += d.z; acc[11] += d.w;
+    acc[12] += e.x; acc[13] += e.y; acc[14] += e.z;
+  }
+#pragma unroll
+  for (int k = 0; k < kCamGradFloats; ++k) red[k][tid] = acc[k];
+  __syncthreads();
+  for (int h = kVgFinalizeThreads / 2; h > 0; h >>= 1) {
+    if (tid < h)
+#pragma unroll
+      for (int k = 0; k < kCamGradFloats; ++k) red[k][tid] += red[k][tid + h];
+    __syncthreads();
+  }
+  float* my_slice = slices + ((size_t)c * S + s) * kCamPartialFloats;
+  if (tid < kCamGradFloats) my_slice[tid] = red[tid][0];
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) last = atomicAdd(counters + c, 1) == S - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  if (tid < kCamGradFloats) {
+    float sum = 0.f;
+    for (int j = 0; j < S; ++j) sum += __ldcg(slices + ((size_t)c * S + j) * kCamPartialFloats + tid);
+    red[tid][0] = sum;
+  }
+  __syncthreads();
+  if (tid == 0) {
+    float vcam[kCamGradFloats], out[16];
+#pragma unroll
+    for (int k = 0; k < kCamGradFloats; ++k) vcam[k] = red[k][0];
+    viewmat_grad_finalize(viewmats + (size_t)c * 16, vcam, out);
+#pragma unroll
+    for (int k = 0; k < 16; ++k) v_viewmats[(size_t)c * 16 + k] = out[k];
+    counters[c] = 0;
+  }
+}
+
 // One thread per Gaussian, looping over cameras: gradients summed over cameras stay in registers,
 // so there are no atomics for any C.  Every output element is written exactly once (zeros for culled
 // Gaussians and inactive SH bands), so the caller does not have to clear the gradient buffers.
-template <bool VEC4>
+// VG: also the view-matrix gradient partials (see store_cam_partial).  Every lane of a warp then runs the camera loop
+// (the shuffles need all 32), lanes past N as if they saw nothing.
+template <bool VEC4, bool VG = false>
 __global__ void __launch_bounds__(kProjBwdThreads) projection_bwd_kernel(const ProjBwdParams p) {
   __shared__ Camera cams[kMaxCamerasSmem];
   for (int c = threadIdx.x; c < p.C && c < kMaxCamerasSmem; c += kProjBwdThreads)
     load_camera(p.viewmats + (size_t)c * 16, p.Ks + (size_t)c * 9, cams[c]);
+  if constexpr (VG) clear_cam_counters(p);
   __syncthreads();
-  const int n = blockIdx.x * kProjBwdThreads + threadIdx.x;
-  if (n >= p.N) return;
+  const int n_lane = blockIdx.x * kProjBwdThreads + threadIdx.x;
+  if (!VG && n_lane >= p.N) return;
+  const bool in_range = !VG || n_lane < p.N;
+  const int n = VG ? min(n_lane, p.N - 1) : n_lane;  // (VG) lanes past N read Gaussian N - 1 and write nothing
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 
   float mean[3], quat[4], scale[3];
   mean[0] = __ldg(p.means + 3 * (size_t)n + 0);
@@ -375,9 +489,14 @@ __global__ void __launch_bounds__(kProjBwdThreads) projection_bwd_kernel(const P
 
   for (int c = 0; c < p.C; ++c) {
     const size_t idx = (size_t)c * p.N + n;
-    const bool vis = p.radii[idx] > 0;
+    const bool vis = in_range && p.radii[idx] > 0;
     float v_rgb[3] = {0.f, 0.f, 0.f};
-    if (p.absgrad != nullptr) {
+    float vcam[kCamGradFloats];
+    if constexpr (VG) {
+#pragma unroll
+      for (int k = 0; k < kCamGradFloats; ++k) vcam[k] = 0.f;
+    }
+    if (p.absgrad != nullptr && in_range) {
       float2 ag = make_float2(0.f, 0.f);
       if (vis) { const float4 g2a = p.v_splats[idx * 3 + 2]; ag = make_float2(g2a.y, g2a.z); }
       p.absgrad[idx] = ag;
@@ -401,22 +520,26 @@ __global__ void __launch_bounds__(kProjBwdThreads) projection_bwd_kernel(const P
       //  off-screen test cannot fire differently because it only depends on the same values.)
       float v_comp = 0.f, w_opac = 1.f;
       if (p.antialiased) { v_comp = g1.y * __ldg(p.opacities + n); w_opac = o.comp; }
-      if (o.radius > 0) project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, v_comp, p.eps2d);
+      if (o.radius > 0)
+        project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, v_comp, p.eps2d,
+                    VG ? vcam : nullptr, mean);
       v_opac += g1.y * w_opac;
       v_rgb[0] = g1.z; v_rgb[1] = g1.w; v_rgb[2] = g2.x;
       if (has_sh) {
         if (!co_loaded) { load_coeffs<VEC4>(p.sh + (size_t)n * p.K * 3, nb * 3, co); co_loaded = true; }
         const float* col = p.colors + idx * 3;
         const float rgb_stored[3] = {col[0], col[1], col[2]};
-        sh_color_bwd(p.sh_degree, mean, *cam, co, rgb_stored, v_rgb, vco, v_mean);
+        sh_color_bwd(p.sh_degree, mean, *cam, co, rgb_stored, v_rgb, vco, v_mean, VG ? vcam : nullptr);
       } else {
         v_rgb_sum[0] += v_rgb[0]; v_rgb_sum[1] += v_rgb[1]; v_rgb_sum[2] += v_rgb[2];
       }
     }
-    if (!has_sh && p.colors_per_camera) {
+    if (!has_sh && p.colors_per_camera && in_range) {
       p.v_sh[idx * 3 + 0] = v_rgb[0]; p.v_sh[idx * 3 + 1] = v_rgb[1]; p.v_sh[idx * 3 + 2] = v_rgb[2];
     }
+    if constexpr (VG) store_cam_partial(vcam, __ballot_sync(0xffffffffu, vis) != 0, cam_partial(p, c, warp), lane);
   }
+  if (!in_range) return;
 
   p.v_means[3 * (size_t)n + 0] = v_mean[0]; p.v_means[3 * (size_t)n + 1] = v_mean[1]; p.v_means[3 * (size_t)n + 2] = v_mean[2];
   reinterpret_cast<float4*>(p.v_quats)[n] = make_float4(v_quat[0], v_quat[1], v_quat[2], v_quat[3]);
@@ -463,12 +586,16 @@ constexpr int kPB2Warps = kPB2Threads / 32;
 #define EGS_PB_MIN_CTAS 3
 #endif
 #define EGS_PB_BOUNDS __launch_bounds__(kPB2Threads, EGS_PB_MIN_CTAS)
-template <bool AA>  // AA: rasterize_mode="antialiased" (a separate instantiation keeps the classic kernel at 128 registers)
+// AA: rasterize_mode="antialiased" (a separate instantiation keeps the classic kernel at 128 registers).
+// VG: also the view-matrix gradient partials (see store_cam_partial).  The camera loop then runs on every lane of a warp
+// that has a seen Gaussian (the shuffles need all 32); lanes that see nothing only take part in the sums.
+template <bool AA, bool VG = false>
 __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) {
   extern __shared__ __align__(16) float smem_pb[];
   __shared__ Camera cams[kMaxCamerasSmem];
   for (int c = threadIdx.x; c < p.C && c < kMaxCamerasSmem; c += kPB2Threads)
     load_camera(p.viewmats + (size_t)c * 16, p.Ks + (size_t)c * 9, cams[c]);
+  if constexpr (VG) clear_cam_counters(p);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float* co_tile = smem_pb + (size_t)warp * 32 * kRowStride;                       // coefficients
@@ -483,6 +610,14 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
   if (in_range)
     for (int c = 0; c < p.C; ++c) seen = seen || (p.radii[(size_t)c * p.N + n] > 0);
   const uint32_t seen_mask = __ballot_sync(0xffffffffu, seen);
+  if constexpr (VG) {
+    if (seen_mask == 0)  // the warp sees nothing: zero partials for every camera
+      for (int c = lane; c < p.C; c += 32) {
+        float4* d = reinterpret_cast<float4*>(cam_partial(p, c, warp));
+        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+        d[0] = z; d[1] = z; d[2] = z; d[3] = z;
+      }
+  }
 
   // phase 1: coalesced load of the coefficient rows that are needed; zero the gradient rows
   if (!p.raw) {
@@ -518,16 +653,17 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
       p.absgrad[idx] = ag;
     }
   }
-  if (seen) {
+  if (VG ? seen_mask != 0 : seen) {
+    const int nl = VG ? (in_range ? n : n_base) : n;  // (VG) a lane past the range reads the warp's first Gaussian
     float mean[3], quat[4], scale[3];
-    mean[0] = __ldg(p.means + 3 * (size_t)n + 0);
-    mean[1] = __ldg(p.means + 3 * (size_t)n + 1);
-    mean[2] = __ldg(p.means + 3 * (size_t)n + 2);
-    const float4 q4 = __ldg(reinterpret_cast<const float4*>(p.quats) + n);
+    mean[0] = __ldg(p.means + 3 * (size_t)nl + 0);
+    mean[1] = __ldg(p.means + 3 * (size_t)nl + 1);
+    mean[2] = __ldg(p.means + 3 * (size_t)nl + 2);
+    const float4 q4 = __ldg(reinterpret_cast<const float4*>(p.quats) + nl);
     quat[0] = q4.x; quat[1] = q4.y; quat[2] = q4.z; quat[3] = q4.w;
-    scale[0] = __ldg(p.scales + 3 * (size_t)n + 0);
-    scale[1] = __ldg(p.scales + 3 * (size_t)n + 1);
-    scale[2] = __ldg(p.scales + 3 * (size_t)n + 2);
+    scale[0] = __ldg(p.scales + 3 * (size_t)nl + 0);
+    scale[1] = __ldg(p.scales + 3 * (size_t)nl + 1);
+    scale[2] = __ldg(p.scales + 3 * (size_t)nl + 2);
     if (p.raw) { scale[0] = act_exp(scale[0]); scale[1] = act_exp(scale[1]); scale[2] = act_exp(scale[2]); }
     const float* co = co_tile + lane * kRowStride;
     float* vc = vc_tile + lane * kRowStride;
@@ -538,8 +674,9 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
     float ncol[3];
     int nrad;
     auto fetch = [&](int c) {
-      const size_t idx = (size_t)c * p.N + n;
+      const size_t idx = (size_t)c * p.N + nl;
       nrad = p.radii[idx];
+      if (VG && !in_range) nrad = 0;
       ng0 = p.v_splats[idx * 3 + 0];
       ng1 = p.v_splats[idx * 3 + 1];
       ng2 = p.v_splats[idx * 3 + 2];
@@ -552,7 +689,15 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
       const float4 g0 = ng0, g1 = ng1, g2 = ng2;
       const float col[3] = {ncol[0], ncol[1], ncol[2]};
       if (c + 1 < p.C) fetch(c + 1);
-      if (!(rad > 0)) continue;
+      float vcam[kCamGradFloats];
+      if constexpr (VG) {
+#pragma unroll
+        for (int k = 0; k < kCamGradFloats; ++k) vcam[k] = 0.f;
+      } else {
+        if (!(rad > 0)) continue;
+      }
+      do {  // (VG: lanes that do not see camera c skip to the warp's sum below)
+      if (VG && !(rad > 0)) break;
       Camera cam_local;
       const Camera* cam = &cams[c < kMaxCamerasSmem ? c : 0];
       if (c >= kMaxCamerasSmem) { load_camera(p.viewmats + (size_t)c * 16, p.Ks + (size_t)c * 9, cam_local); cam = &cam_local; }
@@ -569,10 +714,13 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
           float op = __ldg(p.opacities + n);
           if (p.raw) op = act_sigmoid(op);
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, g1.y * op, p.eps2d);
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, g1.y * op, p.eps2d,
+                        VG ? vcam : nullptr, mean);
           v_opac += g1.y * o.comp;
         } else {
-          if (o.radius > 0) project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale);
+          if (o.radius > 0)
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
+                        VG ? vcam : nullptr, mean);
           v_opac += g1.y;
         }
       }
@@ -616,10 +764,14 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
         float vx, vy, vz;
         sh_basis_vjp(p.sh_degree, x, y, z, g, vx, vy, vz);
         const float dp = vx * x + vy * y + vz * z;
-        v_mean[0] += (vx - dp * x) * inorm;
-        v_mean[1] += (vy - dp * y) * inorm;
-        v_mean[2] += (vz - dp * z) * inorm;
+        const float d0 = (vx - dp * x) * inorm, d1 = (vy - dp * y) * inorm, d2 = (vz - dp * z) * inorm;
+        v_mean[0] += d0;
+        v_mean[1] += d1;
+        v_mean[2] += d2;
+        if constexpr (VG) { vcam[12] -= d0; vcam[13] -= d1; vcam[14] -= d2; }  // dir = mean - campos
       }
+      } while (0);
+      if constexpr (VG) store_cam_partial(vcam, __ballot_sync(0xffffffffu, rad > 0) != 0, cam_partial(p, c, warp), lane);
     }
   }
   __syncwarp();
@@ -748,10 +900,20 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
                                int32_t width, int32_t height, float eps2d, const int32_t* radii, const float* colors,
                                const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
                                float* v_scales, float* v_opacities, float* v_sh_coeffs, float* v_sh_rest, float* absgrad,
-                               egs_stream_t stream, int antialiased = 0, int32_t n_begin = 0, int32_t n_end = -1) {
+                               egs_stream_t stream, int antialiased = 0, int32_t n_begin = 0, int32_t n_end = -1,
+                               float* v_viewmats = nullptr, void* workspace = nullptr, int64_t workspace_bytes = 0) {
   const int raw = sh_rest != nullptr;
   EGS_REQUIRE(C >= 0 && N >= 0, "projection_bwd: negative sizes C=%d N=%d", C, N);
   EGS_REQUIRE(sh_degree <= 3, "projection_bwd: sh_degree %d > 3 is not supported", sh_degree);
+  const bool vg = v_viewmats != nullptr;
+  if (vg) {
+    EGS_REQUIRE(n_begin == 0 && (n_end < 0 || n_end == N), "projection_bwd: viewmat gradients need the whole Gaussian range");
+    EGS_REQUIRE(C <= 65535, "projection_bwd: C=%d exceeds 65535 cameras per call", C);
+    EGS_REQUIRE(workspace != nullptr && workspace_bytes >= egs_projection_bwd_viewmats_workspace_bytes(C, N),
+                "projection_bwd: viewmat gradients need %lld workspace bytes (got %lld)",
+                (long long)egs_projection_bwd_viewmats_workspace_bytes(C, N), (long long)workspace_bytes);
+    if (N == 0 && C > 0) EGS_CUDA(cudaMemsetAsync(v_viewmats, 0, sizeof(float) * 16 * (size_t)C, (cudaStream_t)stream));
+  }
   if (N == 0) return 0;
   if (n_end < 0) n_end = N;
   EGS_REQUIRE(0 <= n_begin && n_begin <= n_end && n_end <= N, "projection_bwd: Gaussian range [%d, %d) outside [0, %d)", n_begin, n_end, N);
@@ -767,7 +929,22 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
   p.absgrad = reinterpret_cast<float2*>(absgrad);
   p.raw = raw; p.sh_rest = sh_rest; p.opacities = opacities_raw; p.v_sh_rest = v_sh_rest;
   p.antialiased = antialiased;
+  p.cam_partials = nullptr; p.cam_counters = nullptr;
   EGS_REQUIRE(!antialiased || opacities_raw != nullptr, "projection_bwd: antialiased mode needs the opacities");
+  const int64_t vg_slots = vg_partial_slots(N);
+  if (vg) {
+    p.cam_partials = static_cast<float*>(workspace);
+    p.cam_counters = reinterpret_cast<int*>(p.cam_partials + (size_t)(C * vg_slots + C * vg_slices(vg_slots)) * kCamPartialFloats);
+  }
+  // viewmat_grad_finalize_kernel, after either backward kernel
+  auto finalize = [&]() -> int {
+    if (C == 0) return 0;
+    const int S = vg_slices(vg_slots);
+    float* slices = p.cam_partials + (size_t)C * vg_slots * kCamPartialFloats;
+    viewmat_grad_finalize_kernel<<<dim3((unsigned)S, (unsigned)C), kVgFinalizeThreads, 0, (cudaStream_t)stream>>>(
+        (int)vg_slots, p.cam_partials, slices, p.cam_counters, viewmats, v_viewmats);
+    return check_launch("viewmat_grad_finalize_kernel");
+  };
   const bool vec4 = sh_degree >= 0 && (K * 3) % 4 == 0 && (reinterpret_cast<uintptr_t>(sh_coeffs) % 16 == 0) &&
                     (reinterpret_cast<uintptr_t>(v_sh_coeffs) % 16 == 0);
   if (raw) {
@@ -777,15 +954,23 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
   if (raw || (vec4 && K == 16)) {
     // the reference's layout (K = 16): coalesced shared-memory staged rows
     constexpr int kSmem = 2 * kPB2Warps * 32 * kRowStride * (int)sizeof(float);
-    auto kern = antialiased ? projection_bwd_sh16_kernel<true> : projection_bwd_sh16_kernel<false>;
+    auto kern = vg ? (antialiased ? projection_bwd_sh16_kernel<true, true> : projection_bwd_sh16_kernel<false, true>)
+                   : (antialiased ? projection_bwd_sh16_kernel<true> : projection_bwd_sh16_kernel<false>);
     const cudaError_t attr_rc =  // per-device attribute: set on every call (cheap), not once per process
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     if (attr_rc != cudaSuccess) return fail((int)attr_rc, "projection_bwd: shared memory opt-in failed: %s", cudaGetErrorString(attr_rc));
     kern<<<(unsigned)ceil_div(n_end - n_begin, kPB2Threads), kPB2Threads, kSmem, (cudaStream_t)stream>>>(p);
-    return check_launch("projection_bwd_sh16_kernel");
+    const int rc = check_launch("projection_bwd_sh16_kernel");
+    return (rc != 0 || !vg) ? rc : finalize();
   }
   EGS_REQUIRE(n_begin == 0 && n_end == N, "projection_bwd: a Gaussian sub-range needs the K = 16 layout (16-byte aligned SH rows)");
   unsigned grid = (unsigned)ceil_div(N, kProjBwdThreads);
+  if (vg) {
+    if (vec4) projection_bwd_kernel<true, true><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
+    else      projection_bwd_kernel<false, true><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
+    const int rc = check_launch("projection_bwd_kernel");
+    return rc != 0 ? rc : finalize();
+  }
   if (vec4) projection_bwd_kernel<true><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
   else      projection_bwd_kernel<false><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
   return check_launch("projection_bwd_kernel");
@@ -858,4 +1043,43 @@ extern "C" int egs_projection_bwd_raw(int32_t C, int32_t N, const float* means, 
   return projection_bwd_impl(C, N, means, quats, log_scales, logit_opacities, sh_0, sh_rest, 16, sh_degree, 0, viewmats,
                              Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means, v_quats,
                              v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream);
+}
+
+/* ---- gradients w.r.t. the view matrices ---- */
+extern "C" int64_t egs_projection_bwd_viewmats_workspace_bytes(int32_t C, int32_t N) {
+  if (C <= 0 || N < 0) return 0;
+  const int64_t slots = vg_partial_slots(N);
+  return (int64_t)C * (slots + vg_slices(slots)) * kCamPartialFloats * (int64_t)sizeof(float) + (int64_t)C * (int64_t)sizeof(int);
+}
+
+extern "C" int egs_projection_bwd_viewmats(
+    int32_t C, int32_t N, const float* means, const float* quats, const float* scales, const float* opacities,
+    const float* sh_coeffs, int32_t K, int32_t sh_degree, int32_t colors_per_camera, const float* viewmats,
+    const float* Ks, int32_t width, int32_t height, float eps2d, const int32_t* radii, const float* colors,
+    const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats, float* v_scales,
+    float* v_opacities, float* v_sh_coeffs, float* absgrad, int32_t antialiased, float* v_viewmats, void* workspace,
+    int64_t workspace_bytes, egs_stream_t stream) {
+  EGS_REQUIRE(v_viewmats != nullptr, "projection_bwd_viewmats: v_viewmats output is required");
+  return projection_bwd_impl(C, N, means, quats, scales, antialiased ? opacities : nullptr, sh_coeffs, nullptr, K,
+                             sh_degree, colors_per_camera, viewmats, Ks, width, height, eps2d, radii, colors, v_splats,
+                             v_means2d_extra, v_means, v_quats, v_scales, v_opacities, v_sh_coeffs, nullptr, absgrad,
+                             stream, antialiased ? 1 : 0, 0, -1, v_viewmats, workspace, workspace_bytes);
+}
+
+extern "C" int egs_projection_bwd_raw_viewmats(
+    int32_t C, int32_t N, const float* means, const float* quats, const float* log_scales, const float* logit_opacities,
+    const float* sh_0, const float* sh_rest, int32_t sh_degree, const float* viewmats, const float* Ks, int32_t width,
+    int32_t height, float eps2d, const int32_t* radii, const float* colors, const float* v_splats,
+    const float* v_means2d_extra, float* v_means, float* v_quats, float* v_log_scales, float* v_logit_opacities,
+    float* v_sh_0, float* v_sh_rest, float* absgrad, float* v_viewmats, void* workspace, int64_t workspace_bytes,
+    egs_stream_t stream) {
+  EGS_REQUIRE(v_viewmats != nullptr, "projection_bwd_raw_viewmats: v_viewmats output is required");
+  EGS_REQUIRE(sh_rest != nullptr && sh_0 != nullptr, "projection_bwd_raw: sh_0 and sh_rest are required");
+  EGS_REQUIRE(reinterpret_cast<uintptr_t>(sh_0) % 16 == 0 && reinterpret_cast<uintptr_t>(sh_rest) % 16 == 0 &&
+                  reinterpret_cast<uintptr_t>(v_sh_0) % 16 == 0 && reinterpret_cast<uintptr_t>(v_sh_rest) % 16 == 0,
+              "projection_bwd_raw: sh_0 / sh_rest and their gradients must be 16-byte aligned");
+  return projection_bwd_impl(C, N, means, quats, log_scales, logit_opacities, sh_0, sh_rest, 16, sh_degree, 0, viewmats,
+                             Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means, v_quats,
+                             v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream, 0, 0, -1, v_viewmats,
+                             workspace, workspace_bytes);
 }

@@ -221,18 +221,22 @@ class _Rasterization(torch.autograd.Function):
                                    render_alphas, last_ids, v_colors, v_alphas, ckpt)
         ref = getattr(ctx, "means2d_ref", None) if cfg["absgrad"] else None
         target = ref() if ref is not None else None
+        # the viewmat keyword is passed only when its gradient is wanted: without it the call is exactly the classic one
+        want_vm = {"want_viewmats_grad": True} if ctx.needs_input_grad[5] else {}
         with stages.nvtx_range("egs.projection_bwd"):
             out = stages.projection_bwd(means, quats, scales, colors, viewmats, Ks, width, height, cfg["sh_degree"],
                                         cfg["eps2d"], radii, colors_rgb, v_splats, v_means2d, want_absgrad=target is not None,
-                                        antialiased_opacities=opacities if cfg["antialiased"] else None, opacities=opacities)
+                                        antialiased_opacities=opacities if cfg["antialiased"] else None, opacities=opacities,
+                                        **want_vm)
         v_means, v_quats, v_scales, v_opac, v_cols = out[:5]
+        v_viewmats = out[-1] if want_vm else None
         if target is not None:
             # same contract as gsplat: attribute tagging on the tensor object handed out in meta
             _tag_absgrad(target, out[5], getattr(ctx, "packed_index", None))
         v_bg = None
         if backgrounds is not None and ctx.needs_input_grad[7]:
             v_bg = ((1.0 - render_alphas) * v_colors).sum(dim=(1, 2))
-        return v_means, v_quats, v_scales, v_opac, v_cols, None, None, v_bg, None
+        return v_means, v_quats, v_scales, v_opac, v_cols, v_viewmats, None, v_bg, None
 
 
 class _RasterizationRaw(torch.autograd.Function):
@@ -280,15 +284,17 @@ class _RasterizationRaw(torch.autograd.Function):
                                    render_alphas, last_ids, v_colors, v_alphas, ckpt)
         ref = getattr(ctx, "means2d_ref", None) if cfg["absgrad"] else None
         target = ref() if ref is not None else None
+        want_vm = {"want_viewmats_grad": True} if ctx.needs_input_grad[6] else {}
         out = stages.projection_bwd_raw(means, quats, log_scales, logit_opacities, sh_0, sh_rest, viewmats, Ks, width,
                                         height, cfg["sh_degree"], cfg["eps2d"], radii, colors_rgb, v_splats, v_means2d,
-                                        want_absgrad=target is not None)
+                                        want_absgrad=target is not None, **want_vm)
+        v_viewmats = out[-1] if want_vm else None
         if target is not None:
             _tag_absgrad(target, out[6], None)
         v_bg = None
         if backgrounds is not None and ctx.needs_input_grad[8]:
             v_bg = ((1.0 - render_alphas) * v_colors).sum(dim=(1, 2))
-        return (*out[:6], None, None, v_bg, None)
+        return (*out[:6], v_viewmats, None, v_bg, None)
 
 
 def _check_inputs(means, quats, scales, opacities, colors, viewmats, Ks, sh_degree, backgrounds):
@@ -363,7 +369,9 @@ def rasterization(
 ) -> Tuple[Tensor, Tensor, Dict]:
     """See module docstring.  The combination the reference uses — SH colours, ``packed=False``,
     ``absgrad=True``, one camera, a [1,3] background — and C > 1 are implemented; modes the
-    reference never requests raise ``NotImplementedError`` instead of silently approximating."""
+    reference never requests raise ``NotImplementedError`` instead of silently approximating.
+    As in gsplat, ``viewmats`` receive a gradient when they require one (camera pose refinement: projection and SH
+    view directions, campos = inverse(viewmats)[:, :3, 3]); ``Ks`` receive none."""
     if render_mode != "RGB":
         raise NotImplementedError(f"render_mode={render_mode!r}: only 'RGB' is implemented (the reference's mode)")
     if rasterize_mode not in ("classic", "antialiased"):
@@ -376,8 +384,6 @@ def rasterization(
     if width < 1 or height < 1:
         raise ValueError(f"width and height must be >= 1, got {width} x {height}")
     _check_inputs(means, quats, scales, opacities, colors, viewmats, Ks, sh_degree, backgrounds)
-    if viewmats.requires_grad and torch.is_grad_enabled():
-        raise NotImplementedError("gradients w.r.t. viewmats are not implemented (the reference never asks for them)")
     C = viewmats.shape[0]
     cfg = dict(width=width, height=height, sh_degree=sh_degree, eps2d=float(eps2d), near_plane=float(near_plane),
                far_plane=float(far_plane), radius_clip=float(radius_clip), absgrad=bool(absgrad),
@@ -482,8 +488,6 @@ def rasterization_from_parameters(
     for name, t in (("sh_0", sh_0), ("sh_rest", sh_rest)):
         if not t.is_cuda or t.dtype != torch.float32:
             raise RuntimeError(f"{name} must be a float32 CUDA tensor: this rasterizer has no CPU path")
-    if viewmats.requires_grad and torch.is_grad_enabled():
-        raise NotImplementedError("gradients w.r.t. viewmats are not implemented")
     cfg = dict(width=width, height=height, sh_degree=int(sh_degree), eps2d=float(eps2d), near_plane=float(near_plane),
                far_plane=float(far_plane), radius_clip=float(radius_clip), absgrad=bool(absgrad),
                grad_enabled=torch.is_grad_enabled())

@@ -224,10 +224,12 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
                    width: int, height: int, sh_degree: Optional[int], eps2d: float, radii: Tensor,
                    colors_rgb: Tensor, v_splats: Tensor, v_means2d_extra: Optional[Tensor] = None,
                    want_absgrad: bool = False, antialiased_opacities: Optional[Tensor] = None,
-                   opacities: Optional[Tensor] = None):
+                   opacities: Optional[Tensor] = None, want_viewmats_grad: bool = False):
     """g8+g9. -> v_means[N,3], v_quats[N,4], v_scales[N,3], v_opacities[N], v_colors (shape of colors)
-    (+ absgrad[C,N,2] when want_absgrad).  antialiased_opacities: the opacities[N] of an antialiased forward;
-    opacities: only consulted for a registered gradient buffer (register_grad_target)."""
+    (+ absgrad[C,N,2] when want_absgrad) (+ v_viewmats[C,4,4] when want_viewmats_grad, always last).
+    antialiased_opacities: the opacities[N] of an antialiased forward; opacities: only consulted for a registered
+    gradient buffer (register_grad_target).  want_viewmats_grad always takes the single launch: the chunked
+    backward of set_grad_chunk_hook (an opt-in overlap of the multi-GPU gradient exchange) does not produce it."""
     lib = _lib.load()
     dev = means.device
     means, quats, scales, colors, viewmats, Ks = dense_inputs(means, quats, scales, colors, viewmats, Ks)
@@ -251,8 +253,16 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
             _ptr(v_scales), _ptr(v_opac), _ptr(v_colors), _ptr(absgrad), _stream(dev))
     hook = _GRAD_CHUNK_HOOK
     chunked = (hook is not None and all_targets and antialiased_opacities is None and deg >= 0 and K == 16 and N >= 4096)
+    v_viewmats = None
     with torch.cuda.device(dev):
-        if antialiased_opacities is not None:
+        if want_viewmats_grad:
+            v_viewmats = torch.empty(C, 4, 4, dtype=torch.float32, device=dev)
+            ws = _viewmats_workspace(lib, C, N, dev)
+            aa = antialiased_opacities is not None
+            aa_op = _f32c(antialiased_opacities, "opacities") if aa else None
+            rc = lib.egs_projection_bwd_viewmats(C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail[:-1],
+                                                 int(aa), _ptr(v_viewmats), _ptr(ws), ws.numel(), tail[-1])
+        elif antialiased_opacities is not None:
             aa_op = _f32c(antialiased_opacities, "opacities")
             rc = lib.egs_projection_bwd_antialiased(C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail)
         elif chunked:
@@ -263,9 +273,13 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
         else:
             rc = lib.egs_projection_bwd(C, N, _ptr(means), _ptr(quats), _ptr(scales), *tail)
     _lib.check(rc, "egs_projection_bwd")
-    if want_absgrad:
-        return v_means, v_quats, v_scales, v_opac, v_colors, absgrad
-    return v_means, v_quats, v_scales, v_opac, v_colors
+    out = (v_means, v_quats, v_scales, v_opac, v_colors) + ((absgrad,) if want_absgrad else ())
+    return out + (v_viewmats,) if want_viewmats_grad else out
+
+
+def _viewmats_workspace(lib, C: int, N: int, dev) -> Tensor:
+    """Scratch of the view-matrix gradient (per-warp partials, see include/egs_raster.h); 16-byte aligned."""
+    return torch.empty(max(lib.egs_projection_bwd_viewmats_workspace_bytes(C, N), 16), dtype=torch.uint8, device=dev)
 
 
 def projection_fwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_opacities: Tensor, sh_0: Tensor,
@@ -308,8 +322,10 @@ def projection_fwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_o
 def projection_bwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_opacities: Tensor, sh_0: Tensor,
                        sh_rest: Tensor, viewmats: Tensor, Ks: Tensor, width: int, height: int, sh_degree: int,
                        eps2d: float, radii: Tensor, colors_rgb: Tensor, v_splats: Tensor,
-                       v_means2d_extra: Optional[Tensor] = None, want_absgrad: bool = False):
-    """-> v_means, v_quats, v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest (, absgrad)."""
+                       v_means2d_extra: Optional[Tensor] = None, want_absgrad: bool = False,
+                       want_viewmats_grad: bool = False):
+    """-> v_means, v_quats, v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest (, absgrad) (, v_viewmats[C,4,4]).
+    want_viewmats_grad always takes the single launch (see projection_bwd)."""
     lib = _lib.load()
     dev = means.device
     means, quats, log_scales, logit_opacities, sh_0, sh_rest, viewmats, Ks = dense_inputs(
@@ -324,8 +340,13 @@ def projection_bwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_o
             int(sh_degree), _ptr(viewmats), _ptr(Ks), int(width), int(height), float(eps2d), _ptr(radii), _ptr(colors_rgb),
             _ptr(v_splats), _ptr(v_means2d_extra), *[_ptr(o) for o in outs], _ptr(absgrad))
     hook = _GRAD_CHUNK_HOOK
+    v_viewmats = None
     with torch.cuda.device(dev):
-        if hook is not None and all_targets and N >= 4096:
+        if want_viewmats_grad:
+            v_viewmats = torch.empty(C, 4, 4, dtype=torch.float32, device=dev)
+            ws = _viewmats_workspace(lib, C, N, dev)
+            rc = lib.egs_projection_bwd_raw_viewmats(*args, _ptr(v_viewmats), _ptr(ws), ws.numel(), _stream(dev))
+        elif hook is not None and all_targets and N >= 4096:
             for i, (n0, n1) in enumerate(_chunk_bounds(N, hook[0])):
                 rc = lib.egs_projection_bwd_raw_range(*args, n0, n1, _stream(dev))
                 _lib.check(rc, "egs_projection_bwd_raw_range")
@@ -333,7 +354,8 @@ def projection_bwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_o
         else:
             rc = lib.egs_projection_bwd_raw(*args, _stream(dev))
     _lib.check(rc, "egs_projection_bwd_raw")
-    return (*outs, absgrad) if want_absgrad else tuple(outs)
+    out = (*outs, absgrad) if want_absgrad else tuple(outs)
+    return out + (v_viewmats,) if want_viewmats_grad else out
 
 
 def exclusive_scan(counts: Tensor) -> Tuple[Tensor, Tensor]:

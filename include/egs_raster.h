@@ -154,6 +154,35 @@ int egs_projection_bwd_raw(int32_t C, int32_t N, const float* means, const float
                            float* v_logit_opacities, float* v_sh_0, float* v_sh_rest, float* absgrad,
                            egs_stream_t stream);
 
+/* ---- gradients w.r.t. the view matrices (camera pose refinement) ------------------------------------------------
+ * The backward entries above, plus v_viewmats[C,4,4]: the gradient of gsplat 1.0.0's `rasterization()` w.r.t.
+ * viewmats, summed over the visible Gaussians of each camera.  Two paths: the projection (mean_c = R m + t,
+ * cov_c = R Sigma R^T; top 3x4 block) and, with SH colours, the view directions m - campos with
+ * campos = inverse(viewmat)[:3,3] (all four rows).  Deterministic: per camera, one partial per warp and a fixed-order
+ * sum in a second, small kernel (no float atomics), so the same inputs give bit-identical v_viewmats.  Every other
+ * output is bit-identical to the entry without viewmat gradients.  Needs the whole Gaussian range (no _range form).
+ *   workspace: egs_projection_bwd_viewmats_workspace_bytes(C, N) bytes of device memory, 16-byte aligned; no need to
+ *   clear it.  One call at a time per workspace.
+ * egs_projection_bwd_viewmats: egs_projection_bwd (antialiased = 0) or egs_projection_bwd_antialiased (antialiased =
+ *   1: opacities[N] required; otherwise it may be NULL). */
+int64_t egs_projection_bwd_viewmats_workspace_bytes(int32_t C, int32_t N);
+int egs_projection_bwd_viewmats(int32_t C, int32_t N, const float* means, const float* quats, const float* scales,
+                                const float* opacities, const float* sh_coeffs, int32_t K, int32_t sh_degree,
+                                int32_t colors_per_camera, const float* viewmats, const float* Ks, int32_t width,
+                                int32_t height, float eps2d, const int32_t* radii, const float* colors,
+                                const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
+                                float* v_scales, float* v_opacities, float* v_sh_coeffs, float* absgrad,
+                                int32_t antialiased, float* v_viewmats, void* workspace, int64_t workspace_bytes,
+                                egs_stream_t stream);
+int egs_projection_bwd_raw_viewmats(int32_t C, int32_t N, const float* means, const float* quats,
+                                    const float* log_scales, const float* logit_opacities, const float* sh_0,
+                                    const float* sh_rest, int32_t sh_degree, const float* viewmats, const float* Ks,
+                                    int32_t width, int32_t height, float eps2d, const int32_t* radii,
+                                    const float* colors, const float* v_splats, const float* v_means2d_extra,
+                                    float* v_means, float* v_quats, float* v_log_scales, float* v_logit_opacities,
+                                    float* v_sh_0, float* v_sh_rest, float* absgrad, float* v_viewmats,
+                                    void* workspace, int64_t workspace_bytes, egs_stream_t stream);
+
 /* ---- g3: exclusive scan of tiles_per_gauss, then key emission -------------------------------------
  * Replaces `torch.cumsum` + the second launch of gsplat `isect_tiles`.
  * egs_exclusive_scan: out[i] = sum_{j<i} in[j] (int64), *total = sum of all (device int64). */
