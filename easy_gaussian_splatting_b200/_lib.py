@@ -25,10 +25,6 @@ _SIGNATURES = {
                                      I32, I32, I32, P, P, P, P, P, P, P, P, P]),
     "egs_projection_bwd": (c_int32, [I32, I32, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, P, P, P, P,
                                      P, P, P, P, P, P, P]),
-    "egs_projection_bwd_range": (c_int32, [I32, I32, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, P, P, P, P,
-                                           P, P, P, P, P, P, I32, I32, P]),
-    "egs_projection_bwd_raw_range": (c_int32, [I32, I32, P, P, P, P, P, P, I32, P, P, I32, I32, F32, P, P, P, P,
-                                               P, P, P, P, P, P, P, I32, I32, P]),
     "egs_projection_fwd_antialiased": (c_int32, [I32, I32, P, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, F32, F32,
                                                  F32, I32, I32, I32, P, P, P, P, P, P, P, P, P, P]),
     "egs_projection_bwd_antialiased": (c_int32, [I32, I32, P, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, P, P, P,
@@ -65,12 +61,8 @@ _SIGNATURES = {
     "egs_densify_stats_update": (c_int32, [I32, I32, P, P, F32, P, P, P, P]),
     "egs_l1_ssim_fwd": (c_int32, [I32, I32, I32, P, P, P, P, P, P]),
     "egs_l1_ssim_bwd": (c_int32, [I32, I32, I32, P, P, P, P, F32, P, P, P]),
-    "egs_allreduce_sum_f32_peer": (c_int32, [I32, I32, P, I64, P]),
-    "egs_allreduce_sum_f32_multimem": (c_int32, [I32, I32, P, I64, P]),
     "egs_allreduce_f32_peer": (c_int32, [I32, I32, P, I64, I64, P]),
     "egs_allreduce_f32_multimem": (c_int32, [I32, I32, P, I64, I64, P]),
-    "egs_allreduce_ranges_f32_peer": (c_int32, [I32, I32, P, I32, P, P, P, P]),
-    "egs_allreduce_ranges_f32_multimem": (c_int32, [I32, I32, P, I32, P, P, P, P]),
     "egs_fused_adam": (c_int32, [I32, P, P, P, P, P, P, F32, F32, F32, I64, P]),
     "egs_probe_fp32_fma": (c_int32, [I32, I32, P, POINTER(ctypes.c_double), P]),
 }

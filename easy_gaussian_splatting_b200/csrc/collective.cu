@@ -19,10 +19,12 @@ constexpr int kArMaxWorld = 16;
 #ifndef EGS_AR_CTAS_PER_SM
 #define EGS_AR_CTAS_PER_SM 8
 #endif
+// Two ranges are used.  With room for fewer than 8, ptxas (CUDA 12.9) copies the kernel argument to a stack frame for
+// the loop over the ranges, and the two-shot kernels for 5-8 GPUs need up to 44 more registers.
 constexpr int kArMaxRanges = 8;
 
-// The float4 ranges one launch reduces, each cut into `world` slices of which this rank owns one.  SUM ranges carry
-// gradients (and the two accumulator rows of the densify statistics), a MAX range the max_radii row.
+// The float4 ranges one launch reduces, each cut into `world` slices of which this rank owns one: the SUM range carries
+// the gradients (and the two accumulator rows of the densify statistics), the MAX range behind it the max_radii row.
 struct ArRanges {
   int n;
   int64_t off4[kArMaxRanges];  // first float4 of the range
@@ -114,19 +116,19 @@ __global__ void __launch_bounds__(kArThreads) allreduce_multimem_kernel(float* _
   }
 }
 
-static int make_ranges(const char* who, int32_t n_ranges, const int64_t* offsets, const int64_t* lengths, const int32_t* is_max,
-                       ArRanges& rg, int64_t& total4) {
-  EGS_REQUIRE(n_ranges >= 0 && n_ranges <= kArMaxRanges, "%s: n_ranges=%d out of [0,%d]", who, n_ranges, kArMaxRanges);
+// [0, n_sum) summed, [n_sum, n_sum + n_max) maximised
+static int make_ranges(const char* who, int64_t n_sum_floats, int64_t n_max_floats, ArRanges& rg, int64_t& total4) {
+  const int64_t offsets[2] = {0, n_sum_floats}, lengths[2] = {n_sum_floats, n_max_floats};
   rg.n = 0;
   total4 = 0;
-  for (int r = 0; r < n_ranges; ++r) {
+  for (int r = 0; r < 2; ++r) {
     EGS_REQUIRE(offsets[r] >= 0 && lengths[r] >= 0 && offsets[r] % 4 == 0 && lengths[r] % 4 == 0,
                 "%s: range %d (offset %lld, length %lld floats) must be non-negative multiples of 4", who, r,
                 (long long)offsets[r], (long long)lengths[r]);
     if (lengths[r] == 0) continue;
     rg.off4[rg.n] = offsets[r] / 4;
     rg.n4[rg.n] = lengths[r] / 4;
-    rg.is_max[rg.n] = is_max != nullptr && is_max[r] != 0;
+    rg.is_max[rg.n] = r == 1;
     total4 += rg.n4[rg.n];
     ++rg.n;
   }
@@ -144,28 +146,26 @@ static unsigned ar_blocks(int64_t total4, int world) {
 
 using namespace egs;
 
-extern "C" int egs_allreduce_ranges_f32_multimem(int32_t world, int32_t rank, void* multicast_ptr, int32_t n_ranges,
-                                                 const int64_t* offsets_floats, const int64_t* lengths_floats,
-                                                 const int32_t* is_max, egs_stream_t stream) {
+extern "C" int egs_allreduce_f32_multimem(int32_t world, int32_t rank, void* multicast_ptr, int64_t n_sum_floats,
+                                          int64_t n_max_floats, egs_stream_t stream) {
   EGS_REQUIRE(world >= 1 && rank >= 0 && rank < world, "allreduce_multimem: bad world=%d rank=%d", world, rank);
   EGS_REQUIRE(multicast_ptr != nullptr, "allreduce_multimem: multicast pointer is required");
   ArRanges rg;
   int64_t total4 = 0;
-  if (int rc = make_ranges("allreduce_multimem", n_ranges, offsets_floats, lengths_floats, is_max, rg, total4)) return rc;
+  if (int rc = make_ranges("allreduce_multimem", n_sum_floats, n_max_floats, rg, total4)) return rc;
   if (total4 == 0 || world == 1) return 0;
   allreduce_multimem_kernel<<<ar_blocks(total4, world), kArThreads, 0, (cudaStream_t)stream>>>(
       reinterpret_cast<float*>(multicast_ptr), world, rank, rg);
   return check_launch("allreduce_multimem_kernel");
 }
 
-extern "C" int egs_allreduce_ranges_f32_peer(int32_t world, int32_t rank, const void* peer_buffers_dev, int32_t n_ranges,
-                                             const int64_t* offsets_floats, const int64_t* lengths_floats,
-                                             const int32_t* is_max, egs_stream_t stream) {
+extern "C" int egs_allreduce_f32_peer(int32_t world, int32_t rank, const void* peer_buffers_dev, int64_t n_sum_floats,
+                                      int64_t n_max_floats, egs_stream_t stream) {
   EGS_REQUIRE(world >= 1 && world <= kArMaxWorld && rank >= 0 && rank < world, "allreduce_peer: bad world=%d rank=%d", world, rank);
   EGS_REQUIRE(peer_buffers_dev != nullptr, "allreduce_peer: peer buffer table is required");
   ArRanges rg;
   int64_t total4 = 0;
-  if (int rc = make_ranges("allreduce_peer", n_ranges, offsets_floats, lengths_floats, is_max, rg, total4)) return rc;
+  if (int rc = make_ranges("allreduce_peer", n_sum_floats, n_max_floats, rg, total4)) return rc;
   if (total4 == 0 || world == 1) return 0;
   float* const* bufs = reinterpret_cast<float* const*>(peer_buffers_dev);
   const unsigned grid = ar_blocks(total4, world);
@@ -181,26 +181,4 @@ extern "C" int egs_allreduce_ranges_f32_peer(int32_t world, int32_t rank, const 
     default: return fail(EGS_ERR_UNSUPPORTED, "allreduce_peer: world=%d is not instantiated (2..8)", world);
   }
   return check_launch("allreduce_two_shot_kernel");
-}
-
-// the whole-buffer forms: [0, n_sum) summed, [n_sum, n_sum + n_max) maximised
-extern "C" int egs_allreduce_f32_multimem(int32_t world, int32_t rank, void* multicast_ptr, int64_t n_sum_floats,
-                                          int64_t n_max_floats, egs_stream_t stream) {
-  const int64_t off[2] = {0, n_sum_floats}, len[2] = {n_sum_floats, n_max_floats};
-  const int32_t mx[2] = {0, 1};
-  return egs_allreduce_ranges_f32_multimem(world, rank, multicast_ptr, 2, off, len, mx, stream);
-}
-extern "C" int egs_allreduce_f32_peer(int32_t world, int32_t rank, const void* peer_buffers_dev, int64_t n_sum_floats,
-                                      int64_t n_max_floats, egs_stream_t stream) {
-  const int64_t off[2] = {0, n_sum_floats}, len[2] = {n_sum_floats, n_max_floats};
-  const int32_t mx[2] = {0, 1};
-  return egs_allreduce_ranges_f32_peer(world, rank, peer_buffers_dev, 2, off, len, mx, stream);
-}
-extern "C" int egs_allreduce_sum_f32_multimem(int32_t world, int32_t rank, void* multicast_ptr, int64_t n_floats,
-                                              egs_stream_t stream) {
-  return egs_allreduce_f32_multimem(world, rank, multicast_ptr, n_floats, 0, stream);
-}
-extern "C" int egs_allreduce_sum_f32_peer(int32_t world, int32_t rank, const void* peer_buffers_dev, int64_t n_floats,
-                                          egs_stream_t stream) {
-  return egs_allreduce_f32_peer(world, rank, peer_buffers_dev, n_floats, 0, stream);
 }

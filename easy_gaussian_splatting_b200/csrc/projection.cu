@@ -333,8 +333,6 @@ struct ProjBwdParams {
   int antialiased;            // v_splats' opacity slot is d L / d (opacity * compensation)
   float* v_sh_rest;
   float2* absgrad;  // nullable [C,N]: sum over pixels of |d L / d means2d|, copied out of the gradient records
-  int n_begin, n_end;  // projection_bwd_sh16_kernel: the Gaussians of this launch (chunked launches let the gradient
-                       // exchange of one chunk overlap the backward pass of the next, egs_projection_bwd_range)
   // viewmat gradients (the VG instantiations only): per camera, one 16-float partial of the camera gradient
   // (egs_math.cuh kCamGradFloats, padded) per warp of the launch, camera-major: [C][gridDim.x * 4][16]; the counters
   // [C] of viewmat_grad_finalize_kernel are cleared by block 0
@@ -600,9 +598,9 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float* co_tile = smem_pb + (size_t)warp * 32 * kRowStride;                       // coefficients
   float* vc_tile = smem_pb + (size_t)(kPB2Warps + warp) * 32 * kRowStride;         // gradient accumulation
-  const int n_base = p.n_begin + blockIdx.x * kPB2Threads + warp * 32;  // a launch covers Gaussians [n_begin, n_end)
+  const int n_base = blockIdx.x * kPB2Threads + warp * 32;
   const int n = n_base + lane;
-  const bool in_range = n < p.n_end;
+  const bool in_range = n < p.N;
   const int nb = (p.sh_degree + 1) * (p.sh_degree + 1);
 
   // which of this warp's Gaussians does any camera see?
@@ -632,7 +630,7 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
       *reinterpret_cast<float4*>(vc_tile + row * kRowStride + c4 * 4) = make_float4(0.f, 0.f, 0.f, 0.f);
     }
   } else {
-    if (p.sh_degree >= 1) load_rows_raw<kRowStride>(co_tile, p.sh, p.sh_rest, n_base, p.n_end, seen_mask, lane);
+    if (p.sh_degree >= 1) load_rows_raw<kRowStride>(co_tile, p.sh, p.sh_rest, n_base, p.N, seen_mask, lane);
 #pragma unroll
     for (int i = 0; i < kRowFloats / 4; ++i) {
       const int f = i * 32 + lane;
@@ -791,10 +789,10 @@ __global__ void EGS_PB_BOUNDS projection_bwd_sh16_kernel(const ProjBwdParams p) 
     for (int i = 0; i < kRowFloats / 4; ++i) {
       const int f = i * 32 + lane;
       const int row = f / 12, c4 = f - row * 12;
-      if (n_base + row < p.n_end) dst[f] = *reinterpret_cast<const float4*>(vc_tile + row * kRowStride + c4 * 4);
+      if (n_base + row < p.N) dst[f] = *reinterpret_cast<const float4*>(vc_tile + row * kRowStride + c4 * 4);
     }
   } else {
-    store_rows_raw<kRowStride>(vc_tile, p.v_sh, p.v_sh_rest, n_base, p.n_end, lane);
+    store_rows_raw<kRowStride>(vc_tile, p.v_sh, p.v_sh_rest, n_base, p.N, lane);
   }
   if (in_range) {
     p.v_means[3 * (size_t)n + 0] = v_mean[0]; p.v_means[3 * (size_t)n + 1] = v_mean[1]; p.v_means[3 * (size_t)n + 2] = v_mean[2];
@@ -900,14 +898,13 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
                                int32_t width, int32_t height, float eps2d, const int32_t* radii, const float* colors,
                                const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
                                float* v_scales, float* v_opacities, float* v_sh_coeffs, float* v_sh_rest, float* absgrad,
-                               egs_stream_t stream, int antialiased = 0, int32_t n_begin = 0, int32_t n_end = -1,
-                               float* v_viewmats = nullptr, void* workspace = nullptr, int64_t workspace_bytes = 0) {
+                               egs_stream_t stream, int antialiased = 0, float* v_viewmats = nullptr,
+                               void* workspace = nullptr, int64_t workspace_bytes = 0) {
   const int raw = sh_rest != nullptr;
   EGS_REQUIRE(C >= 0 && N >= 0, "projection_bwd: negative sizes C=%d N=%d", C, N);
   EGS_REQUIRE(sh_degree <= 3, "projection_bwd: sh_degree %d > 3 is not supported", sh_degree);
   const bool vg = v_viewmats != nullptr;
   if (vg) {
-    EGS_REQUIRE(n_begin == 0 && (n_end < 0 || n_end == N), "projection_bwd: viewmat gradients need the whole Gaussian range");
     EGS_REQUIRE(C <= 65535, "projection_bwd: C=%d exceeds 65535 cameras per call", C);
     EGS_REQUIRE(workspace != nullptr && workspace_bytes >= egs_projection_bwd_viewmats_workspace_bytes(C, N),
                 "projection_bwd: viewmat gradients need %lld workspace bytes (got %lld)",
@@ -915,12 +912,8 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
     if (N == 0 && C > 0) EGS_CUDA(cudaMemsetAsync(v_viewmats, 0, sizeof(float) * 16 * (size_t)C, (cudaStream_t)stream));
   }
   if (N == 0) return 0;
-  if (n_end < 0) n_end = N;
-  EGS_REQUIRE(0 <= n_begin && n_begin <= n_end && n_end <= N, "projection_bwd: Gaussian range [%d, %d) outside [0, %d)", n_begin, n_end, N);
-  if (n_begin == n_end) return 0;
   ProjBwdParams p;
   p.C = C; p.N = N; p.K = K; p.sh_degree = sh_degree; p.colors_per_camera = colors_per_camera;
-  p.n_begin = n_begin; p.n_end = n_end;
   p.means = means; p.quats = quats; p.scales = scales; p.sh = sh_coeffs; p.viewmats = viewmats; p.Ks = Ks;
   p.width = (float)width; p.height = (float)height; p.eps2d = eps2d;
   p.radii = radii; p.colors = colors; p.v_splats = reinterpret_cast<const float4*>(v_splats);
@@ -959,11 +952,10 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
     const cudaError_t attr_rc =  // per-device attribute: set on every call (cheap), not once per process
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     if (attr_rc != cudaSuccess) return fail((int)attr_rc, "projection_bwd: shared memory opt-in failed: %s", cudaGetErrorString(attr_rc));
-    kern<<<(unsigned)ceil_div(n_end - n_begin, kPB2Threads), kPB2Threads, kSmem, (cudaStream_t)stream>>>(p);
+    kern<<<(unsigned)ceil_div(N, kPB2Threads), kPB2Threads, kSmem, (cudaStream_t)stream>>>(p);
     const int rc = check_launch("projection_bwd_sh16_kernel");
     return (rc != 0 || !vg) ? rc : finalize();
   }
-  EGS_REQUIRE(n_begin == 0 && n_end == N, "projection_bwd: a Gaussian sub-range needs the K = 16 layout (16-byte aligned SH rows)");
   unsigned grid = (unsigned)ceil_div(N, kProjBwdThreads);
   if (vg) {
     if (vec4) projection_bwd_kernel<true, true><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
@@ -985,37 +977,6 @@ extern "C" int egs_projection_bwd(int32_t C, int32_t N, const float* means, cons
   return projection_bwd_impl(C, N, means, quats, scales, nullptr, sh_coeffs, nullptr, K, sh_degree, colors_per_camera,
                              viewmats, Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means,
                              v_quats, v_scales, v_opacities, v_sh_coeffs, nullptr, absgrad, stream);
-}
-
-/* One chunk of Gaussians [n_begin, n_end) of egs_projection_bwd: the same kernel on a sub-range, so that a caller can
- * start exchanging the gradients of the first chunks while the later ones are still being computed. */
-extern "C" int egs_projection_bwd_range(int32_t C, int32_t N, const float* means, const float* quats, const float* scales,
-                                        const float* sh_coeffs, int32_t K, int32_t sh_degree, int32_t colors_per_camera,
-                                        const float* viewmats, const float* Ks, int32_t width, int32_t height,
-                                        float eps2d, const int32_t* radii, const float* colors, const float* v_splats,
-                                        const float* v_means2d_extra, float* v_means, float* v_quats, float* v_scales,
-                                        float* v_opacities, float* v_sh_coeffs, float* absgrad, int32_t n_begin,
-                                        int32_t n_end, egs_stream_t stream) {
-  return projection_bwd_impl(C, N, means, quats, scales, nullptr, sh_coeffs, nullptr, K, sh_degree, colors_per_camera,
-                             viewmats, Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means,
-                             v_quats, v_scales, v_opacities, v_sh_coeffs, nullptr, absgrad, stream, 0, n_begin, n_end);
-}
-
-extern "C" int egs_projection_bwd_raw_range(int32_t C, int32_t N, const float* means, const float* quats,
-                                            const float* log_scales, const float* logit_opacities, const float* sh_0,
-                                            const float* sh_rest, int32_t sh_degree, const float* viewmats,
-                                            const float* Ks, int32_t width, int32_t height, float eps2d,
-                                            const int32_t* radii, const float* colors, const float* v_splats,
-                                            const float* v_means2d_extra, float* v_means, float* v_quats,
-                                            float* v_log_scales, float* v_logit_opacities, float* v_sh_0, float* v_sh_rest,
-                                            float* absgrad, int32_t n_begin, int32_t n_end, egs_stream_t stream) {
-  EGS_REQUIRE(sh_rest != nullptr && sh_0 != nullptr, "projection_bwd_raw: sh_0 and sh_rest are required");
-  EGS_REQUIRE(reinterpret_cast<uintptr_t>(sh_0) % 16 == 0 && reinterpret_cast<uintptr_t>(sh_rest) % 16 == 0 &&
-                  reinterpret_cast<uintptr_t>(v_sh_0) % 16 == 0 && reinterpret_cast<uintptr_t>(v_sh_rest) % 16 == 0,
-              "projection_bwd_raw: sh_0 / sh_rest and their gradients must be 16-byte aligned");
-  return projection_bwd_impl(C, N, means, quats, log_scales, logit_opacities, sh_0, sh_rest, 16, sh_degree, 0, viewmats,
-                             Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means, v_quats,
-                             v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream, 0, n_begin, n_end);
 }
 
 extern "C" int egs_projection_bwd_antialiased(
@@ -1063,7 +1024,7 @@ extern "C" int egs_projection_bwd_viewmats(
   return projection_bwd_impl(C, N, means, quats, scales, antialiased ? opacities : nullptr, sh_coeffs, nullptr, K,
                              sh_degree, colors_per_camera, viewmats, Ks, width, height, eps2d, radii, colors, v_splats,
                              v_means2d_extra, v_means, v_quats, v_scales, v_opacities, v_sh_coeffs, nullptr, absgrad,
-                             stream, antialiased ? 1 : 0, 0, -1, v_viewmats, workspace, workspace_bytes);
+                             stream, antialiased ? 1 : 0, v_viewmats, workspace, workspace_bytes);
 }
 
 extern "C" int egs_projection_bwd_raw_viewmats(
@@ -1080,6 +1041,6 @@ extern "C" int egs_projection_bwd_raw_viewmats(
               "projection_bwd_raw: sh_0 / sh_rest and their gradients must be 16-byte aligned");
   return projection_bwd_impl(C, N, means, quats, log_scales, logit_opacities, sh_0, sh_rest, 16, sh_degree, 0, viewmats,
                              Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means, v_quats,
-                             v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream, 0, 0, -1, v_viewmats,
+                             v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream, 0, v_viewmats,
                              workspace, workspace_bytes);
 }

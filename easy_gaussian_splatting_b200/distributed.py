@@ -61,9 +61,6 @@ class FlatGradBucket:
         self.n_max_floats = self.stats_row
         padded = self.n_sum_floats + self.n_max_floats
         self.epoch = 0  # number of completed exchanges
-        self.overlap_chunks = 4  # pieces the projection backward is cut into when its exchange is overlapped
-        self._overlap = None     # state of an overlapped exchange in progress (begin_direct .. all_reduce)
-        self._exchange_stream = None
         self._symm = None
         self._mode = "nccl"
         if symmetric is None:
@@ -80,7 +77,6 @@ class FlatGradBucket:
             p.grad = v
             self.views.append(v)
             off += -(-p.numel() // 4) * 4
-        self._view_offsets = [v.data_ptr() - self.flat.data_ptr() for v in self.views]  # bytes
 
     def _symmetric_buffer(self, n: int, ref: Tensor, world: int) -> Optional[Tensor]:
         buf, ok = None, 0
@@ -119,63 +115,21 @@ class FlatGradBucket:
         buf.zero_()
         return buf
 
-    def _launch_ranges(self, ranges, stream) -> None:
-        """One launch of our all-reduce kernel over [(offset_floats, length_floats, is_max), ...] of the symmetric buffer."""
+    def _peer_all_reduce(self, buf: Tensor) -> None:
         import ctypes
         from . import _lib
-        lib = _lib.load()
         hdl, world, rank = self._symm, dist.get_world_size(), dist.get_rank()
-        n = len(ranges)
-        off = (ctypes.c_int64 * n)(*[r[0] for r in ranges])
-        length = (ctypes.c_int64 * n)(*[r[1] for r in ranges])
-        is_max = (ctypes.c_int32 * n)(*[int(r[2]) for r in ranges])
-        st = ctypes.c_void_p(stream.cuda_stream)
-        if self._mode == "two_shot":
-            rc = lib.egs_allreduce_ranges_f32_peer(world, rank, ctypes.c_void_p(hdl.buffer_ptrs_dev), n, off, length, is_max, st)
-        else:
-            rc = lib.egs_allreduce_ranges_f32_multimem(world, rank, ctypes.c_void_p(hdl.multicast_ptr), n, off, length, is_max, st)
-        _lib.check(rc, "egs_allreduce_ranges_f32")
-
-    def _peer_all_reduce(self, buf: Tensor) -> None:
-        hdl = self._symm
-        stream = torch.cuda.current_stream(buf.device)
+        st = ctypes.c_void_p(torch.cuda.current_stream(buf.device).cuda_stream)
         hdl.barrier(channel=0)  # every bucket is complete
-        self._launch_ranges([(0, self.n_sum_floats, 0), (self.n_sum_floats, self.n_max_floats, 1)], stream)
+        lib = _lib.load()
+        if self._mode == "two_shot":
+            rc = lib.egs_allreduce_f32_peer(world, rank, ctypes.c_void_p(hdl.buffer_ptrs_dev), self.n_sum_floats,
+                                            self.n_max_floats, st)
+        else:
+            rc = lib.egs_allreduce_f32_multimem(world, rank, ctypes.c_void_p(hdl.multicast_ptr), self.n_sum_floats,
+                                                self.n_max_floats, st)
+        _lib.check(rc, "egs_allreduce_f32")
         hdl.barrier(channel=1)  # every slice has landed everywhere
-
-    # ---- exchange overlapped with the projection backward ---------------------------------------------------------
-    def _exchange_chunk(self, i: int, n0: int, n1: int) -> None:
-        """stages' chunk hook: the backward kernel for Gaussians [n0, n1) has just been enqueued on the current stream.
-        On the exchange stream: wait for it, meet the other ranks (all of them have this piece), reduce this piece's
-        slice of every parameter's gradient.  The next piece's backward kernel runs meanwhile."""
-        ov = self._overlap
-        dev = self.flat.device
-        ev = torch.cuda.Event()
-        ev.record(torch.cuda.current_stream(dev))
-        ex = self._exchange_stream
-        ex.wait_event(ev)
-        ranges = []
-        for off_b, w in zip(self._view_offsets, ov["widths"]):
-            length = -(-(n1 - n0) * w // 4) * 4  # a slice's tail padding (< 4 floats, zeros) may ride along
-            ranges.append((off_b // 4 + n0 * w, length, 0))
-        with torch.cuda.stream(ex):
-            self._symm.barrier(channel=0)
-            self._launch_ranges(ranges, ex)
-        ov["covered"] += n1 - n0
-
-    def _finish_overlapped(self) -> None:
-        """The gradients went out piece by piece; what is left is the statistics rows and the closing barrier."""
-        dev = self.flat.device
-        cur, ex = torch.cuda.current_stream(dev), self._exchange_stream
-        ev = torch.cuda.Event()
-        ev.record(cur)  # the densify-stat update of this step (and anything else on the compute stream) is in
-        ex.wait_event(ev)
-        with torch.cuda.stream(ex):
-            if self.stats_size:
-                self._symm.barrier(channel=0)
-                self._launch_ranges([(self.grad_floats, 2 * self.stats_row, 0), (self.n_sum_floats, self.n_max_floats, 1)], ex)
-            self._symm.barrier(channel=1)  # every piece has landed everywhere
-        cur.wait_stream(ex)
 
     @property
     def exchange(self) -> str:
@@ -195,38 +149,20 @@ class FlatGradBucket:
             if p.grad is None or p.grad.data_ptr() != v.data_ptr():
                 p.grad = v
 
-    def begin_direct(self, overlap: Optional[bool] = None) -> None:
-        """For a step with ONE backward pass (all of the step's views in one ``rasterization()`` call): the fused
-        projection backward writes every gradient element exactly once, so it is pointed straight at the bucket —
-        no zero fill before and no accumulate pass after the backward (2 x 236 B/Gaussian of traffic less).  Call
-        ``end_direct()`` after ``backward()``.
-
-        ``overlap=True`` (or EGS_EXCHANGE_OVERLAP=1; needs the peer-memory exchange): the projection backward is
-        launched in ``overlap_chunks`` pieces over the Gaussians and every piece's gradients are exchanged on a second
-        stream while the next piece is computed; ``all_reduce()`` then only finishes (statistics rows, closing
-        barrier).  OFF by default: measured on 4 B200s (1 M Gaussians, 4 views per rank) the step took 5.52 - 5.67 ms
-        with it and 5.50 ms without (gpurun_out/r2h_*.log) — the 0.34 ms projection backward is too short a window
-        for five barriers and five small launches, and the first barrier waits for the slowest rank either way.
-        Every rank must take the same decision (it depends only on the flag, the bucket's mode and the shapes)."""
+    def begin_direct(self) -> None:
+        """For a step with ONE backward pass (all of the step's views in one ``rasterization()`` call): every
+        parameter's bucket slice is registered as the one-shot gradient target of that parameter, so the fused
+        projection backward, which writes every gradient element exactly once, stores straight into the bucket — no
+        zero fill before and no accumulate pass after the backward (2 x 236 B/Gaussian of traffic less).  Call
+        ``end_direct()`` after ``backward()``."""
         from . import stages
         for p, v in zip(self.params, self.views):
             p.grad = None
             stages.register_grad_target(p, v)
-        if overlap is None:
-            overlap = os.environ.get("EGS_EXCHANGE_OVERLAP", "0") == "1"
-        n = self.params[0].shape[0] if self.params[0].dim() > 0 else 0
-        same_n = n > 0 and all(p.dim() > 0 and p.shape[0] == n and p.numel() % n == 0 for p in self.params)
-        self._overlap = None
-        if overlap and self._symm is not None and same_n:
-            if self._exchange_stream is None:
-                self._exchange_stream = torch.cuda.Stream(device=self.flat.device)
-            self._overlap = {"n": n, "covered": 0, "widths": [p.numel() // n for p in self.params]}
-            stages.set_grad_chunk_hook(self.overlap_chunks, self._exchange_chunk)
 
     def end_direct(self) -> None:
         from . import stages
         stages.clear_grad_targets()
-        stages.set_grad_chunk_hook(0, None)
         for p, v in zip(self.params, self.views):
             if p.grad is None:
                 v.zero_()
@@ -252,14 +188,7 @@ class FlatGradBucket:
             if group is not None and group is not dist.group.WORLD:
                 raise ValueError("the symmetric-memory bucket was rendezvoused on the WORLD group; build the bucket with "
                                  "symmetric=False to all-reduce over another group")
-            ov, self._overlap = self._overlap, None
-            if ov is not None and ov["covered"] == ov["n"]:
-                self._finish_overlapped()
-            elif ov is not None and ov["covered"] != 0:
-                raise RuntimeError("the overlapped exchange covered only part of the Gaussians; every rank must run the "
-                                   "same single backward pass between begin_direct() and all_reduce()")
-            else:
-                self._peer_all_reduce(self.flat)
+            self._peer_all_reduce(self.flat)
             self.epoch += 1
             return _CompletedWork() if async_op else None
         self.epoch += 1

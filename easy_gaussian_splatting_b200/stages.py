@@ -85,37 +85,8 @@ def _grad_buffer(inp: Tensor) -> Tensor:
                 if (live is not None and live.data_ptr() == inp.data_ptr() and live.shape == inp.shape
                         and inp.is_contiguous() and tgt.data_ptr() % 16 == 0):
                     del _GRAD_TARGETS[_target_key(inp)]  # one-shot
-                    out = tgt.view(inp.shape)  # a fresh tensor object over the caller's storage: autograd adopts it as .grad
-                    out._egs_target = True
-                    return out
+                    return tgt.view(inp.shape)  # a fresh tensor object over the caller's storage: autograd adopts it as .grad
     return torch.empty(inp.shape, dtype=inp.dtype, device=inp.device)
-
-
-# Chunk hook (distributed.FlatGradBucket.begin_direct(overlap=True)): when set to (n_chunks, fn) and every gradient of
-# a projection backward goes to a registered target, the backward is launched in n_chunks pieces over the Gaussians
-# and fn(i, n_begin, n_end) is called right after piece i is in the queue — the bucket starts exchanging that piece
-# on its own stream while the next piece computes.
-_GRAD_CHUNK_HOOK: Optional[Tuple[int, object]] = None
-
-
-def set_grad_chunk_hook(n_chunks: int, fn) -> None:
-    global _GRAD_CHUNK_HOOK
-    _GRAD_CHUNK_HOOK = (int(n_chunks), fn) if fn is not None and n_chunks > 1 else None
-
-
-def _grad_buffers(inputs) -> Tuple[List[Tensor], bool]:
-    """Gradient storage for every input, and whether ALL of it is caller-registered storage."""
-    outs, all_targets = [], True
-    for t in inputs:
-        buf = _grad_buffer(t)
-        outs.append(buf)
-        all_targets = all_targets and buf.data_ptr() != 0 and getattr(buf, "_egs_target", False)
-    return outs, all_targets
-
-
-def _chunk_bounds(N: int, n_chunks: int) -> List[Tuple[int, int]]:
-    step = max(256, -(-N // n_chunks + 255) // 256 * 256)  # multiples of 256 Gaussians: every slice stays 16-byte aligned
-    return [(a, min(a + step, N)) for a in range(0, N, step)]
 
 
 def _ptr(t: Optional[Tensor]):
@@ -228,8 +199,7 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
     """g8+g9. -> v_means[N,3], v_quats[N,4], v_scales[N,3], v_opacities[N], v_colors (shape of colors)
     (+ absgrad[C,N,2] when want_absgrad) (+ v_viewmats[C,4,4] when want_viewmats_grad, always last).
     antialiased_opacities: the opacities[N] of an antialiased forward; opacities: only consulted for a registered
-    gradient buffer (register_grad_target).  want_viewmats_grad always takes the single launch: the chunked
-    backward of set_grad_chunk_hook (an opt-in overlap of the multi-GPU gradient exchange) does not produce it."""
+    gradient buffer (register_grad_target)."""
     lib = _lib.load()
     dev = means.device
     means, quats, scales, colors, viewmats, Ks = dense_inputs(means, quats, scales, colors, viewmats, Ks)
@@ -241,18 +211,16 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
         K, deg, per_cam = colors.shape[-2], int(sh_degree), 0
     op_ref = antialiased_opacities if antialiased_opacities is not None else opacities
     if op_ref is not None:
-        (v_means, v_quats, v_scales, v_opac, v_colors), all_targets = _grad_buffers((means, quats, scales, op_ref, colors))
+        v_means, v_quats, v_scales, v_opac, v_colors = [_grad_buffer(t) for t in (means, quats, scales, op_ref, colors)]
     else:
-        (v_means, v_quats, v_scales, v_colors), all_targets = _grad_buffers((means, quats, scales, colors))
-        v_opac, all_targets = torch.empty(N, dtype=torch.float32, device=dev), False
+        v_means, v_quats, v_scales, v_colors = [_grad_buffer(t) for t in (means, quats, scales, colors)]
+        v_opac = torch.empty(N, dtype=torch.float32, device=dev)
     if v_means2d_extra is not None:
         v_means2d_extra = _f32c(v_means2d_extra, "v_means2d")
     absgrad = torch.empty(C, N, 2, dtype=torch.float32, device=dev) if want_absgrad else None
     tail = (_ptr(colors), K, deg, per_cam, _ptr(viewmats), _ptr(Ks), int(width), int(height), float(eps2d),
             _ptr(radii), _ptr(colors_rgb), _ptr(v_splats), _ptr(v_means2d_extra), _ptr(v_means), _ptr(v_quats),
             _ptr(v_scales), _ptr(v_opac), _ptr(v_colors), _ptr(absgrad), _stream(dev))
-    hook = _GRAD_CHUNK_HOOK
-    chunked = (hook is not None and all_targets and antialiased_opacities is None and deg >= 0 and K == 16 and N >= 4096)
     v_viewmats = None
     with torch.cuda.device(dev):
         if want_viewmats_grad:
@@ -265,11 +233,6 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
         elif antialiased_opacities is not None:
             aa_op = _f32c(antialiased_opacities, "opacities")
             rc = lib.egs_projection_bwd_antialiased(C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail)
-        elif chunked:
-            for i, (n0, n1) in enumerate(_chunk_bounds(N, hook[0])):
-                rc = lib.egs_projection_bwd_range(C, N, _ptr(means), _ptr(quats), _ptr(scales), *tail[:-1], n0, n1, tail[-1])
-                _lib.check(rc, "egs_projection_bwd_range")
-                hook[1](i, n0, n1)
         else:
             rc = lib.egs_projection_bwd(C, N, _ptr(means), _ptr(quats), _ptr(scales), *tail)
     _lib.check(rc, "egs_projection_bwd")
@@ -324,33 +287,26 @@ def projection_bwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_o
                        eps2d: float, radii: Tensor, colors_rgb: Tensor, v_splats: Tensor,
                        v_means2d_extra: Optional[Tensor] = None, want_absgrad: bool = False,
                        want_viewmats_grad: bool = False):
-    """-> v_means, v_quats, v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest (, absgrad) (, v_viewmats[C,4,4]).
-    want_viewmats_grad always takes the single launch (see projection_bwd)."""
+    """-> v_means, v_quats, v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest (, absgrad) (, v_viewmats[C,4,4])."""
     lib = _lib.load()
     dev = means.device
     means, quats, log_scales, logit_opacities, sh_0, sh_rest, viewmats, Ks = dense_inputs(
         means, quats, log_scales, logit_opacities, sh_0, sh_rest, viewmats, Ks)
     radii, colors_rgb, v_splats = radii.contiguous(), colors_rgb.contiguous(), v_splats.contiguous()
     N, C = means.shape[0], viewmats.shape[0]
-    outs, all_targets = _grad_buffers((means, quats, log_scales, logit_opacities, sh_0, sh_rest))
+    outs = [_grad_buffer(t) for t in (means, quats, log_scales, logit_opacities, sh_0, sh_rest)]
     if v_means2d_extra is not None:
         v_means2d_extra = _f32c(v_means2d_extra, "v_means2d")
     absgrad = torch.empty(C, N, 2, dtype=torch.float32, device=dev) if want_absgrad else None
     args = (C, N, _ptr(means), _ptr(quats), _ptr(log_scales), _ptr(logit_opacities), _ptr(sh_0), _ptr(sh_rest),
             int(sh_degree), _ptr(viewmats), _ptr(Ks), int(width), int(height), float(eps2d), _ptr(radii), _ptr(colors_rgb),
             _ptr(v_splats), _ptr(v_means2d_extra), *[_ptr(o) for o in outs], _ptr(absgrad))
-    hook = _GRAD_CHUNK_HOOK
     v_viewmats = None
     with torch.cuda.device(dev):
         if want_viewmats_grad:
             v_viewmats = torch.empty(C, 4, 4, dtype=torch.float32, device=dev)
             ws = _viewmats_workspace(lib, C, N, dev)
             rc = lib.egs_projection_bwd_raw_viewmats(*args, _ptr(v_viewmats), _ptr(ws), ws.numel(), _stream(dev))
-        elif hook is not None and all_targets and N >= 4096:
-            for i, (n0, n1) in enumerate(_chunk_bounds(N, hook[0])):
-                rc = lib.egs_projection_bwd_raw_range(*args, n0, n1, _stream(dev))
-                _lib.check(rc, "egs_projection_bwd_raw_range")
-                hook[1](i, n0, n1)
         else:
             rc = lib.egs_projection_bwd_raw(*args, _stream(dev))
     _lib.check(rc, "egs_projection_bwd_raw")

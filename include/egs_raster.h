@@ -92,24 +92,6 @@ int egs_projection_bwd(int32_t C, int32_t N, const float* means, const float* qu
                        const float* v_means2d_extra, float* v_means, float* v_quats, float* v_scales,
                        float* v_opacities, float* v_sh_coeffs, float* absgrad, egs_stream_t stream);
 
-/* One chunk of Gaussians [n_begin, n_end) of egs_projection_bwd / egs_projection_bwd_raw (K = 16 layout): the same
- * kernel on a sub-range.  Chunked launches let the multi-GPU gradient exchange of one chunk run while the backward pass of
- * the next chunk is still computing (easy_gaussian_splatting_b200/distributed.py, FlatGradBucket.begin_direct(overlap=True)). */
-int egs_projection_bwd_range(int32_t C, int32_t N, const float* means, const float* quats, const float* scales,
-                             const float* sh_coeffs, int32_t K, int32_t sh_degree, int32_t colors_per_camera,
-                             const float* viewmats, const float* Ks, int32_t width, int32_t height, float eps2d,
-                             const int32_t* radii, const float* colors, const float* v_splats,
-                             const float* v_means2d_extra, float* v_means, float* v_quats, float* v_scales,
-                             float* v_opacities, float* v_sh_coeffs, float* absgrad, int32_t n_begin, int32_t n_end,
-                             egs_stream_t stream);
-int egs_projection_bwd_raw_range(int32_t C, int32_t N, const float* means, const float* quats, const float* log_scales,
-                                 const float* logit_opacities, const float* sh_0, const float* sh_rest, int32_t sh_degree,
-                                 const float* viewmats, const float* Ks, int32_t width, int32_t height, float eps2d,
-                                 const int32_t* radii, const float* colors, const float* v_splats,
-                                 const float* v_means2d_extra, float* v_means, float* v_quats, float* v_log_scales,
-                                 float* v_logit_opacities, float* v_sh_0, float* v_sh_rest, float* absgrad,
-                                 int32_t n_begin, int32_t n_end, egs_stream_t stream);
-
 /* ---- §8f-4: rasterize_mode="antialiased" of the same two kernels ---------------------------------------------
  * gsplat 1.0.0 `fully_fused_projection(calc_compensations=True)` + the Python glue `opacities * compensations`
  * (the reference passes the default rasterize_mode="classic", model/gaussian.py:353-367; this is the other value the
@@ -160,7 +142,7 @@ int egs_projection_bwd_raw(int32_t C, int32_t N, const float* means, const float
  * cov_c = R Sigma R^T; top 3x4 block) and, with SH colours, the view directions m - campos with
  * campos = inverse(viewmat)[:3,3] (all four rows).  Deterministic: per camera, one partial per warp and a fixed-order
  * sum in a second, small kernel (no float atomics), so the same inputs give bit-identical v_viewmats.  Every other
- * output is bit-identical to the entry without viewmat gradients.  Needs the whole Gaussian range (no _range form).
+ * output is bit-identical to the entry without viewmat gradients.
  *   workspace: egs_projection_bwd_viewmats_workspace_bytes(C, N) bytes of device memory, 16-byte aligned; no need to
  *   clear it.  One call at a time per workspace.
  * egs_projection_bwd_viewmats: egs_projection_bwd (antialiased = 0) or egs_projection_bwd_antialiased (antialiased =
@@ -344,35 +326,22 @@ int egs_fused_adam(int32_t n_groups, float* const* params, const float* const* g
                    float eps, int64_t step, egs_stream_t stream);
 
 /* ---- §8e: gradient exchange as a two-shot all-reduce over NVLink peer memory -------------------------------------
- * Every rank's flat fp32 gradient bucket (n_floats, a multiple of 4) is mapped into every peer (symmetric memory);
- * peer_buffers_dev: DEVICE array of `world` device pointers, entry p = rank p's bucket as mapped on this GPU.
- * Rank r sums slice r over all buckets in rank order (peer loads) and writes it into every bucket (peer stores):
- * in-place SUM all-reduce, bit-identical on all replicas.  The caller brackets the call with inter-rank barriers
+ * Every rank's flat fp32 bucket is mapped into every peer (symmetric memory); peer_buffers_dev: DEVICE array of
+ * `world` device pointers, entry p = rank p's bucket as mapped on this GPU.  Both exchanges of the view-sharded step
+ * (SURVEY.md section 8e) go in ONE launch: the first n_sum_floats of the bucket are SUMmed over the ranks (parameter
+ * gradients, then the grad_norm_accum / collecting_counts rows of the step's densify statistics,
+ * model/gaussian.py:196-197), the n_max_floats behind them take the MAXimum (the max_radii row, gaussian.py:194; values
+ * must be >= 0: the NVLS variant compares their bit patterns as unsigned integers).  Both counts are multiples of 4;
+ * n_max_floats = 0 is a plain SUM all-reduce.
+ * Rank r reduces slice r over all buckets in rank order (peer loads) and writes it into every bucket (peer stores):
+ * in place, bit-identical on all replicas.  The caller brackets the call with inter-rank barriers
  * (all buckets complete before, all slices written after); world = 1 is a no-op. */
-int egs_allreduce_sum_f32_peer(int32_t world, int32_t rank, const void* peer_buffers_dev, int64_t n_floats,
-                               egs_stream_t stream);
-/* The same exchange through the NVSwitch (NVLS): multicast_ptr is the multicast mapping of the symmetric bucket;
- * rank r pulls the in-switch SUM of slice r (multimem.ld_reduce) and broadcasts it back (multimem.st). */
-int egs_allreduce_sum_f32_multimem(int32_t world, int32_t rank, void* multicast_ptr, int64_t n_floats,
-                                   egs_stream_t stream);
-/* Both exchanges of the view-sharded step (SURVEY.md section 8e) in ONE launch: the first n_sum_floats of the symmetric
- * buffer are SUMmed over the ranks (parameter gradients, then the grad_norm_accum / collecting_counts rows of the
- * step's densify statistics, model/gaussian.py:196-197), the n_max_floats behind them take the MAXimum (the max_radii
- * row, gaussian.py:194; values must be >= 0: the NVLS variant compares their bit patterns as unsigned integers).
- * Same slicing, same guarantees (one owner GPU per element => bit-identical replicas), same caller-side barriers. */
 int egs_allreduce_f32_peer(int32_t world, int32_t rank, const void* peer_buffers_dev, int64_t n_sum_floats,
                            int64_t n_max_floats, egs_stream_t stream);
+/* The same exchange through the NVSwitch (NVLS): multicast_ptr is the multicast mapping of the symmetric bucket;
+ * rank r pulls the in-switch reduction of slice r (multimem.ld_reduce) and broadcasts it back (multimem.st). */
 int egs_allreduce_f32_multimem(int32_t world, int32_t rank, void* multicast_ptr, int64_t n_sum_floats,
                                int64_t n_max_floats, egs_stream_t stream);
-/* The same exchange restricted to up to 8 ranges of the symmetric buffer (HOST arrays: offsets and lengths in floats,
- * multiples of 4; is_max nullable = all SUM).  Used to exchange the gradients of one chunk of Gaussians — one range per
- * parameter tensor — while the projection backward of the next chunk is still running. */
-int egs_allreduce_ranges_f32_peer(int32_t world, int32_t rank, const void* peer_buffers_dev, int32_t n_ranges,
-                                  const int64_t* offsets_floats, const int64_t* lengths_floats, const int32_t* is_max,
-                                  egs_stream_t stream);
-int egs_allreduce_ranges_f32_multimem(int32_t world, int32_t rank, void* multicast_ptr, int32_t n_ranges,
-                                      const int64_t* offsets_floats, const int64_t* lengths_floats, const int32_t* is_max,
-                                      egs_stream_t stream);
 
 /* ---- measurement utility (bench.py only) -----------------------------------------------------------------
  * Dependent-FMA throughput probe: the FP32-SIMT roofline denominator for the blending kernels

@@ -40,7 +40,7 @@ st = lambda: ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 def peer_allreduce():
     hdl.barrier(channel=0)
-    rc = lib.egs_allreduce_sum_f32_peer(world, rank, ctypes.c_void_p(hdl.buffer_ptrs_dev), n_pad, st())
+    rc = lib.egs_allreduce_f32_peer(world, rank, ctypes.c_void_p(hdl.buffer_ptrs_dev), n_pad, 0, st())
     assert rc == 0, lib.egs_last_error_string()
     hdl.barrier(channel=1)
 
@@ -64,7 +64,7 @@ def tm(fn, reps=20):
 
 def mm_allreduce():
     hdl.barrier(channel=0)
-    rc = lib.egs_allreduce_sum_f32_multimem(world, rank, ctypes.c_void_p(hdl.multicast_ptr), n_pad, st())
+    rc = lib.egs_allreduce_f32_multimem(world, rank, ctypes.c_void_p(hdl.multicast_ptr), n_pad, 0, st())
     assert rc == 0, lib.egs_last_error_string()
     hdl.barrier(channel=1)
 

@@ -489,45 +489,3 @@ def test_automatic_segmentation_from_the_previous_call(monkeypatch):
     torch.cuda.synchronize()
     cuda_run(sc2)
     assert used[-1] == (0, 0), used
-
-
-@pytest.mark.parametrize("raw", [False, True])
-def test_chunked_projection_backward_equals_one_launch(raw):
-    """The multi-GPU exchange overlap launches the projection backward in pieces over the Gaussians
-    (stages.set_grad_chunk_hook): same gradients bit for bit, pieces contiguous, aligned and covering [0, N)."""
-    from easy_gaussian_splatting_b200 import rasterization, rasterization_from_parameters, stages
-    from easy_gaussian_splatting_b200.distributed import FlatGradBucket
-    from easy_gaussian_splatting_b200.synthetic import loss_weights
-    sc = make_scene("outdoor", 20_011, 320, 208, 200.0, 4, n_views=2).to("cuda")
-    C = 2
-    Wc, Wa = (t.cuda() for t in loss_weights(sc.seed, C, sc.height, sc.width))
-    bg = sc.background[None].expand(C, 3).contiguous()
-    src = ([sc.means, sc.quats, torch.log(sc.scales), torch.logit(sc.opacities), sc.colors[:, :1].contiguous(), sc.colors[:, 1:].contiguous()]
-           if raw else [getattr(sc, k) for k in PARAMS])
-
-    def run(hook):
-        params = [t.clone().requires_grad_(True) for t in src]
-        bucket = FlatGradBucket(params)
-        bucket.flat.fill_(float("nan"))
-        bucket.begin_direct(overlap=False)
-        stages.set_grad_chunk_hook(4 if hook else 0, hook)
-        if raw:
-            rc, ra, _ = rasterization_from_parameters(*params, sc.viewmats, sc.Ks, sc.width, sc.height, 3, backgrounds=bg, absgrad=True)
-        else:
-            rc, ra, _ = rasterization(*params, sc.viewmats, sc.Ks, sc.width, sc.height, sh_degree=3, packed=False, absgrad=True, backgrounds=bg)
-        ((rc * Wc).sum() + (ra * Wa).sum()).backward()
-        bucket.end_direct()
-        torch.cuda.synchronize()
-        return torch.cat([v.reshape(-1) for v in bucket.views])  # (the alignment padding between slices is never written)
-
-    pieces = []
-    whole = run(None)
-    chunked = run(lambda i, n0, n1: pieces.append((i, n0, n1)))
-    N = sc.means.shape[0]
-    assert len(pieces) >= 2 and pieces[0][1] == 0 and pieces[-1][2] == N
-    assert all(a[2] == b[1] for a, b in zip(pieces, pieces[1:])) and all(p[1] % 256 == 0 for p in pieces)
-    assert torch.isfinite(chunked).all()
-    # the blend backward's global reductions are not ordered, so two runs differ in the last bits; the projection
-    # backward itself is deterministic, hence the same tolerance as a plain re-run
-    assert float((chunked - whole).norm() / whole.norm()) <= 1e-5
-    assert stages._GRAD_CHUNK_HOOK is None
