@@ -58,6 +58,10 @@ _SIGNATURES = {
     "egs_rasterize_checkpoint_bytes": (c_int64, [I64, I32]),
     "egs_rasterize_fwd_checkpointed": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, I32, I32, P, P]),
     "egs_rasterize_bwd_segmented": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, P, P, I32, I32, P, P, P]),
+    "egs_rasterize_fwd_features": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, I32, P, I32, I32, I32, I32,
+                                             P, P, P, P, P]),
+    "egs_rasterize_bwd_features": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, I32, P, I32, I32, I32, I32,
+                                             P, P, P, P, P, P, P, P]),
     "egs_densify_stats_update": (c_int32, [I32, I32, P, P, F32, P, P, P, P]),
     "egs_l1_ssim_fwd": (c_int32, [I32, I32, I32, P, P, P, P, P, P]),
     "egs_l1_ssim_bwd": (c_int32, [I32, I32, I32, P, P, P, P, F32, P, P, P]),

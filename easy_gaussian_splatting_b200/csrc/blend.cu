@@ -792,6 +792,445 @@ __global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// colours with any number of channels ("features")
+// ------------------------------------------------------------------------------------------------
+// The same blend as above with CH colour channels per launch, read from a separate fp32 row array instead of the r, g, b
+// slots of the splat record (which these kernels do not read).  Row of a list entry: flat id - cam * N when one [N, .]
+// array serves every camera, the flat id for a [C * N, .] array.  A launch covers channels [c0, c0 + CH) of the rows;
+// wider colours are several launches on the same binning result.  The accept / finish tests and the alpha arithmetic are
+// the RGB kernels'; in the <2,2> layout (CH <= 8) alphas and last_ids come out bit-identical to them, while the <1,1>
+// layout's transmittance differs in the last bits (measured on a B200: alphas within 2.4e-7).
+// Pixel layout: CH <= 8 keeps the RGB kernels' <2,2> layout (4 pixels per lane, 4 CH colour registers); CH = 16 / 32
+// use <1,1> (one pixel per lane, 8 warps per tile), which keeps the per-lane colour state at CH registers.  Long lists
+// are always replayed in one piece (no checkpoints).
+constexpr int kFeatRedRows = 16;  // values per warp-sum round of the feature backward (two lanes per value)
+
+template <int CH>
+struct FeatGeo {
+  static constexpr int P = CH <= 8 ? 2 : 1;
+  using G = Geo<P, P>;
+};
+
+// Per-warp shared memory of the feature kernels (dynamic: up to ~111 KB per CTA at CH = 32): the RGB staging plus the
+// colour rows of both batches.  The backward kernel places its warp-sum scratch behind the array of these.
+template <int kBatch, int CH>
+struct FeatStage {
+  WarpStage<kBatch> w;
+  float feat[2][kBatch * CH];
+};
+
+template <int BYTES>
+__device__ __forceinline__ void cp_async_ca(void* smem, const void* gmem) {
+  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
+  asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"(s), "l"(gmem), "n"(BYTES) : "memory");
+}
+
+// One colour row of CH floats: 4- or 8-byte copies for CH = 1 / 2, 16-byte copies from CH = 4 on (the entries check
+// that features, feat_stride and c0 are aligned for that).
+template <int CH>
+__device__ __forceinline__ void cp_async_row(float* dst, const float* src) {
+  if constexpr (CH == 1) {
+    cp_async_ca<4>(dst, src);
+  } else if constexpr (CH == 2) {
+    cp_async_ca<8>(dst, src);
+  } else {
+#pragma unroll
+    for (int i = 0; i < CH; i += 4) cp_async16(dst + i, src + i);
+  }
+}
+
+template <int CH>
+__device__ __forceinline__ void load_row(float (&f)[CH], const float* src) {
+  if constexpr (CH >= 4) {
+#pragma unroll
+    for (int i = 0; i < CH; i += 4) {
+      const float4 t = *reinterpret_cast<const float4*>(src + i);
+      f[i] = t.x; f[i + 1] = t.y; f[i + 2] = t.z; f[i + 3] = t.w;
+    }
+  } else {
+#pragma unroll
+    for (int i = 0; i < CH; ++i) f[i] = src[i];
+  }
+}
+
+// q = -log2(e) * sigma and ov = opacity * 2^q (before the 0.999 clamp) at the lane's pixels, with dx / dy = mean - pixel
+// centre per column / row.  The RGB kernels' operations in the same order: packed FADD2 / FMUL2 / FFMA2 in the <2,2>
+// layout, the same sequence one pixel at a time in <1,1>.
+template <int P>
+__device__ __forceinline__ void splat_eval(const float4 g0, const float4 g1, const float2 npx2, const float2 npy2,
+                                           float (&dx)[P], float (&dy)[P], float (&q)[P * P], float (&ov)[P * P]) {
+  const float la = (0.5f * kNegLog2e) * g0.z, lc = (0.5f * kNegLog2e) * g1.x, lb = kNegLog2e * g0.w;
+  if constexpr (P == 2) {
+    const float2 dx2 = __fadd2_rn(make_float2(g0.x, g0.x), npx2);
+    const float2 dy2 = __fadd2_rn(make_float2(g0.y, g0.y), npy2);
+    const float2 qx = __fmul2_rn(__fmul2_rn(dx2, make_float2(la, la)), dx2);
+    const float2 bx = __fmul2_rn(dx2, make_float2(lb, lb));
+    const float2 qy = __fmul2_rn(__fmul2_rn(dy2, make_float2(lc, lc)), dy2);
+    const float2 o2 = make_float2(g1.y, g1.y);
+    const float2 q0 = __ffma2_rn(bx, make_float2(dy2.x, dy2.x), __fadd2_rn(qx, make_float2(qy.x, qy.x)));
+    const float2 q1 = __ffma2_rn(bx, make_float2(dy2.y, dy2.y), __fadd2_rn(qx, make_float2(qy.y, qy.y)));
+    const float2 a0 = __fmul2_rn(o2, make_float2(fast_ex2(q0.x), fast_ex2(q0.y)));
+    const float2 a1 = __fmul2_rn(o2, make_float2(fast_ex2(q1.x), fast_ex2(q1.y)));
+    dx[0] = dx2.x; dx[1] = dx2.y; dy[0] = dy2.x; dy[1] = dy2.y;
+    q[0] = q0.x; q[1] = q0.y; q[2] = q1.x; q[3] = q1.y;
+    ov[0] = a0.x; ov[1] = a0.y; ov[2] = a1.x; ov[3] = a1.y;
+  } else {
+    static_assert(P == 1, "the feature kernels use the <2,2> and <1,1> layouts");
+    dx[0] = __fadd_rn(g0.x, npx2.x);
+    dy[0] = __fadd_rn(g0.y, npy2.x);
+    const float qx = __fmul_rn(__fmul_rn(dx[0], la), dx[0]), bx = __fmul_rn(dx[0], lb);
+    const float qy = __fmul_rn(__fmul_rn(dy[0], lc), dy[0]);
+    q[0] = __fmaf_rn(bx, dy[0], __fadd_rn(qx, qy));
+    ov[0] = __fmul_rn(g1.y, fast_ex2(q[0]));
+  }
+}
+
+template <int CH>
+__global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_fwd_features_kernel(
+    int64_t n_isects, const float4* __restrict__ splats, const int32_t* __restrict__ tile_offsets,
+    const int32_t* __restrict__ flatten_ids, const float* __restrict__ features, int feat_stride, int row_cam_stride,
+    int D, int c0, const float* __restrict__ backgrounds, int width, int height, int tile_w, int tile_h,
+    int n_tiles_total, float* __restrict__ render_colors, float* __restrict__ render_alphas,
+    int32_t* __restrict__ last_ids, const int32_t* __restrict__ tile_order) {
+  constexpr int P = FeatGeo<CH>::P;
+  using G = typename FeatGeo<CH>::G;
+  constexpr int NP = G::NP, RPL = G::RPL, kBatch = G::kBatch;
+  extern __shared__ __align__(16) unsigned char feat_smem[];
+  FeatStage<kBatch, CH>& fs = reinterpret_cast<FeatStage<kBatch, CH>*>(feat_smem)[threadIdx.x >> 5];
+  WarpStage<kBatch>& st = fs.w;
+  const int lane = threadIdx.x & 31;
+  const int ordered_tile =
+      tile_order != nullptr ? tile_order[(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] : -1;
+  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, ordered_tile);
+  const int nb = (wv.range_end - wv.range_start + kBatch - 1) / kBatch;
+  const int64_t row_off = (int64_t)wv.cam * row_cam_stride;
+
+  float pxf[P], pyf[P];
+#pragma unroll
+  for (int i = 0; i < P; ++i) pxf[i] = opaque((float)(wv.x0 + i) + 0.5f);
+#pragma unroll
+  for (int i = 0; i < P; ++i) pyf[i] = opaque((float)(wv.y0 + i) + 0.5f);
+  const float2 npx2 = make_float2(-pxf[0], -pxf[P - 1]), npy2 = make_float2(-pyf[0], -pyf[P - 1]);
+  const float rx_lo = opaque(wv.rx_lo), rx_hi = opaque(wv.rx_hi), ry_lo = opaque(wv.ry_lo), ry_hi = opaque(wv.ry_hi);
+  // T as in the RGB kernel: > 0 live, < 0 finished with final transmittance |T|
+  float T[NP], col[NP][CH];
+  int last[NP];
+  bool all_done = true;
+#pragma unroll
+  for (int j = 0; j < NP; ++j) {
+    const bool inside = (wv.x0 + (j % P)) < width && (wv.y0 + (j / P)) < height;
+    T[j] = inside ? 1.0f : -1.0f;
+    last[j] = 0;
+#pragma unroll
+    for (int k = 0; k < CH; ++k) col[j][k] = 0.f;
+    all_done = all_done && !inside;
+  }
+
+  auto load_ids = [&](int b, int (&ids)[RPL]) {
+#pragma unroll
+    for (int r = 0; r < RPL; ++r) {
+      const int idx = wv.range_start + b * kBatch + r * 32 + lane;
+      ids[r] = (b < nb && idx < wv.range_end) ? __ldg(flatten_ids + idx) : -1;
+    }
+  };
+  auto issue = [&](int buf, const int (&ids)[RPL]) {
+#pragma unroll
+    for (int r = 0; r < RPL; ++r) {
+      if (ids[r] >= 0) {
+        const int slot = r * 32 + lane;
+        const float4* src = splats + (size_t)ids[r] * 3;
+        float4* dst = &st.rec[buf][slot * 3];
+        cp_async16(dst + 0, src + 0);
+        cp_async16(dst + 1, src + 1);
+        cp_async16(dst + 2, src + 2);
+        cp_async_row<CH>(&fs.feat[buf][slot * CH], features + ((int64_t)ids[r] - row_off) * feat_stride + c0);
+      }
+    }
+    cp_async_commit();
+  };
+
+  if (nb > 0 && !__all_sync(0xffffffffu, all_done)) {
+    int ids[RPL];
+    load_ids(0, ids);
+    issue(0, ids);
+    load_ids(1, ids);
+    for (int b = 0; b < nb; ++b) {
+      if (b + 1 < nb) {
+        issue((b + 1) & 1, ids);
+        load_ids(b + 2, ids);
+        cp_async_wait<1>();
+      } else {
+        cp_async_wait<0>();
+      }
+      __syncwarp();
+      const int batch_start = wv.range_start + b * kBatch;
+      const int batch_size = min(kBatch, wv.range_end - batch_start);
+      const int ns = cull_and_compact<RPL>(st, b & 1, batch_size, lane, rx_lo, rx_hi, ry_lo, ry_hi);
+      const float4* s = st.rec[b & 1];
+      for (int t = 0; t < ns; ++t) {
+        if (__all_sync(0xffffffffu, all_done)) break;  // warp-uniform exit and reconvergence point
+        const int cur = st.list[t];
+        float dx[P], dy[P], q[NP], ov[NP];
+        splat_eval<P>(s[cur * 3 + 0], s[cur * 3 + 1], npx2, npy2, dx, dy, q, ov);
+        float f[CH];
+        load_row<CH>(f, &fs.feat[b & 1][cur * CH]);
+        float tmax = -1.0f;
+#pragma unroll
+        for (int j = 0; j < NP; ++j) {
+          // branch free: a rejected or finished pixel blends with weight 0 and keeps its T (as the RGB kernel)
+          const float alpha = fminf(kAlphaMax, ov[j]);
+          const float nT = __fmul_rn(T[j], __fmaf_rn(alpha, -1.f, 1.f));
+          const bool acc = T[j] > 0.f && q[j] <= 0.f && alpha >= kAlphaMin;
+          const bool bl = acc && nT > kTMin;
+          const float w = bl ? __fmul_rn(alpha, T[j]) : 0.f;
+          if (acc) T[j] = bl ? nT : -T[j];
+          if (bl) last[j] = batch_start + cur;
+#pragma unroll
+          for (int k = 0; k < CH; ++k) col[j][k] = __fmaf_rn(f[k], w, col[j][k]);
+          tmax = fmaxf(tmax, T[j]);
+        }
+        all_done = !(tmax > 0.f);
+      }
+      if (__all_sync(0xffffffffu, all_done)) break;
+      __syncwarp();  // every lane is done with buffer b&1 and the list before they are overwritten
+    }
+    cp_async_wait<0>();
+  }
+
+  const int nc = min(CH, D - c0);
+  float bg[CH];
+#pragma unroll
+  for (int k = 0; k < CH; ++k) bg[k] = (backgrounds != nullptr && k < nc) ? backgrounds[(size_t)wv.cam * D + c0 + k] : 0.f;
+#pragma unroll
+  for (int j = 0; j < NP; ++j) {
+    const int x = wv.x0 + (j % P), y = wv.y0 + (j / P);
+    if (x < width && y < height) {
+      const size_t pix = ((size_t)wv.cam * height + y) * width + x;
+      const float Tf = fabsf(T[j]);
+      float* out = render_colors + pix * D + c0;
+#pragma unroll
+      for (int k = 0; k < CH; ++k)
+        if (k < nc) out[k] = fmaf(Tf, bg[k], col[j][k]);
+      if (render_alphas != nullptr) render_alphas[pix] = 1.0f - Tf;
+      if (last_ids != nullptr) last_ids[pix] = last[j];
+    }
+  }
+}
+
+template <int CH>
+__global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_bwd_features_kernel(
+    int64_t n_isects, const float4* __restrict__ splats, const int32_t* __restrict__ tile_offsets,
+    const int32_t* __restrict__ flatten_ids, const float* __restrict__ features, int feat_stride, int row_cam_stride,
+    int D, int c0, const float* __restrict__ backgrounds, int width, int height, int tile_w, int tile_h,
+    int n_tiles_total, const float* __restrict__ render_alphas, const int32_t* __restrict__ last_ids,
+    const float* __restrict__ v_render_colors, const float* __restrict__ v_render_alphas, float* __restrict__ v_splats,
+    float* __restrict__ v_features, const int32_t* __restrict__ tile_order) {
+  constexpr int P = FeatGeo<CH>::P;
+  using G = typename FeatGeo<CH>::G;
+  constexpr int NP = G::NP, RPL = G::RPL, kBatch = G::kBatch;
+  constexpr int kValues = 8 + CH;  // v_x, v_y, v_conic (3), v_opacity, |v_x|, |v_y|, then the CH colour partials
+  constexpr int kRounds = (kValues + kFeatRedRows - 1) / kFeatRedRows;
+  extern __shared__ __align__(16) unsigned char feat_smem[];
+  FeatStage<kBatch, CH>* stages = reinterpret_cast<FeatStage<kBatch, CH>*>(feat_smem);
+  FeatStage<kBatch, CH>& fs = stages[threadIdx.x >> 5];
+  WarpStage<kBatch>& st = fs.w;
+  float* red = reinterpret_cast<float*>(stages + G::kWarps) + (threadIdx.x >> 5) * (kFeatRedRows * kRedStride);
+  const int lane = threadIdx.x & 31;
+  const int ordered_tile =
+      tile_order != nullptr ? tile_order[(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] : -1;
+  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, ordered_tile);
+  if (wv.range_end - wv.range_start <= 0) return;  // block-uniform
+  const int64_t row_off = (int64_t)wv.cam * row_cam_stride;
+
+  float pxf[P], pyf[P];
+#pragma unroll
+  for (int i = 0; i < P; ++i) pxf[i] = opaque((float)(wv.x0 + i) + 0.5f);
+#pragma unroll
+  for (int i = 0; i < P; ++i) pyf[i] = opaque((float)(wv.y0 + i) + 0.5f);
+  const float2 npx2 = make_float2(-pxf[0], -pxf[P - 1]), npy2 = make_float2(-pyf[0], -pyf[P - 1]);
+  const float rx_lo = opaque(wv.rx_lo), rx_hi = opaque(wv.rx_hi), ry_lo = opaque(wv.ry_lo), ry_hi = opaque(wv.ry_hi);
+
+  // replay state as in the RGB kernel: nbt_ = T_final * (v_alpha_out - bg . v_colour) - (colour behind) . v_colour,
+  // over this chunk's channels; v_alpha_out only where the caller passes it (one chunk of a call)
+  const int nc = min(CH, D - c0);
+  float bg[CH];
+#pragma unroll
+  for (int k = 0; k < CH; ++k) bg[k] = (backgrounds != nullptr && k < nc) ? backgrounds[(size_t)wv.cam * D + c0 + k] : 0.f;
+  float T[NP], nbt_[NP], vc[NP][CH];
+  int bin_final[NP];
+  int my_last = -1;
+#pragma unroll
+  for (int j = 0; j < NP; ++j) {
+    const int x = wv.x0 + (j % P), y = wv.y0 + (j / P);
+    T[j] = 1.f; nbt_[j] = 0.f; bin_final[j] = -1;
+#pragma unroll
+    for (int k = 0; k < CH; ++k) vc[j][k] = 0.f;
+    if (x < width && y < height) {
+      const size_t pix = ((size_t)wv.cam * height + y) * width + x;
+      const float T_final = 1.0f - render_alphas[pix];
+      T[j] = T_final;
+      bin_final[j] = last_ids[pix];
+      float bdot = 0.f;
+#pragma unroll
+      for (int k = 0; k < CH; ++k) {
+        if (k < nc) vc[j][k] = v_render_colors[pix * D + c0 + k];
+        bdot = fmaf(bg[k], vc[j][k], bdot);
+      }
+      nbt_[j] = T_final * ((v_render_alphas != nullptr ? v_render_alphas[pix] : 0.f) - bdot);
+    }
+    my_last = max(my_last, bin_final[j]);
+  }
+  const int warp_last = __reduce_max_sync(0xffffffffu, my_last);
+  const int end_idx = min(wv.range_end - 1, warp_last);
+  if (end_idx < wv.range_start) return;  // warp-uniform
+  const int lo_idx = wv.range_start;
+  const int nb = (end_idx - lo_idx + 1 + kBatch - 1) / kBatch;
+
+  auto load_ids = [&](int b, int (&ids)[RPL]) {
+#pragma unroll
+    for (int r = 0; r < RPL; ++r) {
+      const int idx = end_idx - b * kBatch - (r * 32 + lane);
+      ids[r] = (b < nb && idx >= lo_idx) ? __ldg(flatten_ids + idx) : -1;
+    }
+  };
+  auto issue = [&](int buf, const int (&ids)[RPL]) {
+#pragma unroll
+    for (int r = 0; r < RPL; ++r) {
+      const int slot = r * 32 + lane;
+      if (ids[r] >= 0) {
+        const float4* src = splats + (size_t)ids[r] * 3;
+        float4* dst = &st.rec[buf][slot * 3];
+        cp_async16(dst + 0, src + 0);
+        cp_async16(dst + 1, src + 1);
+        cp_async16(dst + 2, src + 2);
+        cp_async_row<CH>(&fs.feat[buf][slot * CH], features + ((int64_t)ids[r] - row_off) * feat_stride + c0);
+      }
+      st.id[buf][slot] = ids[r];
+    }
+    cp_async_commit();
+  };
+
+  // Warp sum in rounds of 16 values: lane 2k+p adds half p of row k, lane 2k issues the RED of value 16 r + k.
+  // Value v < 8 goes to the gradient record (slots 0-5, then |v_x|, |v_y| in slots 9, 10; the r, g, b slots stay 0),
+  // value 8 + c to v_features (only the chunk's nc real channels, and only when v_features is given).
+  const int out_slot = lane >> 1;
+  const uint32_t red_st = (uint32_t)__cvta_generic_to_shared(red + lane);
+  const float4* row = reinterpret_cast<const float4*>(red + out_slot * kRedStride + (lane & 1) * 16);
+  int rec_off[kRounds], red_flag[kRounds];
+#pragma unroll
+  for (int r = 0; r < kRounds; ++r) {
+    const int v = r * kFeatRedRows + out_slot;
+    const bool is_feat = v >= 8;
+    red_flag[r] = ((lane & 1) == 0 && v < kValues && (!is_feat || (v - 8 < nc && v_features != nullptr))) ? 1 : 0;
+    rec_off[r] = is_feat ? c0 + (v - 8) : (v < 6 ? v : v + 3);
+  }
+
+  int ids[RPL];
+  load_ids(0, ids);
+  issue(0, ids);
+  load_ids(1, ids);
+  for (int b = 0; b < nb; ++b) {
+    if (b + 1 < nb) {
+      issue((b + 1) & 1, ids);
+      load_ids(b + 2, ids);
+      cp_async_wait<1>();
+    } else {
+      cp_async_wait<0>();
+    }
+    __syncwarp();
+    const int batch_end = end_idx - b * kBatch;
+    const int batch_size = min(kBatch, batch_end + 1 - lo_idx);
+    const int ns = cull_and_compact<RPL>(st, b & 1, batch_size, lane, rx_lo, rx_hi, ry_lo, ry_hi);
+    const float4* s = st.rec[b & 1];
+    const int* sid = st.id[b & 1];
+    for (int t = 0; t < ns; ++t) {  // warp-uniform bounds
+      const int cur = st.list[t];
+      const int idx = batch_end - cur;
+      const float4 g0 = s[cur * 3 + 0];
+      const float4 g1 = s[cur * 3 + 1];
+      float dx[P], dy[P], q[NP], ov[NP];
+      splat_eval<P>(g0, g1, npx2, npy2, dx, dy, q, ov);
+      bool valid[NP];
+      bool any_valid = false;
+#pragma unroll
+      for (int j = 0; j < NP; ++j) {
+        valid[j] = idx <= bin_final[j] && q[j] <= 0.f && ov[j] >= kAlphaMin;
+        any_valid = any_valid || valid[j];
+      }
+      if (!__any_sync(0xffffffffu, any_valid)) continue;  // warp-uniform
+      float f[CH];
+      load_row<CH>(f, &fs.feat[b & 1][cur * CH]);
+      const float inv_o = fast_rcp(g1.y);
+      // branch free as the RGB kernel: a pixel that does not take part has ov = 0, hence alpha = 0, 1 - alpha = 1,
+      // MUFU.RCP(1) = 1, and contributes exact zeros
+      float v[8], fac[NP];
+#pragma unroll
+      for (int k = 0; k < 8; ++k) v[k] = 0.f;
+#pragma unroll
+      for (int j = 0; j < NP; ++j) {
+        const float ddx = dx[j % P], ddy = dy[j / P];
+        const float ovj = valid[j] ? ov[j] : 0.f;
+        const float ae = fminf(kAlphaMax, ovj);
+        const float oe = ovj <= kAlphaMax ? ovj : 0.f;  // clamp inactive: alpha depends on sigma and opacity
+        const float ra = fast_rcp(fmaf(ae, -1.f, 1.f));
+        T[j] *= ra;  // transmittance in front of this Gaussian
+        fac[j] = ae * T[j];
+        float cdot = 0.f;
+#pragma unroll
+        for (int k = 0; k < CH; ++k) cdot = fmaf(f[k], vc[j][k], cdot);
+        const float v_alpha = fmaf(T[j], cdot, ra * nbt_[j]);
+        nbt_[j] = fmaf(cdot, -fac[j], nbt_[j]);
+        const float w = oe * v_alpha;  // = -v_sigma
+        const float sx = -w * ddx, sy = -w * ddy;
+        v[2] = fmaf(sx, ddx, v[2]);
+        v[3] = fmaf(sx, ddy, v[3]);
+        v[4] = fmaf(sy, ddy, v[4]);
+        const float gx = fmaf(g0.w, sy, g0.z * sx);
+        const float gy = fmaf(g1.x, sy, g0.w * sx);
+        v[0] += gx;
+        v[1] += gy;
+        v[6] += fabsf(gx);
+        v[7] += fabsf(gy);
+        v[5] += w;
+      }
+      v[2] *= 0.5f; v[4] *= 0.5f; v[5] *= inv_o;
+      const int64_t fid = sid[cur];
+#pragma unroll
+      for (int r = 0; r < kRounds; ++r) {
+        __syncwarp();  // the previous round's (or survivor's) row reads are complete
+#pragma unroll
+        for (int i = 0; i < kFeatRedRows; ++i) {
+          const int vi = r * kFeatRedRows + i;
+          if (vi < 8) {
+            sts_f32(red_st + i * kRedStride * 4, v[vi]);
+          } else if (vi < kValues) {
+            float pf = 0.f;
+#pragma unroll
+            for (int j = 0; j < NP; ++j) pf = fmaf(fac[j], vc[j][vi - 8], pf);
+            sts_f32(red_st + i * kRedStride * 4, pf);
+          }
+        }
+        __syncwarp();
+        // rows past the round's last value hold stale data; no lane issues them
+        const float4 r0 = row[0], r1 = row[1], r2 = row[2], r3 = row[3];
+        float2 s0 = __fadd2_rn(make_float2(r0.x, r0.y), make_float2(r0.z, r0.w));
+        float2 s1 = __fadd2_rn(make_float2(r1.x, r1.y), make_float2(r1.z, r1.w));
+        float2 s2 = __fadd2_rn(make_float2(r2.x, r2.y), make_float2(r2.z, r2.w));
+        float2 s3 = __fadd2_rn(make_float2(r3.x, r3.y), make_float2(r3.z, r3.w));
+        s0 = __fadd2_rn(__fadd2_rn(s0, s1), __fadd2_rn(s2, s3));
+        float total = s0.x + s0.y;
+        total += __shfl_xor_sync(0xffffffffu, total, 1);
+        const bool feat_slot = r * kFeatRedRows + out_slot >= 8;
+        float* dst = feat_slot ? v_features + (fid - row_off) * feat_stride + rec_off[r]
+                               : v_splats + fid * EGS_SPLAT_FLOATS + rec_off[r];
+        red_add_f32_if(red_flag[r], dst, total);
+      }
+    }
+    __syncwarp();  // buffer b&1, its ids and the list are free again
+  }
+}
+
 }  // namespace egs
 
 using namespace egs;
@@ -946,4 +1385,104 @@ extern "C" int egs_rasterize_bwd_segmented(int32_t C, int32_t N, int64_t n_isect
   return launch_bwd(C, n_isects, splats, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height,
                     render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, render_colors, checkpoints,
                     segment, seg_min_len, tile_order, stream);
+}
+
+// ---- colours with any number of channels -------------------------------------------------------------------------
+static int check_feature_args(const char* who, int32_t N, const float* features, int32_t feat_stride,
+                              int32_t shared_rows, int32_t D, int32_t c0, int32_t CH) {
+  EGS_REQUIRE(CH == 1 || CH == 2 || CH == 4 || CH == 8 || CH == 16 || CH == 32,
+              "%s: CH=%d is not an instantiated chunk width (1, 2, 4, 8, 16, 32)", who, CH);
+  EGS_REQUIRE(D >= 1, "%s: D=%d must be >= 1", who, D);
+  EGS_REQUIRE(c0 >= 0 && c0 < D, "%s: c0=%d out of [0, D=%d)", who, c0, D);
+  EGS_REQUIRE(shared_rows == 0 || shared_rows == 1, "%s: shared_rows must be 0 or 1", who);
+  EGS_REQUIRE(N >= 0, "%s: N=%d must be >= 0", who, N);
+  EGS_REQUIRE(features != nullptr, "%s: features is required", who);
+  EGS_REQUIRE(feat_stride >= c0 + CH, "%s: feat_stride=%d < c0 + CH = %d (rows are read CH floats wide)", who,
+              feat_stride, c0 + CH);
+  const int align = CH < 4 ? CH : 4;  // floats per cp.async copy of a row
+  EGS_REQUIRE(feat_stride % align == 0 && c0 % align == 0 && (uintptr_t)features % (4 * align) == 0,
+              "%s: CH=%d reads %d-byte pieces: feat_stride=%d, c0=%d and the features pointer must be aligned to them",
+              who, CH, 4 * align, feat_stride, c0);
+  return 0;
+}
+
+template <int CH>
+static size_t feature_smem_bytes(bool backward) {
+  using G = typename FeatGeo<CH>::G;
+  return G::kWarps * (sizeof(FeatStage<G::kBatch, CH>) + (backward ? kFeatRedRows * kRedStride * sizeof(float) : 0));
+}
+
+template <int CH>
+static int launch_fwd_features(int32_t C, int32_t N, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
+                               const int32_t* flatten_ids, const float* features, int32_t feat_stride,
+                               int32_t shared_rows, int32_t D, int32_t c0, const float* backgrounds, int32_t width,
+                               int32_t height, int32_t tile_width, int32_t tile_height, float* render_colors,
+                               float* render_alphas, int32_t* last_ids, const int32_t* tile_order, cudaStream_t st) {
+  const size_t smem = feature_smem_bytes<CH>(false);
+  EGS_CUDA(cudaFuncSetAttribute(rasterize_fwd_features_kernel<CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  dim3 grid(tile_width, tile_height, C);
+  rasterize_fwd_features_kernel<CH><<<grid, FeatGeo<CH>::G::kThreads, smem, st>>>(
+      n_isects, reinterpret_cast<const float4*>(splats), tile_offsets, flatten_ids, features, feat_stride,
+      shared_rows ? N : 0, D, c0, backgrounds, width, height, tile_width, tile_height, C * tile_width * tile_height,
+      render_colors, render_alphas, last_ids, tile_order);
+  return check_launch("rasterize_fwd_features_kernel");
+}
+
+template <int CH>
+static int launch_bwd_features(int32_t C, int32_t N, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
+                               const int32_t* flatten_ids, const float* features, int32_t feat_stride,
+                               int32_t shared_rows, int32_t D, int32_t c0, const float* backgrounds, int32_t width,
+                               int32_t height, int32_t tile_width, int32_t tile_height, const float* render_alphas,
+                               const int32_t* last_ids, const float* v_render_colors, const float* v_render_alphas,
+                               float* v_splats, float* v_features, const int32_t* tile_order, cudaStream_t st) {
+  const size_t smem = feature_smem_bytes<CH>(true);
+  EGS_CUDA(cudaFuncSetAttribute(rasterize_bwd_features_kernel<CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  dim3 grid(tile_width, tile_height, C);
+  rasterize_bwd_features_kernel<CH><<<grid, FeatGeo<CH>::G::kThreads, smem, st>>>(
+      n_isects, reinterpret_cast<const float4*>(splats), tile_offsets, flatten_ids, features, feat_stride,
+      shared_rows ? N : 0, D, c0, backgrounds, width, height, tile_width, tile_height, C * tile_width * tile_height,
+      render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, v_features, tile_order);
+  return check_launch("rasterize_bwd_features_kernel");
+}
+
+#define EGS_FEATURE_DISPATCH(LAUNCH, ...)        \
+  switch (CH) {                                  \
+    case 1: return LAUNCH<1>(__VA_ARGS__);       \
+    case 2: return LAUNCH<2>(__VA_ARGS__);       \
+    case 4: return LAUNCH<4>(__VA_ARGS__);       \
+    case 8: return LAUNCH<8>(__VA_ARGS__);       \
+    case 16: return LAUNCH<16>(__VA_ARGS__);     \
+    default: return LAUNCH<32>(__VA_ARGS__);     \
+  }
+
+extern "C" int egs_rasterize_fwd_features(int32_t C, int32_t N, int64_t n_isects, const float* splats,
+                                          const int32_t* tile_offsets, const int32_t* flatten_ids,
+                                          const float* features, int32_t feat_stride, int32_t shared_rows, int32_t D,
+                                          int32_t c0, int32_t CH, const float* backgrounds, int32_t width,
+                                          int32_t height, int32_t tile_width, int32_t tile_height,
+                                          float* render_colors, float* render_alphas, int32_t* last_ids,
+                                          const int32_t* tile_order, egs_stream_t stream) {
+  if (int rc = check_raster_args("rasterize_fwd_features", C, n_isects, width, height, tile_width, tile_height)) return rc;
+  if (int rc = check_feature_args("rasterize_fwd_features", N, features, feat_stride, shared_rows, D, c0, CH)) return rc;
+  EGS_REQUIRE(render_colors != nullptr, "rasterize_fwd_features: render_colors is required");
+  if (C == 0) return 0;
+  EGS_FEATURE_DISPATCH(launch_fwd_features, C, N, n_isects, splats, tile_offsets, flatten_ids, features, feat_stride,
+                       shared_rows, D, c0, backgrounds, width, height, tile_width, tile_height, render_colors,
+                       render_alphas, last_ids, tile_order, (cudaStream_t)stream)
+}
+
+extern "C" int egs_rasterize_bwd_features(int32_t C, int32_t N, int64_t n_isects, const float* splats,
+                                          const int32_t* tile_offsets, const int32_t* flatten_ids,
+                                          const float* features, int32_t feat_stride, int32_t shared_rows, int32_t D,
+                                          int32_t c0, int32_t CH, const float* backgrounds, int32_t width,
+                                          int32_t height, int32_t tile_width, int32_t tile_height,
+                                          const float* render_alphas, const int32_t* last_ids,
+                                          const float* v_render_colors, const float* v_render_alphas, float* v_splats,
+                                          float* v_features, const int32_t* tile_order, egs_stream_t stream) {
+  if (int rc = check_raster_args("rasterize_bwd_features", C, n_isects, width, height, tile_width, tile_height)) return rc;
+  if (int rc = check_feature_args("rasterize_bwd_features", N, features, feat_stride, shared_rows, D, c0, CH)) return rc;
+  if (C == 0 || n_isects == 0) return 0;
+  EGS_FEATURE_DISPATCH(launch_bwd_features, C, N, n_isects, splats, tile_offsets, flatten_ids, features, feat_stride,
+                       shared_rows, D, c0, backgrounds, width, height, tile_width, tile_height, render_alphas, last_ids,
+                       v_render_colors, v_render_alphas, v_splats, v_features, tile_order, (cudaStream_t)stream)
 }

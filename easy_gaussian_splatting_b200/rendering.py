@@ -123,19 +123,20 @@ def _tag_absgrad(target: Tensor, absgrad: Tensor, packed_index: Optional[Tensor]
     target.absgrad = absgrad if packed_index is None else absgrad.reshape(-1, 2)[packed_index]
 
 
-def _bin_and_blend(ctx, proj, backgrounds, width, height, grad_enabled=True):
+def _bin_and_blend(ctx, proj, backgrounds, width, height, grad_enabled=True, features=None):
     """Binning + blend forward, enqueued without waiting for the intersection count (stages.isect_sorted_async): the
     buffers are sized from the previous call of this shape, the count is looked at only after the blend forward is
     in the queue, and a guess that turns out too small is repaired by running both again with the exact size.
     When a backward pass will follow and the previous call saw outlier-long tile lists, the checkpointed forward is
     used so that the backward pass can replay those lists in segments (stages.segment_policy).
     (grad_enabled is the CALLER's grad mode: inside Function.forward it is always off, and needs_input_grad stays
-    true under no_grad.)"""
+    true under no_grad.)  features: colours of any width ([N,D] / [C,N,D]) blended by the feature kernels instead of
+    the colours in the splat records; they are never checkpointed."""
     tw, th = stages.tile_grid(width, height)
     C = proj["radii"].shape[0]
     dev = proj["radii"].device
     seg, seg_min = 0, 0
-    if grad_enabled and any(ctx.needs_input_grad):
+    if features is None and grad_enabled and any(ctx.needs_input_grad):
         seg, seg_min = stages.segment_policy(stages.binning_hint(C, tw, th, dev), C * tw * th)
     capacity = None
     while True:
@@ -143,14 +144,17 @@ def _bin_and_blend(ctx, proj, backgrounds, width, height, grad_enabled=True):
             b = stages.isect_sorted_async(proj["means2d"], proj["radii"], proj["depths"], proj["tiles_per_gauss"],
                                           stages.TILE_SIZE, tw, th, capacity=capacity, tight_rects=proj["tight_rects"])
         with stages.nvtx_range("egs.rasterize_fwd"):
-            if seg > 0:
+            ckpt = None
+            if features is not None:
+                rc, ra, last = stages.rasterize_fwd_features(proj["splats"], b.offsets, b.flat_cap, features, backgrounds,
+                                                             width, height, n_isects=b.raster_n, tile_order=b.tile_order)
+            elif seg > 0:
                 rc, ra, last, ckpt = stages.rasterize_fwd_checkpointed(proj["splats"], b.offsets, b.flat_cap, backgrounds, width,
                                                                        height, seg, seg_min_len=seg_min, n_isects=b.raster_n,
                                                                        tile_order=b.tile_order)
             else:
                 rc, ra, last = stages.rasterize_fwd(proj["splats"], b.offsets, b.flat_cap, backgrounds, width, height,
                                                     n_isects=b.raster_n, tile_order=b.tile_order)
-                ckpt = None
         if b.resolve():
             break
         capacity = b.n_isects  # the guess was too small (rare): same route again, exactly sized
@@ -170,6 +174,11 @@ def _blend_backward(ctx, splats, isect_offsets, flatten_ids, backgrounds, width,
                                     v_colors, v_alphas, n_isects=ctx.raster_n, tile_order=ctx.tile_order)
 
 
+def _zero_rgb(means: Tensor) -> Tensor:
+    """The [N,3] colours the projection is given when the blend takes its colours from elsewhere (feature path)."""
+    return torch.zeros(means.shape[0], 3, dtype=torch.float32, device=means.device)
+
+
 class _Rasterization(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means, quats, scales, opacities, colors, viewmats, Ks, backgrounds, cfg):
@@ -180,14 +189,19 @@ class _Rasterization(torch.autograd.Function):
         # input such as ``viewmats = torch.linalg.inv(camtoworlds)`` must not reach it as is.
         means, quats, scales, opacities, colors, viewmats, Ks, backgrounds = stages.dense_inputs(
             means, quats, scales, opacities, colors, viewmats, Ks, backgrounds)
+        # colours that are not RGB (cfg["features"], set by rasterization()) go to the feature blend; the projection gets
+        # zero RGB colours
+        feat = cfg.get("features", False)
+        features = colors if feat else None
+        rgb = _zero_rgb(means) if feat else colors
         with stages.nvtx_range("egs.projection_fwd"):
-            proj = stages.projection_fwd(means, quats, scales, opacities, colors, viewmats, Ks, width, height, sh_degree,
+            proj = stages.projection_fwd(means, quats, scales, opacities, rgb, viewmats, Ks, width, height, sh_degree,
                                          eps2d=cfg["eps2d"], near_plane=cfg["near_plane"], far_plane=cfg["far_plane"],
                                          radius_clip=cfg["radius_clip"], antialiased=cfg["antialiased"])
         cfg["compensations"] = proj.get("compensations")  # non-differentiable side output, like the thunk below
         tiles_per_gauss = proj["tiles_per_gauss"]
         binned, render_colors, render_alphas, last_ids, ckpt = _bin_and_blend(ctx, proj, backgrounds, width, height,
-                                                                             cfg.get("grad_enabled", True))
+                                                                             cfg.get("grad_enabled", True), features)
         # meta's three list entries are gsplat's lists, built on first access (not tensors: cannot be outputs); the
         # outputs below carry the tight lists the kernels used
         cfg["classic_lists"] = _ClassicLists(proj["means2d"], proj["radii"], proj["depths"], tiles_per_gauss,
@@ -213,12 +227,21 @@ class _Rasterization(torch.autograd.Function):
         cfg = ctx.cfg
         width, height = cfg["width"], cfg["height"]
         C = viewmats.shape[0]
+        feat = cfg.get("features", False)
         if v_colors is None:
-            v_colors = torch.zeros(C, height, width, 3, dtype=torch.float32, device=means.device)
+            v_colors = torch.zeros(C, height, width, colors.shape[-1] if feat else 3, dtype=torch.float32, device=means.device)
         if v_alphas is None:
             v_alphas = torch.zeros(C, height, width, 1, dtype=torch.float32, device=means.device)
-        v_splats = _blend_backward(ctx, splats, isect_offsets, flatten_ids, backgrounds, width, height, render_colors,
-                                   render_alphas, last_ids, v_colors, v_alphas, ckpt)
+        if feat:
+            with stages.nvtx_range("egs.rasterize_bwd"):
+                v_splats, v_features = stages.rasterize_bwd_features(
+                    splats, isect_offsets, flatten_ids, colors, backgrounds, width, height, render_alphas, last_ids,
+                    v_colors, v_alphas, n_isects=ctx.raster_n, tile_order=ctx.tile_order,
+                    want_features_grad=ctx.needs_input_grad[4])
+            colors = _zero_rgb(means)  # what the projection saw; its colour gradient is discarded
+        else:
+            v_splats = _blend_backward(ctx, splats, isect_offsets, flatten_ids, backgrounds, width, height, render_colors,
+                                       render_alphas, last_ids, v_colors, v_alphas, ckpt)
         ref = getattr(ctx, "means2d_ref", None) if cfg["absgrad"] else None
         target = ref() if ref is not None else None
         # the viewmat keyword is passed only when its gradient is wanted: without it the call is exactly the classic one
@@ -229,6 +252,8 @@ class _Rasterization(torch.autograd.Function):
                                         antialiased_opacities=opacities if cfg["antialiased"] else None, opacities=opacities,
                                         **want_vm)
         v_means, v_quats, v_scales, v_opac, v_cols = out[:5]
+        if feat:
+            v_cols = v_features
         v_viewmats = out[-1] if want_vm else None
         if target is not None:
             # same contract as gsplat: attribute tagging on the tensor object handed out in meta
@@ -312,12 +337,12 @@ def _check_inputs(means, quats, scales, opacities, colors, viewmats, Ks, sh_degr
         raise ValueError(f"viewmats must be [C,4,4], got {tuple(viewmats.shape)}")
     if Ks.shape != (C, 3, 3):
         raise ValueError(f"Ks must be [C,3,3], got {tuple(Ks.shape)}")
+    D = 3
     if sh_degree is None:
-        ok = (colors.dim() == 2 and colors.shape == (N, 3)) or (colors.dim() == 3 and colors.shape == (C, N, 3))
-        if not ok:
-            if colors.dim() in (2, 3) and colors.shape[-1] != 3:
-                raise NotImplementedError("only 3 colour channels are implemented (the reference renders RGB)")
-            raise ValueError(f"colors must be [N,3] or [C,N,3] when sh_degree is None, got {tuple(colors.shape)}")
+        ok = (colors.dim() == 2 and colors.shape[0] == N) or (colors.dim() == 3 and colors.shape[:2] == (C, N))
+        if not ok or colors.shape[-1] < 1:
+            raise ValueError(f"colors must be [N,D] or [C,N,D] with D >= 1 when sh_degree is None, got {tuple(colors.shape)}")
+        D = colors.shape[-1]
     else:
         if colors.dim() == 4:
             raise NotImplementedError("per-camera SH coefficients [C,N,K,3] are not implemented")
@@ -327,8 +352,8 @@ def _check_inputs(means, quats, scales, opacities, colors, viewmats, Ks, sh_degr
             raise NotImplementedError(f"sh_degree={sh_degree}: degrees 0..3 are implemented (the reference uses <= 3)")
         if (sh_degree + 1) ** 2 > colors.shape[1]:
             raise ValueError(f"sh_degree={sh_degree} needs K >= {(sh_degree + 1) ** 2}, got K={colors.shape[1]}")
-    if backgrounds is not None and backgrounds.shape != (C, 3):
-        raise ValueError(f"backgrounds must be [C,3], got {tuple(backgrounds.shape)}")
+    if backgrounds is not None and backgrounds.shape != (C, D):
+        raise ValueError(f"backgrounds must be [C,{D}], got {tuple(backgrounds.shape)}")
     for name, t in (("means", means), ("quats", quats), ("scales", scales), ("opacities", opacities),
                     ("colors", colors), ("viewmats", viewmats), ("Ks", Ks), ("backgrounds", backgrounds)):
         if t is None:
@@ -348,7 +373,7 @@ def rasterization(
     quats: Tensor,  # [N, 4] wxyz, need not be normalised
     scales: Tensor,  # [N, 3]
     opacities: Tensor,  # [N]
-    colors: Tensor,  # [N, K, 3] SH coefficients (sh_degree given) or [N, 3] / [C, N, 3]
+    colors: Tensor,  # [N, K, 3] SH coefficients (sh_degree given) or [N, D] / [C, N, D], D >= 1
     viewmats: Tensor,  # [C, 4, 4] world -> camera
     Ks: Tensor,  # [C, 3, 3]
     width: int,
@@ -371,7 +396,11 @@ def rasterization(
     ``absgrad=True``, one camera, a [1,3] background — and C > 1 are implemented; modes the
     reference never requests raise ``NotImplementedError`` instead of silently approximating.
     As in gsplat, ``viewmats`` receive a gradient when they require one (camera pose refinement: projection and SH
-    view directions, campos = inverse(viewmats)[:, :3, 3]); ``Ks`` receive none."""
+    view directions, campos = inverse(viewmats)[:, :3, 3]); ``Ks`` receive none.
+    Without SH, colours may have any number of channels D (features, masks, RGB plus extra channels): the images are
+    [C,H,W,D], ``backgrounds`` [C,D], and D != 3 is blended in chunks of 32 channels by the feature kernels.  For
+    D > 32, ``meta["means2d"].absgrad`` is the sum over the chunks of each chunk's absgrad (gsplat 1.0.0 keeps the
+    value of whichever chunk's backward ran last).  ``channel_chunk`` is accepted and has no effect."""
     if render_mode != "RGB":
         raise NotImplementedError(f"render_mode={render_mode!r}: only 'RGB' is implemented (the reference's mode)")
     if rasterize_mode not in ("classic", "antialiased"):
@@ -387,18 +416,25 @@ def rasterization(
     C = viewmats.shape[0]
     cfg = dict(width=width, height=height, sh_degree=sh_degree, eps2d=float(eps2d), near_plane=float(near_plane),
                far_plane=float(far_plane), radius_clip=float(radius_clip), absgrad=bool(absgrad),
-               antialiased=rasterize_mode == "antialiased", grad_enabled=torch.is_grad_enabled())
+               antialiased=rasterize_mode == "antialiased", grad_enabled=torch.is_grad_enabled(),
+               features=sh_degree is None and colors.shape[-1] != 3)
     outs = _Rasterization.apply(means, quats, scales, opacities, colors, viewmats, Ks, backgrounds, cfg)
+    meta_colors = None
+    if cfg["features"]:  # gsplat: the colours as given, per (camera, Gaussian)
+        meta_colors = colors.detach() if colors.dim() == 3 else colors.detach()[None].expand(C, -1, -1)
     opacities_cn = opacities.detach()[None].expand(C, -1)
     comp = cfg.pop("compensations", None)
     if comp is not None:
         opacities_cn = opacities_cn * comp  # gsplat: meta["opacities"] = opacities * compensations
-    return _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad, packed=bool(packed))
+    return _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad, packed=bool(packed),
+                   meta_colors=meta_colors)
 
 
-def _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad, packed=False):
+def _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad, packed=False, meta_colors=None):
     (render_colors, render_alphas, means2d, radii, depths, conics, colors_rgb, tiles_per_gauss,
      _blend_flatten_ids, _blend_offsets, _last_ids) = outs
+    if meta_colors is not None:
+        colors_rgb = meta_colors
     classic = cfg.pop("classic_lists")
     isect_ids, flatten_ids, isect_offsets = classic.isect_ids, classic.flatten_ids, classic.isect_offsets
     cfg.pop("compensations", None)
@@ -419,7 +455,7 @@ def _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad, packe
         flatten_ids = lambda: rank[dense_flatten_ids().long()]  # stays lazy: built from gsplat's list on first access
         means2d = means2d.reshape(-1, 2)[packed_index]  # differentiable gather: gradients on it reach the dense one
         radii, depths, tiles_per_gauss = (t.reshape(-1)[packed_index] for t in (radii, depths, tiles_per_gauss))
-        conics, colors_rgb = (t.reshape(-1, 3)[packed_index] for t in (conics, colors_rgb))
+        conics, colors_rgb = (t.reshape(-1, t.shape[-1])[packed_index] for t in (conics, colors_rgb))
         opacities_cn = opacities_cn.reshape(-1)[packed_index]
         if node is not None:
             node.packed_index = packed_index

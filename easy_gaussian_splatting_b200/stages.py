@@ -835,6 +835,94 @@ def rasterize_bwd(splats: Tensor, isect_offsets: Tensor, flatten_ids: Tensor, ba
     return v_splats
 
 
+FEATURE_CHUNK = 32  # colour channels per blend launch: gsplat's default channel_chunk
+FEATURE_WIDTHS = (1, 2, 4, 8, 16, 32)  # chunk widths the feature kernels are instantiated for
+
+
+def feature_chunks(D: int) -> List[Tuple[int, int]]:
+    """(c0, CH) of the blend launches for D colour channels: 32-channel chunks, the last one narrowed to the smallest
+    instantiated width that holds the remaining channels (the rows are padded with zero channels up to it)."""
+    if D < 1:
+        raise ValueError(f"colours need at least one channel, got D={D}")
+    return [(c0, next(w for w in FEATURE_WIDTHS if w >= min(FEATURE_CHUNK, D - c0))) for c0 in range(0, D, FEATURE_CHUNK)]
+
+
+def _feature_rows(features: Tensor, chunks: List[Tuple[int, int]]) -> Tensor:
+    """features [N,D] / [C,N,D] -> dense fp32 rows [rows, stride] from which every chunk reads its CH channels:
+    stride = the padded width, rounded up to the row alignment the widest chunk needs (4 floats from CH = 4 on).
+    The tensor itself (a view) when it already is such an array, a zero-padded copy otherwise."""
+    D = features.shape[-1]
+    c0, ch = chunks[-1]
+    align = min(4, max(w for _, w in chunks))
+    stride = -(-(c0 + ch) // align) * align
+    rows = _f32c(features, "colors").reshape(-1, D)
+    if stride == D:
+        return rows
+    out = torch.zeros(rows.shape[0], stride, dtype=torch.float32, device=rows.device)
+    out[:, :D] = rows
+    return out
+
+
+def rasterize_fwd_features(splats: Tensor, isect_offsets: Tensor, flatten_ids: Tensor, features: Tensor,
+                           backgrounds: Optional[Tensor], width: int, height: int, n_isects: Optional[int] = None,
+                           tile_order: Optional[Tensor] = None):
+    """g6 for colours of any width: features [N,D] (shared by the cameras) or [C,N,D], backgrounds [C,D] ->
+    render_colors[C,H,W,D], render_alphas[C,H,W,1], last_ids[C,H,W].  One launch per 32-channel chunk on the same
+    lists; the first chunk writes the alphas and last_ids (every chunk would write the same)."""
+    lib = _lib.load()
+    dev = splats.device
+    C, N = splats.shape[:2]
+    th, tw = isect_offsets.shape[1:]
+    D = features.shape[-1]
+    chunks = feature_chunks(D)
+    rows = _feature_rows(features, chunks)
+    colors = torch.empty(C, height, width, D, dtype=torch.float32, device=dev)
+    alphas = torch.empty(C, height, width, 1, dtype=torch.float32, device=dev)
+    last = torch.empty(C, height, width, dtype=torch.int32, device=dev)
+    bg = None if backgrounds is None else _f32c(backgrounds, "backgrounds")
+    n = flatten_ids.numel() if n_isects is None else int(n_isects)
+    with torch.cuda.device(dev):
+        for i, (c0, ch) in enumerate(chunks):
+            rc = lib.egs_rasterize_fwd_features(C, N, n, _ptr(splats), _ptr(isect_offsets), _ptr(flatten_ids), _ptr(rows),
+                                                rows.shape[1], int(features.dim() == 2), D, c0, ch, _ptr(bg), int(width),
+                                                int(height), tw, th, _ptr(colors), _ptr(alphas) if i == 0 else None,
+                                                _ptr(last) if i == 0 else None, _ptr(tile_order), _stream(dev))
+            _lib.check(rc, "egs_rasterize_fwd_features")
+    return colors, alphas, last
+
+
+def rasterize_bwd_features(splats: Tensor, isect_offsets: Tensor, flatten_ids: Tensor, features: Tensor,
+                           backgrounds: Optional[Tensor], width: int, height: int, render_alphas: Tensor,
+                           last_ids: Tensor, v_render_colors: Tensor, v_render_alphas: Tensor,
+                           n_isects: Optional[int] = None, tile_order: Optional[Tensor] = None,
+                           want_features_grad: bool = True) -> Tuple[Tensor, Optional[Tensor]]:
+    """g7 for colours of any width -> (v_splats[C,N,12] with the geometry slots filled and v_r, v_g, v_b = 0,
+    v_features in the shape of features, or None without want_features_grad).  One launch per chunk; the geometry
+    gradients, |v_x| and |v_y| included, sum over the chunks."""
+    lib = _lib.load()
+    dev = splats.device
+    C, N = splats.shape[:2]
+    th, tw = isect_offsets.shape[1:]
+    D = features.shape[-1]
+    chunks = feature_chunks(D)
+    rows = _feature_rows(features, chunks)
+    v_splats = torch.zeros(C, N, SPLAT_FLOATS, dtype=torch.float32, device=dev)
+    v_rows = torch.zeros_like(rows) if want_features_grad else None
+    bg = None if backgrounds is None else _f32c(backgrounds, "backgrounds")
+    v_c, v_a = _f32c(v_render_colors, "v_render_colors"), _f32c(v_render_alphas, "v_render_alphas")
+    n = flatten_ids.numel() if n_isects is None else int(n_isects)
+    with torch.cuda.device(dev):
+        for i, (c0, ch) in enumerate(chunks):
+            rc = lib.egs_rasterize_bwd_features(C, N, n, _ptr(splats), _ptr(isect_offsets), _ptr(flatten_ids), _ptr(rows),
+                                                rows.shape[1], int(features.dim() == 2), D, c0, ch, _ptr(bg), int(width),
+                                                int(height), tw, th, _ptr(render_alphas), _ptr(last_ids), _ptr(v_c),
+                                                _ptr(v_a) if i == 0 else None, _ptr(v_splats), _ptr(v_rows),
+                                                _ptr(tile_order), _stream(dev))
+            _lib.check(rc, "egs_rasterize_bwd_features")
+    v_features = None if v_rows is None else v_rows[:, :D].reshape(features.shape)
+    return v_splats, v_features
+
+
 def densify_stats_update(max_radii: Tensor, grad_norm_accum: Tensor, collecting_counts: Tensor, radii: Tensor,
                          absgrad: Tensor, width: int, height: int) -> None:
     """§8f-1: in-place, sync-free equivalent of GaussianModel.update_statistics

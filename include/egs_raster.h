@@ -308,6 +308,44 @@ int egs_rasterize_bwd_segmented(int32_t C, int32_t N, int64_t n_isects, const fl
                                 int32_t segment, int32_t seg_min_len, float* v_splats, const int32_t* tile_order,
                                 egs_stream_t stream);
 
+/* ---- g6 / g7 with colours of any number of channels ("features") ---------------------------------------------------
+ * gsplat 1.0.0 `rasterize_to_pixels` with colors[..., D], D >= 1 (rasterization() with sh_degree=None and [N,D] or
+ * [C,N,D] colours).  The splat records still carry the geometry (their r, g, b slots are not read); the colours come
+ * from a separate row array:
+ *   features [rows, feat_stride] fp32, row = flat id - cam * N (shared_rows = 1: one [N, .] array for all cameras) or
+ *            the flat id (shared_rows = 0: [C*N, .]).  A call reads channels [c0, c0 + CH) of every row it blends, so
+ *            feat_stride >= c0 + CH: pad the rows with zero channels up to the chunk width.  CH is one of 1, 2, 4, 8, 16,
+ *            32; features, feat_stride and c0 must be aligned to min(CH, 4) floats (rows are copied in 4 / 8 / 16-byte
+ *            pieces).  0 <= c0 < D.
+ *   A call covers channels [c0, c0 + min(CH, D - c0)) of the [C,H,W,D] images; colours wider than 32 channels take one
+ *   call per chunk on the same binning result.  CH <= 8 reproduces egs_rasterize_fwd's render_alphas and last_ids bit
+ *   for bit; CH = 16 / 32 blend one pixel per lane and their transmittance can differ from that in the last bits
+ *   (measured: alphas within 2.4e-7).  Take render_alphas / last_ids from one chunk and pass those to every backward
+ *   chunk of the call.
+ *   backgrounds[C,D] (nullable): the call adds T_final * backgrounds[cam, c0 + k].
+ * egs_rasterize_fwd_features: render_colors[C,H,W,D] (channels of this chunk written); render_alphas, last_ids as in
+ *   egs_rasterize_fwd, both nullable (chunks after the first need not write them again).
+ * egs_rasterize_bwd_features: render_alphas / last_ids from the forward; v_render_colors[C,H,W,D];
+ *   v_render_alphas (nullable: pass it to exactly one chunk of a call; the others get NULL).  Adds (RED.ADD) into
+ *   caller-zeroed buffers: the geometry slots of v_splats[C,N,12] (v_x, v_y, v_conic, v_opacity, |v_x|, |v_y|; the
+ *   v_r, v_g, v_b slots are left alone, so egs_projection_bwd* consume the records unchanged) and, when v_features is
+ *   given, v_features [rows, feat_stride] (same layout as features; only the chunk's real channels).  With several
+ *   chunks the geometry slots, |v_x| and |v_y| included, sum over the chunks.
+ * No segmented replay: long lists are replayed in one piece. */
+int egs_rasterize_fwd_features(int32_t C, int32_t N, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
+                               const int32_t* flatten_ids, const float* features, int32_t feat_stride,
+                               int32_t shared_rows, int32_t D, int32_t c0, int32_t CH, const float* backgrounds,
+                               int32_t width, int32_t height, int32_t tile_width, int32_t tile_height,
+                               float* render_colors, float* render_alphas, int32_t* last_ids, const int32_t* tile_order,
+                               egs_stream_t stream);
+int egs_rasterize_bwd_features(int32_t C, int32_t N, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
+                               const int32_t* flatten_ids, const float* features, int32_t feat_stride,
+                               int32_t shared_rows, int32_t D, int32_t c0, int32_t CH, const float* backgrounds,
+                               int32_t width, int32_t height, int32_t tile_width, int32_t tile_height,
+                               const float* render_alphas, const int32_t* last_ids, const float* v_render_colors,
+                               const float* v_render_alphas, float* v_splats, float* v_features,
+                               const int32_t* tile_order, egs_stream_t stream);
+
 /* ---- §8f-1: fused, sync-free densification statistics (C-aware) ----------------------------------------
  * Replaces GaussianModel.update_statistics, /root/reference/model/gaussian.py:188-197, applied once
  * per camera: visible = radii > 0; max_radii = max(max_radii, radii / max_hw);
