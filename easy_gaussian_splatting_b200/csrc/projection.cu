@@ -903,6 +903,7 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
   const int raw = sh_rest != nullptr;
   EGS_REQUIRE(C >= 0 && N >= 0, "projection_bwd: negative sizes C=%d N=%d", C, N);
   EGS_REQUIRE(sh_degree <= 3, "projection_bwd: sh_degree %d > 3 is not supported", sh_degree);
+  EGS_REQUIRE(sh_degree < 0 || K >= (sh_degree + 1) * (sh_degree + 1), "projection_bwd: K=%d too small for sh_degree=%d", K, sh_degree);
   const bool vg = v_viewmats != nullptr;
   if (vg) {
     EGS_REQUIRE(C <= 65535, "projection_bwd: C=%d exceeds 65535 cameras per call", C);

@@ -44,6 +44,27 @@ def test_workspace_queries_and_argument_errors_without_gpu():
     assert rc == -1 and b"sh_degree" in lib.egs_last_error_string()
 
 
+def test_projection_backward_rejects_too_few_sh_coefficients_without_gpu():
+    """K < (sh_degree + 1)^2 would make the backward kernels read past each SH row: every backward entry rejects it
+    before any launch, as the forward does."""
+    from easy_gaussian_splatting_b200 import _lib
+    lib = _lib.load()
+    n0 = lib.egs_kernel_launch_count()
+    fake = ctypes.c_void_p(0x1000)  # a non-null v_viewmats that is never touched
+    for K, deg in ((9, 3), (4, 2), (1, 1), (15, 3)):
+        rc = lib.egs_projection_bwd(1, 10, None, None, None, None, K, deg, 0, None, None, 64, 64, 0.3, None, None, None,
+                                    None, None, None, None, None, None, None, None)
+        assert rc == -1 and f"K={K} too small".encode() in lib.egs_last_error_string(), (K, deg)
+        rc = lib.egs_projection_bwd_antialiased(1, 10, None, None, None, None, None, K, deg, 0, None, None, 64, 64, 0.3,
+                                                None, None, None, None, None, None, None, None, None, None, None)
+        assert rc == -1 and f"K={K} too small".encode() in lib.egs_last_error_string(), (K, deg)
+        rc = lib.egs_projection_bwd_viewmats(1, 10, None, None, None, None, None, K, deg, 0, None, None, 64, 64, 0.3,
+                                             None, None, None, None, None, None, None, None, None, None, 0, fake, None, 0,
+                                             None)
+        assert rc == -1 and f"K={K} too small".encode() in lib.egs_last_error_string(), (K, deg)
+    assert lib.egs_kernel_launch_count() == n0
+
+
 def test_product_never_imports_the_oracle_and_has_no_cpu_path():
     pkg = ROOT / "easy_gaussian_splatting_b200"
     for f in pkg.rglob("*.py"):
