@@ -344,14 +344,13 @@ def _check_inputs(means, quats, scales, opacities, colors, viewmats, Ks, sh_degr
             raise ValueError(f"colors must be [N,D] or [C,N,D] with D >= 1 when sh_degree is None, got {tuple(colors.shape)}")
         D = colors.shape[-1]
     else:
-        if colors.dim() == 4:
-            raise NotImplementedError("per-camera SH coefficients [C,N,K,3] are not implemented")
-        if not (colors.dim() == 3 and colors.shape[0] == N and colors.shape[2] == 3):
-            raise ValueError(f"colors must be [N,K,3] SH coefficients, got {tuple(colors.shape)}")
+        ok = (colors.dim() == 3 and colors.shape[0] == N) or (colors.dim() == 4 and colors.shape[:2] == (C, N))
+        if not ok or colors.shape[-1] != 3:
+            raise ValueError(f"colors must be [N,K,3] or per-camera [C,N,K,3] SH coefficients, got {tuple(colors.shape)}")
         if not 0 <= sh_degree <= 3:
             raise NotImplementedError(f"sh_degree={sh_degree}: degrees 0..3 are implemented (the reference uses <= 3)")
-        if (sh_degree + 1) ** 2 > colors.shape[1]:
-            raise ValueError(f"sh_degree={sh_degree} needs K >= {(sh_degree + 1) ** 2}, got K={colors.shape[1]}")
+        if (sh_degree + 1) ** 2 > colors.shape[-2]:
+            raise ValueError(f"sh_degree={sh_degree} needs K >= {(sh_degree + 1) ** 2}, got K={colors.shape[-2]}")
     if backgrounds is not None and backgrounds.shape != (C, D):
         raise ValueError(f"backgrounds must be [C,{D}], got {tuple(backgrounds.shape)}")
     for name, t in (("means", means), ("quats", quats), ("scales", scales), ("opacities", opacities),
@@ -373,7 +372,7 @@ def rasterization(
     quats: Tensor,  # [N, 4] wxyz, need not be normalised
     scales: Tensor,  # [N, 3]
     opacities: Tensor,  # [N]
-    colors: Tensor,  # [N, K, 3] SH coefficients (sh_degree given) or [N, D] / [C, N, D], D >= 1
+    colors: Tensor,  # [N, K, 3] / [C, N, K, 3] SH coefficients (sh_degree given) or [N, D] / [C, N, D], D >= 1
     viewmats: Tensor,  # [C, 4, 4] world -> camera
     Ks: Tensor,  # [C, 3, 3]
     width: int,
@@ -400,7 +399,10 @@ def rasterization(
     Without SH, colours may have any number of channels D (features, masks, RGB plus extra channels): the images are
     [C,H,W,D], ``backgrounds`` [C,D], and D != 3 is blended in chunks of 32 channels by the feature kernels.  For
     D > 32, ``meta["means2d"].absgrad`` is the sum over the chunks of each chunk's absgrad (gsplat 1.0.0 keeps the
-    value of whichever chunk's backward ran last).  ``channel_chunk`` is accepted and has no effect."""
+    value of whichever chunk's backward ran last).  ``channel_chunk`` is accepted and has no effect.
+    With SH, coefficients may also be per camera, [C,N,K,3] (e.g. shared coefficients plus a learned per-view
+    offset): camera c colours Gaussian n from its own row colors[c, n], and colors.grad is [C,N,K,3], one row per
+    (camera, Gaussian), 0 for pairs the camera culls."""
     if render_mode != "RGB":
         raise NotImplementedError(f"render_mode={render_mode!r}: only 'RGB' is implemented (the reference's mode)")
     if rasterize_mode not in ("classic", "antialiased"):

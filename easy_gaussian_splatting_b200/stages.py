@@ -152,7 +152,8 @@ def projection_fwd(means: Tensor, quats: Tensor, scales: Tensor, opacities: Tens
                    eps2d: float = 0.3, near_plane: float = 0.01, far_plane: float = 1e10,
                    radius_clip: float = 0.0, tile_size: int = TILE_SIZE,
                    antialiased: bool = False) -> Dict[str, Tensor]:
-    """g1+g2+count(g3).  colors: [N,K,3] SH coefficients when sh_degree is not None, else [N,3]/[C,N,3].
+    """g1+g2+count(g3).  colors: [N,K,3] or per-camera [C,N,K,3] SH coefficients when sh_degree is not None, else
+    [N,3]/[C,N,3].
     antialiased: gsplat's rasterize_mode="antialiased" — adds out["compensations"] [C,N]; the splat records then
     carry opacity * compensation."""
     lib = _lib.load()
@@ -164,7 +165,7 @@ def projection_fwd(means: Tensor, quats: Tensor, scales: Tensor, opacities: Tens
     if sh_degree is None:
         K, deg, per_cam = 1, -1, int(colors.dim() == 3)
     else:
-        K, deg, per_cam = colors.shape[-2], int(sh_degree), 0
+        K, deg, per_cam = colors.shape[-2], int(sh_degree), int(colors.dim() == 4)
     tw, th = tile_grid(width, height, tile_size)
     out = {
         "radii": torch.empty(C, N, dtype=torch.int32, device=dev),
@@ -208,7 +209,7 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
     if sh_degree is None:
         K, deg, per_cam = 1, -1, int(colors.dim() == 3)
     else:
-        K, deg, per_cam = colors.shape[-2], int(sh_degree), 0
+        K, deg, per_cam = colors.shape[-2], int(sh_degree), int(colors.dim() == 4)
     op_ref = antialiased_opacities if antialiased_opacities is not None else opacities
     if op_ref is not None:
         v_means, v_quats, v_scales, v_opac, v_colors = [_grad_buffer(t) for t in (means, quats, scales, op_ref, colors)]

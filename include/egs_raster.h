@@ -57,9 +57,12 @@ int64_t egs_kernel_launch_count(void);
  * `dirs = means - inverse(viewmats)[:3,3]`, `clamp_min(rgb + 0.5, 0)` and the first launch of
  * `isect_tiles`, all reached from model/gaussian.py:353-367.
  *   means[N,3] quats[N,4](wxyz, unnormalised) scales[N,3] opacities[N]
- *   sh_coeffs: sh_degree >= 0 → [N,K,3] SH coefficients (K >= (sh_degree+1)^2, sh_degree <= 3);
+ *   sh_coeffs: sh_degree >= 0 → SH coefficients (K >= (sh_degree+1)^2, sh_degree <= 3), [N,K,3] shared by all
+ *              cameras (colors_per_camera = 0) or [C,N,K,3], one row per (camera, Gaussian) (colors_per_camera = 1);
  *              sh_degree <  0 → colours used as they are, [N,3] (colors_per_camera = 0)
  *              or [C,N,3] (colors_per_camera = 1)
+ *   colors_per_camera must be 0 or 1 (rejected before any launch otherwise), here and in every entry below that
+ *   takes it; the _raw entries have shared coefficients by construction
  *   viewmats[C,4,4] Ks[C,3,3]
  * outputs (culled entries are zero-filled, radii == 0):
  *   radii[C,N] i32, means2d[C,N,2], depths[C,N], conics[C,N,3], colors[C,N,3],
@@ -82,7 +85,8 @@ int egs_projection_fwd(int32_t C, int32_t N, const float* means, const float* qu
  *   v_splats[C,N,12]: packed gradient records produced by egs_rasterize_bwd
  *   v_means2d_extra[C,N,2] (nullable): user gradient that arrived on meta["means2d"] itself
  * outputs (dense, written for every Gaussian): v_means[N,3], v_quats[N,4], v_scales[N,3],
- *   v_opacities[N], v_sh_coeffs (same shape as sh_coeffs; inactive bands and culled entries are 0);
+ *   v_opacities[N], v_sh_coeffs (same shape as sh_coeffs; inactive bands and culled entries are 0; per-camera
+ *   coefficients get one gradient row per (camera, Gaussian), not summed over cameras);
  *   absgrad[C,N,2] (nullable): the |v_x|,|v_y| slots of the gradient records as a dense tensor — what the
  *   reference reads as meta["means2d"].absgrad (model/gaussian.py:191). */
 int egs_projection_bwd(int32_t C, int32_t N, const float* means, const float* quats, const float* scales,
