@@ -41,19 +41,18 @@ constexpr int kTileSize = 16;
 // Resident CTAs per SM the compiler must leave room for (register cap = 65536 / (threads * this)); tuning knobs,
 // overridable at build time for A/B runs (scripts/build_variant.py).
 #ifdef EGS_FWD_MIN_CTAS
-#define EGS_FWD_BOUNDS(T, PX) __launch_bounds__(T, (PX) == 2 ? EGS_FWD_MIN_CTAS : 1)
+#define EGS_FWD_BOUNDS(T) __launch_bounds__(T, EGS_FWD_MIN_CTAS)
 #else
-#define EGS_FWD_BOUNDS(T, PX) __launch_bounds__(T)
+#define EGS_FWD_BOUNDS(T) __launch_bounds__(T)
 #endif
 #ifdef EGS_BWD_MIN_CTAS
-#define EGS_BWD_BOUNDS(T, PX) __launch_bounds__(T, (PX) == 2 ? EGS_BWD_MIN_CTAS : 1)
+#define EGS_BWD_BOUNDS(T) __launch_bounds__(T, EGS_BWD_MIN_CTAS)
 #else
-#define EGS_BWD_BOUNDS(T, PX) __launch_bounds__(T)
+#define EGS_BWD_BOUNDS(T) __launch_bounds__(T)
 #endif
 // A lane owns PX x PY pixels, a warp 8 x 4 lanes = (8 PX) x (4 PY) pixels.  <2,2>: 2 warps of 16x8 pixels per
-// tile — the throughput configuration.  <1,1>: 8 warps of 8x4 pixels per tile — more warps, smaller culling
-// rectangles and a shorter per-entry chain; used only for tiles whose list is so long that the serial walk of
-// one warp would become the tail of the whole launch.
+// tile — the RGB kernels and the feature kernels up to 8 channels.  <1,1>: 8 warps of 8x4 pixels per tile, one
+// pixel per lane — the 16- and 32-channel feature kernels, whose per-lane colour state would not fit 4 pixels.
 template <int PX, int PY>
 struct Geo {
   static constexpr int NP = PX * PY;
@@ -117,18 +116,23 @@ struct WarpStage {
 };
 
 struct WarpView {
-  int cam, x0, y0;               // first pixel of this lane's 2x2 block
+  int cam, x0, y0;               // first pixel of this lane's block
   int range_start, range_end;    // the tile's slice of the sorted intersection list
-  float rx_lo, rx_hi, ry_lo, ry_hi;  // pixel-centre rectangle of the warp (16 x 8 pixels)
+  float2 npx2, npy2;             // minus the pixel centres of the block's first / last column, first / last row
+  float rx_lo, rx_hi, ry_lo, ry_hi;  // pixel-centre rectangle of the warp
 };
 
-// tile_id < 0: the tile is the block's position in the (tile_w, tile_h, C) grid; otherwise the given flat tile index
-// (cam * tile_h + ty) * tile_w + tx (the segment launch of the backward pass maps blocks to list segments).
+// The block's tile: the given flat tile index (cam * tile_h + ty) * tile_w + tx when tile_id >= 0 (the segment launch
+// of the backward pass maps blocks to list segments), else tile_order[block] when tile_order is given (longest lists
+// first, egs_isect_sorted), else the block's position in the (tile_w, tile_h, C) grid.
 template <class G>
 __device__ __forceinline__ WarpView warp_setup(int tile_w, int tile_h, int64_t n_isects,
                                                const int32_t* __restrict__ tile_offsets, int n_tiles_total,
-                                               int tile_id = -1) {
+                                               const int32_t* __restrict__ tile_order, int tile_id = -1) {
+  constexpr int PX = G::kWarpW / 8, PY = G::kWarpH / 4;
   WarpView v;
+  if (tile_id < 0 && tile_order != nullptr)
+    tile_id = tile_order[(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x];
   int bx = blockIdx.x, by = blockIdx.y;
   v.cam = blockIdx.z;
   if (tile_id < 0) {
@@ -142,16 +146,24 @@ __device__ __forceinline__ WarpView warp_setup(int tile_w, int tile_h, int64_t n
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int wx = warp % G::kWarpsX, wy = warp / G::kWarpsX;
   const int wx0 = bx * kTileSize + wx * G::kWarpW, wy0 = by * kTileSize + wy * G::kWarpH;
-  v.x0 = wx0 + (lane & 7) * (G::kWarpW / 8);
-  v.y0 = wy0 + (lane >> 3) * (G::kWarpH / 4);
+  v.x0 = wx0 + (lane & 7) * PX;
+  v.y0 = wy0 + (lane >> 3) * PY;
   v.range_start = tile_offsets[tile_id];
   // n_isects < 0: the offsets carry a sentinel entry behind the last tile (the live list length, written on the
   // device by egs_isect_sorted); otherwise the last tile ends at n_isects
   v.range_end = (tile_id == n_tiles_total - 1 && n_isects >= 0) ? (int)n_isects : tile_offsets[tile_id + 1];
-  v.rx_lo = (float)wx0 + 0.5f;
-  v.rx_hi = v.rx_lo + (float)(G::kWarpW - 1);
-  v.ry_lo = (float)wy0 + 0.5f;
-  v.ry_hi = v.ry_lo + (float)(G::kWarpH - 1);
+  float pxf[PX], pyf[PY];
+#pragma unroll
+  for (int i = 0; i < PX; ++i) pxf[i] = opaque((float)(v.x0 + i) + 0.5f);
+#pragma unroll
+  for (int i = 0; i < PY; ++i) pyf[i] = opaque((float)(v.y0 + i) + 0.5f);
+  v.npx2 = make_float2(-pxf[0], -pxf[PX - 1]);
+  v.npy2 = make_float2(-pyf[0], -pyf[PY - 1]);
+  const float rx_lo = (float)wx0 + 0.5f, ry_lo = (float)wy0 + 0.5f;
+  v.rx_lo = opaque(rx_lo);
+  v.rx_hi = opaque(rx_lo + (float)(G::kWarpW - 1));
+  v.ry_lo = opaque(ry_lo);
+  v.ry_hi = opaque(ry_lo + (float)(G::kWarpH - 1));
   return v;
 }
 
@@ -187,8 +199,8 @@ __device__ __forceinline__ bool splat_touches_rect(const float4 g0, const float4
 // Tests this lane's RPL records of raw batch `buf` (record slots lane, lane+32, ...), writes the survivor
 // slots, in order, to st.list and returns the number of survivors (warp-uniform).
 template <int RPL>
-__device__ __forceinline__ int cull_and_compact(WarpStage<32 * RPL>& st, int buf, int batch_size, int lane, float rx_lo,
-                                                float rx_hi, float ry_lo, float ry_hi) {
+__device__ __forceinline__ int cull_and_compact(WarpStage<32 * RPL>& st, int buf, int batch_size, int lane,
+                                                const WarpView& wv) {
   bool keep[RPL];
 #pragma unroll
   for (int r = 0; r < RPL; ++r) {
@@ -198,7 +210,7 @@ __device__ __forceinline__ int cull_and_compact(WarpStage<32 * RPL>& st, int buf
       const float4 g0 = st.rec[buf][slot * 3 + 0];
       const float4 g1 = st.rec[buf][slot * 3 + 1];
       const float cut = st.rec[buf][slot * 3 + 2].w;
-      keep[r] = splat_touches_rect(g0, g1, cut, rx_lo, rx_hi, ry_lo, ry_hi);
+      keep[r] = splat_touches_rect(g0, g1, cut, wv.rx_lo, wv.rx_hi, wv.ry_lo, wv.ry_hi);
     }
   }
   const uint32_t lt = (1u << lane) - 1u;
@@ -213,42 +225,151 @@ __device__ __forceinline__ int cull_and_compact(WarpStage<32 * RPL>& st, int buf
   return base;
 }
 
+// The staging pipeline of all four blend kernels.  Walks the sorted list entries first, first + 1, ..., end - 1 (front
+// to back) or, with BACK, first, first - 1, ..., end + 1, in batches of kBatch records; the walk must hold at least one
+// entry.  The flatten ids of the batch after next are prefetched into registers, each record is copied with three
+// 16-byte cp.async (double buffered), and extra(buf, slot, id) may issue one more copy per record into the same group
+// (the feature kernels' colour row).  KEEP_IDS also stores the batch's flatten ids in st.id.  Once a batch has landed
+// it is culled against the warp's rectangle and body(b, ns, base) runs on batch b: st.rec[b & 1] holds its records,
+// st.list[0, ns) the surviving slots in walk order, and slot s is sorted entry base + s (front to back) or base - s
+// (back to front).  The walk ends when body returns true.
+template <bool BACK, bool KEEP_IDS, int RPL, class Extra, class Body>
+__device__ __forceinline__ void stage_batches(WarpStage<32 * RPL>& st, const float4* __restrict__ splats,
+                                              const int32_t* __restrict__ flatten_ids, int first, int end, int lane,
+                                              const WarpView& wv, Extra&& extra, Body&& body) {
+  constexpr int kBatch = 32 * RPL;
+  const int nb = ((BACK ? first - end : end - first) + kBatch - 1) / kBatch;
+  // the callers guarantee it; without the hint the loop below gets a second entry test and the kernels more registers
+  __builtin_assume(nb > 0);
+  auto load_ids = [&](int b, int (&ids)[RPL]) {
+#pragma unroll
+    for (int r = 0; r < RPL; ++r) {
+      const int k = b * kBatch + r * 32 + lane;
+      const int idx = BACK ? first - k : first + k;
+      ids[r] = (BACK ? idx > end : idx < end) ? __ldg(flatten_ids + idx) : -1;  // b >= nb: past the end
+    }
+  };
+  auto issue = [&](int buf, const int (&ids)[RPL]) {
+#pragma unroll
+    for (int r = 0; r < RPL; ++r) {
+      const int slot = r * 32 + lane;
+      if (ids[r] >= 0) {
+        const float4* src = splats + (size_t)ids[r] * 3;
+        float4* dst = &st.rec[buf][slot * 3];
+        cp_async16(dst + 0, src + 0);
+        cp_async16(dst + 1, src + 1);
+        cp_async16(dst + 2, src + 2);
+        extra(buf, slot, ids[r]);
+      }
+      if constexpr (KEEP_IDS) st.id[buf][slot] = ids[r];
+    }
+    cp_async_commit();
+  };
+
+  int ids[RPL];
+  load_ids(0, ids);
+  issue(0, ids);
+  load_ids(1, ids);
+  for (int b = 0; b < nb; ++b) {
+    if (b + 1 < nb) {
+      issue((b + 1) & 1, ids);
+      load_ids(b + 2, ids);
+      cp_async_wait<1>();
+    } else {
+      cp_async_wait<0>();
+    }
+    __syncwarp();  // batch b has landed for every lane of this warp
+    const int base = BACK ? first - b * kBatch : first + b * kBatch;
+    const int batch_size = min(kBatch, BACK ? base - end : end - base);
+    const int ns = cull_and_compact<RPL>(st, b & 1, batch_size, lane, wv);
+    if (body(b, ns, base)) {
+      cp_async_wait<0>();  // the next batch may still be in flight
+      return;
+    }
+    __syncwarp();  // every lane is done with buffer b&1, its ids and the list before they are overwritten
+  }
+}
+
+// q = -log2(e) * sigma and ov = opacity * 2^q (before the 0.999 clamp) at the lane's pixels, with dx / dy = mean - pixel
+// centre per column / row.  Packed FADD2 / FMUL2 / FFMA2 in the <2,2> layout (sm_100: the two pixels of a row share one
+// instruction; the kernels are issue bound, not FMA-pipe bound, profiles/r1g, so halving the issue slots of the
+// arithmetic is what counts), the same sequence one pixel at a time in <1,1>.  Every kernel evaluates alphas here, so
+// their alphas agree bit for bit.
+template <int P>
+__device__ __forceinline__ void splat_eval(const float4 g0, const float4 g1, const float2 npx2, const float2 npy2,
+                                           float (&dx)[P], float (&dy)[P], float (&q)[P * P], float (&ov)[P * P]) {
+  // q(dx,dy) = -log2(e) * sigma, separable parts shared by the rows / columns of the pixel block
+  const float la = (0.5f * kNegLog2e) * g0.z, lc = (0.5f * kNegLog2e) * g1.x, lb = kNegLog2e * g0.w;
+  if constexpr (P == 2) {
+    const float2 dx2 = __fadd2_rn(make_float2(g0.x, g0.x), npx2);
+    const float2 dy2 = __fadd2_rn(make_float2(g0.y, g0.y), npy2);
+    const float2 qx = __fmul2_rn(__fmul2_rn(dx2, make_float2(la, la)), dx2);
+    const float2 bx = __fmul2_rn(dx2, make_float2(lb, lb));
+    const float2 qy = __fmul2_rn(__fmul2_rn(dy2, make_float2(lc, lc)), dy2);
+    const float2 o2 = make_float2(g1.y, g1.y);
+    const float2 q0 = __ffma2_rn(bx, make_float2(dy2.x, dy2.x), __fadd2_rn(qx, make_float2(qy.x, qy.x)));
+    const float2 q1 = __ffma2_rn(bx, make_float2(dy2.y, dy2.y), __fadd2_rn(qx, make_float2(qy.y, qy.y)));
+    const float2 a0 = __fmul2_rn(o2, make_float2(fast_ex2(q0.x), fast_ex2(q0.y)));
+    const float2 a1 = __fmul2_rn(o2, make_float2(fast_ex2(q1.x), fast_ex2(q1.y)));
+    dx[0] = dx2.x; dx[1] = dx2.y; dy[0] = dy2.x; dy[1] = dy2.y;
+    q[0] = q0.x; q[1] = q0.y; q[2] = q1.x; q[3] = q1.y;
+    ov[0] = a0.x; ov[1] = a0.y; ov[2] = a1.x; ov[3] = a1.y;
+  } else {
+    static_assert(P == 1, "the blend kernels use the <2,2> and <1,1> layouts");
+    dx[0] = __fadd_rn(g0.x, npx2.x);
+    dy[0] = __fadd_rn(g0.y, npy2.x);
+    const float qx = __fmul_rn(__fmul_rn(dx[0], la), dx[0]), bx = __fmul_rn(dx[0], lb);
+    const float qy = __fmul_rn(__fmul_rn(dy[0], lc), dy[0]);
+    q[0] = __fmaf_rn(bx, dy[0], __fadd_rn(qx, qy));
+    ov[0] = __fmul_rn(g1.y, fast_ex2(q[0]));
+  }
+}
+
+// Warp sum of up to 16 per-lane values and one RED per value, the tail of both backward kernels.  Every lane stores its
+// values v[0, n) to the rows of its warp's scratch (row k = value k, row stride kRedStride words: conflict free;
+// red_st = this lane's column), then lane 2k+p adds half p of row k (`row`: 4 LDS.128, a packed add tree), one shuffle
+// joins the halves and the lanes with `flag` set (lane 2k, k < n) issue the RED of their row's total to `dst`.
+// ~40 issue slots against ~90 for the 16-slot shuffle reduce-scatter (32 selects + 16 SHFL + 16 FADD) — the kernels
+// are issue bound.
+template <int N>
+__device__ __forceinline__ void warp_sum_red(const float (&v)[N], int n, uint32_t red_st, const float4* row, int flag,
+                                             float* dst) {
+  __syncwarp();  // the previous round's (or survivor's) row reads are complete
+#pragma unroll
+  for (int k = 0; k < N; ++k)
+    if (k < n) sts_f32(red_st + k * kRedStride * 4, v[k]);
+  __syncwarp();
+  // rows past n hold stale data; no lane issues them
+  const float4 r0 = row[0], r1 = row[1], r2 = row[2], r3 = row[3];
+  float2 s0 = __fadd2_rn(make_float2(r0.x, r0.y), make_float2(r0.z, r0.w));
+  float2 s1 = __fadd2_rn(make_float2(r1.x, r1.y), make_float2(r1.z, r1.w));
+  float2 s2 = __fadd2_rn(make_float2(r2.x, r2.y), make_float2(r2.z, r2.w));
+  float2 s3 = __fadd2_rn(make_float2(r3.x, r3.y), make_float2(r3.z, r3.w));
+  s0 = __fadd2_rn(__fadd2_rn(s0, s1), __fadd2_rn(s2, s3));
+  float total = s0.x + s0.y;
+  total += __shfl_xor_sync(0xffffffffu, total, 1);
+  red_add_f32_if(flag, dst, total);
+}
+
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
-// The CTA handles its tile only when len_lo <= (tile list length) < len_hi: the <2,2> launch takes the
-// ordinary tiles, the <1,1> launch the very long ones (see Geo).
-template <int PX, int PY, bool COUNT>
-__global__ void EGS_FWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_fwd_kernel(
+template <bool COUNT>
+__global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
     int64_t n_isects, const float4* __restrict__ splats, const int32_t* __restrict__ tile_offsets,
     const int32_t* __restrict__ flatten_ids, const float* __restrict__ backgrounds, int width, int height, int tile_w,
-    int tile_h, int n_tiles_total, int len_lo, int len_hi, float* __restrict__ render_colors,
-    float* __restrict__ render_alphas, int32_t* __restrict__ last_ids, unsigned long long* __restrict__ pair_counters,
-    float4* __restrict__ ckpt, int ckpt_k, int seg_min_len,
+    int tile_h, int n_tiles_total, float* __restrict__ render_colors, float* __restrict__ render_alphas,
+    int32_t* __restrict__ last_ids, unsigned long long* __restrict__ pair_counters, float4* __restrict__ ckpt,
+    int ckpt_k, int seg_min_len,
     // nullable: block b handles tile tile_order[b] (longest lists first, egs_isect_sorted) instead of the tile at its grid position
     const int32_t* __restrict__ tile_order) {
-  using G = Geo<PX, PY>;
+  using G = Geo<2, 2>;
   constexpr int NP = G::NP;
   constexpr int RPL = G::RPL, kBatch = G::kBatch;
   __shared__ __align__(16) WarpStage<kBatch> stage[G::kWarps];
   const int lane = threadIdx.x & 31;
   WarpStage<kBatch>& st = stage[threadIdx.x >> 5];
-  const int ordered_tile =
-      tile_order != nullptr ? tile_order[(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] : -1;
-  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, ordered_tile);
-  {
-    const int len = wv.range_end - wv.range_start;
-    if (len < len_lo || len >= len_hi) return;  // block-uniform: the other launch owns this tile
-  }
-  const int nb = (wv.range_end - wv.range_start + kBatch - 1) / kBatch;
-
-  float pxf[PX], pyf[PY];
-#pragma unroll
-  for (int i = 0; i < PX; ++i) pxf[i] = opaque((float)(wv.x0 + i) + 0.5f);
-#pragma unroll
-  for (int i = 0; i < PY; ++i) pyf[i] = opaque((float)(wv.y0 + i) + 0.5f);
-  const float2 npx2 = make_float2(-pxf[0], -pxf[PX - 1]), npy2 = make_float2(-pyf[0], -pyf[PY - 1]);
-  const float rx_lo = opaque(wv.rx_lo), rx_hi = opaque(wv.rx_hi), ry_lo = opaque(wv.ry_lo), ry_hi = opaque(wv.ry_hi);
+  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, tile_order);
   // T[j] > 0: transmittance of a live pixel; T[j] < 0: pixel finished, |T[j]| is its final transmittance
   // (the "done" flag lives in the sign bit, so liveness is one more FSETP in the accept test).
   float T[NP], cr[NP], cg[NP], cb[NP];
@@ -256,173 +377,88 @@ __global__ void EGS_FWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_fwd_kernel
   bool all_done = true;
 #pragma unroll
   for (int j = 0; j < NP; ++j) {
-    const bool inside = (wv.x0 + (j % PX)) < width && (wv.y0 + (j / PX)) < height;
+    const bool inside = (wv.x0 + (j % 2)) < width && (wv.y0 + (j / 2)) < height;
     T[j] = inside ? 1.0f : -1.0f; cr[j] = 0.f; cg[j] = 0.f; cb[j] = 0.f; last[j] = 0; term[j] = -1;
     all_done = all_done && !inside;
   }
   unsigned int n_acc = 0;
 
-  auto load_ids = [&](int b, int (&ids)[RPL]) {
+  if (wv.range_end > wv.range_start && !__all_sync(0xffffffffu, all_done)) {
+    stage_batches<false, false, RPL>(
+        st, splats, flatten_ids, wv.range_start, wv.range_end, lane, wv, [](int, int, int) {},
+        [&](int b, int ns, int batch_start) {
+          const float4* s = st.rec[b & 1];
+          // Two survivors per trip: their alphas do not depend on the running transmittance, so both are evaluated
+          // up front (independent LDS / FMA / MUFU chains = twice the ILP for a warp that walks a long list alone),
+          // then blended in order.  The vote at the top is the warp-uniform exit and the reconvergence point.
+          for (int t = 0; t < ns; t += 2) {
+            if (__all_sync(0xffffffffu, all_done)) break;
+            const bool has_b = t + 1 < ns;  // warp-uniform
+            const int cur_a = st.list[t], cur_b = st.list[has_b ? t + 1 : t];
+            float4 g0[2], g1[2];
+            float cbl[2], alpha[2][NP], q[2][NP];
+            g0[0] = s[cur_a * 3 + 0]; g1[0] = s[cur_a * 3 + 1]; cbl[0] = s[cur_a * 3 + 2].x;
+            g0[1] = s[cur_b * 3 + 0]; g1[1] = s[cur_b * 3 + 1]; cbl[1] = s[cur_b * 3 + 2].x;
 #pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      const int idx = wv.range_start + b * kBatch + r * 32 + lane;
-      ids[r] = (b < nb && idx < wv.range_end) ? __ldg(flatten_ids + idx) : -1;
-    }
-  };
-  auto issue = [&](int buf, const int (&ids)[RPL]) {
+            for (int e = 0; e < 2; ++e) {
+              float dx[2], dy[2];
+              splat_eval<2>(g0[e], g1[e], wv.npx2, wv.npy2, dx, dy, q[e], alpha[e]);
 #pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      if (ids[r] >= 0) {
-        const float4* src = splats + (size_t)ids[r] * 3;
-        float4* dst = &st.rec[buf][(r * 32 + lane) * 3];
-        cp_async16(dst + 0, src + 0);
-        cp_async16(dst + 1, src + 1);
-        cp_async16(dst + 2, src + 2);
-      }
-    }
-    cp_async_commit();
-  };
-
-  if (nb > 0 && !__all_sync(0xffffffffu, all_done)) {
-    int ids[RPL];
-    load_ids(0, ids);
-    issue(0, ids);
-    load_ids(1, ids);
-    for (int b = 0; b < nb; ++b) {
-      if (b + 1 < nb) {
-        issue((b + 1) & 1, ids);
-        load_ids(b + 2, ids);
-        cp_async_wait<1>();
-      } else {
-        cp_async_wait<0>();
-      }
-      __syncwarp();  // batch b has landed for every lane of this warp
-      const int batch_start = wv.range_start + b * kBatch;
-      const int batch_size = min(kBatch, wv.range_end - batch_start);
-      const int ns = cull_and_compact<RPL>(st, b & 1, batch_size, lane, rx_lo, rx_hi, ry_lo, ry_hi);
-      const float4* s = st.rec[b & 1];
-      // Two survivors per trip: their alphas do not depend on the running transmittance, so both are evaluated
-      // up front (independent LDS / FMA / MUFU chains = twice the ILP for a warp that walks a long list alone),
-      // then blended in order.  The vote at the top is the warp-uniform exit and the reconvergence point.
-      for (int t = 0; t < ns; t += 2) {
-        if (__all_sync(0xffffffffu, all_done)) break;
-        const bool has_b = t + 1 < ns;  // warp-uniform
-        const int cur_a = st.list[t], cur_b = st.list[has_b ? t + 1 : t];
-        float4 g0[2], g1[2];
-        float cbl[2], alpha[2][NP], q[2][NP];
-        g0[0] = s[cur_a * 3 + 0]; g1[0] = s[cur_a * 3 + 1]; cbl[0] = s[cur_a * 3 + 2].x;
-        g0[1] = s[cur_b * 3 + 0]; g1[1] = s[cur_b * 3 + 1]; cbl[1] = s[cur_b * 3 + 2].x;
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-          // q(dx,dy) = -log2(e) * sigma, separable parts shared by the rows / columns of the pixel block
-          const float la = (0.5f * kNegLog2e) * g0[e].z, lc = (0.5f * kNegLog2e) * g1[e].x, lb = kNegLog2e * g0[e].w;
-          if constexpr (PX == 2 && PY == 2) {
-            // packed fp32 (FADD2 / FMUL2 / FFMA2, sm_100): the two pixels of a row share one instruction.  The
-            // kernel is issue bound, not FMA-pipe bound (profiles/r1g), so halving the issue slots of the
-            // arithmetic is what counts.
-            const float2 dx = __fadd2_rn(make_float2(g0[e].x, g0[e].x), npx2);
-            const float2 dyv = __fadd2_rn(make_float2(g0[e].y, g0[e].y), npy2);
-            const float2 qx = __fmul2_rn(__fmul2_rn(dx, make_float2(la, la)), dx);
-            const float2 bx = __fmul2_rn(dx, make_float2(lb, lb));
-            const float2 qy = __fmul2_rn(__fmul2_rn(dyv, make_float2(lc, lc)), dyv);
-            const float2 o2 = make_float2(g1[e].y, g1[e].y);
-            const float2 q0 = __ffma2_rn(bx, make_float2(dyv.x, dyv.x), __fadd2_rn(qx, make_float2(qy.x, qy.x)));
-            const float2 q1 = __ffma2_rn(bx, make_float2(dyv.y, dyv.y), __fadd2_rn(qx, make_float2(qy.y, qy.y)));
-            const float2 a0 = __fmul2_rn(o2, make_float2(fast_ex2(q0.x), fast_ex2(q0.y)));
-            const float2 a1 = __fmul2_rn(o2, make_float2(fast_ex2(q1.x), fast_ex2(q1.y)));
-            q[e][0] = q0.x; q[e][1] = q0.y; q[e][2] = q1.x; q[e][3] = q1.y;
-            alpha[e][0] = fminf(kAlphaMax, a0.x); alpha[e][1] = fminf(kAlphaMax, a0.y);
-            alpha[e][2] = fminf(kAlphaMax, a1.x); alpha[e][3] = fminf(kAlphaMax, a1.y);
-          } else {
-            float qx[PX], bx[PX], dy[PY], qy[PY];
-#pragma unroll
-            for (int i = 0; i < PX; ++i) { const float dx = g0[e].x - pxf[i]; qx[i] = la * dx * dx; bx[i] = lb * dx; }
-#pragma unroll
-            for (int i = 0; i < PY; ++i) { dy[i] = g0[e].y - pyf[i]; qy[i] = lc * dy[i] * dy[i]; }
-#pragma unroll
-            for (int j = 0; j < NP; ++j) {
-              q[e][j] = fmaf(bx[j % PX], dy[j / PX], qx[j % PX] + qy[j / PX]);
-              alpha[e][j] = fminf(kAlphaMax, g1[e].y * fast_ex2(q[e][j]));
+              for (int j = 0; j < NP; ++j) alpha[e][j] = fminf(kAlphaMax, alpha[e][j]);
             }
-          }
-        }
-        float tmax = -1.0f;
+            float tmax = -1.0f;
 #pragma unroll
-        for (int e = 0; e < 2; ++e) {
-          if (e == 0 || has_b) {
-            const int cur = e == 0 ? cur_a : cur_b;
-            if constexpr (PX == 2 && PY == 2) {
-              // branch-free, two pixels (one row of the lane's block) per packed instruction: a rejected or
-              // finished pixel blends with weight 0 (exact: c + g * 0 = c) and keeps its T
+            for (int e = 0; e < 2; ++e) {
+              if (e == 0 || has_b) {
+                const int cur = e == 0 ? cur_a : cur_b;
+                // branch-free, two pixels (one row of the lane's block) per packed instruction: a rejected or
+                // finished pixel blends with weight 0 (exact: c + g * 0 = c) and keeps its T
 #pragma unroll
-              for (int r = 0; r < 2; ++r) {
-                const int j0 = 2 * r, j1 = 2 * r + 1;
-                const float2 a2 = make_float2(alpha[e][j0], alpha[e][j1]);
-                const float2 T2 = make_float2(T[j0], T[j1]);
-                const float2 nT = __fmul2_rn(T2, __ffma2_rn(a2, make_float2(-1.f, -1.f), make_float2(1.f, 1.f)));
-                float2 w = __fmul2_rn(a2, T2);
-                const bool acc0 = T[j0] > 0.f && q[e][j0] <= 0.f && alpha[e][j0] >= kAlphaMin;
-                const bool acc1 = T[j1] > 0.f && q[e][j1] <= 0.f && alpha[e][j1] >= kAlphaMin;
-                const bool bl0 = acc0 && nT.x > kTMin, bl1 = acc1 && nT.y > kTMin;
-                w.x = bl0 ? w.x : 0.f;
-                w.y = bl1 ? w.y : 0.f;
-                if (acc0) T[j0] = bl0 ? nT.x : -T[j0];  // not blended: finished, sign flags it
-                if (acc1) T[j1] = bl1 ? nT.y : -T[j1];
-                if (bl0) last[j0] = batch_start + cur;
-                if (bl1) last[j1] = batch_start + cur;
-                if (COUNT) {
-                  if (acc0 && !bl0) term[j0] = batch_start + cur;
-                  if (acc1 && !bl1) term[j1] = batch_start + cur;
-                  n_acc += (bl0 ? 1u : 0u) + (bl1 ? 1u : 0u);
-                }
-                const float2 c_r = __ffma2_rn(make_float2(g1[e].z, g1[e].z), w, make_float2(cr[j0], cr[j1]));
-                const float2 c_g = __ffma2_rn(make_float2(g1[e].w, g1[e].w), w, make_float2(cg[j0], cg[j1]));
-                const float2 c_b = __ffma2_rn(make_float2(cbl[e], cbl[e]), w, make_float2(cb[j0], cb[j1]));
-                cr[j0] = c_r.x; cr[j1] = c_r.y; cg[j0] = c_g.x; cg[j1] = c_g.y; cb[j0] = c_b.x; cb[j1] = c_b.y;
-              }
-            } else {
-#pragma unroll
-              for (int j = 0; j < NP; ++j) {
-                if (T[j] > 0.f && q[e][j] <= 0.f && alpha[e][j] >= kAlphaMin) {  // sigma >= 0  <=>  q <= 0
-                  const float next_T = T[j] * (1.0f - alpha[e][j]);
-                  if (next_T <= kTMin) {
-                    T[j] = -T[j];  // finished: this Gaussian is not blended
-                    if (COUNT) term[j] = batch_start + cur;
-                  } else {
-                    const float w = alpha[e][j] * T[j];
-                    cr[j] = fmaf(g1[e].z, w, cr[j]);
-                    cg[j] = fmaf(g1[e].w, w, cg[j]);
-                    cb[j] = fmaf(cbl[e], w, cb[j]);
-                    last[j] = batch_start + cur;
-                    T[j] = next_T;
-                    if (COUNT) ++n_acc;
+                for (int r = 0; r < 2; ++r) {
+                  const int j0 = 2 * r, j1 = 2 * r + 1;
+                  const float2 a2 = make_float2(alpha[e][j0], alpha[e][j1]);
+                  const float2 T2 = make_float2(T[j0], T[j1]);
+                  const float2 nT = __fmul2_rn(T2, __ffma2_rn(a2, make_float2(-1.f, -1.f), make_float2(1.f, 1.f)));
+                  float2 w = __fmul2_rn(a2, T2);
+                  const bool acc0 = T[j0] > 0.f && q[e][j0] <= 0.f && alpha[e][j0] >= kAlphaMin;
+                  const bool acc1 = T[j1] > 0.f && q[e][j1] <= 0.f && alpha[e][j1] >= kAlphaMin;
+                  const bool bl0 = acc0 && nT.x > kTMin, bl1 = acc1 && nT.y > kTMin;
+                  w.x = bl0 ? w.x : 0.f;
+                  w.y = bl1 ? w.y : 0.f;
+                  if (acc0) T[j0] = bl0 ? nT.x : -T[j0];  // not blended: finished, sign flags it
+                  if (acc1) T[j1] = bl1 ? nT.y : -T[j1];
+                  if (bl0) last[j0] = batch_start + cur;
+                  if (bl1) last[j1] = batch_start + cur;
+                  if (COUNT) {
+                    if (acc0 && !bl0) term[j0] = batch_start + cur;
+                    if (acc1 && !bl1) term[j1] = batch_start + cur;
+                    n_acc += (bl0 ? 1u : 0u) + (bl1 ? 1u : 0u);
                   }
+                  const float2 c_r = __ffma2_rn(make_float2(g1[e].z, g1[e].z), w, make_float2(cr[j0], cr[j1]));
+                  const float2 c_g = __ffma2_rn(make_float2(g1[e].w, g1[e].w), w, make_float2(cg[j0], cg[j1]));
+                  const float2 c_b = __ffma2_rn(make_float2(cbl[e], cbl[e]), w, make_float2(cb[j0], cb[j1]));
+                  cr[j0] = c_r.x; cr[j1] = c_r.y; cg[j0] = c_g.x; cg[j1] = c_g.y; cb[j0] = c_b.x; cb[j1] = c_b.y;
                 }
               }
             }
+#pragma unroll
+            for (int j = 0; j < NP; ++j) tmax = fmaxf(tmax, T[j]);
+            all_done = !(tmax > 0.f);
           }
-        }
+          if (__all_sync(0xffffffffu, all_done)) return true;  // this warp needs nothing further down the list
+          // Per-pixel state after every ckpt_k entries of a long list: lets the backward pass start its back-to-front
+          // replay at any of these boundaries, one warp per segment (see rasterize_bwd_kernel).  Slot numbering
+          // floor(start / K) + k is collision free across tiles because their list ranges are disjoint and ordered.
+          const int done_local = (b + 1) * kBatch;
+          if (ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len && done_local % ckpt_k == 0 &&
+              done_local < wv.range_end - wv.range_start) {
+            const size_t slot = (size_t)(wv.range_start / ckpt_k + done_local / ckpt_k);
+            float4* dst = ckpt + ((slot * G::kWarps + (threadIdx.x >> 5)) * NP) * 32 + lane;
 #pragma unroll
-        for (int j = 0; j < NP; ++j) tmax = fmaxf(tmax, T[j]);
-        all_done = !(tmax > 0.f);
-      }
-      if (__all_sync(0xffffffffu, all_done)) break;  // this warp needs nothing further down the list
-      if constexpr (PX == 2 && PY == 2) {
-        // Per-pixel state after every ckpt_k entries of a long list: lets the backward pass start its back-to-front
-        // replay at any of these boundaries, one warp per segment (see rasterize_bwd_kernel).  Slot numbering
-        // floor(start / K) + k is collision free across tiles because their list ranges are disjoint and ordered.
-        const int done_local = (b + 1) * kBatch;
-        if (ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len && done_local % ckpt_k == 0 &&
-            done_local < wv.range_end - wv.range_start) {
-          const size_t slot = (size_t)(wv.range_start / ckpt_k + done_local / ckpt_k);
-          float4* dst = ckpt + ((slot * G::kWarps + (threadIdx.x >> 5)) * NP) * 32 + lane;
-#pragma unroll
-          for (int j = 0; j < NP; ++j) dst[j * 32] = make_float4(T[j], cr[j], cg[j], cb[j]);
-        }
-      }
-      __syncwarp();  // every lane is done with buffer b&1 and the list before they are overwritten
-    }
-    cp_async_wait<0>();
+            for (int j = 0; j < NP; ++j) dst[j * 32] = make_float4(T[j], cr[j], cg[j], cb[j]);
+          }
+          return false;
+        });
   }
 
   float bgr = 0.f, bgg = 0.f, bgb = 0.f;
@@ -432,7 +468,7 @@ __global__ void EGS_FWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_fwd_kernel
   unsigned int n_eval = 0;
 #pragma unroll
   for (int j = 0; j < NP; ++j) {
-    const int x = wv.x0 + (j % PX), y = wv.y0 + (j / PX);
+    const int x = wv.x0 + (j % 2), y = wv.y0 + (j / 2);
     if (x < width && y < height) {
       const size_t pix = ((size_t)wv.cam * height + y) * width + x;
       const float Tf = fabsf(T[j]);
@@ -461,11 +497,10 @@ __global__ void EGS_FWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_fwd_kernel
 // backward
 // ------------------------------------------------------------------------------------------------
 
-template <int PX, int PY>
-__global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel(
+__global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
     int64_t n_isects, const float4* __restrict__ splats, const int32_t* __restrict__ tile_offsets,
     const int32_t* __restrict__ flatten_ids, const float* __restrict__ backgrounds, int width, int height, int tile_w,
-    int tile_h, int n_tiles_total, int len_lo, int len_hi, const float* __restrict__ render_alphas,
+    int tile_h, int n_tiles_total, const float* __restrict__ render_alphas,
     const int32_t* __restrict__ last_ids, const float* __restrict__ v_render_colors,
     const float* __restrict__ v_render_alphas, float* __restrict__ v_splats,
     // Segmented replay of long lists (ckpt != nullptr): the forward pass left the per-pixel state after every ckpt_k
@@ -476,7 +511,7 @@ __global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel
     // Only lists of at least seg_min_len (> ckpt_k) entries are replayed in segments; shorter ones as one piece.
     const float* __restrict__ render_colors, const float4* __restrict__ ckpt, int ckpt_k, int seg_min_len, int seg_launch,
     const int32_t* __restrict__ tile_order /* nullable, tile launch only: see the forward kernel */) {
-  using G = Geo<PX, PY>;
+  using G = Geo<2, 2>;
   constexpr int NP = G::NP;
   constexpr int RPL = G::RPL, kBatch = G::kBatch;
   __shared__ __align__(16) WarpStage<kBatch> stage[G::kWarps];
@@ -496,23 +531,13 @@ __global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel
     }
     seg_tile = lo_t;
     seg_k = (int)(blockIdx.x + 1) - tile_offsets[seg_tile] / ckpt_k;
-  } else if (tile_order != nullptr) {
-    seg_tile = tile_order[(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x];
   }
-  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, seg_tile);
+  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, tile_order, seg_tile);
   {
     const int len = wv.range_end - wv.range_start;
-    if (len <= 0 || len < len_lo || len >= len_hi) return;  // block-uniform: empty, or owned by the other launch
+    if (len <= 0) return;  // block-uniform
     if (seg_launch && (len < seg_min_len || seg_k < 1 || (int64_t)seg_k * ckpt_k >= len)) return;  // block-uniform: slot not in use
   }
-
-  float pxf[PX], pyf[PY];
-#pragma unroll
-  for (int i = 0; i < PX; ++i) pxf[i] = opaque((float)(wv.x0 + i) + 0.5f);
-#pragma unroll
-  for (int i = 0; i < PY; ++i) pyf[i] = opaque((float)(wv.y0 + i) + 0.5f);
-  const float2 npx2 = make_float2(-pxf[0], -pxf[PX - 1]), npy2 = make_float2(-pyf[0], -pyf[PY - 1]);
-  const float rx_lo = opaque(wv.rx_lo), rx_hi = opaque(wv.rx_hi), ry_lo = opaque(wv.ry_lo), ry_hi = opaque(wv.ry_hi);
 
   // per-pixel replay state.  nbt_ = tfv - bdot with bdot = sum over the Gaussians behind of fac * (rgb . v_colour),
   // which is all the backward pass needs of the colour accumulated behind, and
@@ -526,7 +551,7 @@ __global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel
   }
 #pragma unroll
   for (int j = 0; j < NP; ++j) {
-    const int x = wv.x0 + (j % PX), y = wv.y0 + (j / PX);
+    const int x = wv.x0 + (j % 2), y = wv.y0 + (j / 2);
     T[j] = 1.f; nbt_[j] = 0.f; vcr[j] = 0.f; vcg[j] = 0.f; vcb[j] = 0.f;
     bin_final[j] = -1;  // pixels outside the image never match any index
     if (x < width && y < height) {
@@ -546,62 +571,36 @@ __global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel
   int end_idx = min(wv.range_end - 1, warp_last);
   if (end_idx < wv.range_start) return;  // warp-uniform
   int lo_idx = wv.range_start;  // the replay walks end_idx, end_idx - 1, ..., lo_idx
-  if constexpr (PX == 2 && PY == 2) {
-    if (ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len) {
-      const int last_seg = (end_idx - wv.range_start) / ckpt_k;  // segment that holds the warp's last blended entry
-      if (!seg_launch) {
-        lo_idx = wv.range_start + last_seg * ckpt_k;
-      } else {
-        if (seg_k > last_seg) return;  // warp-uniform: nothing of this warp reaches into or beyond this segment
-        end_idx = wv.range_start + seg_k * ckpt_k - 1;
-        lo_idx = end_idx + 1 - ckpt_k;
-        // state after entry end_idx: transmittance and colour accumulated in front of the boundary (the forward
-        // checkpoint); what lies behind it is the final colour minus that
-        const size_t slot = (size_t)(wv.range_start / ckpt_k + seg_k);
-        const float4* src = ckpt + ((slot * G::kWarps + (threadIdx.x >> 5)) * NP) * 32 + lane;
+  if (ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len) {
+    const int last_seg = (end_idx - wv.range_start) / ckpt_k;  // segment that holds the warp's last blended entry
+    if (!seg_launch) {
+      lo_idx = wv.range_start + last_seg * ckpt_k;
+    } else {
+      if (seg_k > last_seg) return;  // warp-uniform: nothing of this warp reaches into or beyond this segment
+      end_idx = wv.range_start + seg_k * ckpt_k - 1;
+      lo_idx = end_idx + 1 - ckpt_k;
+      // state after entry end_idx: transmittance and colour accumulated in front of the boundary (the forward
+      // checkpoint); what lies behind it is the final colour minus that
+      const size_t slot = (size_t)(wv.range_start / ckpt_k + seg_k);
+      const float4* src = ckpt + ((slot * G::kWarps + (threadIdx.x >> 5)) * NP) * 32 + lane;
 #pragma unroll
-        for (int j = 0; j < NP; ++j) {
-          const int x = wv.x0 + (j % PX), y = wv.y0 + (j / PX);
-          if (x < width && y < height) {
-            const size_t pix = ((size_t)wv.cam * height + y) * width + x;
-            const float4 ck = src[j * 32];
-            const float T_final = T[j];
-            const float br = render_colors[pix * 3 + 0] - T_final * bgr - ck.y;
-            const float bgn = render_colors[pix * 3 + 1] - T_final * bgg - ck.z;
-            const float bb = render_colors[pix * 3 + 2] - T_final * bgb - ck.w;
-            nbt_[j] -= br * vcr[j] + bgn * vcg[j] + bb * vcb[j];
-            T[j] = fabsf(ck.x);
-          }
+      for (int j = 0; j < NP; ++j) {
+        const int x = wv.x0 + (j % 2), y = wv.y0 + (j / 2);
+        if (x < width && y < height) {
+          const size_t pix = ((size_t)wv.cam * height + y) * width + x;
+          const float4 ck = src[j * 32];
+          const float T_final = T[j];
+          const float br = render_colors[pix * 3 + 0] - T_final * bgr - ck.y;
+          const float bgn = render_colors[pix * 3 + 1] - T_final * bgg - ck.z;
+          const float bb = render_colors[pix * 3 + 2] - T_final * bgb - ck.w;
+          nbt_[j] -= br * vcr[j] + bgn * vcg[j] + bb * vcb[j];
+          T[j] = fabsf(ck.x);
         }
       }
-    } else if (seg_launch) {
-      return;
     }
+  } else if (seg_launch) {
+    return;
   }
-  const int nb = (end_idx - lo_idx + 1 + kBatch - 1) / kBatch;
-
-  auto load_ids = [&](int b, int (&ids)[RPL]) {
-#pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      const int idx = end_idx - b * kBatch - (r * 32 + lane);
-      ids[r] = (b < nb && idx >= lo_idx) ? __ldg(flatten_ids + idx) : -1;
-    }
-  };
-  auto issue = [&](int buf, const int (&ids)[RPL]) {
-#pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      const int slot = r * 32 + lane;
-      if (ids[r] >= 0) {
-        const float4* src = splats + (size_t)ids[r] * 3;
-        float4* dst = &st.rec[buf][slot * 3];
-        cp_async16(dst + 0, src + 0);
-        cp_async16(dst + 1, src + 1);
-        cp_async16(dst + 2, src + 2);
-      }
-      st.id[buf][slot] = ids[r];
-    }
-    cp_async_commit();
-  };
 
   // Addresses of the warp-sum scratch and of the gradient slot this lane reduces, pinned in registers: ptxas
   // otherwise re-derives them from %tid / the CTA's shared window for every survivor (~12 of the loop's ~200
@@ -615,181 +614,91 @@ __global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel
   float* out_base = v_splats + min(out_slot, kGradValues - 1);
   asm volatile("" : "+l"(out_base));
 
-  int ids[RPL];
-  load_ids(0, ids);
-  issue(0, ids);
-  load_ids(1, ids);
-  for (int b = 0; b < nb; ++b) {
-    if (b + 1 < nb) {
-      issue((b + 1) & 1, ids);
-      load_ids(b + 2, ids);
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncwarp();
-    const int batch_end = end_idx - b * kBatch;  // sorted index held in slot 0 (the one furthest back)
-    const int batch_size = min(kBatch, batch_end + 1 - lo_idx);
-    const int ns = cull_and_compact<RPL>(st, b & 1, batch_size, lane, rx_lo, rx_hi, ry_lo, ry_hi);
-    const float4* s = st.rec[b & 1];
-    const int* sid = st.id[b & 1];
-    int slot = st.list[0];
-    for (int t = 0; t < ns; ++t) {  // warp-uniform bounds
-      const int cur = slot;
-      slot = st.list[min(t + 1, kBatch - 1)];
-      const int idx = batch_end - cur;
-      const float4 g0 = s[cur * 3 + 0];  // x, y, conic_a, conic_b
-      const float4 g1 = s[cur * 3 + 1];  // conic_c, opacity, r, g
-      const float la = (0.5f * kNegLog2e) * g0.z, lc = (0.5f * kNegLog2e) * g1.x, lb = kNegLog2e * g0.w;
-      const float cbl = s[cur * 3 + 2].x;
-      const float inv_o = fast_rcp(g1.y);
-      // v[2], v[3], v[4] accumulate sx*dx, sx*dy, sy*dy (the 0.5 of the conic gradient is applied once, after
-      // the per-lane sum); v[5] accumulates ov * v_alpha (the 1/opacity is applied after the per-lane sum).
-      float v[kGradValues];
+  stage_batches<true, true, RPL>(
+      st, splats, flatten_ids, end_idx, lo_idx - 1, lane, wv, [](int, int, int) {},
+      [&](int b, int ns, int batch_end) {  // batch_end: sorted index held in slot 0 (the one furthest back)
+        const float4* s = st.rec[b & 1];
+        const int* sid = st.id[b & 1];
+        int slot = st.list[0];
+        for (int t = 0; t < ns; ++t) {  // warp-uniform bounds
+          const int cur = slot;
+          slot = st.list[min(t + 1, kBatch - 1)];
+          const int idx = batch_end - cur;
+          const float4 g0 = s[cur * 3 + 0];  // x, y, conic_a, conic_b
+          const float4 g1 = s[cur * 3 + 1];  // conic_c, opacity, r, g
+          const float cbl = s[cur * 3 + 2].x;
+          const float inv_o = fast_rcp(g1.y);
+          // Packed fp32 (FADD2 / FMUL2 / FFMA2): the two pixels of a row of the lane's block share one instruction,
+          // and the replay is branch free — a pixel that does not take part gets alpha = 0 and ov = 0, which makes
+          // every one of its contributions an exact zero and leaves its running state untouched.
+          float dx[2], dy[2], q[NP], ov[NP];
+          splat_eval<2>(g0, g1, wv.npx2, wv.npy2, dx, dy, q, ov);
+          const float2 dx2 = make_float2(dx[0], dx[1]);
+          bool valid[NP];
+          bool any_valid = false;
 #pragma unroll
-      for (int k = 0; k < kGradValues; ++k) v[k] = 0.f;
-      if constexpr (PX == 2 && PY == 2) {
-        // Packed fp32 (FADD2 / FMUL2 / FFMA2): the two pixels of a row of the lane's block share one instruction,
-        // and the replay is branch free — a pixel that does not take part gets alpha = 0 and ov = 0, which makes
-        // every one of its contributions an exact zero and leaves its running state untouched.
-        const float2 dx2 = __fadd2_rn(make_float2(g0.x, g0.x), npx2);
-        const float2 dy2 = __fadd2_rn(make_float2(g0.y, g0.y), npy2);
-        const float2 qx = __fmul2_rn(__fmul2_rn(dx2, make_float2(la, la)), dx2);
-        const float2 bx = __fmul2_rn(dx2, make_float2(lb, lb));
-        const float2 qy = __fmul2_rn(__fmul2_rn(dy2, make_float2(lc, lc)), dy2);
-        const float2 o2 = make_float2(g1.y, g1.y);
-        float2 ov2[2];
-        bool valid[NP];
-        bool any_valid = false;
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-          const float dyr = r == 0 ? dy2.x : dy2.y, qyr = r == 0 ? qy.x : qy.y;
-          const float2 q = __ffma2_rn(bx, make_float2(dyr, dyr), __fadd2_rn(qx, make_float2(qyr, qyr)));
-          ov2[r] = __fmul2_rn(o2, make_float2(fast_ex2(q.x), fast_ex2(q.y)));
-          valid[2 * r] = idx <= bin_final[2 * r] && q.x <= 0.f && ov2[r].x >= kAlphaMin;
-          valid[2 * r + 1] = idx <= bin_final[2 * r + 1] && q.y <= 0.f && ov2[r].y >= kAlphaMin;
-          any_valid = any_valid || valid[2 * r] || valid[2 * r + 1];
-        }
-        if (!__any_sync(0xffffffffu, any_valid)) continue;  // warp-uniform
-        float2 s_gx = make_float2(0.f, 0.f), s_gy = s_gx, s_xx = s_gx, s_xy = s_gx, s_yy = s_gx, s_w = s_gx, s_r = s_gx,
-               s_g = s_gx, s_b = s_gx, s_ax = s_gx, s_ay = s_gx;
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-          const int j0 = 2 * r, j1 = 2 * r + 1;
-          const float dyr = r == 0 ? dy2.x : dy2.y;
-          const float2 dyb = make_float2(dyr, dyr);
-          float2 ae, oe;  // alpha and ov of the pixels that take part, 0 for the others
-          // ov of the pixels that take part, 0 for the others; everything downstream is then an exact no-op for
-          // a pixel that does not take part: alpha = 0, 1 - alpha = 1, MUFU.RCP(1) = 1 exactly
-          // (scripts/probes/rcp_one.cu), so T * 1 = T needs no select
-          const float ovx = valid[j0] ? ov2[r].x : 0.f, ovy = valid[j1] ? ov2[r].y : 0.f;
-          ae.x = fminf(kAlphaMax, ovx);
-          ae.y = fminf(kAlphaMax, ovy);
-          oe.x = ovx <= kAlphaMax ? ovx : 0.f;  // clamp inactive: alpha depends on sigma, opacity
-          oe.y = ovy <= kAlphaMax ? ovy : 0.f;
-          const float2 om = __ffma2_rn(ae, make_float2(-1.f, -1.f), make_float2(1.f, 1.f));
-          const float2 ra = make_float2(fast_rcp(om.x), fast_rcp(om.y));
-          const float2 Tf = __fmul2_rn(make_float2(T[j0], T[j1]), ra);  // transmittance in front of this Gaussian
-          T[j0] = Tf.x; T[j1] = Tf.y;
-          const float2 fac = __fmul2_rn(ae, Tf);
-          const float2 vr2 = make_float2(vcr[j0], vcr[j1]), vg2 = make_float2(vcg[j0], vcg[j1]), vb2 = make_float2(vcb[j0], vcb[j1]);
-          s_r = __ffma2_rn(fac, vr2, s_r);
-          s_g = __ffma2_rn(fac, vg2, s_g);
-          s_b = __ffma2_rn(fac, vb2, s_b);
-          const float2 cdot = __ffma2_rn(make_float2(cbl, cbl), vb2,
-                                         __ffma2_rn(make_float2(g1.w, g1.w), vg2, __fmul2_rn(make_float2(g1.z, g1.z), vr2)));
-          // nbt = tfv - bdot (kept negated so that v_alpha is one FMUL2 + one FFMA2)
-          const float2 nbt = make_float2(nbt_[j0], nbt_[j1]);
-          const float2 v_alpha = __ffma2_rn(Tf, cdot, __fmul2_rn(ra, nbt));
-          const float2 nfac = make_float2(-fac.x, -fac.y);
-          const float2 nbt_new = __ffma2_rn(cdot, nfac, nbt);
-          nbt_[j0] = nbt_new.x; nbt_[j1] = nbt_new.y;
-          const float2 w = __fmul2_rn(oe, v_alpha);  // = opacity * d(alpha)/d(opacity) * v_alpha = -v_sigma
-          const float2 nw = make_float2(-w.x, -w.y);
-          const float2 sx = __fmul2_rn(nw, dx2), sy = __fmul2_rn(nw, dyb);
-          s_xx = __ffma2_rn(sx, dx2, s_xx);
-          s_xy = __ffma2_rn(sx, dyb, s_xy);
-          s_yy = __ffma2_rn(sy, dyb, s_yy);
-          const float2 gx = __ffma2_rn(make_float2(g0.w, g0.w), sy, __fmul2_rn(make_float2(g0.z, g0.z), sx));
-          const float2 gy = __ffma2_rn(make_float2(g1.x, g1.x), sy, __fmul2_rn(make_float2(g0.w, g0.w), sx));
-          s_gx = __fadd2_rn(s_gx, gx);
-          s_gy = __fadd2_rn(s_gy, gy);
-          s_ax = __fadd2_rn(s_ax, make_float2(fabsf(gx.x), fabsf(gx.y)));
-          s_ay = __fadd2_rn(s_ay, make_float2(fabsf(gy.x), fabsf(gy.y)));
-          s_w = __fadd2_rn(s_w, w);
-        }
-        v[0] = s_gx.x + s_gx.y; v[1] = s_gy.x + s_gy.y; v[2] = s_xx.x + s_xx.y; v[3] = s_xy.x + s_xy.y;
-        v[4] = s_yy.x + s_yy.y; v[5] = s_w.x + s_w.y; v[6] = s_r.x + s_r.y; v[7] = s_g.x + s_g.y;
-        v[8] = s_b.x + s_b.y; v[9] = s_ax.x + s_ax.y; v[10] = s_ay.x + s_ay.y;
-      } else {
-        float dx[PX], qx[PX], bx[PX], dy[PY], qy[PY];
-#pragma unroll
-        for (int i = 0; i < PX; ++i) { dx[i] = g0.x - pxf[i]; qx[i] = la * dx[i] * dx[i]; bx[i] = lb * dx[i]; }
-#pragma unroll
-        for (int i = 0; i < PY; ++i) { dy[i] = g0.y - pyf[i]; qy[i] = lc * dy[i] * dy[i]; }
-        float ov[NP];  // opacity * exp(-sigma), before the 0.999 clamp
-        bool valid[NP];
-        bool any_valid = false;
-#pragma unroll
-        for (int j = 0; j < NP; ++j) {
-          const float q = fmaf(bx[j % PX], dy[j / PX], qx[j % PX] + qy[j / PX]);  // -log2(e) * sigma
-          ov[j] = g1.y * fast_ex2(q);
-          valid[j] = idx <= bin_final[j] && q <= 0.f && ov[j] >= kAlphaMin;  // min(.999, ov) >= 1/255 <=> ov >= 1/255
-          any_valid = any_valid || valid[j];
-        }
-        if (!__any_sync(0xffffffffu, any_valid)) continue;  // warp-uniform
-#pragma unroll
-        for (int j = 0; j < NP; ++j) {
-          if (valid[j]) {
-            const float ddx = dx[j % PX], ddy = dy[j / PX];
-            const float alpha = fminf(kAlphaMax, ov[j]);
-            const float ra = fast_rcp(1.0f - alpha);
-            T[j] *= ra;  // transmittance in front of this Gaussian
-            const float fac = alpha * T[j];
-            v[6] = fmaf(fac, vcr[j], v[6]);
-            v[7] = fmaf(fac, vcg[j], v[7]);
-            v[8] = fmaf(fac, vcb[j], v[8]);
-            const float cdot = fmaf(cbl, vcb[j], fmaf(g1.w, vcg[j], g1.z * vcr[j]));
-            const float v_alpha = fmaf(T[j], cdot, ra * nbt_[j]);
-            nbt_[j] = fmaf(cdot, -fac, nbt_[j]);
-            if (ov[j] <= kAlphaMax) {  // the clamp was inactive: alpha depends on sigma and opacity
-              const float w = ov[j] * v_alpha;  // = opacity * d(alpha)/d(opacity) * v_alpha = -v_sigma
-              const float sx = -w * ddx, sy = -w * ddy;
-              v[2] = fmaf(sx, ddx, v[2]);
-              v[3] = fmaf(sx, ddy, v[3]);
-              v[4] = fmaf(sy, ddy, v[4]);
-              const float gx = fmaf(g0.w, sy, g0.z * sx);
-              const float gy = fmaf(g1.x, sy, g0.w * sx);
-              v[0] += gx;
-              v[1] += gy;
-              v[9] += fabsf(gx);
-              v[10] += fabsf(gy);
-              v[5] += w;
-            }
+          for (int j = 0; j < NP; ++j) {
+            valid[j] = idx <= bin_final[j] && q[j] <= 0.f && ov[j] >= kAlphaMin;  // min(.999, ov) >= 1/255 <=> ov >= 1/255
+            any_valid = any_valid || valid[j];
           }
-        }
-      }
-      v[2] *= 0.5f; v[4] *= 0.5f; v[5] *= inv_o;
-      // Warp sum of the 11 values through shared memory: every lane stores its 11 partials (row k = value k,
-      // row stride 36 words: conflict free), then lane 2k+p adds half p of row k (4 LDS.128, a packed add tree),
-      // one shuffle joins the halves and lane 2k issues the RED.  ~40 issue slots against ~90 for the 16-slot
-      // shuffle reduce-scatter (32 selects + 16 SHFL + 16 FADD) — the kernel is issue bound.
-      __syncwarp();  // the previous survivor's row reads are complete
+          if (!__any_sync(0xffffffffu, any_valid)) continue;  // warp-uniform
+          float2 s_gx = make_float2(0.f, 0.f), s_gy = s_gx, s_xx = s_gx, s_xy = s_gx, s_yy = s_gx, s_w = s_gx, s_r = s_gx,
+                 s_g = s_gx, s_b = s_gx, s_ax = s_gx, s_ay = s_gx;
 #pragma unroll
-      for (int k = 0; k < kGradValues; ++k) sts_f32(red_st + k * kRedStride * 4, v[k]);
-      __syncwarp();
-      const float4 r0 = row[0], r1 = row[1], r2 = row[2], r3 = row[3];
-      float2 s0 = __fadd2_rn(make_float2(r0.x, r0.y), make_float2(r0.z, r0.w));
-      float2 s1 = __fadd2_rn(make_float2(r1.x, r1.y), make_float2(r1.z, r1.w));
-      float2 s2 = __fadd2_rn(make_float2(r2.x, r2.y), make_float2(r2.z, r2.w));
-      float2 s3 = __fadd2_rn(make_float2(r3.x, r3.y), make_float2(r3.z, r3.w));
-      s0 = __fadd2_rn(__fadd2_rn(s0, s1), __fadd2_rn(s2, s3));
-      float total = s0.x + s0.y;
-      total += __shfl_xor_sync(0xffffffffu, total, 1);
-      red_add_f32_if(red_flag, out_base + (size_t)sid[cur] * EGS_SPLAT_FLOATS, total);
-    }
-    __syncwarp();  // buffer b&1, its ids and the list are free again
-  }
+          for (int r = 0; r < 2; ++r) {
+            const int j0 = 2 * r, j1 = 2 * r + 1;
+            const float2 dyb = make_float2(dy[r], dy[r]);
+            float2 ae, oe;  // alpha and ov of the pixels that take part, 0 for the others
+            // ov of the pixels that take part, 0 for the others; everything downstream is then an exact no-op for
+            // a pixel that does not take part: alpha = 0, 1 - alpha = 1, MUFU.RCP(1) = 1 exactly
+            // (scripts/probes/rcp_one.cu), so T * 1 = T needs no select
+            const float ovx = valid[j0] ? ov[j0] : 0.f, ovy = valid[j1] ? ov[j1] : 0.f;
+            ae.x = fminf(kAlphaMax, ovx);
+            ae.y = fminf(kAlphaMax, ovy);
+            oe.x = ovx <= kAlphaMax ? ovx : 0.f;  // clamp inactive: alpha depends on sigma, opacity
+            oe.y = ovy <= kAlphaMax ? ovy : 0.f;
+            const float2 om = __ffma2_rn(ae, make_float2(-1.f, -1.f), make_float2(1.f, 1.f));
+            const float2 ra = make_float2(fast_rcp(om.x), fast_rcp(om.y));
+            const float2 Tf = __fmul2_rn(make_float2(T[j0], T[j1]), ra);  // transmittance in front of this Gaussian
+            T[j0] = Tf.x; T[j1] = Tf.y;
+            const float2 fac = __fmul2_rn(ae, Tf);
+            const float2 vr2 = make_float2(vcr[j0], vcr[j1]), vg2 = make_float2(vcg[j0], vcg[j1]), vb2 = make_float2(vcb[j0], vcb[j1]);
+            s_r = __ffma2_rn(fac, vr2, s_r);
+            s_g = __ffma2_rn(fac, vg2, s_g);
+            s_b = __ffma2_rn(fac, vb2, s_b);
+            const float2 cdot = __ffma2_rn(make_float2(cbl, cbl), vb2,
+                                           __ffma2_rn(make_float2(g1.w, g1.w), vg2, __fmul2_rn(make_float2(g1.z, g1.z), vr2)));
+            // nbt = tfv - bdot (kept negated so that v_alpha is one FMUL2 + one FFMA2)
+            const float2 nbt = make_float2(nbt_[j0], nbt_[j1]);
+            const float2 v_alpha = __ffma2_rn(Tf, cdot, __fmul2_rn(ra, nbt));
+            const float2 nfac = make_float2(-fac.x, -fac.y);
+            const float2 nbt_new = __ffma2_rn(cdot, nfac, nbt);
+            nbt_[j0] = nbt_new.x; nbt_[j1] = nbt_new.y;
+            const float2 w = __fmul2_rn(oe, v_alpha);  // = opacity * d(alpha)/d(opacity) * v_alpha = -v_sigma
+            const float2 nw = make_float2(-w.x, -w.y);
+            const float2 sx = __fmul2_rn(nw, dx2), sy = __fmul2_rn(nw, dyb);
+            s_xx = __ffma2_rn(sx, dx2, s_xx);
+            s_xy = __ffma2_rn(sx, dyb, s_xy);
+            s_yy = __ffma2_rn(sy, dyb, s_yy);
+            const float2 gx = __ffma2_rn(make_float2(g0.w, g0.w), sy, __fmul2_rn(make_float2(g0.z, g0.z), sx));
+            const float2 gy = __ffma2_rn(make_float2(g1.x, g1.x), sy, __fmul2_rn(make_float2(g0.w, g0.w), sx));
+            s_gx = __fadd2_rn(s_gx, gx);
+            s_gy = __fadd2_rn(s_gy, gy);
+            s_ax = __fadd2_rn(s_ax, make_float2(fabsf(gx.x), fabsf(gx.y)));
+            s_ay = __fadd2_rn(s_ay, make_float2(fabsf(gy.x), fabsf(gy.y)));
+            s_w = __fadd2_rn(s_w, w);
+          }
+          // v[2], v[3], v[4] are the sums of sx*dx, sx*dy, sy*dy (the 0.5 of the conic gradient is applied once, after
+          // the per-lane sum); v[5] the sum of ov * v_alpha (the 1/opacity is applied after the per-lane sum).
+          float v[kGradValues];
+          v[0] = s_gx.x + s_gx.y; v[1] = s_gy.x + s_gy.y; v[2] = s_xx.x + s_xx.y; v[3] = s_xy.x + s_xy.y;
+          v[4] = s_yy.x + s_yy.y; v[5] = s_w.x + s_w.y; v[6] = s_r.x + s_r.y; v[7] = s_g.x + s_g.y;
+          v[8] = s_b.x + s_b.y; v[9] = s_ax.x + s_ax.y; v[10] = s_ay.x + s_ay.y;
+          v[2] *= 0.5f; v[4] *= 0.5f; v[5] *= inv_o;
+          warp_sum_red(v, kGradValues, red_st, row, red_flag, out_base + (size_t)sid[cur] * EGS_SPLAT_FLOATS);
+        }
+        return false;
+      });
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -798,7 +707,8 @@ __global__ void EGS_BWD_BOUNDS((Geo<PX, PY>::kThreads), PX) rasterize_bwd_kernel
 // The same blend as above with CH colour channels per launch, read from a separate fp32 row array instead of the r, g, b
 // slots of the splat record (which these kernels do not read).  Row of a list entry: flat id - cam * N when one [N, .]
 // array serves every camera, the flat id for a [C * N, .] array.  A launch covers channels [c0, c0 + CH) of the rows;
-// wider colours are several launches on the same binning result.  The accept / finish tests and the alpha arithmetic are
+// wider colours are several launches on the same binning result.  The prologue (warp_setup), the staging and culling
+// (stage_batches), the alpha evaluation (splat_eval), the accept / finish tests and the warp-sum tail (warp_sum_red) are
 // the RGB kernels'; in the <2,2> layout (CH <= 8) alphas and last_ids come out bit-identical to them, while the <1,1>
 // layout's transmittance differs in the last bits (measured on a B200: alphas within 2.4e-7).
 // Pixel layout: CH <= 8 keeps the RGB kernels' <2,2> layout (4 pixels per lane, 4 CH colour registers); CH = 16 / 32
@@ -854,38 +764,6 @@ __device__ __forceinline__ void load_row(float (&f)[CH], const float* src) {
   }
 }
 
-// q = -log2(e) * sigma and ov = opacity * 2^q (before the 0.999 clamp) at the lane's pixels, with dx / dy = mean - pixel
-// centre per column / row.  The RGB kernels' operations in the same order: packed FADD2 / FMUL2 / FFMA2 in the <2,2>
-// layout, the same sequence one pixel at a time in <1,1>.
-template <int P>
-__device__ __forceinline__ void splat_eval(const float4 g0, const float4 g1, const float2 npx2, const float2 npy2,
-                                           float (&dx)[P], float (&dy)[P], float (&q)[P * P], float (&ov)[P * P]) {
-  const float la = (0.5f * kNegLog2e) * g0.z, lc = (0.5f * kNegLog2e) * g1.x, lb = kNegLog2e * g0.w;
-  if constexpr (P == 2) {
-    const float2 dx2 = __fadd2_rn(make_float2(g0.x, g0.x), npx2);
-    const float2 dy2 = __fadd2_rn(make_float2(g0.y, g0.y), npy2);
-    const float2 qx = __fmul2_rn(__fmul2_rn(dx2, make_float2(la, la)), dx2);
-    const float2 bx = __fmul2_rn(dx2, make_float2(lb, lb));
-    const float2 qy = __fmul2_rn(__fmul2_rn(dy2, make_float2(lc, lc)), dy2);
-    const float2 o2 = make_float2(g1.y, g1.y);
-    const float2 q0 = __ffma2_rn(bx, make_float2(dy2.x, dy2.x), __fadd2_rn(qx, make_float2(qy.x, qy.x)));
-    const float2 q1 = __ffma2_rn(bx, make_float2(dy2.y, dy2.y), __fadd2_rn(qx, make_float2(qy.y, qy.y)));
-    const float2 a0 = __fmul2_rn(o2, make_float2(fast_ex2(q0.x), fast_ex2(q0.y)));
-    const float2 a1 = __fmul2_rn(o2, make_float2(fast_ex2(q1.x), fast_ex2(q1.y)));
-    dx[0] = dx2.x; dx[1] = dx2.y; dy[0] = dy2.x; dy[1] = dy2.y;
-    q[0] = q0.x; q[1] = q0.y; q[2] = q1.x; q[3] = q1.y;
-    ov[0] = a0.x; ov[1] = a0.y; ov[2] = a1.x; ov[3] = a1.y;
-  } else {
-    static_assert(P == 1, "the feature kernels use the <2,2> and <1,1> layouts");
-    dx[0] = __fadd_rn(g0.x, npx2.x);
-    dy[0] = __fadd_rn(g0.y, npy2.x);
-    const float qx = __fmul_rn(__fmul_rn(dx[0], la), dx[0]), bx = __fmul_rn(dx[0], lb);
-    const float qy = __fmul_rn(__fmul_rn(dy[0], lc), dy[0]);
-    q[0] = __fmaf_rn(bx, dy[0], __fadd_rn(qx, qy));
-    ov[0] = __fmul_rn(g1.y, fast_ex2(q[0]));
-  }
-}
-
 template <int CH>
 __global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_fwd_features_kernel(
     int64_t n_isects, const float4* __restrict__ splats, const int32_t* __restrict__ tile_offsets,
@@ -900,19 +778,9 @@ __global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_fwd_featur
   FeatStage<kBatch, CH>& fs = reinterpret_cast<FeatStage<kBatch, CH>*>(feat_smem)[threadIdx.x >> 5];
   WarpStage<kBatch>& st = fs.w;
   const int lane = threadIdx.x & 31;
-  const int ordered_tile =
-      tile_order != nullptr ? tile_order[(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] : -1;
-  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, ordered_tile);
-  const int nb = (wv.range_end - wv.range_start + kBatch - 1) / kBatch;
+  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, tile_order);
   const int64_t row_off = (int64_t)wv.cam * row_cam_stride;
 
-  float pxf[P], pyf[P];
-#pragma unroll
-  for (int i = 0; i < P; ++i) pxf[i] = opaque((float)(wv.x0 + i) + 0.5f);
-#pragma unroll
-  for (int i = 0; i < P; ++i) pyf[i] = opaque((float)(wv.y0 + i) + 0.5f);
-  const float2 npx2 = make_float2(-pxf[0], -pxf[P - 1]), npy2 = make_float2(-pyf[0], -pyf[P - 1]);
-  const float rx_lo = opaque(wv.rx_lo), rx_hi = opaque(wv.rx_hi), ry_lo = opaque(wv.ry_lo), ry_hi = opaque(wv.ry_hi);
   // T as in the RGB kernel: > 0 live, < 0 finished with final transmittance |T|
   float T[NP], col[NP][CH];
   int last[NP];
@@ -927,75 +795,40 @@ __global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_fwd_featur
     all_done = all_done && !inside;
   }
 
-  auto load_ids = [&](int b, int (&ids)[RPL]) {
+  if (wv.range_end > wv.range_start && !__all_sync(0xffffffffu, all_done)) {
+    stage_batches<false, false, RPL>(
+        st, splats, flatten_ids, wv.range_start, wv.range_end, lane, wv,
+        [&](int buf, int slot, int id) {
+          cp_async_row<CH>(&fs.feat[buf][slot * CH], features + ((int64_t)id - row_off) * feat_stride + c0);
+        },
+        [&](int b, int ns, int batch_start) {
+          const float4* s = st.rec[b & 1];
+          for (int t = 0; t < ns; ++t) {
+            if (__all_sync(0xffffffffu, all_done)) break;  // warp-uniform exit and reconvergence point
+            const int cur = st.list[t];
+            float dx[P], dy[P], q[NP], ov[NP];
+            splat_eval<P>(s[cur * 3 + 0], s[cur * 3 + 1], wv.npx2, wv.npy2, dx, dy, q, ov);
+            float f[CH];
+            load_row<CH>(f, &fs.feat[b & 1][cur * CH]);
+            float tmax = -1.0f;
 #pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      const int idx = wv.range_start + b * kBatch + r * 32 + lane;
-      ids[r] = (b < nb && idx < wv.range_end) ? __ldg(flatten_ids + idx) : -1;
-    }
-  };
-  auto issue = [&](int buf, const int (&ids)[RPL]) {
+            for (int j = 0; j < NP; ++j) {
+              // branch free: a rejected or finished pixel blends with weight 0 and keeps its T (as the RGB kernel)
+              const float alpha = fminf(kAlphaMax, ov[j]);
+              const float nT = __fmul_rn(T[j], __fmaf_rn(alpha, -1.f, 1.f));
+              const bool acc = T[j] > 0.f && q[j] <= 0.f && alpha >= kAlphaMin;
+              const bool bl = acc && nT > kTMin;
+              const float w = bl ? __fmul_rn(alpha, T[j]) : 0.f;
+              if (acc) T[j] = bl ? nT : -T[j];
+              if (bl) last[j] = batch_start + cur;
 #pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      if (ids[r] >= 0) {
-        const int slot = r * 32 + lane;
-        const float4* src = splats + (size_t)ids[r] * 3;
-        float4* dst = &st.rec[buf][slot * 3];
-        cp_async16(dst + 0, src + 0);
-        cp_async16(dst + 1, src + 1);
-        cp_async16(dst + 2, src + 2);
-        cp_async_row<CH>(&fs.feat[buf][slot * CH], features + ((int64_t)ids[r] - row_off) * feat_stride + c0);
-      }
-    }
-    cp_async_commit();
-  };
-
-  if (nb > 0 && !__all_sync(0xffffffffu, all_done)) {
-    int ids[RPL];
-    load_ids(0, ids);
-    issue(0, ids);
-    load_ids(1, ids);
-    for (int b = 0; b < nb; ++b) {
-      if (b + 1 < nb) {
-        issue((b + 1) & 1, ids);
-        load_ids(b + 2, ids);
-        cp_async_wait<1>();
-      } else {
-        cp_async_wait<0>();
-      }
-      __syncwarp();
-      const int batch_start = wv.range_start + b * kBatch;
-      const int batch_size = min(kBatch, wv.range_end - batch_start);
-      const int ns = cull_and_compact<RPL>(st, b & 1, batch_size, lane, rx_lo, rx_hi, ry_lo, ry_hi);
-      const float4* s = st.rec[b & 1];
-      for (int t = 0; t < ns; ++t) {
-        if (__all_sync(0xffffffffu, all_done)) break;  // warp-uniform exit and reconvergence point
-        const int cur = st.list[t];
-        float dx[P], dy[P], q[NP], ov[NP];
-        splat_eval<P>(s[cur * 3 + 0], s[cur * 3 + 1], npx2, npy2, dx, dy, q, ov);
-        float f[CH];
-        load_row<CH>(f, &fs.feat[b & 1][cur * CH]);
-        float tmax = -1.0f;
-#pragma unroll
-        for (int j = 0; j < NP; ++j) {
-          // branch free: a rejected or finished pixel blends with weight 0 and keeps its T (as the RGB kernel)
-          const float alpha = fminf(kAlphaMax, ov[j]);
-          const float nT = __fmul_rn(T[j], __fmaf_rn(alpha, -1.f, 1.f));
-          const bool acc = T[j] > 0.f && q[j] <= 0.f && alpha >= kAlphaMin;
-          const bool bl = acc && nT > kTMin;
-          const float w = bl ? __fmul_rn(alpha, T[j]) : 0.f;
-          if (acc) T[j] = bl ? nT : -T[j];
-          if (bl) last[j] = batch_start + cur;
-#pragma unroll
-          for (int k = 0; k < CH; ++k) col[j][k] = __fmaf_rn(f[k], w, col[j][k]);
-          tmax = fmaxf(tmax, T[j]);
-        }
-        all_done = !(tmax > 0.f);
-      }
-      if (__all_sync(0xffffffffu, all_done)) break;
-      __syncwarp();  // every lane is done with buffer b&1 and the list before they are overwritten
-    }
-    cp_async_wait<0>();
+              for (int k = 0; k < CH; ++k) col[j][k] = __fmaf_rn(f[k], w, col[j][k]);
+              tmax = fmaxf(tmax, T[j]);
+            }
+            all_done = !(tmax > 0.f);
+          }
+          return __all_sync(0xffffffffu, all_done);
+        });
   }
 
   const int nc = min(CH, D - c0);
@@ -1037,19 +870,9 @@ __global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_bwd_featur
   WarpStage<kBatch>& st = fs.w;
   float* red = reinterpret_cast<float*>(stages + G::kWarps) + (threadIdx.x >> 5) * (kFeatRedRows * kRedStride);
   const int lane = threadIdx.x & 31;
-  const int ordered_tile =
-      tile_order != nullptr ? tile_order[(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] : -1;
-  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, ordered_tile);
+  const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, tile_order);
   if (wv.range_end - wv.range_start <= 0) return;  // block-uniform
   const int64_t row_off = (int64_t)wv.cam * row_cam_stride;
-
-  float pxf[P], pyf[P];
-#pragma unroll
-  for (int i = 0; i < P; ++i) pxf[i] = opaque((float)(wv.x0 + i) + 0.5f);
-#pragma unroll
-  for (int i = 0; i < P; ++i) pyf[i] = opaque((float)(wv.y0 + i) + 0.5f);
-  const float2 npx2 = make_float2(-pxf[0], -pxf[P - 1]), npy2 = make_float2(-pyf[0], -pyf[P - 1]);
-  const float rx_lo = opaque(wv.rx_lo), rx_hi = opaque(wv.rx_hi), ry_lo = opaque(wv.ry_lo), ry_hi = opaque(wv.ry_hi);
 
   // replay state as in the RGB kernel: nbt_ = T_final * (v_alpha_out - bg . v_colour) - (colour behind) . v_colour,
   // over this chunk's channels; v_alpha_out only where the caller passes it (one chunk of a call)
@@ -1084,32 +907,6 @@ __global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_bwd_featur
   const int warp_last = __reduce_max_sync(0xffffffffu, my_last);
   const int end_idx = min(wv.range_end - 1, warp_last);
   if (end_idx < wv.range_start) return;  // warp-uniform
-  const int lo_idx = wv.range_start;
-  const int nb = (end_idx - lo_idx + 1 + kBatch - 1) / kBatch;
-
-  auto load_ids = [&](int b, int (&ids)[RPL]) {
-#pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      const int idx = end_idx - b * kBatch - (r * 32 + lane);
-      ids[r] = (b < nb && idx >= lo_idx) ? __ldg(flatten_ids + idx) : -1;
-    }
-  };
-  auto issue = [&](int buf, const int (&ids)[RPL]) {
-#pragma unroll
-    for (int r = 0; r < RPL; ++r) {
-      const int slot = r * 32 + lane;
-      if (ids[r] >= 0) {
-        const float4* src = splats + (size_t)ids[r] * 3;
-        float4* dst = &st.rec[buf][slot * 3];
-        cp_async16(dst + 0, src + 0);
-        cp_async16(dst + 1, src + 1);
-        cp_async16(dst + 2, src + 2);
-        cp_async_row<CH>(&fs.feat[buf][slot * CH], features + ((int64_t)ids[r] - row_off) * feat_stride + c0);
-      }
-      st.id[buf][slot] = ids[r];
-    }
-    cp_async_commit();
-  };
 
   // Warp sum in rounds of 16 values: lane 2k+p adds half p of row k, lane 2k issues the RED of value 16 r + k.
   // Value v < 8 goes to the gradient record (slots 0-5, then |v_x|, |v_y| in slots 9, 10; the r, g, b slots stay 0),
@@ -1126,109 +923,88 @@ __global__ void __launch_bounds__(FeatGeo<CH>::G::kThreads) rasterize_bwd_featur
     rec_off[r] = is_feat ? c0 + (v - 8) : (v < 6 ? v : v + 3);
   }
 
-  int ids[RPL];
-  load_ids(0, ids);
-  issue(0, ids);
-  load_ids(1, ids);
-  for (int b = 0; b < nb; ++b) {
-    if (b + 1 < nb) {
-      issue((b + 1) & 1, ids);
-      load_ids(b + 2, ids);
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncwarp();
-    const int batch_end = end_idx - b * kBatch;
-    const int batch_size = min(kBatch, batch_end + 1 - lo_idx);
-    const int ns = cull_and_compact<RPL>(st, b & 1, batch_size, lane, rx_lo, rx_hi, ry_lo, ry_hi);
-    const float4* s = st.rec[b & 1];
-    const int* sid = st.id[b & 1];
-    for (int t = 0; t < ns; ++t) {  // warp-uniform bounds
-      const int cur = st.list[t];
-      const int idx = batch_end - cur;
-      const float4 g0 = s[cur * 3 + 0];
-      const float4 g1 = s[cur * 3 + 1];
-      float dx[P], dy[P], q[NP], ov[NP];
-      splat_eval<P>(g0, g1, npx2, npy2, dx, dy, q, ov);
-      bool valid[NP];
-      bool any_valid = false;
+  stage_batches<true, true, RPL>(
+      st, splats, flatten_ids, end_idx, wv.range_start - 1, lane, wv,
+      [&](int buf, int slot, int id) {
+        cp_async_row<CH>(&fs.feat[buf][slot * CH], features + ((int64_t)id - row_off) * feat_stride + c0);
+      },
+      [&](int b, int ns, int batch_end) {
+        const float4* s = st.rec[b & 1];
+        const int* sid = st.id[b & 1];
+        for (int t = 0; t < ns; ++t) {  // warp-uniform bounds
+          const int cur = st.list[t];
+          const int idx = batch_end - cur;
+          const float4 g0 = s[cur * 3 + 0];
+          const float4 g1 = s[cur * 3 + 1];
+          float dx[P], dy[P], q[NP], ov[NP];
+          splat_eval<P>(g0, g1, wv.npx2, wv.npy2, dx, dy, q, ov);
+          bool valid[NP];
+          bool any_valid = false;
 #pragma unroll
-      for (int j = 0; j < NP; ++j) {
-        valid[j] = idx <= bin_final[j] && q[j] <= 0.f && ov[j] >= kAlphaMin;
-        any_valid = any_valid || valid[j];
-      }
-      if (!__any_sync(0xffffffffu, any_valid)) continue;  // warp-uniform
-      float f[CH];
-      load_row<CH>(f, &fs.feat[b & 1][cur * CH]);
-      const float inv_o = fast_rcp(g1.y);
-      // branch free as the RGB kernel: a pixel that does not take part has ov = 0, hence alpha = 0, 1 - alpha = 1,
-      // MUFU.RCP(1) = 1, and contributes exact zeros
-      float v[8], fac[NP];
+          for (int j = 0; j < NP; ++j) {
+            valid[j] = idx <= bin_final[j] && q[j] <= 0.f && ov[j] >= kAlphaMin;
+            any_valid = any_valid || valid[j];
+          }
+          if (!__any_sync(0xffffffffu, any_valid)) continue;  // warp-uniform
+          float f[CH];
+          load_row<CH>(f, &fs.feat[b & 1][cur * CH]);
+          const float inv_o = fast_rcp(g1.y);
+          // branch free as the RGB kernel: a pixel that does not take part has ov = 0, hence alpha = 0, 1 - alpha = 1,
+          // MUFU.RCP(1) = 1, and contributes exact zeros
+          float v[8], fac[NP];
 #pragma unroll
-      for (int k = 0; k < 8; ++k) v[k] = 0.f;
+          for (int k = 0; k < 8; ++k) v[k] = 0.f;
 #pragma unroll
-      for (int j = 0; j < NP; ++j) {
-        const float ddx = dx[j % P], ddy = dy[j / P];
-        const float ovj = valid[j] ? ov[j] : 0.f;
-        const float ae = fminf(kAlphaMax, ovj);
-        const float oe = ovj <= kAlphaMax ? ovj : 0.f;  // clamp inactive: alpha depends on sigma and opacity
-        const float ra = fast_rcp(fmaf(ae, -1.f, 1.f));
-        T[j] *= ra;  // transmittance in front of this Gaussian
-        fac[j] = ae * T[j];
-        float cdot = 0.f;
+          for (int j = 0; j < NP; ++j) {
+            const float ddx = dx[j % P], ddy = dy[j / P];
+            const float ovj = valid[j] ? ov[j] : 0.f;
+            const float ae = fminf(kAlphaMax, ovj);
+            const float oe = ovj <= kAlphaMax ? ovj : 0.f;  // clamp inactive: alpha depends on sigma and opacity
+            const float ra = fast_rcp(fmaf(ae, -1.f, 1.f));
+            T[j] *= ra;  // transmittance in front of this Gaussian
+            fac[j] = ae * T[j];
+            float cdot = 0.f;
 #pragma unroll
-        for (int k = 0; k < CH; ++k) cdot = fmaf(f[k], vc[j][k], cdot);
-        const float v_alpha = fmaf(T[j], cdot, ra * nbt_[j]);
-        nbt_[j] = fmaf(cdot, -fac[j], nbt_[j]);
-        const float w = oe * v_alpha;  // = -v_sigma
-        const float sx = -w * ddx, sy = -w * ddy;
-        v[2] = fmaf(sx, ddx, v[2]);
-        v[3] = fmaf(sx, ddy, v[3]);
-        v[4] = fmaf(sy, ddy, v[4]);
-        const float gx = fmaf(g0.w, sy, g0.z * sx);
-        const float gy = fmaf(g1.x, sy, g0.w * sx);
-        v[0] += gx;
-        v[1] += gy;
-        v[6] += fabsf(gx);
-        v[7] += fabsf(gy);
-        v[5] += w;
-      }
-      v[2] *= 0.5f; v[4] *= 0.5f; v[5] *= inv_o;
-      const int64_t fid = sid[cur];
+            for (int k = 0; k < CH; ++k) cdot = fmaf(f[k], vc[j][k], cdot);
+            const float v_alpha = fmaf(T[j], cdot, ra * nbt_[j]);
+            nbt_[j] = fmaf(cdot, -fac[j], nbt_[j]);
+            const float w = oe * v_alpha;  // = -v_sigma
+            const float sx = -w * ddx, sy = -w * ddy;
+            v[2] = fmaf(sx, ddx, v[2]);
+            v[3] = fmaf(sx, ddy, v[3]);
+            v[4] = fmaf(sy, ddy, v[4]);
+            const float gx = fmaf(g0.w, sy, g0.z * sx);
+            const float gy = fmaf(g1.x, sy, g0.w * sx);
+            v[0] += gx;
+            v[1] += gy;
+            v[6] += fabsf(gx);
+            v[7] += fabsf(gy);
+            v[5] += w;
+          }
+          v[2] *= 0.5f; v[4] *= 0.5f; v[5] *= inv_o;
+          const int64_t fid = sid[cur];
 #pragma unroll
-      for (int r = 0; r < kRounds; ++r) {
-        __syncwarp();  // the previous round's (or survivor's) row reads are complete
+          for (int r = 0; r < kRounds; ++r) {
+            float rv[kFeatRedRows];  // the round's values: geometry partials, then colour partials
 #pragma unroll
-        for (int i = 0; i < kFeatRedRows; ++i) {
-          const int vi = r * kFeatRedRows + i;
-          if (vi < 8) {
-            sts_f32(red_st + i * kRedStride * 4, v[vi]);
-          } else if (vi < kValues) {
-            float pf = 0.f;
+            for (int i = 0; i < kFeatRedRows; ++i) {
+              const int vi = r * kFeatRedRows + i;
+              rv[i] = 0.f;
+              if (vi < 8) {
+                rv[i] = v[vi];
+              } else if (vi < kValues) {
 #pragma unroll
-            for (int j = 0; j < NP; ++j) pf = fmaf(fac[j], vc[j][vi - 8], pf);
-            sts_f32(red_st + i * kRedStride * 4, pf);
+                for (int j = 0; j < NP; ++j) rv[i] = fmaf(fac[j], vc[j][vi - 8], rv[i]);
+              }
+            }
+            const bool feat_slot = r * kFeatRedRows + out_slot >= 8;
+            float* dst = feat_slot ? v_features + (fid - row_off) * feat_stride + rec_off[r]
+                                   : v_splats + fid * EGS_SPLAT_FLOATS + rec_off[r];
+            warp_sum_red(rv, min(kFeatRedRows, kValues - r * kFeatRedRows), red_st, row, red_flag[r], dst);
           }
         }
-        __syncwarp();
-        // rows past the round's last value hold stale data; no lane issues them
-        const float4 r0 = row[0], r1 = row[1], r2 = row[2], r3 = row[3];
-        float2 s0 = __fadd2_rn(make_float2(r0.x, r0.y), make_float2(r0.z, r0.w));
-        float2 s1 = __fadd2_rn(make_float2(r1.x, r1.y), make_float2(r1.z, r1.w));
-        float2 s2 = __fadd2_rn(make_float2(r2.x, r2.y), make_float2(r2.z, r2.w));
-        float2 s3 = __fadd2_rn(make_float2(r3.x, r3.y), make_float2(r3.z, r3.w));
-        s0 = __fadd2_rn(__fadd2_rn(s0, s1), __fadd2_rn(s2, s3));
-        float total = s0.x + s0.y;
-        total += __shfl_xor_sync(0xffffffffu, total, 1);
-        const bool feat_slot = r * kFeatRedRows + out_slot >= 8;
-        float* dst = feat_slot ? v_features + (fid - row_off) * feat_stride + rec_off[r]
-                               : v_splats + fid * EGS_SPLAT_FLOATS + rec_off[r];
-        red_add_f32_if(red_flag[r], dst, total);
-      }
-    }
-    __syncwarp();  // buffer b&1, its ids and the list are free again
-  }
+        return false;
+      });
 }
 
 }  // namespace egs
@@ -1247,12 +1023,11 @@ static int check_raster_args(const char* who, int32_t C, int64_t n_isects, int32
   return 0;
 }
 
-// Every tile is handled by the <2,2> layout.  A second launch with the 8-warps-per-tile <1,1> layout for very long
+// The RGB kernels handle every tile in the <2,2> layout.  A second launch with the 8-warps-per-tile <1,1> layout for very long
 // lists was measured twice (round 1: object scene, 4 views per call: forward 0.48 -> 0.42 ms, backward 0.59 -> 0.72 ms;
 // round 2, one view per call: 1.224 -> 1.225 ms per view, gpurun_out/r2c_knobs.log) and is no longer built: the busy
 // tiles of an object scene are bound by their serial walk, and eight warps that each cull the whole list do 1.5 x the
 // instructions of two.
-constexpr int kNoLengthLimit = 0x7fffffff;
 
 template <bool COUNT>
 static int launch_fwd(int32_t C, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
@@ -1266,9 +1041,9 @@ static int launch_fwd(int32_t C, int64_t n_isects, const float* splats, const in
   const float4* sp = reinterpret_cast<const float4*>(splats);
   unsigned long long* pc = reinterpret_cast<unsigned long long*>(pair_counters);
   cudaStream_t st = (cudaStream_t)stream;
-  rasterize_fwd_kernel<2, 2, COUNT><<<grid, Geo<2, 2>::kThreads, 0, st>>>(
-      n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles, 0,
-      kNoLengthLimit, render_colors, render_alphas, last_ids, pc, ck, segment, seg_min_len > segment ? seg_min_len : segment + 1,
+  rasterize_fwd_kernel<COUNT><<<grid, Geo<2, 2>::kThreads, 0, st>>>(
+      n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles,
+      render_colors, render_alphas, last_ids, pc, ck, segment, seg_min_len > segment ? seg_min_len : segment + 1,
       tile_order);
   return check_launch("rasterize_fwd_kernel");
 }
@@ -1338,18 +1113,17 @@ static int launch_bwd(int32_t C, int64_t n_isects, const float* splats, const in
   seg_min_len = seg_min_len > segment ? seg_min_len : segment + 1;
   dim3 grid(tile_width, tile_height, C);
   const int n_tiles = C * tile_width * tile_height;
-  const int thr = kNoLengthLimit;
   const float4* sp = reinterpret_cast<const float4*>(splats);
   const float4* ck = segment > 0 ? reinterpret_cast<const float4*>(checkpoints) : nullptr;
   cudaStream_t st = (cudaStream_t)stream;
   // the segment launch goes first: its warps all have full segments to replay, the tile launch then fills in
   const int64_t n_slots = ck != nullptr ? (n_isects < 0 ? -n_isects : n_isects) / segment : 0;
   if (n_slots > 0)
-    rasterize_bwd_kernel<2, 2><<<(unsigned)n_slots, Geo<2, 2>::kThreads, 0, st>>>(
-        n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles, 0, thr,
+    rasterize_bwd_kernel<<<(unsigned)n_slots, Geo<2, 2>::kThreads, 0, st>>>(
+        n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles,
         render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, render_colors, ck, segment, seg_min_len, 1, nullptr);
-  rasterize_bwd_kernel<2, 2><<<grid, Geo<2, 2>::kThreads, 0, st>>>(
-      n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles, 0, thr,
+  rasterize_bwd_kernel<<<grid, Geo<2, 2>::kThreads, 0, st>>>(
+      n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles,
       render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, render_colors, ck, segment, seg_min_len, 0, tile_order);
   return check_launch("rasterize_bwd_kernel", 1 + (n_slots > 0 ? 1 : 0));
 }
