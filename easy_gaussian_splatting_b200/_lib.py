@@ -38,6 +38,11 @@ _SIGNATURES = {
                                               P, P, P, P, P, P, I32, P, P, I64, P]),
     "egs_projection_bwd_raw_viewmats": (c_int32, [I32, I32, P, P, P, P, P, P, I32, P, P, I32, I32, F32, P, P, P, P,
                                                   P, P, P, P, P, P, P, P, P, I64, P]),
+    "egs_projection_bwd_intrinsics_workspace_bytes": (c_int64, [I32, I32]),
+    "egs_projection_bwd_intrinsics": (c_int32, [I32, I32, P, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, P, P, P,
+                                                P, P, P, P, P, P, P, I32, P, P, P, I64, P]),
+    "egs_projection_bwd_raw_intrinsics": (c_int32, [I32, I32, P, P, P, P, P, P, I32, P, P, I32, I32, F32, P, P, P, P,
+                                                    P, P, P, P, P, P, P, P, P, P, I64, P]),
     "egs_exclusive_scan_workspace_bytes": (c_int64, [I64]),
     "egs_exclusive_scan": (c_int32, [I64, P, P, P, P, I64, P]),
     "egs_isect_emit": (c_int32, [I32, I32, P, P, P, P, I32, I32, I32, I32, I64, P, P, P]),

@@ -246,15 +246,19 @@ EGS_HD void pack_tile_rect(int32_t x0, int32_t y0, int32_t x1, int32_t y1, int32
 // Camera gradient of one (camera, Gaussian) pair, 15 floats: v_R[9] (row major) and v_t[3] of the view matrix's
 // top 3x4 block, then v_campos[3], the gradient w.r.t. the camera centre the SH directions are taken from.
 constexpr int kCamGradFloats = 15;
+// Intrinsics gradient of one (camera, Gaussian) pair, 4 floats: v_fx, v_fy, v_cx, v_cy.
+constexpr int kKsGradFloats = 4;
 
 // VJP of project_fwd for a visible Gaussian (SURVEY.md A-8).  Accumulates (+=) into
 // v_mean[3], v_quat[4], v_scale[3].
 // v_cam (nullable, with the Gaussian's world-space mean): also accumulates v_R and v_t (entries 0..11 of the camera
 // gradient above) through mean_c = R m + t and cov_c = R Sigma R^T.  A literal nullptr compiles the block out.
+// v_K (nullable): also accumulates the intrinsics gradient above through means2d and the Jacobian J (which carries the
+// conic's and the compensation's cotangents).  A literal nullptr compiles the block out.
 EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera& cam, float v_m2x, float v_m2y,
                         float v_depth, float v_ca, float v_cb, float v_cc, const ProjOut& o, float v_mean[3],
                         float v_quat[4], float v_scale[3], float v_comp = 0.f, float eps2d = 0.f,
-                        float* v_cam = nullptr, const float* mean = nullptr) {
+                        float* v_cam = nullptr, const float* mean = nullptr, float* v_K = nullptr) {
   // conic = inverse(cov2d'):  V = -Q * G * Q with G = [[v_ca, v_cb/2],[v_cb/2, v_cc]]
   float q00 = o.ca, q01 = o.cb, q11 = o.cc;
   float g00 = v_ca, g01 = 0.5f * v_cb, g11 = v_cc;
@@ -290,6 +294,18 @@ EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera&
   float vJ12 = 2.f * (VJ10 * k[2] + VJ11 * k[4] + VJ12 * k[5]);
   float fx = cam.fx, fy = cam.fy, rz = st.rz, rz2 = st.rz2, rz3 = st.rz2 * st.rz;
   float x = st.x, y = st.y;
+  if (v_K != nullptr) {
+    // mean2d = (fx x rz + cx, fy y rz + cy); J00 = fx rz; J02 = -fx tx rz^2 depends on fx only while the fov clamp is
+    // off (clamped, fx tx = z * 1.3 * 0.5 * width does not); likewise for y
+    float vfx = v_m2x * x * rz + vJ00 * rz;
+    float vfy = v_m2y * y * rz + vJ11 * rz;
+    if (!st.clamp_x) vfx -= vJ02 * st.tx * rz2;
+    if (!st.clamp_y) vfy -= vJ12 * st.ty * rz2;
+    v_K[0] += vfx;
+    v_K[1] += vfy;
+    v_K[2] += v_m2x;
+    v_K[3] += v_m2y;
+  }
   // mean2d = (fx x rz + cx, fy y rz + cy); depth = z
   float vx = fx * rz * v_m2x;
   float vy = fy * rz * v_m2y;
@@ -539,6 +555,14 @@ EGS_HD void viewmat_grad_finalize(const float* V, const float vcam[kCamGradFloat
     out[12 + i] = -(cg * c[i]);
   }
   out[15] = -cg;
+}
+
+// The [3,3] gradient of one K from its intrinsics gradient summed over the Gaussians (v_fx, v_fy, v_cx, v_cy, see
+// project_bwd).  The projection reads no other entry, so the skew and the last row get 0.
+EGS_HD void ks_grad_finalize(const float vk[kKsGradFloats], float out[9]) {
+  out[0] = vk[0]; out[1] = 0.f;   out[2] = vk[2];
+  out[3] = 0.f;   out[4] = vk[1]; out[5] = vk[3];
+  out[6] = 0.f;   out[7] = 0.f;   out[8] = 0.f;
 }
 
 }  // namespace egs

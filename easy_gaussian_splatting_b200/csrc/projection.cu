@@ -160,7 +160,8 @@ struct ProjBwdParams {
   float2* absgrad;  // nullable [C,N]: sum over pixels of |d L / d means2d|, copied out of the gradient records
   // viewmat gradients (the VG instantiations only): per camera, one 16-float partial of the camera gradient
   // (egs_math.cuh kCamGradFloats, padded) per warp of the launch, camera-major: [C][gridDim.x * 4][16]; the counters
-  // [C] of viewmat_grad_finalize_kernel are cleared by block 0
+  // [C] of viewmat_grad_finalize_kernel are cleared by block 0.  The egs::ksgrad kernels store 20-float partials
+  // (kCamGradFloats + kKsGradFloats, padded) for intrinsics_grad_finalize_kernel.
   float* cam_partials;
   int* cam_counters;
 };
@@ -173,6 +174,9 @@ constexpr int kMaxCamerasSmem = 64;
 // with a fixed shuffle tree and lane 0 stores the warp's partial; viewmat_grad_finalize_kernel then sums the partials
 // in a fixed order.  No float atomics anywhere: the same gradient records give bit-identical v_viewmats.
 constexpr int kCamPartialFloats = 16;
+// With intrinsics gradients (the egs::ksgrad kernels) a partial is 15 + 4 floats, padded to 20.
+constexpr int kCamKsGradFloats = kCamGradFloats + kKsGradFloats;
+constexpr int kCamKsPartialFloats = 20;
 constexpr int kVgFinalizeThreads = 256;
 constexpr int kVgMaxSlices = 32;
 
@@ -206,9 +210,34 @@ __device__ __forceinline__ void store_cam_partial(float (&v)[kCamGradFloats], bo
   }
 }
 
+// The same with the intrinsics gradient: 19 floats, stored as 20.
+__device__ __forceinline__ void store_cam_partial(float (&v)[kCamKsGradFloats], bool any, float* __restrict__ dst, int lane) {
+  if (any) {
+#pragma unroll
+    for (int k = 0; k < kCamKsGradFloats; ++k)
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) v[k] += __shfl_down_sync(0xffffffffu, v[k], off);
+  }
+  if (lane == 0) {
+    float4* d = reinterpret_cast<float4*>(dst);
+    if (any) {
+      d[0] = make_float4(v[0], v[1], v[2], v[3]);
+      d[1] = make_float4(v[4], v[5], v[6], v[7]);
+      d[2] = make_float4(v[8], v[9], v[10], v[11]);
+      d[3] = make_float4(v[12], v[13], v[14], v[15]);
+      d[4] = make_float4(v[16], v[17], v[18], 0.f);
+    } else {
+      const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+      d[0] = z; d[1] = z; d[2] = z; d[3] = z; d[4] = z;
+    }
+  }
+}
+
+// Partial of warp `warp` of this block for camera c; kStride floats per partial.
+template <int kStride>
 __device__ __forceinline__ float* cam_partial(const ProjBwdParams& p, int c, int warp) {
   const size_t slots = (size_t)gridDim.x * 4;
-  return p.cam_partials + ((size_t)c * slots + (size_t)blockIdx.x * 4 + warp) * kCamPartialFloats;
+  return p.cam_partials + ((size_t)c * slots + (size_t)blockIdx.x * 4 + warp) * kStride;
 }
 
 __device__ __forceinline__ void clear_cam_counters(const ProjBwdParams& p) {
@@ -271,6 +300,70 @@ __global__ void __launch_bounds__(kVgFinalizeThreads) viewmat_grad_finalize_kern
   }
 }
 
+// As viewmat_grad_finalize_kernel, for the 20-float partials of the egs::ksgrad kernels: writes v_Ks[c] (9 floats) and,
+// when v_viewmats is not null, v_viewmats[c] (16 floats).
+__global__ void __launch_bounds__(kVgFinalizeThreads) intrinsics_grad_finalize_kernel(
+    int n_slots, const float* __restrict__ partials, float* __restrict__ slices, int* __restrict__ counters,
+    const float* __restrict__ viewmats, float* __restrict__ v_viewmats, float* __restrict__ v_Ks) {
+  __shared__ float red[kCamKsGradFloats][kVgFinalizeThreads];
+  __shared__ bool last;
+  const int s = blockIdx.x, S = gridDim.x, c = blockIdx.y, tid = threadIdx.x;
+  const int per = (n_slots + S - 1) / S;
+  const int begin = s * per, end = min(n_slots, begin + per);
+  float acc[kCamKsGradFloats];
+#pragma unroll
+  for (int k = 0; k < kCamKsGradFloats; ++k) acc[k] = 0.f;
+  const float4* src = reinterpret_cast<const float4*>(partials + (size_t)c * n_slots * kCamKsPartialFloats);
+  for (int i = begin + tid; i < end; i += kVgFinalizeThreads) {
+    const float4* q = src + (size_t)i * (kCamKsPartialFloats / 4);
+    const float4 a = q[0], b = q[1], d = q[2], e = q[3], f = q[4];
+    acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
+    acc[4] += b.x; acc[5] += b.y; acc[6] += b.z; acc[7] += b.w;
+    acc[8] += d.x; acc[9] += d.y; acc[10] += d.z; acc[11] += d.w;
+    acc[12] += e.x; acc[13] += e.y; acc[14] += e.z; acc[15] += e.w;
+    acc[16] += f.x; acc[17] += f.y; acc[18] += f.z;
+  }
+#pragma unroll
+  for (int k = 0; k < kCamKsGradFloats; ++k) red[k][tid] = acc[k];
+  __syncthreads();
+  for (int h = kVgFinalizeThreads / 2; h > 0; h >>= 1) {
+    if (tid < h)
+#pragma unroll
+      for (int k = 0; k < kCamKsGradFloats; ++k) red[k][tid] += red[k][tid + h];
+    __syncthreads();
+  }
+  float* my_slice = slices + ((size_t)c * S + s) * kCamKsPartialFloats;
+  if (tid < kCamKsGradFloats) my_slice[tid] = red[tid][0];
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) last = atomicAdd(counters + c, 1) == S - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  if (tid < kCamKsGradFloats) {
+    float sum = 0.f;
+    for (int j = 0; j < S; ++j) sum += __ldcg(slices + ((size_t)c * S + j) * kCamKsPartialFloats + tid);
+    red[tid][0] = sum;
+  }
+  __syncthreads();
+  if (tid == 0) {
+    float vcam[kCamGradFloats], vk[kKsGradFloats], out[16], kout[9];
+#pragma unroll
+    for (int k = 0; k < kCamGradFloats; ++k) vcam[k] = red[k][0];
+#pragma unroll
+    for (int k = 0; k < kKsGradFloats; ++k) vk[k] = red[kCamGradFloats + k][0];
+    if (v_viewmats != nullptr) {
+      viewmat_grad_finalize(viewmats + (size_t)c * 16, vcam, out);
+#pragma unroll
+      for (int k = 0; k < 16; ++k) v_viewmats[(size_t)c * 16 + k] = out[k];
+    }
+    ks_grad_finalize(vk, kout);
+#pragma unroll
+    for (int k = 0; k < 9; ++k) v_Ks[(size_t)c * 9 + k] = kout[k];
+    counters[c] = 0;
+  }
+}
+
 // Store one SH gradient row of `total` = K * 3 floats: the 48 of bands 0..3 from registers, zeros past them.
 template <bool VEC4>
 __device__ __forceinline__ void store_coeff_grads(float* __restrict__ out, int total, const float (&vco)[48]) {
@@ -311,8 +404,9 @@ constexpr int kPB2Warps = kPB2Threads / 32;
 #define EGS_PB_MIN_CTAS 3
 #endif
 // The per-camera-SH form with viewmat gradients holds the camera gradient and the staged rows' loop state at once: it
-// runs 2 CTAs per SM (255 registers) instead of spilling at 168.
-#define EGS_PB_BOUNDS(PER_CAMERA_VG) __launch_bounds__(kPB2Threads, (PER_CAMERA_VG) ? 2 : EGS_PB_MIN_CTAS)
+// runs 2 CTAs per SM (255 registers) instead of spilling at 168.  So do the forms with intrinsics gradients, whose 4
+// more accumulators spill the classic form at 168.
+#define EGS_PB_BOUNDS(TWO_CTAS) __launch_bounds__(kPB2Threads, (TWO_CTAS) ? 2 : EGS_PB_MIN_CTAS)
 
 // Per-camera SH rows of a warp's 32 Gaussians (rows of camera c start at (c * N + n_base) * 48 floats), copied in and
 // out with the same coalesced float4 pattern as the shared rows.
@@ -348,12 +442,25 @@ __device__ __forceinline__ void store_sh_grad_rows(float* __restrict__ tile, flo
 }
 
 constexpr bool kPerCameraSh = false;
+constexpr bool kKsGrad = false;
 #include "projection_kernels.cuh"
 
 namespace percam {
 constexpr bool kPerCameraSh = true;
 #include "projection_kernels.cuh"
 }  // namespace percam
+
+// Intrinsics gradients: only the VG forms of the backward kernels are instantiated here.  They are separate kernels so
+// that the pose-only forms keep their registers (the classic sh16 one sits at the 168-register cap of 3 CTAs/SM).
+namespace ksgrad {
+constexpr bool kKsGrad = true;
+#include "projection_bwd_kernels.cuh"
+
+namespace percam {
+constexpr bool kPerCameraSh = true;
+#include "projection_bwd_kernels.cuh"
+}  // namespace percam
+}  // namespace ksgrad
 
 }  // namespace egs
 
@@ -457,15 +564,24 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
                                const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
                                float* v_scales, float* v_opacities, float* v_sh_coeffs, float* v_sh_rest, float* absgrad,
                                egs_stream_t stream, int antialiased = 0, float* v_viewmats = nullptr,
-                               void* workspace = nullptr, int64_t workspace_bytes = 0) {
+                               void* workspace = nullptr, int64_t workspace_bytes = 0, float* v_Ks = nullptr) {
   const int raw = sh_rest != nullptr;
   EGS_REQUIRE(C >= 0 && N >= 0, "projection_bwd: negative sizes C=%d N=%d", C, N);
   EGS_REQUIRE(sh_degree <= 3, "projection_bwd: sh_degree %d > 3 is not supported", sh_degree);
   EGS_REQUIRE(sh_degree < 0 || K >= (sh_degree + 1) * (sh_degree + 1), "projection_bwd: K=%d too small for sh_degree=%d", K, sh_degree);
   EGS_REQUIRE(colors_per_camera == 0 || colors_per_camera == 1, "projection_bwd: colors_per_camera=%d must be 0 or 1",
               colors_per_camera);
-  const bool vg = v_viewmats != nullptr;
-  if (vg) {
+  const bool kg = v_Ks != nullptr;              // intrinsics gradients: the egs::ksgrad kernels, 20-float partials
+  const bool vg = kg || v_viewmats != nullptr;  // camera-gradient partials and a finalize launch
+  if (kg) {
+    EGS_REQUIRE(C <= 65535, "projection_bwd: C=%d exceeds 65535 cameras per call", C);
+    EGS_REQUIRE(workspace != nullptr && workspace_bytes >= egs_projection_bwd_intrinsics_workspace_bytes(C, N),
+                "projection_bwd: intrinsics gradients need %lld workspace bytes (got %lld)",
+                (long long)egs_projection_bwd_intrinsics_workspace_bytes(C, N), (long long)workspace_bytes);
+    if (N == 0 && C > 0) EGS_CUDA(cudaMemsetAsync(v_Ks, 0, sizeof(float) * 9 * (size_t)C, (cudaStream_t)stream));
+    if (N == 0 && C > 0 && v_viewmats != nullptr)
+      EGS_CUDA(cudaMemsetAsync(v_viewmats, 0, sizeof(float) * 16 * (size_t)C, (cudaStream_t)stream));
+  } else if (vg) {
     EGS_REQUIRE(C <= 65535, "projection_bwd: C=%d exceeds 65535 cameras per call", C);
     EGS_REQUIRE(workspace != nullptr && workspace_bytes >= egs_projection_bwd_viewmats_workspace_bytes(C, N),
                 "projection_bwd: viewmat gradients need %lld workspace bytes (got %lld)",
@@ -486,15 +602,21 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
   p.cam_partials = nullptr; p.cam_counters = nullptr;
   EGS_REQUIRE(!antialiased || opacities_raw != nullptr, "projection_bwd: antialiased mode needs the opacities");
   const int64_t vg_slots = vg_partial_slots(N);
+  const int partial_floats = kg ? kCamKsPartialFloats : kCamPartialFloats;
   if (vg) {
     p.cam_partials = static_cast<float*>(workspace);
-    p.cam_counters = reinterpret_cast<int*>(p.cam_partials + (size_t)(C * vg_slots + C * vg_slices(vg_slots)) * kCamPartialFloats);
+    p.cam_counters = reinterpret_cast<int*>(p.cam_partials + (size_t)(C * vg_slots + C * vg_slices(vg_slots)) * partial_floats);
   }
-  // viewmat_grad_finalize_kernel, after either backward kernel
+  // viewmat_grad_finalize_kernel / intrinsics_grad_finalize_kernel, after either backward kernel
   auto finalize = [&]() -> int {
     if (C == 0) return 0;
     const int S = vg_slices(vg_slots);
-    float* slices = p.cam_partials + (size_t)C * vg_slots * kCamPartialFloats;
+    float* slices = p.cam_partials + (size_t)C * vg_slots * partial_floats;
+    if (kg) {
+      intrinsics_grad_finalize_kernel<<<dim3((unsigned)S, (unsigned)C), kVgFinalizeThreads, 0, (cudaStream_t)stream>>>(
+          (int)vg_slots, p.cam_partials, slices, p.cam_counters, viewmats, v_viewmats, v_Ks);
+      return check_launch("intrinsics_grad_finalize_kernel");
+    }
     viewmat_grad_finalize_kernel<<<dim3((unsigned)S, (unsigned)C), kVgFinalizeThreads, 0, (cudaStream_t)stream>>>(
         (int)vg_slots, p.cam_partials, slices, p.cam_counters, viewmats, v_viewmats);
     return check_launch("viewmat_grad_finalize_kernel");
@@ -509,7 +631,11 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
   if (raw || (vec4 && K == 16)) {
     // the reference's layout (K = 16): coalesced shared-memory staged rows
     constexpr int kSmem = 2 * kPB2Warps * 32 * kRowStride * (int)sizeof(float);
-    auto kern = pc ? (vg ? (antialiased ? percam::projection_bwd_sh16_kernel<true, true> : percam::projection_bwd_sh16_kernel<false, true>)
+    auto kern = kg ? (pc ? (antialiased ? ksgrad::percam::projection_bwd_sh16_kernel<true, true>
+                                        : ksgrad::percam::projection_bwd_sh16_kernel<false, true>)
+                         : (antialiased ? ksgrad::projection_bwd_sh16_kernel<true, true>
+                                        : ksgrad::projection_bwd_sh16_kernel<false, true>))
+              : pc ? (vg ? (antialiased ? percam::projection_bwd_sh16_kernel<true, true> : percam::projection_bwd_sh16_kernel<false, true>)
                          : (antialiased ? percam::projection_bwd_sh16_kernel<true> : percam::projection_bwd_sh16_kernel<false>))
                    : vg ? (antialiased ? projection_bwd_sh16_kernel<true, true> : projection_bwd_sh16_kernel<false, true>)
                         : (antialiased ? projection_bwd_sh16_kernel<true> : projection_bwd_sh16_kernel<false>);
@@ -521,6 +647,13 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
     return (rc != 0 || !vg) ? rc : finalize();
   }
   unsigned grid = (unsigned)ceil_div(N, kProjBwdThreads);
+  if (kg) {
+    auto kern = pc ? (vec4 ? ksgrad::percam::projection_bwd_kernel<true, true> : ksgrad::percam::projection_bwd_kernel<false, true>)
+                   : (vec4 ? ksgrad::projection_bwd_kernel<true, true> : ksgrad::projection_bwd_kernel<false, true>);
+    kern<<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
+    const int rc = check_launch("projection_bwd_kernel");
+    return rc != 0 ? rc : finalize();
+  }
   if (pc) {
     auto kern = vg ? (vec4 ? percam::projection_bwd_kernel<true, true> : percam::projection_bwd_kernel<false, true>)
                    : (vec4 ? percam::projection_bwd_kernel<true> : percam::projection_bwd_kernel<false>);
@@ -614,4 +747,44 @@ extern "C" int egs_projection_bwd_raw_viewmats(
                              Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means, v_quats,
                              v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream, 0, v_viewmats,
                              workspace, workspace_bytes);
+}
+
+/* ---- gradients w.r.t. the intrinsics ---- */
+extern "C" int64_t egs_projection_bwd_intrinsics_workspace_bytes(int32_t C, int32_t N) {
+  if (C <= 0 || N < 0) return 0;
+  const int64_t slots = vg_partial_slots(N);
+  return (int64_t)C * (slots + vg_slices(slots)) * kCamKsPartialFloats * (int64_t)sizeof(float) +
+         (int64_t)C * (int64_t)sizeof(int);
+}
+
+extern "C" int egs_projection_bwd_intrinsics(
+    int32_t C, int32_t N, const float* means, const float* quats, const float* scales, const float* opacities,
+    const float* sh_coeffs, int32_t K, int32_t sh_degree, int32_t colors_per_camera, const float* viewmats,
+    const float* Ks, int32_t width, int32_t height, float eps2d, const int32_t* radii, const float* colors,
+    const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats, float* v_scales,
+    float* v_opacities, float* v_sh_coeffs, float* absgrad, int32_t antialiased, float* v_viewmats, float* v_Ks,
+    void* workspace, int64_t workspace_bytes, egs_stream_t stream) {
+  EGS_REQUIRE(v_Ks != nullptr, "projection_bwd_intrinsics: v_Ks output is required");
+  return projection_bwd_impl(C, N, means, quats, scales, antialiased ? opacities : nullptr, sh_coeffs, nullptr, K,
+                             sh_degree, colors_per_camera, viewmats, Ks, width, height, eps2d, radii, colors, v_splats,
+                             v_means2d_extra, v_means, v_quats, v_scales, v_opacities, v_sh_coeffs, nullptr, absgrad,
+                             stream, antialiased ? 1 : 0, v_viewmats, workspace, workspace_bytes, v_Ks);
+}
+
+extern "C" int egs_projection_bwd_raw_intrinsics(
+    int32_t C, int32_t N, const float* means, const float* quats, const float* log_scales, const float* logit_opacities,
+    const float* sh_0, const float* sh_rest, int32_t sh_degree, const float* viewmats, const float* Ks, int32_t width,
+    int32_t height, float eps2d, const int32_t* radii, const float* colors, const float* v_splats,
+    const float* v_means2d_extra, float* v_means, float* v_quats, float* v_log_scales, float* v_logit_opacities,
+    float* v_sh_0, float* v_sh_rest, float* absgrad, float* v_viewmats, float* v_Ks, void* workspace,
+    int64_t workspace_bytes, egs_stream_t stream) {
+  EGS_REQUIRE(v_Ks != nullptr, "projection_bwd_raw_intrinsics: v_Ks output is required");
+  EGS_REQUIRE(sh_rest != nullptr && sh_0 != nullptr, "projection_bwd_raw: sh_0 and sh_rest are required");
+  EGS_REQUIRE(reinterpret_cast<uintptr_t>(sh_0) % 16 == 0 && reinterpret_cast<uintptr_t>(sh_rest) % 16 == 0 &&
+                  reinterpret_cast<uintptr_t>(v_sh_0) % 16 == 0 && reinterpret_cast<uintptr_t>(v_sh_rest) % 16 == 0,
+              "projection_bwd_raw: sh_0 / sh_rest and their gradients must be 16-byte aligned");
+  return projection_bwd_impl(C, N, means, quats, log_scales, logit_opacities, sh_0, sh_rest, 16, sh_degree, 0, viewmats,
+                             Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means, v_quats,
+                             v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream, 0, v_viewmats,
+                             workspace, workspace_bytes, v_Ks);
 }

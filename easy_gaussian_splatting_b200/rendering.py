@@ -244,24 +244,42 @@ class _Rasterization(torch.autograd.Function):
                                        render_alphas, last_ids, v_colors, v_alphas, ckpt)
         ref = getattr(ctx, "means2d_ref", None) if cfg["absgrad"] else None
         target = ref() if ref is not None else None
-        # the viewmat keyword is passed only when its gradient is wanted: without it the call is exactly the classic one
-        want_vm = {"want_viewmats_grad": True} if ctx.needs_input_grad[5] else {}
+        # the camera keywords are passed only when their gradients are wanted: without them the call is exactly the
+        # classic one
+        want_cam = _camera_grad_keywords(ctx.needs_input_grad[5], ctx.needs_input_grad[6])
         with stages.nvtx_range("egs.projection_bwd"):
             out = stages.projection_bwd(means, quats, scales, colors, viewmats, Ks, width, height, cfg["sh_degree"],
                                         cfg["eps2d"], radii, colors_rgb, v_splats, v_means2d, want_absgrad=target is not None,
                                         antialiased_opacities=opacities if cfg["antialiased"] else None, opacities=opacities,
-                                        **want_vm)
+                                        **want_cam)
         v_means, v_quats, v_scales, v_opac, v_cols = out[:5]
         if feat:
             v_cols = v_features
-        v_viewmats = out[-1] if want_vm else None
+        v_viewmats, v_Ks = _camera_grads(out, want_cam)
         if target is not None:
             # same contract as gsplat: attribute tagging on the tensor object handed out in meta
             _tag_absgrad(target, out[5], getattr(ctx, "packed_index", None))
         v_bg = None
         if backgrounds is not None and ctx.needs_input_grad[7]:
             v_bg = ((1.0 - render_alphas) * v_colors).sum(dim=(1, 2))
-        return v_means, v_quats, v_scales, v_opac, v_cols, v_viewmats, None, v_bg, None
+        return v_means, v_quats, v_scales, v_opac, v_cols, v_viewmats, v_Ks, v_bg, None
+
+
+def _camera_grad_keywords(want_viewmats: bool, want_Ks: bool) -> Dict[str, bool]:
+    """The keywords of the projection backward stages for the camera gradients that are wanted (none: {})."""
+    kw = {}
+    if want_viewmats:
+        kw["want_viewmats_grad"] = True
+    if want_Ks:
+        kw["want_Ks_grad"] = True
+    return kw
+
+
+def _camera_grads(out: tuple, kw: Dict[str, bool]) -> Tuple[Optional[Tensor], Optional[Tensor]]:
+    """(v_viewmats, v_Ks) from the end of a projection backward stage's outputs; None for those not requested."""
+    v_Ks = out[-1] if "want_Ks_grad" in kw else None
+    v_viewmats = out[-2 if v_Ks is not None else -1] if "want_viewmats_grad" in kw else None
+    return v_viewmats, v_Ks
 
 
 class _RasterizationRaw(torch.autograd.Function):
@@ -309,17 +327,17 @@ class _RasterizationRaw(torch.autograd.Function):
                                    render_alphas, last_ids, v_colors, v_alphas, ckpt)
         ref = getattr(ctx, "means2d_ref", None) if cfg["absgrad"] else None
         target = ref() if ref is not None else None
-        want_vm = {"want_viewmats_grad": True} if ctx.needs_input_grad[6] else {}
+        want_cam = _camera_grad_keywords(ctx.needs_input_grad[6], ctx.needs_input_grad[7])
         out = stages.projection_bwd_raw(means, quats, log_scales, logit_opacities, sh_0, sh_rest, viewmats, Ks, width,
                                         height, cfg["sh_degree"], cfg["eps2d"], radii, colors_rgb, v_splats, v_means2d,
-                                        want_absgrad=target is not None, **want_vm)
-        v_viewmats = out[-1] if want_vm else None
+                                        want_absgrad=target is not None, **want_cam)
+        v_viewmats, v_Ks = _camera_grads(out, want_cam)
         if target is not None:
             _tag_absgrad(target, out[6], None)
         v_bg = None
         if backgrounds is not None and ctx.needs_input_grad[8]:
             v_bg = ((1.0 - render_alphas) * v_colors).sum(dim=(1, 2))
-        return (*out[:6], v_viewmats, None, v_bg, None)
+        return (*out[:6], v_viewmats, v_Ks, v_bg, None)
 
 
 def _check_inputs(means, quats, scales, opacities, colors, viewmats, Ks, sh_degree, backgrounds):
@@ -395,7 +413,10 @@ def rasterization(
     ``absgrad=True``, one camera, a [1,3] background — and C > 1 are implemented; modes the
     reference never requests raise ``NotImplementedError`` instead of silently approximating.
     As in gsplat, ``viewmats`` receive a gradient when they require one (camera pose refinement: projection and SH
-    view directions, campos = inverse(viewmats)[:, :3, 3]); ``Ks`` receive none.
+    view directions, campos = inverse(viewmats)[:, :3, 3]).  Beyond gsplat 1.0.0, which gives ``Ks`` no gradient,
+    ``Ks`` receive one when they require it (intrinsics refinement): [C,3,3] with v_fx, v_fy, v_cx, v_cy at (0,0),
+    (1,1), (0,2), (1,2) and 0 elsewhere, the exact derivative of the projection (means2d, conics and, in antialiased
+    mode, the compensation), summed over each camera's visible Gaussians.
     Without SH, colours may have any number of channels D (features, masks, RGB plus extra channels): the images are
     [C,H,W,D], ``backgrounds`` [C,D], and D != 3 is blended in chunks of 32 channels by the feature kernels.  For
     D > 32, ``meta["means2d"].absgrad`` is the sum over the chunks of each chunk's absgrad (gsplat 1.0.0 keeps the
@@ -512,7 +533,8 @@ def rasterization_from_parameters(
     packed=False)`` — what ``GaussianModel.forward`` computes through its ``scales`` / ``opacities`` / ``shs``
     properties (/root/reference/model/gaussian.py:97-107, 353-367) — but the three activations and their backward
     passes run inside the projection kernels: no ``cat`` (384 B/Gaussian each way), no separate exp / sigmoid
-    kernels, and gradients arrive directly on the six parameter tensors."""
+    kernels, and gradients arrive directly on the six parameter tensors.  ``viewmats`` and ``Ks`` receive gradients
+    when they require them, as in ``rasterization()``."""
     width, height = int(width), int(height)
     if width < 1 or height < 1:
         raise ValueError(f"width and height must be >= 1, got {width} x {height}")

@@ -196,9 +196,10 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
                    width: int, height: int, sh_degree: Optional[int], eps2d: float, radii: Tensor,
                    colors_rgb: Tensor, v_splats: Tensor, v_means2d_extra: Optional[Tensor] = None,
                    want_absgrad: bool = False, antialiased_opacities: Optional[Tensor] = None,
-                   opacities: Optional[Tensor] = None, want_viewmats_grad: bool = False):
+                   opacities: Optional[Tensor] = None, want_viewmats_grad: bool = False, want_Ks_grad: bool = False):
     """g8+g9. -> v_means[N,3], v_quats[N,4], v_scales[N,3], v_opacities[N], v_colors (shape of colors)
-    (+ absgrad[C,N,2] when want_absgrad) (+ v_viewmats[C,4,4] when want_viewmats_grad, always last).
+    (+ absgrad[C,N,2] when want_absgrad) (+ v_viewmats[C,4,4] when want_viewmats_grad) (+ v_Ks[C,3,3] when
+    want_Ks_grad, always last).
     antialiased_opacities: the opacities[N] of an antialiased forward; opacities: only consulted for a registered
     gradient buffer (register_grad_target)."""
     lib = _lib.load()
@@ -222,15 +223,21 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
     tail = (_ptr(colors), K, deg, per_cam, _ptr(viewmats), _ptr(Ks), int(width), int(height), float(eps2d),
             _ptr(radii), _ptr(colors_rgb), _ptr(v_splats), _ptr(v_means2d_extra), _ptr(v_means), _ptr(v_quats),
             _ptr(v_scales), _ptr(v_opac), _ptr(v_colors), _ptr(absgrad), _stream(dev))
-    v_viewmats = None
+    v_viewmats = v_Ks = None
     with torch.cuda.device(dev):
         if want_viewmats_grad:
             v_viewmats = torch.empty(C, 4, 4, dtype=torch.float32, device=dev)
-            ws = _viewmats_workspace(lib, C, N, dev)
+        if want_Ks_grad or want_viewmats_grad:
             aa = antialiased_opacities is not None
             aa_op = _f32c(antialiased_opacities, "opacities") if aa else None
-            rc = lib.egs_projection_bwd_viewmats(C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail[:-1],
-                                                 int(aa), _ptr(v_viewmats), _ptr(ws), ws.numel(), tail[-1])
+            head = (C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail[:-1], int(aa), _ptr(v_viewmats))
+        if want_Ks_grad:  # one launch for both camera gradients
+            v_Ks = torch.empty(C, 3, 3, dtype=torch.float32, device=dev)
+            ws = _intrinsics_workspace(lib, C, N, dev)
+            rc = lib.egs_projection_bwd_intrinsics(*head, _ptr(v_Ks), _ptr(ws), ws.numel(), tail[-1])
+        elif want_viewmats_grad:
+            ws = _viewmats_workspace(lib, C, N, dev)
+            rc = lib.egs_projection_bwd_viewmats(*head, _ptr(ws), ws.numel(), tail[-1])
         elif antialiased_opacities is not None:
             aa_op = _f32c(antialiased_opacities, "opacities")
             rc = lib.egs_projection_bwd_antialiased(C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail)
@@ -238,12 +245,22 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
             rc = lib.egs_projection_bwd(C, N, _ptr(means), _ptr(quats), _ptr(scales), *tail)
     _lib.check(rc, "egs_projection_bwd")
     out = (v_means, v_quats, v_scales, v_opac, v_colors) + ((absgrad,) if want_absgrad else ())
-    return out + (v_viewmats,) if want_viewmats_grad else out
+    return _with_camera_grads(out, v_viewmats, v_Ks)
+
+
+def _with_camera_grads(out: tuple, v_viewmats: Optional[Tensor], v_Ks: Optional[Tensor]) -> tuple:
+    """out (+ v_viewmats) (+ v_Ks): only the camera gradients that were asked for, v_Ks last."""
+    return out + tuple(t for t in (v_viewmats, v_Ks) if t is not None)
 
 
 def _viewmats_workspace(lib, C: int, N: int, dev) -> Tensor:
     """Scratch of the view-matrix gradient (per-warp partials, see include/egs_raster.h); 16-byte aligned."""
     return torch.empty(max(lib.egs_projection_bwd_viewmats_workspace_bytes(C, N), 16), dtype=torch.uint8, device=dev)
+
+
+def _intrinsics_workspace(lib, C: int, N: int, dev) -> Tensor:
+    """Scratch of the intrinsics (and view-matrix) gradients: wider per-warp partials; 16-byte aligned."""
+    return torch.empty(max(lib.egs_projection_bwd_intrinsics_workspace_bytes(C, N), 16), dtype=torch.uint8, device=dev)
 
 
 def projection_fwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_opacities: Tensor, sh_0: Tensor,
@@ -287,8 +304,9 @@ def projection_bwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_o
                        sh_rest: Tensor, viewmats: Tensor, Ks: Tensor, width: int, height: int, sh_degree: int,
                        eps2d: float, radii: Tensor, colors_rgb: Tensor, v_splats: Tensor,
                        v_means2d_extra: Optional[Tensor] = None, want_absgrad: bool = False,
-                       want_viewmats_grad: bool = False):
-    """-> v_means, v_quats, v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest (, absgrad) (, v_viewmats[C,4,4])."""
+                       want_viewmats_grad: bool = False, want_Ks_grad: bool = False):
+    """-> v_means, v_quats, v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest (, absgrad) (, v_viewmats[C,4,4])
+    (, v_Ks[C,3,3])."""
     lib = _lib.load()
     dev = means.device
     means, quats, log_scales, logit_opacities, sh_0, sh_rest, viewmats, Ks = dense_inputs(
@@ -302,17 +320,23 @@ def projection_bwd_raw(means: Tensor, quats: Tensor, log_scales: Tensor, logit_o
     args = (C, N, _ptr(means), _ptr(quats), _ptr(log_scales), _ptr(logit_opacities), _ptr(sh_0), _ptr(sh_rest),
             int(sh_degree), _ptr(viewmats), _ptr(Ks), int(width), int(height), float(eps2d), _ptr(radii), _ptr(colors_rgb),
             _ptr(v_splats), _ptr(v_means2d_extra), *[_ptr(o) for o in outs], _ptr(absgrad))
-    v_viewmats = None
+    v_viewmats = v_Ks = None
     with torch.cuda.device(dev):
         if want_viewmats_grad:
             v_viewmats = torch.empty(C, 4, 4, dtype=torch.float32, device=dev)
+        if want_Ks_grad:  # one launch for both camera gradients
+            v_Ks = torch.empty(C, 3, 3, dtype=torch.float32, device=dev)
+            ws = _intrinsics_workspace(lib, C, N, dev)
+            rc = lib.egs_projection_bwd_raw_intrinsics(*args, _ptr(v_viewmats), _ptr(v_Ks), _ptr(ws), ws.numel(),
+                                                       _stream(dev))
+        elif want_viewmats_grad:
             ws = _viewmats_workspace(lib, C, N, dev)
             rc = lib.egs_projection_bwd_raw_viewmats(*args, _ptr(v_viewmats), _ptr(ws), ws.numel(), _stream(dev))
         else:
             rc = lib.egs_projection_bwd_raw(*args, _stream(dev))
     _lib.check(rc, "egs_projection_bwd_raw")
     out = (*outs, absgrad) if want_absgrad else tuple(outs)
-    return out + (v_viewmats,) if want_viewmats_grad else out
+    return _with_camera_grads(out, v_viewmats, v_Ks)
 
 
 def exclusive_scan(counts: Tensor) -> Tuple[Tensor, Tensor]:

@@ -169,6 +169,36 @@ int egs_projection_bwd_raw_viewmats(int32_t C, int32_t N, const float* means, co
                                     float* v_sh_0, float* v_sh_rest, float* absgrad, float* v_viewmats,
                                     void* workspace, int64_t workspace_bytes, egs_stream_t stream);
 
+/* ---- gradients w.r.t. the intrinsics (camera intrinsics refinement) ---------------------------------------------
+ * The viewmat entries above with a required v_Ks[C,3,3] and a nullable v_viewmats[C,4,4].  gsplat 1.0.0 returns no
+ * Ks gradient; this is the exact derivative of its projection, summed over the visible Gaussians of each camera:
+ *   v_Ks[c] = [[v_fx, 0, v_cx], [0, v_fy, v_cy], [0, 0, 0]]
+ * v_cx / v_cy sum the means2d cotangents (v_means2d_extra included); v_fx / v_fy also take the conic's and, in
+ * antialiased mode, the compensation's cotangents through the Jacobian (J02 = -fx tx / z^2 does not depend on fx where
+ * the fov clamp is active).  The skew and the last row are not read by the projection: 0.  Deterministic in the same
+ * way as v_viewmats (one backward launch and one finalize launch, also when v_viewmats is requested), and every other
+ * output is bit-identical to the entry without camera gradients.  C = 0 or N = 0: v_Ks (and v_viewmats) are zeros.
+ *   workspace: egs_projection_bwd_intrinsics_workspace_bytes(C, N) bytes (wider partials than the viewmat entries'),
+ *   16-byte aligned; no need to clear it.  One call at a time per workspace.
+ * Rejected before any launch: v_Ks NULL, too small a workspace, C > 65535. */
+int64_t egs_projection_bwd_intrinsics_workspace_bytes(int32_t C, int32_t N);
+int egs_projection_bwd_intrinsics(int32_t C, int32_t N, const float* means, const float* quats, const float* scales,
+                                  const float* opacities, const float* sh_coeffs, int32_t K, int32_t sh_degree,
+                                  int32_t colors_per_camera, const float* viewmats, const float* Ks, int32_t width,
+                                  int32_t height, float eps2d, const int32_t* radii, const float* colors,
+                                  const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
+                                  float* v_scales, float* v_opacities, float* v_sh_coeffs, float* absgrad,
+                                  int32_t antialiased, float* v_viewmats, float* v_Ks, void* workspace,
+                                  int64_t workspace_bytes, egs_stream_t stream);
+int egs_projection_bwd_raw_intrinsics(int32_t C, int32_t N, const float* means, const float* quats,
+                                      const float* log_scales, const float* logit_opacities, const float* sh_0,
+                                      const float* sh_rest, int32_t sh_degree, const float* viewmats, const float* Ks,
+                                      int32_t width, int32_t height, float eps2d, const int32_t* radii,
+                                      const float* colors, const float* v_splats, const float* v_means2d_extra,
+                                      float* v_means, float* v_quats, float* v_log_scales, float* v_logit_opacities,
+                                      float* v_sh_0, float* v_sh_rest, float* absgrad, float* v_viewmats, float* v_Ks,
+                                      void* workspace, int64_t workspace_bytes, egs_stream_t stream);
+
 /* ---- g3: exclusive scan of tiles_per_gauss, then key emission -------------------------------------
  * Replaces `torch.cumsum` + the second launch of gsplat `isect_tiles`.
  * egs_exclusive_scan: out[i] = sum_{j<i} in[j] (int64), *total = sum of all (device int64). */
