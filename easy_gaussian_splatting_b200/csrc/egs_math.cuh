@@ -519,6 +519,109 @@ EGS_HD void sh_color_bwd(int degree, const float mean[3], const Camera& cam, con
   }
 }
 
+// ---- spherical harmonics, degree 4: 25 bands ------------------------------------------------------
+// Bands 0..3 are sh_basis / sh_basis_vjp / sh_color_fwd / sh_color_bwd at degree 3, term for term and in the same
+// order, and band 4 is added after them: with zero band-4 coefficients the results equal degree 3's bit for bit.
+// Band 4 is the real SH basis of the lower bands' convention (sqrt(2) Re / Im of Y_4^|m| with the Condon-Shortley
+// phase, m = -4..4), written with fCm / fSm = Re / Im (x + iy)^(m+1) as in sh_basis.
+constexpr int kSh4Bands = 25;
+
+EGS_HD void sh_basis4(float x, float y, float z, float Y[kSh4Bands]) {
+  sh_basis(3, x, y, z, Y);
+  float z2 = z * z;
+  float fC1 = x * x - y * y;
+  float fS1 = 2.f * x * y;
+  float fC2 = x * fC1 - y * fS1;
+  float fS2 = x * fS1 + y * fC1;
+  float fC3 = x * fC2 - y * fS2;
+  float fS3 = x * fS2 + y * fC2;
+  float fTmp0D = 3.31161143515146f * z2 - 0.47308734787878f;
+  float fTmp1C = z * (-4.683325804901025f * z2 + 2.007139630671868f);
+  float fTmp2B = -1.770130769779931f * z;
+  Y[16] = 0.6258357354491763f * fS3;
+  Y[17] = fTmp2B * fS2;
+  Y[18] = fTmp0D * fS1;
+  Y[19] = fTmp1C * y;
+  Y[20] = 1.984313483298443f * z * Y[12] - 1.006230589874905f * Y[6];
+  Y[21] = fTmp1C * x;
+  Y[22] = fTmp0D * fC1;
+  Y[23] = fTmp2B * fC2;
+  Y[24] = 0.6258357354491763f * fC3;
+}
+
+// d(sum_k g[k] * Y_k)/d(x,y,z) of sh_basis4.  d(fCm, fSm)/dx = (m+1) (fC(m-1), fS(m-1)), d/dy = (m+1) (-fS(m-1), fC(m-1)).
+EGS_HD void sh_basis4_vjp(float x, float y, float z, const float g[kSh4Bands], float& vx, float& vy, float& vz) {
+  sh_basis_vjp(3, x, y, z, g, vx, vy, vz);
+  float z2 = z * z;
+  float fC1 = x * x - y * y;
+  float fS1 = 2.f * x * y;
+  float fC2 = x * fC1 - y * fS1;
+  float fS2 = x * fS1 + y * fC1;
+  float fTmp0D = 3.31161143515146f * z2 - 0.47308734787878f;
+  float fTmp1C = z * (-4.683325804901025f * z2 + 2.007139630671868f);
+  float fTmp2B = -1.770130769779931f * z;
+  const float k4 = 0.6258357354491763f;
+  const float dTmp1C = -3.f * 4.683325804901025f * z2 + 2.007139630671868f;  // d fTmp1C / dz
+  // d Y20 / dz with Y6 = 0.946.. z^2 - 0.315.. and Y12 = z (1.865.. z^2 - 1.119..)
+  const float dY20 = 1.984313483298443f * (z * (3.f * 1.865881662950577f * z2 - 1.119528997770346f) +
+                                           z * (1.865881662950577f * z2 - 1.119528997770346f)) -
+                     1.006230589874905f * (2.f * 0.9461746957575601f * z);
+  vx += g[16] * (k4 * 4.f * fS2) + g[17] * (fTmp2B * 3.f * fS1) + g[18] * (fTmp0D * 2.f * y) + g[21] * fTmp1C +
+        g[22] * (fTmp0D * 2.f * x) + g[23] * (fTmp2B * 3.f * fC1) + g[24] * (k4 * 4.f * fC2);
+  vy += g[16] * (k4 * 4.f * fC2) + g[17] * (fTmp2B * 3.f * fC1) + g[18] * (fTmp0D * 2.f * x) + g[19] * fTmp1C -
+        g[22] * (fTmp0D * 2.f * y) - g[23] * (fTmp2B * 3.f * fS1) - g[24] * (k4 * 4.f * fS2);
+  vz += g[17] * (-1.770130769779931f * fS2) + g[18] * (2.f * 3.31161143515146f * z * fS1) + g[19] * (dTmp1C * y) +
+        g[20] * dY20 + g[21] * (dTmp1C * x) + g[22] * (2.f * 3.31161143515146f * z * fC1) +
+        g[23] * (-1.770130769779931f * fC2);
+}
+
+// sh_color_fwd at degree 4.  co: the first 25 coefficient rows, [k][channel] (75 floats; shared memory in the kernels).
+EGS_HD void sh4_color_fwd(const float mean[3], const Camera& cam, const float* co, float rgb[3]) {
+  float dx = mean[0] - cam.campos[0], dy = mean[1] - cam.campos[1], dz = mean[2] - cam.campos[2];
+  float inorm = 1.0f / sqrtf(dx * dx + dy * dy + dz * dz);
+  float Y[kSh4Bands];
+  sh_basis4(dx * inorm, dy * inorm, dz * inorm, Y);
+  float r = 0.f, g = 0.f, b = 0.f;
+#pragma unroll
+  for (int k = 0; k < kSh4Bands; ++k) {
+    r += Y[k] * co[3 * k + 0];
+    g += Y[k] * co[3 * k + 1];
+    b += Y[k] * co[3 * k + 2];
+  }
+  rgb[0] = fmaxf(r + 0.5f, 0.f);
+  rgb[1] = fmaxf(g + 0.5f, 0.f);
+  rgb[2] = fmaxf(b + 0.5f, 0.f);
+}
+
+// sh_color_bwd at degree 4: accumulates (+=) into vco (75 floats) and v_mean[3]; v_cam (nullable) as in sh_color_bwd.
+EGS_HD void sh4_color_bwd(const float mean[3], const Camera& cam, const float* co, const float rgb_stored[3],
+                          const float v_rgb_in[3], float* vco, float v_mean[3], float* v_cam = nullptr) {
+  float v_rgb[3];
+  v_rgb[0] = (rgb_stored[0] > 0.f) ? v_rgb_in[0] : 0.f;
+  v_rgb[1] = (rgb_stored[1] > 0.f) ? v_rgb_in[1] : 0.f;
+  v_rgb[2] = (rgb_stored[2] > 0.f) ? v_rgb_in[2] : 0.f;
+  float dx = mean[0] - cam.campos[0], dy = mean[1] - cam.campos[1], dz = mean[2] - cam.campos[2];
+  float inorm = 1.0f / sqrtf(dx * dx + dy * dy + dz * dz);
+  float x = dx * inorm, y = dy * inorm, z = dz * inorm;
+  float Y[kSh4Bands], g[kSh4Bands];
+  sh_basis4(x, y, z, Y);
+#pragma unroll
+  for (int k = 0; k < kSh4Bands; ++k) {
+    vco[3 * k + 0] += Y[k] * v_rgb[0];
+    vco[3 * k + 1] += Y[k] * v_rgb[1];
+    vco[3 * k + 2] += Y[k] * v_rgb[2];
+    g[k] = co[3 * k + 0] * v_rgb[0] + co[3 * k + 1] * v_rgb[1] + co[3 * k + 2] * v_rgb[2];
+  }
+  float vx, vy, vz;
+  sh_basis4_vjp(x, y, z, g, vx, vy, vz);
+  float dp = vx * x + vy * y + vz * z;
+  const float d0 = (vx - dp * x) * inorm, d1 = (vy - dp * y) * inorm, d2 = (vz - dp * z) * inorm;
+  v_mean[0] += d0;
+  v_mean[1] += d1;
+  v_mean[2] += d2;
+  if (v_cam != nullptr) { v_cam[12] -= d0; v_cam[13] -= d1; v_cam[14] -= d2; }
+}
+
 // The [4,4] gradient of one view matrix V from its camera gradient summed over the Gaussians (v_R, v_t, g = v_campos,
 // see project_bwd).  campos = inv(V)[:3,3] with inv(V) = [[A, c], [0, 1]] (A = R^-1 by the same adjugate as
 // load_camera, c = campos), and the VJP of a matrix inverse is -inv(V)^T G inv(V)^T with g in column 3 of G:

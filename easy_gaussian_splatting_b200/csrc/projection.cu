@@ -441,6 +441,84 @@ __device__ __forceinline__ void store_sh_grad_rows(float* __restrict__ tile, flo
   __syncwarp();
 }
 
+// ------------------------------------------------------------------------------------------------
+// SH degree 4 (K >= 25): the first 25 bands of a row are 75 floats, 300 B.  A warp stages the rows of its 32 Gaussians
+// (rows row0 .. row0 + 31 of the [rows, K, 3] coefficient block: n_base, or c * N + n_base with per-camera rows) as a
+// dense 32 x 75 tile; the odd row stride keeps a lane's row-wise reads conflict free.  For K = 25 the tile has the
+// layout of the warp's 9600-byte span, so a full warp whose span is 16-byte aligned copies it with 19 128-bit accesses
+// per lane, all in flight at once (a float4 that straddles two rows is needed when either row is).  Whether the span is
+// aligned depends on the base pointer and, for per-camera rows, on N mod 4; unaligned spans, the last partial warp and
+// K > 25 take 4-byte accesses, which are coalesced whatever the alignment (the latter skip the bands past 4).
+// ------------------------------------------------------------------------------------------------
+constexpr int kSh4RowFloats = kSh4Bands * 3;           // 75
+constexpr int kSh4TileFloats = 32 * kSh4RowFloats;     // one warp's tile
+constexpr int kSh4TileVec4 = kSh4TileFloats / 4;       // 600
+constexpr int kSh4BwdMinCtas = 2;                      // 2 x 76.8 KB of tiles per SM
+
+__device__ __forceinline__ bool sh4_span_vec4(const float* span, int K3, int rows) {
+  return K3 == kSh4RowFloats && rows == 32 && (reinterpret_cast<uintptr_t>(span) & 15u) == 0;
+}
+
+// Rows in `mask` of the warp's `rows` into `tile` (other rows are zero-filled, nothing is read for them).
+__device__ __forceinline__ void stage_sh4_rows(float* __restrict__ tile, const float* __restrict__ sh, size_t row0,
+                                               int rows, int K3, uint32_t mask, int lane) {
+  const float* src = sh + row0 * K3;
+  if (sh4_span_vec4(src, K3, rows)) {
+    const float4* s4 = reinterpret_cast<const float4*>(src);
+    float4* t4 = reinterpret_cast<float4*>(tile);
+#pragma unroll
+    for (int i = 0; i < (kSh4TileVec4 + 31) / 32; ++i) {
+      const int f = i * 32 + lane;
+      if (f < kSh4TileVec4) {
+        const int r0 = (4 * f) / kSh4RowFloats, r1 = (4 * f + 3) / kSh4RowFloats;
+        const bool need = ((mask >> r0) | (mask >> r1)) & 1u;
+        t4[f] = need ? __ldg(s4 + f) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    }
+  } else {
+#pragma unroll 5
+    for (int e = lane; e < kSh4TileFloats; e += 32) {
+      const int row = e / kSh4RowFloats, col = e - row * kSh4RowFloats;
+      tile[e] = ((mask >> row) & 1u) ? __ldg(src + (size_t)row * K3 + col) : 0.f;
+    }
+  }
+  __syncwarp();
+}
+
+// The warp's gradient tile -> rows row0 .. row0 + rows - 1 of v_sh, zeros for the bands past 4, and the tile cleared.
+// Every element of those rows is written exactly once.
+__device__ __forceinline__ void store_sh4_rows(float* __restrict__ tile, float* __restrict__ v_sh, size_t row0, int rows,
+                                               int K3, int lane) {
+  __syncwarp();
+  float* dst = v_sh + row0 * K3;
+  if (sh4_span_vec4(dst, K3, rows)) {
+    float4* d4 = reinterpret_cast<float4*>(dst);
+    float4* t4 = reinterpret_cast<float4*>(tile);
+#pragma unroll
+    for (int i = 0; i < (kSh4TileVec4 + 31) / 32; ++i) {
+      const int f = i * 32 + lane;
+      if (f < kSh4TileVec4) {
+        d4[f] = t4[f];
+        t4[f] = make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    }
+  } else {
+#pragma unroll 5
+    for (int e = lane; e < kSh4TileFloats; e += 32) {
+      const int row = e / kSh4RowFloats, col = e - row * kSh4RowFloats;
+      if (row < rows) dst[(size_t)row * K3 + col] = tile[e];
+      tile[e] = 0.f;
+    }
+    const int extra = K3 - kSh4RowFloats;
+    if (extra > 0)
+      for (int e = lane; e < rows * extra; e += 32) {
+        const int row = e / extra;
+        dst[(size_t)row * K3 + kSh4RowFloats + (e - row * extra)] = 0.f;
+      }
+  }
+  __syncwarp();
+}
+
 constexpr bool kPerCameraSh = false;
 constexpr bool kKsGrad = false;
 #include "projection_kernels.cuh"
@@ -479,7 +557,7 @@ static int projection_fwd_impl(int32_t C, int32_t N, const float* means, const f
   EGS_REQUIRE(C <= 65535, "projection_fwd: C=%d exceeds 65535 cameras per call", C);
   EGS_REQUIRE(width >= 1 && height >= 1, "projection_fwd: width/height must be >= 1 (got %d x %d)", width, height);
   EGS_REQUIRE(tile_size >= 1 && (tile_size & (tile_size - 1)) == 0, "projection_fwd: tile_size must be a power of two");
-  EGS_REQUIRE(sh_degree <= 3, "projection_fwd: sh_degree %d > 3 is not supported", sh_degree);
+  EGS_REQUIRE(sh_degree <= 4, "projection_fwd: sh_degree %d > 4 is not supported", sh_degree);
   EGS_REQUIRE(tight_rects == nullptr || (tile_width < 65536 && tile_height < 65536),
               "projection_fwd: tile grid %d x %d too large for the packed tight rectangles", tile_width, tile_height);
   EGS_REQUIRE(sh_degree < 0 || K >= (sh_degree + 1) * (sh_degree + 1), "projection_fwd: K=%d too small for sh_degree=%d", K, sh_degree);
@@ -502,6 +580,12 @@ static int projection_fwd_impl(int32_t C, int32_t N, const float* means, const f
   const bool pc = sh_degree >= 0 && colors_per_camera;  // per-camera SH coefficients [C,N,K,3]
   if (raw) {
     EGS_REQUIRE(K == 16 && sh_degree >= 0, "projection_fwd_raw: needs sh_0 [N,1,3] + sh_rest [N,15,3] and sh_degree >= 0");
+  }
+  if (sh_degree == 4) {
+    const unsigned grid2 = (unsigned)(ceil_div(N, kPF2Threads) * C);
+    auto kern = pc ? percam::projection_fwd_sh4_kernel : projection_fwd_sh4_kernel;
+    kern<<<grid2, kPF2Threads, 0, (cudaStream_t)stream>>>(p);
+    return check_launch("projection_fwd_sh4_kernel");
   }
   if (raw || (vec4 && K == 16)) {
     const unsigned grid2 = (unsigned)(ceil_div(N, kPF2Threads) * C);
@@ -567,7 +651,7 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
                                void* workspace = nullptr, int64_t workspace_bytes = 0, float* v_Ks = nullptr) {
   const int raw = sh_rest != nullptr;
   EGS_REQUIRE(C >= 0 && N >= 0, "projection_bwd: negative sizes C=%d N=%d", C, N);
-  EGS_REQUIRE(sh_degree <= 3, "projection_bwd: sh_degree %d > 3 is not supported", sh_degree);
+  EGS_REQUIRE(sh_degree <= 4, "projection_bwd: sh_degree %d > 4 is not supported", sh_degree);
   EGS_REQUIRE(sh_degree < 0 || K >= (sh_degree + 1) * (sh_degree + 1), "projection_bwd: K=%d too small for sh_degree=%d", K, sh_degree);
   EGS_REQUIRE(colors_per_camera == 0 || colors_per_camera == 1, "projection_bwd: colors_per_camera=%d must be 0 or 1",
               colors_per_camera);
@@ -628,6 +712,22 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
                 "projection_bwd_raw: needs sh_0 / sh_rest (K = 16), logits and sh_degree >= 0");
   }
   const bool pc = sh_degree >= 0 && colors_per_camera;  // per-camera SH coefficients [C,N,K,3]
+  if (sh_degree == 4) {  // (raw mode has K = 16 and cannot get here)
+    constexpr int kSmem = 2 * kPB2Warps * kSh4TileFloats * (int)sizeof(float);
+    auto kern = kg ? (pc ? (antialiased ? ksgrad::percam::projection_bwd_sh4_kernel<true, true>
+                                        : ksgrad::percam::projection_bwd_sh4_kernel<false, true>)
+                         : (antialiased ? ksgrad::projection_bwd_sh4_kernel<true, true>
+                                        : ksgrad::projection_bwd_sh4_kernel<false, true>))
+              : pc ? (vg ? (antialiased ? percam::projection_bwd_sh4_kernel<true, true> : percam::projection_bwd_sh4_kernel<false, true>)
+                         : (antialiased ? percam::projection_bwd_sh4_kernel<true> : percam::projection_bwd_sh4_kernel<false>))
+                   : vg ? (antialiased ? projection_bwd_sh4_kernel<true, true> : projection_bwd_sh4_kernel<false, true>)
+                        : (antialiased ? projection_bwd_sh4_kernel<true> : projection_bwd_sh4_kernel<false>);
+    const cudaError_t attr_rc = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+    if (attr_rc != cudaSuccess) return fail((int)attr_rc, "projection_bwd: shared memory opt-in failed: %s", cudaGetErrorString(attr_rc));
+    kern<<<(unsigned)ceil_div(N, kPB2Threads), kPB2Threads, kSmem, (cudaStream_t)stream>>>(p);
+    const int rc = check_launch("projection_bwd_sh4_kernel");
+    return (rc != 0 || !vg) ? rc : finalize();
+  }
   if (raw || (vec4 && K == 16)) {
     // the reference's layout (K = 16): coalesced shared-memory staged rows
     constexpr int kSmem = 2 * kPB2Warps * 32 * kRowStride * (int)sizeof(float);

@@ -1,5 +1,6 @@
-// The two projection backward kernels, compiled four times, each with two flags (projection_kernels.cuh includes this
-// file in egs and egs::percam, projection.cu includes it in egs::ksgrad and egs::ksgrad::percam):
+// The projection backward kernels (generic, K = 16, SH degree 4), compiled four times, each with two flags
+// (projection_kernels.cuh includes this file in egs and egs::percam, projection.cu includes it in egs::ksgrad and
+// egs::ksgrad::percam):
 // - kPerCameraSh: SH coefficients [N,K,3] shared by all cameras (or direct colours), or [C,N,K,3], one row per
 //   (camera, Gaussian);
 // - kKsGrad: the camera-gradient (VG) forms also reduce the intrinsics gradient, 4 more floats per partial.
@@ -353,6 +354,155 @@ __global__ void EGS_PB_BOUNDS((kPerCameraSh || kKsGrad) && VG) projection_bwd_sh
     }
   } else if (!kPerCameraSh) {
     store_rows_raw<kRowStride>(vc_tile, p.v_sh, p.v_sh_rest, n_base, p.N, lane);
+  }
+  if (in_range) {
+    p.v_means[3 * (size_t)n + 0] = v_mean[0]; p.v_means[3 * (size_t)n + 1] = v_mean[1]; p.v_means[3 * (size_t)n + 2] = v_mean[2];
+    reinterpret_cast<float4*>(p.v_quats)[n] = make_float4(v_quat[0], v_quat[1], v_quat[2], v_quat[3]);
+    p.v_scales[3 * (size_t)n + 0] = v_scale[0]; p.v_scales[3 * (size_t)n + 1] = v_scale[1]; p.v_scales[3 * (size_t)n + 2] = v_scale[2];
+    p.v_opacities[n] = v_opac;
+  }
+}
+
+// Backward, SH degree 4 (K >= 25), the structure of projection_bwd_sh16_kernel: the coefficient rows and the gradient
+// rows of a warp's 32 Gaussians go through two shared-memory tiles (stage_sh4_rows / store_sh4_rows), every gradient
+// element is written once (zeros for Gaussians or pairs no camera sees and for the bands past 4).  2 x 38.4 KB of tiles
+// per block: 2 CTAs per SM.
+template <bool AA, bool VG = false>
+__global__ void __launch_bounds__(kPB2Threads, kSh4BwdMinCtas) projection_bwd_sh4_kernel(const ProjBwdParams p) {
+  static_assert(VG || !kKsGrad, "intrinsics gradients are reduced with the view-matrix gradient partials");
+  extern __shared__ __align__(16) float smem_pb[];
+  __shared__ Camera cams[kMaxCamerasSmem];
+  for (int c = threadIdx.x; c < p.C && c < kMaxCamerasSmem; c += kPB2Threads)
+    load_camera(p.viewmats + (size_t)c * 16, p.Ks + (size_t)c * 9, cams[c]);
+  if constexpr (VG) clear_cam_counters(p);
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float* co_tile = smem_pb + (size_t)warp * kSh4TileFloats;                // coefficients
+  float* vc_tile = smem_pb + (size_t)(kPB2Warps + warp) * kSh4TileFloats;  // gradient accumulation
+  const int n_base = blockIdx.x * kPB2Threads + warp * 32;
+  const int n = n_base + lane;
+  const bool in_range = n < p.N;
+  const int rows = min(32, p.N - n_base);
+  const int K3 = p.K * 3;
+
+  bool seen = false;
+  if (in_range)
+    for (int c = 0; c < p.C; ++c) seen = seen || (p.radii[(size_t)c * p.N + n] > 0);
+  const uint32_t seen_mask = __ballot_sync(0xffffffffu, seen);
+  if constexpr (VG) {
+    if (seen_mask == 0)  // the warp sees nothing: zero partials for every camera
+      for (int c = lane; c < p.C; c += 32) {
+        float4* d = reinterpret_cast<float4*>(cam_partial<kCamPartialStride>(p, c, warp));
+        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+        d[0] = z; d[1] = z; d[2] = z; d[3] = z;
+        if constexpr (kKsGrad) d[4] = z;
+      }
+  }
+
+  // phase 1: the shared coefficient rows that are needed (per camera, below, for per-camera SH); zero gradient rows
+  if (!kPerCameraSh && seen_mask != 0) stage_sh4_rows(co_tile, p.sh, (size_t)n_base, rows, K3, seen_mask, lane);
+  for (int f = lane; f < kSh4TileVec4; f += 32) reinterpret_cast<float4*>(vc_tile)[f] = make_float4(0.f, 0.f, 0.f, 0.f);
+  __syncwarp();
+
+  // phase 2: thread-private work on its own Gaussian / its own two rows
+  float v_mean[3] = {0.f, 0.f, 0.f}, v_quat[4] = {0.f, 0.f, 0.f, 0.f}, v_scale[3] = {0.f, 0.f, 0.f};
+  float v_opac = 0.f;
+  if (in_range && p.absgrad != nullptr) {
+    for (int c = 0; c < p.C; ++c) {
+      const size_t idx = (size_t)c * p.N + n;
+      float2 ag = make_float2(0.f, 0.f);
+      if (p.radii[idx] > 0) { const float4 g2a = p.v_splats[idx * 3 + 2]; ag = make_float2(g2a.y, g2a.z); }
+      p.absgrad[idx] = ag;
+    }
+  }
+  constexpr bool kWarpLoop = VG || kPerCameraSh;  // the camera loop runs on every lane of the warp
+  if (kWarpLoop ? seen_mask != 0 : seen) {
+    const int nl = kWarpLoop ? (in_range ? n : n_base) : n;  // a lane past the range reads the warp's first Gaussian
+    float mean[3], quat[4], scale[3];
+    mean[0] = __ldg(p.means + 3 * (size_t)nl + 0);
+    mean[1] = __ldg(p.means + 3 * (size_t)nl + 1);
+    mean[2] = __ldg(p.means + 3 * (size_t)nl + 2);
+    const float4 q4 = __ldg(reinterpret_cast<const float4*>(p.quats) + nl);
+    quat[0] = q4.x; quat[1] = q4.y; quat[2] = q4.z; quat[3] = q4.w;
+    scale[0] = __ldg(p.scales + 3 * (size_t)nl + 0);
+    scale[1] = __ldg(p.scales + 3 * (size_t)nl + 1);
+    scale[2] = __ldg(p.scales + 3 * (size_t)nl + 2);
+    const float* co = co_tile + lane * kSh4RowFloats;
+    float* vc = vc_tile + lane * kSh4RowFloats;
+    // the records of camera c + 1 are requested before camera c is worked on, as in projection_bwd_sh16_kernel
+    float4 ng0, ng1, ng2;
+    float ncol[3];
+    int nrad;
+    auto fetch = [&](int c) {
+      const size_t idx = (size_t)c * p.N + nl;
+      nrad = p.radii[idx];
+      if (kWarpLoop && !in_range) nrad = 0;
+      ng0 = p.v_splats[idx * 3 + 0];
+      ng1 = p.v_splats[idx * 3 + 1];
+      ng2 = p.v_splats[idx * 3 + 2];
+      ncol[0] = p.colors[idx * 3 + 0]; ncol[1] = p.colors[idx * 3 + 1]; ncol[2] = p.colors[idx * 3 + 2];
+    };
+    fetch(0);
+    for (int c = 0; c < p.C; ++c) {
+      const size_t idx = (size_t)c * p.N + n;
+      const int rad = nrad;
+      const float4 g0 = ng0, g1 = ng1, g2 = ng2;
+      const float col[3] = {ncol[0], ncol[1], ncol[2]};
+      if (c + 1 < p.C) fetch(c + 1);
+      if constexpr (kPerCameraSh) {
+        const uint32_t cam_mask = __ballot_sync(0xffffffffu, rad > 0);
+        if (cam_mask != 0) stage_sh4_rows(co_tile, p.sh, (size_t)c * p.N + n_base, rows, K3, cam_mask, lane);
+      }
+      float vcam[kCamAccFloats];
+      if constexpr (VG) {
+#pragma unroll
+        for (int k = 0; k < kCamAccFloats; ++k) vcam[k] = 0.f;
+      } else if constexpr (!kPerCameraSh) {
+        if (!(rad > 0)) continue;
+      }
+      do {  // (VG, per-camera SH: lanes that do not see camera c skip to the warp's sum / row store below)
+      if (kWarpLoop && !(rad > 0)) break;
+      Camera cam_local;
+      const Camera* cam = &cams[c < kMaxCamerasSmem ? c : 0];
+      if (c >= kMaxCamerasSmem) { load_camera(p.viewmats + (size_t)c * 16, p.Ks + (size_t)c * 9, cam_local); cam = &cam_local; }
+      float v_m2x = g0.x, v_m2y = g0.y;
+      if (p.v_means2d_extra != nullptr) {
+        v_m2x += p.v_means2d_extra[idx * 2 + 0];
+        v_m2y += p.v_means2d_extra[idx * 2 + 1];
+      }
+      {
+        ProjState st;
+        ProjOut o;
+        project_fwd(mean, quat, scale, *cam, p.width, p.height, p.eps2d, 0.f, INFINITY, -1.f, st, o);
+        if constexpr (AA) {
+          if (o.radius > 0)
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale,
+                        g1.y * __ldg(p.opacities + n), p.eps2d, VG ? vcam : nullptr, mean,
+                        kKsGrad ? vcam + kCamGradFloats : nullptr);
+          v_opac += g1.y * o.comp;
+        } else {
+          if (o.radius > 0)
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
+                        VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
+          v_opac += g1.y;
+        }
+      }
+      const float v_rgb[3] = {g1.z, g1.w, g2.x};
+      sh4_color_bwd(mean, *cam, co, col, v_rgb, vc, v_mean, VG ? vcam : nullptr);
+      } while (0);
+      if constexpr (VG)
+        store_cam_partial(vcam, __ballot_sync(0xffffffffu, rad > 0) != 0, cam_partial<kCamPartialStride>(p, c, warp), lane);
+      if constexpr (kPerCameraSh) store_sh4_rows(vc_tile, p.v_sh, (size_t)c * p.N + n_base, rows, K3, lane);
+    }
+  }
+  __syncwarp();
+
+  // phase 3: the gradient rows; small per-Gaussian outputs directly
+  if constexpr (kPerCameraSh) {
+    if (seen_mask == 0)  // no camera sees the warp's Gaussians: zero rows for every camera (stored per camera otherwise)
+      for (int c = 0; c < p.C; ++c) store_sh4_rows(vc_tile, p.v_sh, (size_t)c * p.N + n_base, rows, K3, lane);
+  } else {
+    store_sh4_rows(vc_tile, p.v_sh, (size_t)n_base, rows, K3, lane);
   }
   if (in_range) {
     p.v_means[3 * (size_t)n + 0] = v_mean[0]; p.v_means[3 * (size_t)n + 1] = v_mean[1]; p.v_means[3 * (size_t)n + 2] = v_mean[2];

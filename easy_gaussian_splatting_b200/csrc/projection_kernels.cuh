@@ -1,5 +1,5 @@
-// The four projection kernels: the two forward kernels below and the two backward kernels of
-// projection_bwd_kernels.cuh.  projection.cu includes this file twice: in namespace egs with kPerCameraSh = false (SH
+// The projection kernels: the three forward kernels below (generic, K = 16, SH degree 4) and the three backward kernels
+// of projection_bwd_kernels.cuh.  projection.cu includes this file twice: in namespace egs with kPerCameraSh = false (SH
 // coefficients [N,K,3] shared by all cameras, or direct colours) and in egs::percam with kPerCameraSh = true (SH
 // coefficients [C,N,K,3], one row per (camera, Gaussian)).  The per-camera code is behind `if constexpr`, so the
 // shared-coefficient kernels keep their names and compile exactly as without it.
@@ -161,6 +161,72 @@ __global__ void __launch_bounds__(kPF2Threads) projection_fwd_sh16_kernel(const 
     rgb[2] = fmaxf(b + 0.5f, 0.f);
     float opac = __ldg(p.opacities + n);
     if (p.raw) opac = act_sigmoid(opac);
+    if (p.antialiased) opac = opac * o.comp;
+    float4* s = p.splats + idx * 3;
+    s[0] = make_float4(o.m2x, o.m2y, o.ca, o.cb);
+    s[1] = make_float4(o.cc, opac, rgb[0], rgb[1]);
+    const float cut = sigma_cutoff(opac);
+    s[2] = make_float4(rgb[2], o.depth, 0.f, cut);
+    if (p.tight_rects != nullptr) {
+      tighten_tile_rect(o.m2x, o.m2y, o.ca, o.cb, o.cc, cut, p.tile_size, x0, y0, x1, y1);
+      pack_tile_rect(x0, y0, x1, y1, tight.x, tight.y);
+    }
+  }
+  p.radii[idx] = o.radius;
+  p.tiles_per_gauss[idx] = ntiles;
+  if (p.tight_rects != nullptr) reinterpret_cast<int2*>(p.tight_rects)[idx] = tight;
+  reinterpret_cast<float2*>(p.means2d)[idx] = make_float2(o.m2x, o.m2y);
+  p.depths[idx] = o.depth;
+  p.conics[idx * 3 + 0] = o.ca; p.conics[idx * 3 + 1] = o.cb; p.conics[idx * 3 + 2] = o.cc;
+  p.colors[idx * 3 + 0] = rgb[0]; p.colors[idx * 3 + 1] = rgb[1]; p.colors[idx * 3 + 2] = rgb[2];
+  if (p.antialiased) p.compensations[idx] = o.comp;
+}
+
+// Forward, SH degree 4 (K >= 25): as projection_fwd_sh16_kernel, the coefficient rows of the warp's VISIBLE Gaussians
+// go through a shared-memory tile (stage_sh4_rows), camera-fastest blocks.
+__global__ void __launch_bounds__(kPF2Threads) projection_fwd_sh4_kernel(const ProjFwdParams p) {
+  __shared__ Camera cam;
+  __shared__ __align__(16) float tile[kPF2Threads / 32][kSh4TileFloats];
+  const int c = blockIdx.x % p.C, chunk = blockIdx.x / p.C;
+  if (threadIdx.x == 0) load_camera(p.viewmats + (size_t)c * 16, p.Ks + (size_t)c * 9, cam);
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int n_base = chunk * kPF2Threads + warp * 32;
+  const int n = n_base + lane;
+  const bool in_range = n < p.N;
+  const size_t idx = (size_t)c * p.N + (in_range ? n : 0);
+
+  float mean[3] = {0.f, 0.f, 0.f};
+  ProjOut o;
+  o.m2x = 0.f; o.m2y = 0.f; o.depth = 0.f; o.ca = 0.f; o.cb = 0.f; o.cc = 0.f; o.radius = 0; o.lambda_max = 0.f; o.comp = 0.f;
+  bool vis = false;
+  if (in_range) {
+    float quat[4], scale[3];
+    mean[0] = __ldg(p.means + 3 * (size_t)n + 0);
+    mean[1] = __ldg(p.means + 3 * (size_t)n + 1);
+    mean[2] = __ldg(p.means + 3 * (size_t)n + 2);
+    const float4 q4 = __ldg(reinterpret_cast<const float4*>(p.quats) + n);
+    quat[0] = q4.x; quat[1] = q4.y; quat[2] = q4.z; quat[3] = q4.w;
+    scale[0] = __ldg(p.scales + 3 * (size_t)n + 0);
+    scale[1] = __ldg(p.scales + 3 * (size_t)n + 1);
+    scale[2] = __ldg(p.scales + 3 * (size_t)n + 2);
+    ProjState st;
+    vis = project_fwd(mean, quat, scale, cam, p.width, p.height, p.eps2d, p.near_plane, p.far_plane, p.radius_clip, st, o);
+  }
+  const uint32_t vis_mask = __ballot_sync(0xffffffffu, vis);
+  if (vis_mask != 0)
+    stage_sh4_rows(tile[warp], p.sh, (kPerCameraSh ? (size_t)c * p.N : 0) + n_base, min(32, p.N - n_base), p.K * 3,
+                   vis_mask, lane);
+  if (!in_range) return;
+  int32_t ntiles = 0;
+  int2 tight = make_int2(0, 0);
+  float rgb[3] = {0.f, 0.f, 0.f};
+  if (vis) {
+    int32_t x0, y0, x1, y1;
+    tile_rect(o.m2x, o.m2y, o.radius, p.tile_size, p.tile_w, p.tile_h, x0, y0, x1, y1);
+    ntiles = (x1 - x0) * (y1 - y0);
+    sh4_color_fwd(mean, cam, tile[warp] + lane * kSh4RowFloats, rgb);
+    float opac = __ldg(p.opacities + n);
     if (p.antialiased) opac = opac * o.comp;
     float4* s = p.splats + idx * 3;
     s[0] = make_float4(o.m2x, o.m2y, o.ca, o.cb);

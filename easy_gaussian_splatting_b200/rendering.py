@@ -365,8 +365,8 @@ def _check_inputs(means, quats, scales, opacities, colors, viewmats, Ks, sh_degr
         ok = (colors.dim() == 3 and colors.shape[0] == N) or (colors.dim() == 4 and colors.shape[:2] == (C, N))
         if not ok or colors.shape[-1] != 3:
             raise ValueError(f"colors must be [N,K,3] or per-camera [C,N,K,3] SH coefficients, got {tuple(colors.shape)}")
-        if not 0 <= sh_degree <= 3:
-            raise NotImplementedError(f"sh_degree={sh_degree}: degrees 0..3 are implemented (the reference uses <= 3)")
+        if not 0 <= sh_degree <= 4:
+            raise NotImplementedError(f"sh_degree={sh_degree}: degrees 0..4 are implemented (gsplat's fast SH evaluates 0..4)")
         if (sh_degree + 1) ** 2 > colors.shape[-2]:
             raise ValueError(f"sh_degree={sh_degree} needs K >= {(sh_degree + 1) ** 2}, got K={colors.shape[-2]}")
     if backgrounds is not None and backgrounds.shape != (C, D):
@@ -423,7 +423,9 @@ def rasterization(
     value of whichever chunk's backward ran last).  ``channel_chunk`` is accepted and has no effect.
     With SH, coefficients may also be per camera, [C,N,K,3] (e.g. shared coefficients plus a learned per-view
     offset): camera c colours Gaussian n from its own row colors[c, n], and colors.grad is [C,N,K,3], one row per
-    (camera, Gaussian), 0 for pairs the camera culls."""
+    (camera, Gaussian), 0 for pairs the camera culls.
+    ``sh_degree`` may be 0..4, as gsplat's fast SH evaluates; degree 4 needs K >= 25 and leaves the bands past 4 a
+    zero gradient."""
     if render_mode != "RGB":
         raise NotImplementedError(f"render_mode={render_mode!r}: only 'RGB' is implemented (the reference's mode)")
     if rasterize_mode not in ("classic", "antialiased"):

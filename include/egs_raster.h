@@ -57,7 +57,8 @@ int64_t egs_kernel_launch_count(void);
  * `dirs = means - inverse(viewmats)[:3,3]`, `clamp_min(rgb + 0.5, 0)` and the first launch of
  * `isect_tiles`, all reached from model/gaussian.py:353-367.
  *   means[N,3] quats[N,4](wxyz, unnormalised) scales[N,3] opacities[N]
- *   sh_coeffs: sh_degree >= 0 → SH coefficients (K >= (sh_degree+1)^2, sh_degree <= 3), [N,K,3] shared by all
+ *   sh_coeffs: sh_degree >= 0 → SH coefficients (K >= (sh_degree+1)^2, sh_degree <= 4; the _raw entries take
+ *              K = 16, so degree <= 3), [N,K,3] shared by all
  *              cameras (colors_per_camera = 0) or [C,N,K,3], one row per (camera, Gaussian) (colors_per_camera = 1);
  *              sh_degree <  0 → colours used as they are, [N,3] (colors_per_camera = 0)
  *              or [C,N,3] (colors_per_camera = 1)
