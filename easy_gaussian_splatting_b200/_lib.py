@@ -43,6 +43,8 @@ _SIGNATURES = {
                                                 P, P, P, P, P, P, P, I32, P, P, P, I64, P]),
     "egs_projection_bwd_raw_intrinsics": (c_int32, [I32, I32, P, P, P, P, P, P, I32, P, P, I32, I32, F32, P, P, P, P,
                                                     P, P, P, P, P, P, P, P, P, P, I64, P]),
+    "egs_projection_bwd_depth": (c_int32, [I32, I32, P, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, P, P, P, P,
+                                          P, P, P, P, P, P, I32, P, P, P, I64, P]),
     "egs_exclusive_scan_workspace_bytes": (c_int64, [I64]),
     "egs_exclusive_scan": (c_int32, [I64, P, P, P, P, I64, P]),
     "egs_isect_emit": (c_int32, [I32, I32, P, P, P, P, I32, I32, I32, I32, I64, P, P, P]),
@@ -60,6 +62,8 @@ _SIGNATURES = {
     "egs_rasterize_fwd": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, P]),
     "egs_rasterize_fwd_count": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, P]),
     "egs_rasterize_bwd": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, P, P, P]),
+    "egs_rasterize_fwd_depth": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, P]),
+    "egs_rasterize_bwd_depth": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, P, P, P]),
     "egs_rasterize_checkpoint_bytes": (c_int64, [I64, I32]),
     "egs_rasterize_fwd_checkpointed": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, I32, I32, P, P]),
     "egs_rasterize_bwd_segmented": (c_int32, [I32, I32, I64, P, P, P, P, I32, I32, I32, I32, P, P, P, P, P, P, I32, I32, P, P, P]),

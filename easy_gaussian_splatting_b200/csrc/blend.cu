@@ -27,7 +27,7 @@
 // the 2x2 layout the two pixels of a row share FADD2 / FMUL2 / FFMA2 instructions (sm_100) and the per-pixel
 // updates are branch free: a pixel that does not take part blends with weight 0.
 //
-// Backward: per-pixel back-to-front replay from the warp's own last blended index; the 11 per-Gaussian
+// Backward: per-pixel back-to-front replay from the warp's own last blended index; the 11 (12 with depth) per-Gaussian
 // partial gradients are summed over the lane's 4 pixels in registers, then over the warp through a 1.6 KB
 // shared-memory scratch (11 conflict-free row stores, 4 LDS.128 + a packed add tree per lane, one shuffle), and
 // 11 lanes issue one coalesced RED.ADD.F32 into the packed 48-byte gradient record of the Gaussian.
@@ -354,7 +354,9 @@ __device__ __forceinline__ void warp_sum_red(const float (&v)[N], int n, uint32_
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
-template <bool COUNT>
+// DEPTH: a fourth channel, the camera-space depth of record slot 9, blended like r, g, b with background 0 (render_colors
+// then has 4 floats per pixel); never with COUNT or checkpoints.
+template <bool COUNT, bool DEPTH = false>
 __global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
     int64_t n_isects, const float4* __restrict__ splats, const int32_t* __restrict__ tile_offsets,
     const int32_t* __restrict__ flatten_ids, const float* __restrict__ backgrounds, int width, int height, int tile_w,
@@ -372,13 +374,14 @@ __global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
   const WarpView wv = warp_setup<G>(tile_w, tile_h, n_isects, tile_offsets, n_tiles_total, tile_order);
   // T[j] > 0: transmittance of a live pixel; T[j] < 0: pixel finished, |T[j]| is its final transmittance
   // (the "done" flag lives in the sign bit, so liveness is one more FSETP in the accept test).
-  float T[NP], cr[NP], cg[NP], cb[NP];
+  float T[NP], cr[NP], cg[NP], cb[NP], cd[NP];
   int last[NP], term[NP];
   bool all_done = true;
 #pragma unroll
   for (int j = 0; j < NP; ++j) {
     const bool inside = (wv.x0 + (j % 2)) < width && (wv.y0 + (j / 2)) < height;
     T[j] = inside ? 1.0f : -1.0f; cr[j] = 0.f; cg[j] = 0.f; cb[j] = 0.f; last[j] = 0; term[j] = -1;
+    if constexpr (DEPTH) cd[j] = 0.f;
     all_done = all_done && !inside;
   }
   unsigned int n_acc = 0;
@@ -396,9 +399,10 @@ __global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
             const bool has_b = t + 1 < ns;  // warp-uniform
             const int cur_a = st.list[t], cur_b = st.list[has_b ? t + 1 : t];
             float4 g0[2], g1[2];
-            float cbl[2], alpha[2][NP], q[2][NP];
+            float cbl[2], dep[2], alpha[2][NP], q[2][NP];
             g0[0] = s[cur_a * 3 + 0]; g1[0] = s[cur_a * 3 + 1]; cbl[0] = s[cur_a * 3 + 2].x;
             g0[1] = s[cur_b * 3 + 0]; g1[1] = s[cur_b * 3 + 1]; cbl[1] = s[cur_b * 3 + 2].x;
+            if constexpr (DEPTH) { dep[0] = s[cur_a * 3 + 2].y; dep[1] = s[cur_b * 3 + 2].y; }
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
               float dx[2], dy[2];
@@ -438,6 +442,10 @@ __global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
                   const float2 c_g = __ffma2_rn(make_float2(g1[e].w, g1[e].w), w, make_float2(cg[j0], cg[j1]));
                   const float2 c_b = __ffma2_rn(make_float2(cbl[e], cbl[e]), w, make_float2(cb[j0], cb[j1]));
                   cr[j0] = c_r.x; cr[j1] = c_r.y; cg[j0] = c_g.x; cg[j1] = c_g.y; cb[j0] = c_b.x; cb[j1] = c_b.y;
+                  if constexpr (DEPTH) {
+                    const float2 c_d = __ffma2_rn(make_float2(dep[e], dep[e]), w, make_float2(cd[j0], cd[j1]));
+                    cd[j0] = c_d.x; cd[j1] = c_d.y;
+                  }
                 }
               }
             }
@@ -450,7 +458,7 @@ __global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
           // replay at any of these boundaries, one warp per segment (see rasterize_bwd_kernel).  Slot numbering
           // floor(start / K) + k is collision free across tiles because their list ranges are disjoint and ordered.
           const int done_local = (b + 1) * kBatch;
-          if (ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len && done_local % ckpt_k == 0 &&
+          if (!DEPTH && ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len && done_local % ckpt_k == 0 &&
               done_local < wv.range_end - wv.range_start) {
             const size_t slot = (size_t)(wv.range_start / ckpt_k + done_local / ckpt_k);
             float4* dst = ckpt + ((slot * G::kWarps + (threadIdx.x >> 5)) * NP) * 32 + lane;
@@ -472,9 +480,11 @@ __global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
     if (x < width && y < height) {
       const size_t pix = ((size_t)wv.cam * height + y) * width + x;
       const float Tf = fabsf(T[j]);
-      render_colors[pix * 3 + 0] = fmaf(Tf, bgr, cr[j]);
-      render_colors[pix * 3 + 1] = fmaf(Tf, bgg, cg[j]);
-      render_colors[pix * 3 + 2] = fmaf(Tf, bgb, cb[j]);
+      constexpr int PS = DEPTH ? 4 : 3;  // floats per pixel of render_colors
+      render_colors[pix * PS + 0] = fmaf(Tf, bgr, cr[j]);
+      render_colors[pix * PS + 1] = fmaf(Tf, bgg, cg[j]);
+      render_colors[pix * PS + 2] = fmaf(Tf, bgb, cb[j]);
+      if constexpr (DEPTH) render_colors[pix * PS + 3] = cd[j];
       render_alphas[pix] = 1.0f - Tf;
       last_ids[pix] = last[j];
       // P_eval in the reference's sense: list entries up to and including the terminating one
@@ -496,7 +506,10 @@ __global__ void EGS_FWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_fwd_kernel(
 // ------------------------------------------------------------------------------------------------
 // backward
 // ------------------------------------------------------------------------------------------------
-
+// DEPTH: the backward of the DEPTH forward.  v_render_colors has 4 floats per pixel; the depth channel (background 0)
+// enters v_alpha through depth * v_d, and sum fac * v_d is reduced as a twelfth value into gradient-record slot 11
+// (v_depth).  No segmented replay.
+template <bool DEPTH = false>
 __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
     int64_t n_isects, const float4* __restrict__ splats, const int32_t* __restrict__ tile_offsets,
     const int32_t* __restrict__ flatten_ids, const float* __restrict__ backgrounds, int width, int height, int tile_w,
@@ -514,8 +527,10 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
   using G = Geo<2, 2>;
   constexpr int NP = G::NP;
   constexpr int RPL = G::RPL, kBatch = G::kBatch;
+  constexpr int NV = DEPTH ? kGradValues + 1 : kGradValues;  // values reduced per Gaussian
+  constexpr int PS = DEPTH ? 4 : 3;                           // floats per pixel of v_render_colors
   __shared__ __align__(16) WarpStage<kBatch> stage[G::kWarps];
-  __shared__ __align__(16) float red_all[G::kWarps][kGradValues * kRedStride];
+  __shared__ __align__(16) float red_all[G::kWarps][NV * kRedStride];
   const int lane = threadIdx.x & 31;
   WarpStage<kBatch>& st = stage[threadIdx.x >> 5];
   float* red = red_all[threadIdx.x >> 5];
@@ -542,7 +557,7 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
   // per-pixel replay state.  nbt_ = tfv - bdot with bdot = sum over the Gaussians behind of fac * (rgb . v_colour),
   // which is all the backward pass needs of the colour accumulated behind, and
   // tfv = T_final * (v_alpha_out - bg . v_colour).
-  float T[NP], nbt_[NP], vcr[NP], vcg[NP], vcb[NP];
+  float T[NP], nbt_[NP], vcr[NP], vcg[NP], vcb[NP], vcd[NP];
   int bin_final[NP];
   int my_last = -1;
   float bgr = 0.f, bgg = 0.f, bgb = 0.f;
@@ -553,15 +568,17 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
   for (int j = 0; j < NP; ++j) {
     const int x = wv.x0 + (j % 2), y = wv.y0 + (j / 2);
     T[j] = 1.f; nbt_[j] = 0.f; vcr[j] = 0.f; vcg[j] = 0.f; vcb[j] = 0.f;
+    if constexpr (DEPTH) vcd[j] = 0.f;
     bin_final[j] = -1;  // pixels outside the image never match any index
     if (x < width && y < height) {
       const size_t pix = ((size_t)wv.cam * height + y) * width + x;
       const float T_final = 1.0f - render_alphas[pix];
       T[j] = T_final;
       bin_final[j] = last_ids[pix];
-      vcr[j] = v_render_colors[pix * 3 + 0];
-      vcg[j] = v_render_colors[pix * 3 + 1];
-      vcb[j] = v_render_colors[pix * 3 + 2];
+      vcr[j] = v_render_colors[pix * PS + 0];
+      vcg[j] = v_render_colors[pix * PS + 1];
+      vcb[j] = v_render_colors[pix * PS + 2];
+      if constexpr (DEPTH) vcd[j] = v_render_colors[pix * PS + 3];
       nbt_[j] = T_final * (v_render_alphas[pix] - (bgr * vcr[j] + bgg * vcg[j] + bgb * vcb[j]));
     }
     my_last = max(my_last, bin_final[j]);
@@ -571,7 +588,7 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
   int end_idx = min(wv.range_end - 1, warp_last);
   if (end_idx < wv.range_start) return;  // warp-uniform
   int lo_idx = wv.range_start;  // the replay walks end_idx, end_idx - 1, ..., lo_idx
-  if (ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len) {
+  if (!DEPTH && ckpt != nullptr && wv.range_end - wv.range_start >= seg_min_len) {
     const int last_seg = (end_idx - wv.range_start) / ckpt_k;  // segment that holds the warp's last blended entry
     if (!seg_launch) {
       lo_idx = wv.range_start + last_seg * ckpt_k;
@@ -606,12 +623,12 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
   // otherwise re-derives them from %tid / the CTA's shared window for every survivor (~12 of the loop's ~200
   // instructions).
   const int out_slot = lane >> 1;
-  int red_flag = ((lane & 1) == 0 && out_slot < kGradValues) ? 1 : 0;
+  int red_flag = ((lane & 1) == 0 && out_slot < NV) ? 1 : 0;
   asm volatile("" : "+r"(red_flag));
   uint32_t red_st = (uint32_t)__cvta_generic_to_shared(red + lane);
   asm volatile("" : "+r"(red_st));
-  const float4* row = reinterpret_cast<const float4*>(red + min(out_slot, kGradValues - 1) * kRedStride + (lane & 1) * 16);
-  float* out_base = v_splats + min(out_slot, kGradValues - 1);
+  const float4* row = reinterpret_cast<const float4*>(red + min(out_slot, NV - 1) * kRedStride + (lane & 1) * 16);
+  float* out_base = v_splats + min(out_slot, NV - 1);
   asm volatile("" : "+l"(out_base));
 
   stage_batches<true, true, RPL>(
@@ -627,6 +644,8 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
           const float4 g0 = s[cur * 3 + 0];  // x, y, conic_a, conic_b
           const float4 g1 = s[cur * 3 + 1];  // conic_c, opacity, r, g
           const float cbl = s[cur * 3 + 2].x;
+          float dep = 0.f;
+          if constexpr (DEPTH) dep = s[cur * 3 + 2].y;
           const float inv_o = fast_rcp(g1.y);
           // Packed fp32 (FADD2 / FMUL2 / FFMA2): the two pixels of a row of the lane's block share one instruction,
           // and the replay is branch free — a pixel that does not take part gets alpha = 0 and ov = 0, which makes
@@ -643,7 +662,7 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
           }
           if (!__any_sync(0xffffffffu, any_valid)) continue;  // warp-uniform
           float2 s_gx = make_float2(0.f, 0.f), s_gy = s_gx, s_xx = s_gx, s_xy = s_gx, s_yy = s_gx, s_w = s_gx, s_r = s_gx,
-                 s_g = s_gx, s_b = s_gx, s_ax = s_gx, s_ay = s_gx;
+                 s_g = s_gx, s_b = s_gx, s_ax = s_gx, s_ay = s_gx, s_d = s_gx;
 #pragma unroll
           for (int r = 0; r < 2; ++r) {
             const int j0 = 2 * r, j1 = 2 * r + 1;
@@ -666,8 +685,13 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
             s_r = __ffma2_rn(fac, vr2, s_r);
             s_g = __ffma2_rn(fac, vg2, s_g);
             s_b = __ffma2_rn(fac, vb2, s_b);
-            const float2 cdot = __ffma2_rn(make_float2(cbl, cbl), vb2,
-                                           __ffma2_rn(make_float2(g1.w, g1.w), vg2, __fmul2_rn(make_float2(g1.z, g1.z), vr2)));
+            float2 cdot = __ffma2_rn(make_float2(cbl, cbl), vb2,
+                                     __ffma2_rn(make_float2(g1.w, g1.w), vg2, __fmul2_rn(make_float2(g1.z, g1.z), vr2)));
+            if constexpr (DEPTH) {
+              const float2 vd2 = make_float2(vcd[j0], vcd[j1]);
+              s_d = __ffma2_rn(fac, vd2, s_d);
+              cdot = __ffma2_rn(make_float2(dep, dep), vd2, cdot);
+            }
             // nbt = tfv - bdot (kept negated so that v_alpha is one FMUL2 + one FFMA2)
             const float2 nbt = make_float2(nbt_[j0], nbt_[j1]);
             const float2 v_alpha = __ffma2_rn(Tf, cdot, __fmul2_rn(ra, nbt));
@@ -690,12 +714,13 @@ __global__ void EGS_BWD_BOUNDS((Geo<2, 2>::kThreads)) rasterize_bwd_kernel(
           }
           // v[2], v[3], v[4] are the sums of sx*dx, sx*dy, sy*dy (the 0.5 of the conic gradient is applied once, after
           // the per-lane sum); v[5] the sum of ov * v_alpha (the 1/opacity is applied after the per-lane sum).
-          float v[kGradValues];
+          float v[NV];
           v[0] = s_gx.x + s_gx.y; v[1] = s_gy.x + s_gy.y; v[2] = s_xx.x + s_xx.y; v[3] = s_xy.x + s_xy.y;
           v[4] = s_yy.x + s_yy.y; v[5] = s_w.x + s_w.y; v[6] = s_r.x + s_r.y; v[7] = s_g.x + s_g.y;
           v[8] = s_b.x + s_b.y; v[9] = s_ax.x + s_ax.y; v[10] = s_ay.x + s_ay.y;
+          if constexpr (DEPTH) v[11] = s_d.x + s_d.y;
           v[2] *= 0.5f; v[4] *= 0.5f; v[5] *= inv_o;
-          warp_sum_red(v, kGradValues, red_st, row, red_flag, out_base + (size_t)sid[cur] * EGS_SPLAT_FLOATS);
+          warp_sum_red(v, NV, red_st, row, red_flag, out_base + (size_t)sid[cur] * EGS_SPLAT_FLOATS);
         }
         return false;
       });
@@ -1029,7 +1054,7 @@ static int check_raster_args(const char* who, int32_t C, int64_t n_isects, int32
 // tiles of an object scene are bound by their serial walk, and eight warps that each cull the whole list do 1.5 x the
 // instructions of two.
 
-template <bool COUNT>
+template <bool COUNT, bool DEPTH = false>
 static int launch_fwd(int32_t C, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
                       const int32_t* flatten_ids, const float* backgrounds, int32_t width, int32_t height,
                       int32_t tile_width, int32_t tile_height, float* render_colors, float* render_alphas,
@@ -1041,7 +1066,7 @@ static int launch_fwd(int32_t C, int64_t n_isects, const float* splats, const in
   const float4* sp = reinterpret_cast<const float4*>(splats);
   unsigned long long* pc = reinterpret_cast<unsigned long long*>(pair_counters);
   cudaStream_t st = (cudaStream_t)stream;
-  rasterize_fwd_kernel<COUNT><<<grid, Geo<2, 2>::kThreads, 0, st>>>(
+  rasterize_fwd_kernel<COUNT, DEPTH><<<grid, Geo<2, 2>::kThreads, 0, st>>>(
       n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles,
       render_colors, render_alphas, last_ids, pc, ck, segment, seg_min_len > segment ? seg_min_len : segment + 1,
       tile_order);
@@ -1104,6 +1129,7 @@ extern "C" int egs_rasterize_fwd_checkpointed(int32_t C, int32_t N, int64_t n_is
                            segment, seg_min_len);
 }
 
+template <bool DEPTH = false>
 static int launch_bwd(int32_t C, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
                       const int32_t* flatten_ids, const float* backgrounds, int32_t width, int32_t height,
                       int32_t tile_width, int32_t tile_height, const float* render_alphas, const int32_t* last_ids,
@@ -1119,10 +1145,10 @@ static int launch_bwd(int32_t C, int64_t n_isects, const float* splats, const in
   // the segment launch goes first: its warps all have full segments to replay, the tile launch then fills in
   const int64_t n_slots = ck != nullptr ? (n_isects < 0 ? -n_isects : n_isects) / segment : 0;
   if (n_slots > 0)
-    rasterize_bwd_kernel<<<(unsigned)n_slots, Geo<2, 2>::kThreads, 0, st>>>(
+    rasterize_bwd_kernel<DEPTH><<<(unsigned)n_slots, Geo<2, 2>::kThreads, 0, st>>>(
         n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles,
         render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, render_colors, ck, segment, seg_min_len, 1, nullptr);
-  rasterize_bwd_kernel<<<grid, Geo<2, 2>::kThreads, 0, st>>>(
+  rasterize_bwd_kernel<DEPTH><<<grid, Geo<2, 2>::kThreads, 0, st>>>(
       n_isects, sp, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height, n_tiles,
       render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, render_colors, ck, segment, seg_min_len, 0, tile_order);
   return check_launch("rasterize_bwd_kernel", 1 + (n_slots > 0 ? 1 : 0));
@@ -1159,6 +1185,33 @@ extern "C" int egs_rasterize_bwd_segmented(int32_t C, int32_t N, int64_t n_isect
   return launch_bwd(C, n_isects, splats, tile_offsets, flatten_ids, backgrounds, width, height, tile_width, tile_height,
                     render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, render_colors, checkpoints,
                     segment, seg_min_len, tile_order, stream);
+}
+
+// ---- RGB plus expected depth: the DEPTH forms, 4 floats per pixel, no checkpoints --------------------------------------
+extern "C" int egs_rasterize_fwd_depth(int32_t C, int32_t N, int64_t n_isects, const float* splats,
+                                       const int32_t* tile_offsets, const int32_t* flatten_ids, const float* backgrounds,
+                                       int32_t width, int32_t height, int32_t tile_width, int32_t tile_height,
+                                       float* render_colors, float* render_alphas, int32_t* last_ids,
+                                       const int32_t* tile_order, egs_stream_t stream) {
+  (void)N;
+  if (int rc = check_raster_args("rasterize_fwd_depth", C, n_isects, width, height, tile_width, tile_height)) return rc;
+  if (C == 0) return 0;
+  return launch_fwd<false, true>(C, n_isects, splats, tile_offsets, flatten_ids, backgrounds, width, height, tile_width,
+                                 tile_height, render_colors, render_alphas, last_ids, nullptr, tile_order, stream);
+}
+
+extern "C" int egs_rasterize_bwd_depth(int32_t C, int32_t N, int64_t n_isects, const float* splats,
+                                       const int32_t* tile_offsets, const int32_t* flatten_ids, const float* backgrounds,
+                                       int32_t width, int32_t height, int32_t tile_width, int32_t tile_height,
+                                       const float* render_alphas, const int32_t* last_ids,
+                                       const float* v_render_colors, const float* v_render_alphas, float* v_splats,
+                                       const int32_t* tile_order, egs_stream_t stream) {
+  (void)N;
+  if (int rc = check_raster_args("rasterize_bwd_depth", C, n_isects, width, height, tile_width, tile_height)) return rc;
+  if (C == 0 || n_isects == 0) return 0;
+  return launch_bwd<true>(C, n_isects, splats, tile_offsets, flatten_ids, backgrounds, width, height, tile_width,
+                          tile_height, render_alphas, last_ids, v_render_colors, v_render_alphas, v_splats, nullptr,
+                          nullptr, 0, 0, tile_order, stream);
 }
 
 // ---- colours with any number of channels -------------------------------------------------------------------------

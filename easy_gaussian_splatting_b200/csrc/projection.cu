@@ -521,6 +521,7 @@ __device__ __forceinline__ void store_sh4_rows(float* __restrict__ tile, float* 
 
 constexpr bool kPerCameraSh = false;
 constexpr bool kKsGrad = false;
+constexpr bool kDepthGrad = false;
 #include "projection_kernels.cuh"
 
 namespace percam {
@@ -539,6 +540,32 @@ constexpr bool kPerCameraSh = true;
 #include "projection_bwd_kernels.cuh"
 }  // namespace percam
 }  // namespace ksgrad
+
+#include "projection_bwd_launch.cuh"
+
+// The backward kernels once more, with the depth cotangent of gradient-record slot 11 (render modes with expected
+// depth): every form above, in a namespace of its own so that the kernels above keep their code and registers.
+namespace depth {
+constexpr bool kDepthGrad = true;
+#include "projection_bwd_kernels.cuh"
+
+namespace percam {
+constexpr bool kPerCameraSh = true;
+#include "projection_bwd_kernels.cuh"
+}  // namespace percam
+
+namespace ksgrad {
+constexpr bool kKsGrad = true;
+#include "projection_bwd_kernels.cuh"
+
+namespace percam {
+constexpr bool kPerCameraSh = true;
+#include "projection_bwd_kernels.cuh"
+}  // namespace percam
+}  // namespace ksgrad
+
+#include "projection_bwd_launch.cuh"
+}  // namespace depth
 
 }  // namespace egs
 
@@ -648,7 +675,8 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
                                const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
                                float* v_scales, float* v_opacities, float* v_sh_coeffs, float* v_sh_rest, float* absgrad,
                                egs_stream_t stream, int antialiased = 0, float* v_viewmats = nullptr,
-                               void* workspace = nullptr, int64_t workspace_bytes = 0, float* v_Ks = nullptr) {
+                               void* workspace = nullptr, int64_t workspace_bytes = 0, float* v_Ks = nullptr,
+                               int depth_grad = 0) {
   const int raw = sh_rest != nullptr;
   EGS_REQUIRE(C >= 0 && N >= 0, "projection_bwd: negative sizes C=%d N=%d", C, N);
   EGS_REQUIRE(sh_degree <= 4, "projection_bwd: sh_degree %d > 4 is not supported", sh_degree);
@@ -712,64 +740,9 @@ static int projection_bwd_impl(int32_t C, int32_t N, const float* means, const f
                 "projection_bwd_raw: needs sh_0 / sh_rest (K = 16), logits and sh_degree >= 0");
   }
   const bool pc = sh_degree >= 0 && colors_per_camera;  // per-camera SH coefficients [C,N,K,3]
-  if (sh_degree == 4) {  // (raw mode has K = 16 and cannot get here)
-    constexpr int kSmem = 2 * kPB2Warps * kSh4TileFloats * (int)sizeof(float);
-    auto kern = kg ? (pc ? (antialiased ? ksgrad::percam::projection_bwd_sh4_kernel<true, true>
-                                        : ksgrad::percam::projection_bwd_sh4_kernel<false, true>)
-                         : (antialiased ? ksgrad::projection_bwd_sh4_kernel<true, true>
-                                        : ksgrad::projection_bwd_sh4_kernel<false, true>))
-              : pc ? (vg ? (antialiased ? percam::projection_bwd_sh4_kernel<true, true> : percam::projection_bwd_sh4_kernel<false, true>)
-                         : (antialiased ? percam::projection_bwd_sh4_kernel<true> : percam::projection_bwd_sh4_kernel<false>))
-                   : vg ? (antialiased ? projection_bwd_sh4_kernel<true, true> : projection_bwd_sh4_kernel<false, true>)
-                        : (antialiased ? projection_bwd_sh4_kernel<true> : projection_bwd_sh4_kernel<false>);
-    const cudaError_t attr_rc = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-    if (attr_rc != cudaSuccess) return fail((int)attr_rc, "projection_bwd: shared memory opt-in failed: %s", cudaGetErrorString(attr_rc));
-    kern<<<(unsigned)ceil_div(N, kPB2Threads), kPB2Threads, kSmem, (cudaStream_t)stream>>>(p);
-    const int rc = check_launch("projection_bwd_sh4_kernel");
-    return (rc != 0 || !vg) ? rc : finalize();
-  }
-  if (raw || (vec4 && K == 16)) {
-    // the reference's layout (K = 16): coalesced shared-memory staged rows
-    constexpr int kSmem = 2 * kPB2Warps * 32 * kRowStride * (int)sizeof(float);
-    auto kern = kg ? (pc ? (antialiased ? ksgrad::percam::projection_bwd_sh16_kernel<true, true>
-                                        : ksgrad::percam::projection_bwd_sh16_kernel<false, true>)
-                         : (antialiased ? ksgrad::projection_bwd_sh16_kernel<true, true>
-                                        : ksgrad::projection_bwd_sh16_kernel<false, true>))
-              : pc ? (vg ? (antialiased ? percam::projection_bwd_sh16_kernel<true, true> : percam::projection_bwd_sh16_kernel<false, true>)
-                         : (antialiased ? percam::projection_bwd_sh16_kernel<true> : percam::projection_bwd_sh16_kernel<false>))
-                   : vg ? (antialiased ? projection_bwd_sh16_kernel<true, true> : projection_bwd_sh16_kernel<false, true>)
-                        : (antialiased ? projection_bwd_sh16_kernel<true> : projection_bwd_sh16_kernel<false>);
-    const cudaError_t attr_rc =  // per-device attribute: set on every call (cheap), not once per process
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-    if (attr_rc != cudaSuccess) return fail((int)attr_rc, "projection_bwd: shared memory opt-in failed: %s", cudaGetErrorString(attr_rc));
-    kern<<<(unsigned)ceil_div(N, kPB2Threads), kPB2Threads, kSmem, (cudaStream_t)stream>>>(p);
-    const int rc = check_launch("projection_bwd_sh16_kernel");
-    return (rc != 0 || !vg) ? rc : finalize();
-  }
-  unsigned grid = (unsigned)ceil_div(N, kProjBwdThreads);
-  if (kg) {
-    auto kern = pc ? (vec4 ? ksgrad::percam::projection_bwd_kernel<true, true> : ksgrad::percam::projection_bwd_kernel<false, true>)
-                   : (vec4 ? ksgrad::projection_bwd_kernel<true, true> : ksgrad::projection_bwd_kernel<false, true>);
-    kern<<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
-    const int rc = check_launch("projection_bwd_kernel");
-    return rc != 0 ? rc : finalize();
-  }
-  if (pc) {
-    auto kern = vg ? (vec4 ? percam::projection_bwd_kernel<true, true> : percam::projection_bwd_kernel<false, true>)
-                   : (vec4 ? percam::projection_bwd_kernel<true> : percam::projection_bwd_kernel<false>);
-    kern<<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
-    const int rc = check_launch("projection_bwd_kernel");
-    return (rc != 0 || !vg) ? rc : finalize();
-  }
-  if (vg) {
-    if (vec4) projection_bwd_kernel<true, true><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
-    else      projection_bwd_kernel<false, true><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
-    const int rc = check_launch("projection_bwd_kernel");
-    return rc != 0 ? rc : finalize();
-  }
-  if (vec4) projection_bwd_kernel<true><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
-  else      projection_bwd_kernel<false><<<grid, kProjBwdThreads, 0, (cudaStream_t)stream>>>(p);
-  return check_launch("projection_bwd_kernel");
+  const int rc = depth_grad ? depth::launch_projection_bwd(p, kg, vg, pc, vec4, antialiased, raw, (cudaStream_t)stream)
+                            : launch_projection_bwd(p, kg, vg, pc, vec4, antialiased, raw, (cudaStream_t)stream);
+  return (rc != 0 || !vg) ? rc : finalize();
 }
 
 extern "C" int egs_projection_bwd(int32_t C, int32_t N, const float* means, const float* quats, const float* scales,
@@ -887,4 +860,18 @@ extern "C" int egs_projection_bwd_raw_intrinsics(
                              Ks, width, height, eps2d, radii, colors, v_splats, v_means2d_extra, v_means, v_quats,
                              v_log_scales, v_logit_opacities, v_sh_0, v_sh_rest, absgrad, stream, 0, v_viewmats,
                              workspace, workspace_bytes, v_Ks);
+}
+
+/* ---- with the depth cotangent of the gradient records (render modes with expected depth) ---- */
+extern "C" int egs_projection_bwd_depth(
+    int32_t C, int32_t N, const float* means, const float* quats, const float* scales, const float* opacities,
+    const float* sh_coeffs, int32_t K, int32_t sh_degree, int32_t colors_per_camera, const float* viewmats,
+    const float* Ks, int32_t width, int32_t height, float eps2d, const int32_t* radii, const float* colors,
+    const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats, float* v_scales,
+    float* v_opacities, float* v_sh_coeffs, float* absgrad, int32_t antialiased, float* v_viewmats, float* v_Ks,
+    void* workspace, int64_t workspace_bytes, egs_stream_t stream) {
+  return projection_bwd_impl(C, N, means, quats, scales, antialiased ? opacities : nullptr, sh_coeffs, nullptr, K,
+                             sh_degree, colors_per_camera, viewmats, Ks, width, height, eps2d, radii, colors, v_splats,
+                             v_means2d_extra, v_means, v_quats, v_scales, v_opacities, v_sh_coeffs, nullptr, absgrad,
+                             stream, antialiased ? 1 : 0, v_viewmats, workspace, workspace_bytes, v_Ks, 1);
 }

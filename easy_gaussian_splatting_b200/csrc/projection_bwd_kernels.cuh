@@ -1,4 +1,5 @@
-// The projection backward kernels (generic, K = 16, SH degree 4), compiled four times, each with two flags
+// The projection backward kernels (generic, K = 16, SH degree 4), compiled four times, each with two flags (and the
+// four again with the depth flag below)
 // (projection_kernels.cuh includes this file in egs and egs::percam, projection.cu includes it in egs::ksgrad and
 // egs::ksgrad::percam):
 // - kPerCameraSh: SH coefficients [N,K,3] shared by all cameras (or direct colours), or [C,N,K,3], one row per
@@ -6,6 +7,9 @@
 // - kKsGrad: the camera-gradient (VG) forms also reduce the intrinsics gradient, 4 more floats per partial.
 // egs and egs::percam hold the kernels without intrinsics gradients, egs::ksgrad and egs::ksgrad::percam those with.
 // Both flags are behind `if constexpr`, so the kernels of egs keep their names and compile exactly as without them.
+// A third flag, kDepthGrad, passes the depth cotangent of gradient-record slot 11 (written by the depth blend) to
+// project_bwd; projection.cu includes the file again under egs::depth with it set.  The forms without it read 0, so
+// their registers and code are those of the kernels before the flag existed.
 // (No include guard on purpose.)
 
 // Camera-gradient floats per (camera, Gaussian) pair and per warp partial: 15 padded to 16 for the view matrices, with
@@ -94,7 +98,7 @@ __global__ void __launch_bounds__(kProjBwdThreads) projection_bwd_kernel(const P
       float v_comp = 0.f, w_opac = 1.f;
       if (p.antialiased) { v_comp = g1.y * __ldg(p.opacities + n); w_opac = o.comp; }
       if (o.radius > 0)
-        project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, v_comp, p.eps2d,
+        project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, v_comp, p.eps2d,
                     VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
       v_opac += g1.y * w_opac;
       v_rgb[0] = g1.z; v_rgb[1] = g1.w; v_rgb[2] = g2.x;
@@ -137,8 +141,9 @@ __global__ void __launch_bounds__(kProjBwdThreads) projection_bwd_kernel(const P
 // stages that camera's rows of the Gaussians it sees in co_tile, accumulates into vc_tile and stores all 32 gradient
 // rows of the camera (zeros for rows it does not see) coalesced before moving on.
 // kKsGrad (VG forms only): the partials also carry v_fx, v_fy, v_cx, v_cy.
+// kDepthGrad: the per-camera form spills 16 bytes at 168 registers even without VG, so it runs 2 CTAs per SM as well.
 template <bool AA, bool VG = false>
-__global__ void EGS_PB_BOUNDS((kPerCameraSh || kKsGrad) && VG) projection_bwd_sh16_kernel(const ProjBwdParams p) {
+__global__ void EGS_PB_BOUNDS(((kPerCameraSh || kKsGrad) && VG) || (kDepthGrad && kPerCameraSh)) projection_bwd_sh16_kernel(const ProjBwdParams p) {
   static_assert(VG || !kKsGrad, "intrinsics gradients are reduced with the view-matrix gradient partials");
   extern __shared__ __align__(16) float smem_pb[];
   __shared__ Camera cams[kMaxCamerasSmem];
@@ -267,12 +272,12 @@ __global__ void EGS_PB_BOUNDS((kPerCameraSh || kKsGrad) && VG) projection_bwd_sh
           float op = __ldg(p.opacities + n);
           if (p.raw) op = act_sigmoid(op);
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, g1.y * op, p.eps2d,
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, g1.y * op, p.eps2d,
                         VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y * o.comp;
         } else {
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
                         VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y;
         }
@@ -476,13 +481,13 @@ __global__ void __launch_bounds__(kPB2Threads, kSh4BwdMinCtas) projection_bwd_sh
         project_fwd(mean, quat, scale, *cam, p.width, p.height, p.eps2d, 0.f, INFINITY, -1.f, st, o);
         if constexpr (AA) {
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale,
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale,
                         g1.y * __ldg(p.opacities + n), p.eps2d, VG ? vcam : nullptr, mean,
                         kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y * o.comp;
         } else {
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
+            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
                         VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y;
         }

@@ -123,7 +123,7 @@ def _tag_absgrad(target: Tensor, absgrad: Tensor, packed_index: Optional[Tensor]
     target.absgrad = absgrad if packed_index is None else absgrad.reshape(-1, 2)[packed_index]
 
 
-def _bin_and_blend(ctx, proj, backgrounds, width, height, grad_enabled=True, features=None):
+def _bin_and_blend(ctx, proj, backgrounds, width, height, grad_enabled=True, features=None, depth=False):
     """Binning + blend forward, enqueued without waiting for the intersection count (stages.isect_sorted_async): the
     buffers are sized from the previous call of this shape, the count is looked at only after the blend forward is
     in the queue, and a guess that turns out too small is repaired by running both again with the exact size.
@@ -131,12 +131,13 @@ def _bin_and_blend(ctx, proj, backgrounds, width, height, grad_enabled=True, fea
     used so that the backward pass can replay those lists in segments (stages.segment_policy).
     (grad_enabled is the CALLER's grad mode: inside Function.forward it is always off, and needs_input_grad stays
     true under no_grad.)  features: colours of any width ([N,D] / [C,N,D]) blended by the feature kernels instead of
-    the colours in the splat records; they are never checkpointed."""
+    the colours in the splat records; they are never checkpointed.  depth: the RGB blend with the depth as a fourth
+    channel (stages.rasterize_fwd_depth), never checkpointed either."""
     tw, th = stages.tile_grid(width, height)
     C = proj["radii"].shape[0]
     dev = proj["radii"].device
     seg, seg_min = 0, 0
-    if features is None and grad_enabled and any(ctx.needs_input_grad):
+    if features is None and not depth and grad_enabled and any(ctx.needs_input_grad):
         seg, seg_min = stages.segment_policy(stages.binning_hint(C, tw, th, dev), C * tw * th)
     capacity = None
     while True:
@@ -148,6 +149,9 @@ def _bin_and_blend(ctx, proj, backgrounds, width, height, grad_enabled=True, fea
             if features is not None:
                 rc, ra, last = stages.rasterize_fwd_features(proj["splats"], b.offsets, b.flat_cap, features, backgrounds,
                                                              width, height, n_isects=b.raster_n, tile_order=b.tile_order)
+            elif depth:
+                rc, ra, last = stages.rasterize_fwd_depth(proj["splats"], b.offsets, b.flat_cap, backgrounds, width, height,
+                                                          n_isects=b.raster_n, tile_order=b.tile_order)
             elif seg > 0:
                 rc, ra, last, ckpt = stages.rasterize_fwd_checkpointed(proj["splats"], b.offsets, b.flat_cap, backgrounds, width,
                                                                        height, seg, seg_min_len=seg_min, n_isects=b.raster_n,
@@ -179,6 +183,24 @@ def _zero_rgb(means: Tensor) -> Tensor:
     return torch.zeros(means.shape[0], 3, dtype=torch.float32, device=means.device)
 
 
+DEPTH_MODES = ("ED", "RGB+ED")
+
+
+def _depth_blend_inputs(mode: str, features: Optional[Tensor], backgrounds: Optional[Tensor], depths: Tensor):
+    """What the blend of a depth mode takes, as gsplat builds it: (features, backgrounds).  With feature colours the
+    depth is one more feature column ("RGB+ED": [C,N,D+1] rows of the colours and the depth, "ED": the depth alone)
+    and its background is 0; with RGB colours the depth comes from the splat records and features stays None.  In "ED"
+    the output does not depend on the background, which is not passed."""
+    if mode == "ED":
+        return (None if features is None else depths[..., None]), None
+    if features is None:
+        return None, backgrounds
+    C, N = depths.shape
+    rows = features if features.dim() == 3 else features[None].expand(C, N, -1)
+    bg = None if backgrounds is None else torch.cat([backgrounds, backgrounds.new_zeros(C, 1)], -1)
+    return torch.cat([rows, depths[..., None]], -1), bg
+
+
 class _Rasterization(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means, quats, scales, opacities, colors, viewmats, Ks, backgrounds, cfg):
@@ -194,14 +216,19 @@ class _Rasterization(torch.autograd.Function):
         feat = cfg.get("features", False)
         features = colors if feat else None
         rgb = _zero_rgb(means) if feat else colors
+        depth = cfg.get("render_mode", "RGB") in DEPTH_MODES
         with stages.nvtx_range("egs.projection_fwd"):
             proj = stages.projection_fwd(means, quats, scales, opacities, rgb, viewmats, Ks, width, height, sh_degree,
                                          eps2d=cfg["eps2d"], near_plane=cfg["near_plane"], far_plane=cfg["far_plane"],
                                          radius_clip=cfg["radius_clip"], antialiased=cfg["antialiased"])
         cfg["compensations"] = proj.get("compensations")  # non-differentiable side output, like the thunk below
         tiles_per_gauss = proj["tiles_per_gauss"]
-        binned, render_colors, render_alphas, last_ids, ckpt = _bin_and_blend(ctx, proj, backgrounds, width, height,
-                                                                             cfg.get("grad_enabled", True), features)
+        blend_bg = backgrounds
+        if depth:
+            features, blend_bg = _depth_blend_inputs(cfg["render_mode"], features, backgrounds, proj["depths"])
+        binned, render_colors, render_alphas, last_ids, ckpt = _bin_and_blend(ctx, proj, blend_bg, width, height,
+                                                                             cfg.get("grad_enabled", True), features,
+                                                                             depth=depth and features is None)
         # meta's three list entries are gsplat's lists, built on first access (not tensors: cannot be outputs); the
         # outputs below carry the tight lists the kernels used
         cfg["classic_lists"] = _ClassicLists(proj["means2d"], proj["radii"], proj["depths"], tiles_per_gauss,
@@ -214,7 +241,8 @@ class _Rasterization(torch.autograd.Function):
         # the backward pass walks the same (capacity-sized) list buffer the forward kernels used
         ctx.save_for_backward(means, quats, scales, colors, viewmats, Ks, backgrounds, proj["radii"], proj["colors"],
                               proj["splats"], isect_offsets, binned.flat_cap, render_alphas, last_ids,
-                              opacities, ckpt, render_colors if ckpt is not None else None)
+                              opacities, ckpt, render_colors if ckpt is not None else None,
+                              *((features, blend_bg) if depth else ()))
         nondiff = (proj["radii"], proj["depths"], proj["conics"], proj["colors"], tiles_per_gauss,
                    flatten_ids, isect_offsets, last_ids)
         ctx.mark_non_differentiable(*nondiff)
@@ -223,22 +251,37 @@ class _Rasterization(torch.autograd.Function):
     @staticmethod
     def backward(ctx, v_colors, v_alphas, v_means2d, *_unused):
         (means, quats, scales, colors, viewmats, Ks, backgrounds, radii, colors_rgb, splats, isect_offsets,
-         flatten_ids, render_alphas, last_ids, opacities, ckpt, render_colors) = ctx.saved_tensors
+         flatten_ids, render_alphas, last_ids, opacities, ckpt, render_colors, *depth_saved) = ctx.saved_tensors
         cfg = ctx.cfg
         width, height = cfg["width"], cfg["height"]
         C = viewmats.shape[0]
         feat = cfg.get("features", False)
+        mode = cfg.get("render_mode", "RGB")
+        depth = mode in DEPTH_MODES
+        # what the blend took: the colours and backgrounds as given, or in a depth mode _depth_blend_inputs'
+        blend_feat, blend_bg = depth_saved if depth else (colors if feat else None, backgrounds)
         if v_colors is None:
-            v_colors = torch.zeros(C, height, width, colors.shape[-1] if feat else 3, dtype=torch.float32, device=means.device)
+            n_out = blend_feat.shape[-1] if blend_feat is not None else 4 if depth else 3
+            v_colors = torch.zeros(C, height, width, n_out, dtype=torch.float32, device=means.device)
         if v_alphas is None:
             v_alphas = torch.zeros(C, height, width, 1, dtype=torch.float32, device=means.device)
-        if feat:
+        if blend_feat is not None:
             with stages.nvtx_range("egs.rasterize_bwd"):
                 v_splats, v_features = stages.rasterize_bwd_features(
-                    splats, isect_offsets, flatten_ids, colors, backgrounds, width, height, render_alphas, last_ids,
+                    splats, isect_offsets, flatten_ids, blend_feat, blend_bg, width, height, render_alphas, last_ids,
                     v_colors, v_alphas, n_isects=ctx.raster_n, tile_order=ctx.tile_order,
-                    want_features_grad=ctx.needs_input_grad[4])
+                    want_features_grad=ctx.needs_input_grad[4] or depth)
+            if depth:  # the depth column's gradient is the v_depth slot of the records; the rest the colours'
+                v_splats[..., 11] = v_features[..., -1]
+                v_features = v_features[..., :-1]
+                if colors.dim() == 2 and mode != "ED":
+                    v_features = v_features.sum(0)  # [N,D] colours were expanded to every camera's rows
             colors = _zero_rgb(means)  # what the projection saw; its colour gradient is discarded
+        elif depth:
+            with stages.nvtx_range("egs.rasterize_bwd"):
+                v_splats = stages.rasterize_bwd_depth(splats, isect_offsets, flatten_ids, blend_bg, width, height,
+                                                      render_alphas, last_ids, v_colors, v_alphas, n_isects=ctx.raster_n,
+                                                      tile_order=ctx.tile_order)
         else:
             v_splats = _blend_backward(ctx, splats, isect_offsets, flatten_ids, backgrounds, width, height, render_colors,
                                        render_alphas, last_ids, v_colors, v_alphas, ckpt)
@@ -247,6 +290,8 @@ class _Rasterization(torch.autograd.Function):
         # the camera keywords are passed only when their gradients are wanted: without them the call is exactly the
         # classic one
         want_cam = _camera_grad_keywords(ctx.needs_input_grad[5], ctx.needs_input_grad[6])
+        if depth:
+            want_cam["depth_grad"] = True
         with stages.nvtx_range("egs.projection_bwd"):
             out = stages.projection_bwd(means, quats, scales, colors, viewmats, Ks, width, height, cfg["sh_degree"],
                                         cfg["eps2d"], radii, colors_rgb, v_splats, v_means2d, want_absgrad=target is not None,
@@ -260,8 +305,11 @@ class _Rasterization(torch.autograd.Function):
             # same contract as gsplat: attribute tagging on the tensor object handed out in meta
             _tag_absgrad(target, out[5], getattr(ctx, "packed_index", None))
         v_bg = None
-        if backgrounds is not None and ctx.needs_input_grad[7]:
-            v_bg = ((1.0 - render_alphas) * v_colors).sum(dim=(1, 2))
+        if mode == "ED":  # gsplat: the output depends neither on the colours nor on the background
+            v_cols = None
+        elif backgrounds is not None and ctx.needs_input_grad[7]:
+            vc = v_colors[..., :backgrounds.shape[-1]] if depth else v_colors  # the colour channels only
+            v_bg = ((1.0 - render_alphas) * vc).sum(dim=(1, 2))
         return v_means, v_quats, v_scales, v_opac, v_cols, v_viewmats, v_Ks, v_bg, None
 
 
@@ -425,9 +473,15 @@ def rasterization(
     offset): camera c colours Gaussian n from its own row colors[c, n], and colors.grad is [C,N,K,3], one row per
     (camera, Gaussian), 0 for pairs the camera culls.
     ``sh_degree`` may be 0..4, as gsplat's fast SH evaluates; degree 4 needs K >= 25 and leaves the bands past 4 a
-    zero gradient."""
-    if render_mode != "RGB":
-        raise NotImplementedError(f"render_mode={render_mode!r}: only 'RGB' is implemented (the reference's mode)")
+    zero gradient.
+    ``render_mode`` "RGB", "ED" or "RGB+ED" (gsplat's expected depth): the camera-space depth of each Gaussian
+    (``meta["depths"]``) is blended as one more channel with background 0 and divided by
+    ``render_alphas.clamp(min=1e-10)``.  "RGB+ED" returns [C,H,W,D+1] (the colours, then the expected depth), "ED"
+    [C,H,W,1]; ``render_alphas`` and ``meta`` are those of "RGB".  Gradients of the depth reach the geometry,
+    ``viewmats`` and absgrad; in "ED" ``colors`` and ``backgrounds`` get none, in "RGB+ED" ``backgrounds`` [C,D] get the
+    colour channels' gradient.  "D" and "RGB+D" raise ``NotImplementedError``."""
+    if render_mode not in ("RGB",) + DEPTH_MODES:
+        raise NotImplementedError(f"render_mode={render_mode!r}: 'RGB', 'ED' and 'RGB+ED' are implemented")
     if rasterize_mode not in ("classic", "antialiased"):
         raise ValueError(f"rasterize_mode must be 'classic' or 'antialiased', got {rasterize_mode!r}")
     if sparse_grad:
@@ -442,7 +496,7 @@ def rasterization(
     cfg = dict(width=width, height=height, sh_degree=sh_degree, eps2d=float(eps2d), near_plane=float(near_plane),
                far_plane=float(far_plane), radius_clip=float(radius_clip), absgrad=bool(absgrad),
                antialiased=rasterize_mode == "antialiased", grad_enabled=torch.is_grad_enabled(),
-               features=sh_degree is None and colors.shape[-1] != 3)
+               features=sh_degree is None and colors.shape[-1] != 3, render_mode=render_mode)
     outs = _Rasterization.apply(means, quats, scales, opacities, colors, viewmats, Ks, backgrounds, cfg)
     meta_colors = None
     if cfg["features"]:  # gsplat: the colours as given, per (camera, Gaussian)
@@ -451,8 +505,14 @@ def rasterization(
     comp = cfg.pop("compensations", None)
     if comp is not None:
         opacities_cn = opacities_cn * comp  # gsplat: meta["opacities"] = opacities * compensations
-    return _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad, packed=bool(packed),
-                   meta_colors=meta_colors)
+    render_colors, render_alphas, meta = _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad,
+                                                 packed=bool(packed), meta_colors=meta_colors)
+    if render_mode in DEPTH_MODES:
+        # gsplat: the accumulated depth (last channel) over the alpha is the expected depth; autograd carries the
+        # division into the alpha gradient
+        ed = render_colors[..., -1:] / render_alphas.clamp(min=1e-10)
+        render_colors = ed if render_mode == "ED" else torch.cat([render_colors[..., :-1], ed], dim=-1)
+    return render_colors, render_alphas, meta
 
 
 def _finish(outs, cfg, opacities_cn, width, height, tile_size, C, absgrad, packed=False, meta_colors=None):

@@ -196,12 +196,15 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
                    width: int, height: int, sh_degree: Optional[int], eps2d: float, radii: Tensor,
                    colors_rgb: Tensor, v_splats: Tensor, v_means2d_extra: Optional[Tensor] = None,
                    want_absgrad: bool = False, antialiased_opacities: Optional[Tensor] = None,
-                   opacities: Optional[Tensor] = None, want_viewmats_grad: bool = False, want_Ks_grad: bool = False):
+                   opacities: Optional[Tensor] = None, want_viewmats_grad: bool = False, want_Ks_grad: bool = False,
+                   depth_grad: bool = False):
     """g8+g9. -> v_means[N,3], v_quats[N,4], v_scales[N,3], v_opacities[N], v_colors (shape of colors)
     (+ absgrad[C,N,2] when want_absgrad) (+ v_viewmats[C,4,4] when want_viewmats_grad) (+ v_Ks[C,3,3] when
     want_Ks_grad, always last).
     antialiased_opacities: the opacities[N] of an antialiased forward; opacities: only consulted for a registered
-    gradient buffer (register_grad_target)."""
+    gradient buffer (register_grad_target).
+    depth_grad: also take slot 11 of v_splats (v_depth, from rasterize_bwd_depth) as the gradient w.r.t. the
+    camera-space depths (egs_projection_bwd_depth); otherwise that slot is not read."""
     lib = _lib.load()
     dev = means.device
     means, quats, scales, colors, viewmats, Ks = dense_inputs(means, quats, scales, colors, viewmats, Ks)
@@ -227,11 +230,17 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
     with torch.cuda.device(dev):
         if want_viewmats_grad:
             v_viewmats = torch.empty(C, 4, 4, dtype=torch.float32, device=dev)
-        if want_Ks_grad or want_viewmats_grad:
+        if want_Ks_grad or want_viewmats_grad or depth_grad:
             aa = antialiased_opacities is not None
             aa_op = _f32c(antialiased_opacities, "opacities") if aa else None
             head = (C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail[:-1], int(aa), _ptr(v_viewmats))
-        if want_Ks_grad:  # one launch for both camera gradients
+        if depth_grad:
+            if want_Ks_grad:
+                v_Ks = torch.empty(C, 3, 3, dtype=torch.float32, device=dev)
+            ws = (_intrinsics_workspace(lib, C, N, dev) if want_Ks_grad else _viewmats_workspace(lib, C, N, dev)
+                  if want_viewmats_grad else None)
+            rc = lib.egs_projection_bwd_depth(*head, _ptr(v_Ks), _ptr(ws), 0 if ws is None else ws.numel(), tail[-1])
+        elif want_Ks_grad:  # one launch for both camera gradients
             v_Ks = torch.empty(C, 3, 3, dtype=torch.float32, device=dev)
             ws = _intrinsics_workspace(lib, C, N, dev)
             rc = lib.egs_projection_bwd_intrinsics(*head, _ptr(v_Ks), _ptr(ws), ws.numel(), tail[-1])
@@ -857,6 +866,48 @@ def rasterize_bwd(splats: Tensor, isect_offsets: Tensor, flatten_ids: Tensor, ba
                                    _ptr(bg), int(width), int(height), tw, th, _ptr(render_alphas), _ptr(last_ids),
                                    _ptr(v_c), _ptr(v_a), _ptr(v_splats), _ptr(tile_order), _stream(dev))
     _lib.check(rc, "egs_rasterize_bwd")
+    return v_splats
+
+
+def rasterize_fwd_depth(splats: Tensor, isect_offsets: Tensor, flatten_ids: Tensor, backgrounds: Optional[Tensor],
+                        width: int, height: int, n_isects: Optional[int] = None, tile_order: Optional[Tensor] = None):
+    """g6 with the depth (record slot 9) as a fourth channel -> render_colors[C,H,W,4] = (r, g, b, accumulated depth),
+    render_alphas[C,H,W,1], last_ids[C,H,W].  backgrounds [C,3] apply to r, g, b; the depth's background is 0.
+    Arguments as rasterize_fwd."""
+    lib = _lib.load()
+    dev = splats.device
+    C, N = splats.shape[:2]
+    th, tw = isect_offsets.shape[1:]
+    colors = torch.empty(C, height, width, 4, dtype=torch.float32, device=dev)
+    alphas = torch.empty(C, height, width, 1, dtype=torch.float32, device=dev)
+    last = torch.empty(C, height, width, dtype=torch.int32, device=dev)
+    bg = None if backgrounds is None else _f32c(backgrounds, "backgrounds")
+    with torch.cuda.device(dev):
+        rc = lib.egs_rasterize_fwd_depth(C, N, flatten_ids.numel() if n_isects is None else int(n_isects), _ptr(splats),
+                                         _ptr(isect_offsets), _ptr(flatten_ids), _ptr(bg), int(width), int(height), tw, th,
+                                         _ptr(colors), _ptr(alphas), _ptr(last), _ptr(tile_order), _stream(dev))
+    _lib.check(rc, "egs_rasterize_fwd_depth")
+    return colors, alphas, last
+
+
+def rasterize_bwd_depth(splats: Tensor, isect_offsets: Tensor, flatten_ids: Tensor, backgrounds: Optional[Tensor],
+                        width: int, height: int, render_alphas: Tensor, last_ids: Tensor, v_render_colors: Tensor,
+                        v_render_alphas: Tensor, n_isects: Optional[int] = None,
+                        tile_order: Optional[Tensor] = None) -> Tensor:
+    """g7 of rasterize_fwd_depth: v_render_colors [C,H,W,4] -> v_splats[C,N,12] with v_depth in slot 11."""
+    lib = _lib.load()
+    dev = splats.device
+    C, N = splats.shape[:2]
+    th, tw = isect_offsets.shape[1:]
+    v_splats = torch.zeros(C, N, SPLAT_FLOATS, dtype=torch.float32, device=dev)
+    bg = None if backgrounds is None else _f32c(backgrounds, "backgrounds")
+    v_c, v_a = _f32c(v_render_colors, "v_render_colors"), _f32c(v_render_alphas, "v_render_alphas")
+    with torch.cuda.device(dev):
+        rc = lib.egs_rasterize_bwd_depth(C, N, flatten_ids.numel() if n_isects is None else int(n_isects), _ptr(splats),
+                                         _ptr(isect_offsets), _ptr(flatten_ids), _ptr(bg), int(width), int(height), tw, th,
+                                         _ptr(render_alphas), _ptr(last_ids), _ptr(v_c), _ptr(v_a), _ptr(v_splats),
+                                         _ptr(tile_order), _stream(dev))
+    _lib.check(rc, "egs_rasterize_bwd_depth")
     return v_splats
 
 

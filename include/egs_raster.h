@@ -42,7 +42,9 @@ enum egs_status {
  *                sigma_cut = ln(255 * opacity) (+ margin): the largest sigma at which alpha can reach 1/255.  The
  *                blending kernels drop a Gaussian for a warp when min sigma over the warp's pixels exceeds it
  *                (+inf disables that culling; <= 0 = never visible)
- * grad  record : {v_x, v_y, v_conic_a, v_conic_b | v_conic_c, v_opacity, v_r, v_g | v_b, |v_x|, |v_y|, 0} */
+ * grad  record : {v_x, v_y, v_conic_a, v_conic_b | v_conic_c, v_opacity, v_r, v_g | v_b, |v_x|, |v_y|, v_depth}
+ *                v_depth: gradient w.r.t. the camera-space depth of slot 9, written by egs_rasterize_bwd_depth (0 from
+ *                every other blend backward); egs_projection_bwd_depth routes it into v_means and v_viewmats */
 #define EGS_SPLAT_FLOATS 12
 
 int egs_abi_version(void);
@@ -200,6 +202,23 @@ int egs_projection_bwd_raw_intrinsics(int32_t C, int32_t N, const float* means, 
                                       float* v_sh_0, float* v_sh_rest, float* absgrad, float* v_viewmats, float* v_Ks,
                                       void* workspace, int64_t workspace_bytes, egs_stream_t stream);
 
+/* ---- the depth cotangent (render modes with expected depth) ---------------------------------------------------------
+ * The backward entries above also take slot 11 of the gradient records (v_depth, written by egs_rasterize_bwd_depth) as
+ * the gradient w.r.t. the camera-space depth z = R[2,:] m + t[2] of each visible (camera, Gaussian): it adds
+ * v_depth * R[2,:] to v_means and, when v_viewmats is requested, v_depth * (m, 1) to row 2 of v_viewmats.  v_Ks does not
+ * depend on it (z does not depend on K).  One entry for every form: antialiased as in egs_projection_bwd_viewmats;
+ * v_viewmats and v_Ks both nullable, with egs_projection_bwd_intrinsics_workspace_bytes(C, N) bytes of workspace when
+ * v_Ks is given, egs_projection_bwd_viewmats_workspace_bytes(C, N) when only v_viewmats is, none otherwise.  The entries
+ * above read v_depth as 0; their kernels are compiled separately from these. */
+int egs_projection_bwd_depth(int32_t C, int32_t N, const float* means, const float* quats, const float* scales,
+                             const float* opacities, const float* sh_coeffs, int32_t K, int32_t sh_degree,
+                             int32_t colors_per_camera, const float* viewmats, const float* Ks, int32_t width,
+                             int32_t height, float eps2d, const int32_t* radii, const float* colors,
+                             const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
+                             float* v_scales, float* v_opacities, float* v_sh_coeffs, float* absgrad,
+                             int32_t antialiased, float* v_viewmats, float* v_Ks, void* workspace,
+                             int64_t workspace_bytes, egs_stream_t stream);
+
 /* ---- g3: exclusive scan of tiles_per_gauss, then key emission -------------------------------------
  * Replaces `torch.cumsum` + the second launch of gsplat `isect_tiles`.
  * egs_exclusive_scan: out[i] = sum_{j<i} in[j] (int64), *total = sum of all (device int64). */
@@ -318,6 +337,24 @@ int egs_rasterize_bwd(int32_t C, int32_t N, int64_t n_isects, const float* splat
                       int32_t tile_width, int32_t tile_height, const float* render_alphas,
                       const int32_t* last_ids, const float* v_render_colors, const float* v_render_alphas,
                       float* v_splats, const int32_t* tile_order, egs_stream_t stream);
+
+/* ---- g6 / g7 with the depth as a fourth channel (gsplat's render_mode "ED" / "RGB+ED") ------------------------------
+ * egs_rasterize_fwd / _bwd with one more blended channel: the camera-space depth of splat-record slot 9, background 0.
+ * egs_rasterize_fwd_depth: render_colors[C,H,W,4] = {r, g, b, accumulated depth}; backgrounds[C,3] (nullable) apply to
+ *   r, g, b only.  render_alphas and last_ids, and the r, g, b channels, are bit-identical to egs_rasterize_fwd's.
+ * egs_rasterize_bwd_depth: v_render_colors[C,H,W,4].  The depth channel enters v_alpha like a colour channel, and
+ *   sum fac * v_depth_channel is added into slot 11 (v_depth) of the gradient records.  With a zero depth cotangent,
+ *   slots 0-10 equal egs_rasterize_bwd's.
+ * Neither has a segmented / checkpointed form: long lists are replayed in one piece. */
+int egs_rasterize_fwd_depth(int32_t C, int32_t N, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
+                            const int32_t* flatten_ids, const float* backgrounds, int32_t width, int32_t height,
+                            int32_t tile_width, int32_t tile_height, float* render_colors, float* render_alphas,
+                            int32_t* last_ids, const int32_t* tile_order, egs_stream_t stream);
+int egs_rasterize_bwd_depth(int32_t C, int32_t N, int64_t n_isects, const float* splats, const int32_t* tile_offsets,
+                            const int32_t* flatten_ids, const float* backgrounds, int32_t width, int32_t height,
+                            int32_t tile_width, int32_t tile_height, const float* render_alphas,
+                            const int32_t* last_ids, const float* v_render_colors, const float* v_render_alphas,
+                            float* v_splats, const int32_t* tile_order, egs_stream_t stream);
 
 /* ---- g7 on long lists: segmented replay ---------------------------------------------------------------------------
  * A tile whose list has thousands of entries (object-centric scenes: a few hundred tiles hold the whole object) makes
