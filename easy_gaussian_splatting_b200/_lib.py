@@ -45,6 +45,10 @@ _SIGNATURES = {
                                                     P, P, P, P, P, P, P, P, P, P, I64, P]),
     "egs_projection_bwd_depth": (c_int32, [I32, I32, P, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, P, P, P, P,
                                           P, P, P, P, P, P, I32, P, P, P, I64, P]),
+    "egs_projection_fwd_camera_model": (c_int32, [I32, I32, I32, P, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, F32,
+                                                  F32, F32, I32, I32, I32, P, P, P, P, P, P, P, P, P, P]),
+    "egs_projection_bwd_camera_model": (c_int32, [I32, I32, I32, P, P, P, P, P, I32, I32, I32, P, P, I32, I32, F32, P,
+                                                  P, P, P, P, P, P, P, P, P, I32, P, P, P, I64, P]),
     "egs_exclusive_scan_workspace_bytes": (c_int64, [I64]),
     "egs_exclusive_scan": (c_int32, [I64, P, P, P, P, I64, P]),
     "egs_isect_emit": (c_int32, [I32, I32, P, P, P, P, I32, I32, I32, I32, I64, P, P, P]),

@@ -24,10 +24,12 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler",
           "-Xptxas", "-v", f"-I{INCLUDE}"]
 # Translation units whose fp32 results must be bit-identical to the oracle: no FMA contraction,
 # IEEE division / sqrt (nvcc defaults), no fast-math.
-EXACT_UNITS = {"projection.cu", "binning.cu"}
+EXACT_UNITS = {"projection.cu", "projection_ortho.cu", "projection_fisheye.cu", "binning.cu"}
 # FP32-throughput-bound units: FMA contraction on, fast intrinsics are explicit in the source.
 FLAGS = {
     "projection.cu": ["-fmad=false"],
+    "projection_ortho.cu": ["-fmad=false"],
+    "projection_fisheye.cu": ["-fmad=false"],
     "binning.cu": ["-fmad=false"],
 }
 

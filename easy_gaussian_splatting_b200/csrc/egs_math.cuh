@@ -85,7 +85,98 @@ struct ProjState {
   float a, b, d, det;         // blurred 2D covariance and its determinant
   float det_orig;             // determinant before the eps2d blur (antialiased mode: compensation factor)
   bool clamp_x, clamp_y;      // fov clamp active
+  float J01, J10;             // kOrtho / kFisheye: the rest of the 2x3 Jacobian (0 for kOrtho)
+  float fs, fg, fq, r2;       // kFisheye: theta / r, g (fisheye_theta_over_r), 1 / (r^2 + z^2), r^2 = x^2 + y^2
 };
+
+// ---- camera models -------------------------------------------------------------------------------------------------
+// The camera enters the projection only through (x, y, z, Sigma_cam) -> (means2d, cov2d = J Sigma_cam J^T) and its VJP;
+// project_fwd / project_bwd take the model as a template argument, kPinhole by default.
+//   kPinhole: means2d = (fx x / z + cx, fy y / z + cy), gsplat's persp_proj J with the 1.3 x fov clamp (the code below
+//             the model switch is the one every pinhole kernel has always compiled).
+//   kOrtho:   means2d = (fx x + cx, fy y + cy), J = [[fx, 0, 0], [0, fy, 0]], no clamp.
+//   kFisheye: equidistant, r = sqrt(x^2 + y^2), theta = atan2(r, z): means2d = (fx x theta / r + cx, fy y theta / r + cy),
+//             J the exact Jacobian of means2d (gsplat's fisheye_proj J), no clamp.
+// Culling (near / far on z, eps2d blur, radius, off-screen test) and the compensation are the same for all three.
+constexpr int kPinhole = 0, kOrtho = 1, kFisheye = 2;
+
+// atan(sqrt(u)) / sqrt(u) and (1 / (1 + u) - atan(sqrt(u)) / sqrt(u)) / u on u in [0, 1]: fp32 polynomials fitted by
+// scripts/fit_fisheye_theta.py (0.86 and 2.6 ulp there), evaluated by Horner from the highest term, mul then add.
+EGS_HD float fisheye_poly_p(float u) {
+  float p = 0.0010774789843708277f;
+  p = p * u + -0.007134431507438421f;
+  p = p * u + 0.022145025432109833f;
+  p = p * u + -0.044218774884939194f;
+  p = p * u + 0.0670754536986351f;
+  p = p * u + -0.0879582092165947f;
+  p = p * u + 0.11054043471813202f;
+  p = p * u + -0.142791748046875f;
+  p = p * u + 0.1999961882829666f;
+  p = p * u + -0.33333325386047363f;
+  p = p * u + 1.0f;
+  return p;
+}
+
+EGS_HD float fisheye_poly_h(float u) {
+  float p = -0.015319157391786575f;
+  p = p * u + 0.09921801835298538f;
+  p = p * u + -0.29700547456741333f;
+  p = p * u + 0.5588876008987427f;
+  p = p * u + -0.7710589170455933f;
+  p = p * u + 0.876106321811676f;
+  p = p * u + -0.9004436731338501f;
+  p = p * u + 0.8879852890968323f;
+  p = p * u + -0.8571013808250427f;
+  p = p * u + 0.7999998927116394f;
+  p = p * u + -0.6666666865348816f;
+  return p;
+}
+
+// a * b = p + e exactly: Dekker's product with Veltkamp's split (round to nearest, no FMA, |a|, |b| < 1e34)
+EGS_HD void two_prod(float a, float b, float& p, float& e) {
+  const float ca = 4097.0f * a, cb = 4097.0f * b;
+  const float ah = ca - (ca - a), bh = cb - (cb - b);
+  const float al = a - ah, bl = b - bh;
+  p = a * b;
+  e = ((ah * bh - p) + ah * bl + al * bh) + al * bl;
+}
+
+// s = theta / r with theta = atan2(r, z) in [0, pi], and g = (1 / r) ds/dr = (z q - s) / r^2, q = 1 / (r^2 + z^2), for
+// r = sqrt(r2) >= 0.  Built only from +, x, / (no atan2f, whose device and host results differ), so that a CPU
+// reference reproduces it bit for bit.  CANONICAL OP ORDER, four ranges of theta (r > z in all but the first):
+//   r <= z     (theta <= pi/4):           u = r2 / (z * z), s = P(u) / z,  g = H(u) / ((z * z) * z)
+//   z >= r / 2 (theta <= atan 2):         t = (r - z) / (r + z), d = (pi/4)_lo + t * P(t * t), hi = (pi/4)_hi
+//   r > -z     (theta < 3pi/4):           t = z / r,             d = (pi/2)_lo - t * P(t * t), hi = (pi/2)_hi
+//   otherwise  (theta >= 3pi/4):          t = r / (-z),          d = pi_lo - t * P(t * t),     hi = pi_hi
+//   then s = (d + hi) / r corrected by the remainder of the division as written below, g = (z * q - s) / r2
+//   (_hi + _lo is the fp32 split of the constant).  The second range keeps |atan t| below 0.42 theta, so that its
+//   error stays small against theta.  Measured error of s against fp64: 1.6 ulp at most over [0, pi).
+// The first range does not use r at all: s and g are exact limits at r = 0 (s = 1/z) and keep full precision for any
+// r / z (g by its own polynomial; the direct formula cancels there).  r = 0 with z <= 0 gives non-finite values, which
+// the projection culls.
+EGS_HD void fisheye_theta_over_r(float r, float r2, float z, float q, float& s, float& g) {
+  if (r <= z) {
+    const float u = r2 / (z * z);
+    s = fisheye_poly_p(u) / z;
+    g = fisheye_poly_h(u) / ((z * z) * z);
+    return;
+  }
+  const bool low = z >= 0.5f * r, mid = r > -z;
+  const float t = low ? (r - z) / (r + z) : mid ? z / r : r / (-z);
+  const float u = t * t;
+  const float at = t * fisheye_poly_p(u);
+  const float hi = low ? 0.7853981852531433f : mid ? 1.5707963705062866f : 3.1415927410125732f;
+  const float d = low ? -2.1855694143368964e-08f + at : (mid ? -4.371138828673793e-08f : -8.742277657347586e-08f) - at;
+  // theta = th + tl exactly (|d| < hi), s0 = th / r, and the remainder th + tl - s0 r of that division (s0 r = p + e
+  // exactly, th - p exact) corrects it: neither the rounding of theta nor that of the division reaches s
+  const float th = d + hi;
+  const float tl = d - (th - hi);
+  const float s0 = th / r;
+  float p, e;
+  two_prod(s0, r, p, e);
+  s = s0 + (((th - p) - e) + tl) / r;
+  g = (z * q - s) / r2;
+}
 
 struct ProjOut {
   float m2x, m2y, depth, ca, cb, cc;
@@ -94,7 +185,8 @@ struct ProjOut {
   int32_t radius;             // 0 = culled
 };
 
-// Returns true when the Gaussian is visible.  st is filled as far as the computation went.
+// Returns true when the Gaussian is visible.  st is filled as far as the computation went.  CM: the camera model.
+template <int CM = kPinhole>
 EGS_HD bool project_fwd(const float mean[3], const float quat[4], const float scale[3], const Camera& cam,
                         float width, float height, float eps2d, float near_plane, float far_plane,
                         float radius_clip, ProjState& st, ProjOut& o) {
@@ -132,6 +224,8 @@ EGS_HD bool project_fwd(const float mean[3], const float quat[4], const float sc
 #undef EGS_SC
   st.k[0] = k00; st.k[1] = k01; st.k[2] = k02; st.k[3] = k11; st.k[4] = k12; st.k[5] = k22;
   float fx = cam.fx, fy = cam.fy;
+  float a, b, d, m2x, m2y;
+  if constexpr (CM == kPinhole) {
   float tan_fovx = (0.5f * width) / fx;
   float tan_fovy = (0.5f * height) / fy;
   float lim_x = 1.3f * tan_fovx;
@@ -154,11 +248,48 @@ EGS_HD bool project_fwd(const float mean[3], const float quat[4], const float sc
   float B02 = J00 * k02 + J02 * k22;
   float B11 = J11 * k11 + J12 * k12;
   float B12 = J11 * k12 + J12 * k22;
-  float a = B00 * J00 + B02 * J02;
-  float b = B01 * J11 + B02 * J12;
-  float d = B11 * J11 + B12 * J12;
-  float m2x = (fx * x) * rz + cam.cx;
-  float m2y = (fy * y) * rz + cam.cy;
+  a = B00 * J00 + B02 * J02;
+  b = B01 * J11 + B02 * J12;
+  d = B11 * J11 + B12 * J12;
+  m2x = (fx * x) * rz + cam.cx;
+  m2y = (fy * y) * rz + cam.cy;
+  } else if constexpr (CM == kOrtho) {
+    // CANONICAL: cov2d = (fx k00 fx, fx k01 fy, fy k11 fy) in that order; means2d = fx x + cx
+    st.J00 = fx; st.J01 = 0.f; st.J02 = 0.f; st.J10 = 0.f; st.J11 = fy; st.J12 = 0.f;
+    a = (fx * k00) * fx;
+    b = (fx * k01) * fy;
+    d = (fy * k11) * fy;
+    m2x = fx * x + cam.cx;
+    m2y = fy * y + cam.cy;
+  } else {
+    static_assert(CM == kFisheye, "unknown camera model");
+    // CANONICAL: r2 = x*x + y*y, r = sqrt(r2), q = 1 / (r2 + z*z), (s, g) = fisheye_theta_over_r, then
+    // J0. = fx (s + (x*x) g, (x*y) g, -(x q)), J1. = fy ((x*y) g, s + (y*y) g, -(y q)) (fx times the bracket),
+    // B = J Sc row by row, B_ij = (J_i0 k0j + J_i1 k1j) + J_i2 k2j, cov2d_ij = (B_i0 J_j0 + B_i1 J_j1) + B_i2 J_j2,
+    // means2d = (fx x) s + cx
+    const float xx = x * x, yy = y * y;
+    const float r2 = xx + yy;
+    const float r = sqrtf(r2);
+    const float q = 1.0f / (r2 + z * z);
+    float s, g;
+    fisheye_theta_over_r(r, r2, z, q, s, g);
+    const float xyg = (x * y) * g;
+    const float J00 = fx * (s + xx * g), J01 = fx * xyg, J02 = -(fx * (x * q));
+    const float J10 = fy * xyg, J11 = fy * (s + yy * g), J12 = -(fy * (y * q));
+    st.J00 = J00; st.J01 = J01; st.J02 = J02; st.J10 = J10; st.J11 = J11; st.J12 = J12;
+    st.fs = s; st.fg = g; st.fq = q; st.r2 = r2;
+    const float B00 = (J00 * k00 + J01 * k01) + J02 * k02;
+    const float B01 = (J00 * k01 + J01 * k11) + J02 * k12;
+    const float B02 = (J00 * k02 + J01 * k12) + J02 * k22;
+    const float B10 = (J10 * k00 + J11 * k01) + J12 * k02;
+    const float B11 = (J10 * k01 + J11 * k11) + J12 * k12;
+    const float B12 = (J10 * k02 + J11 * k12) + J12 * k22;
+    a = (B00 * J00 + B01 * J01) + B02 * J02;
+    b = (B00 * J10 + B01 * J11) + B02 * J12;
+    d = (B10 * J10 + B11 * J11) + B12 * J12;
+    m2x = (fx * x) * s + cam.cx;
+    m2y = (fy * y) * s + cam.cy;
+  }
   const float det_orig = a * d - b * b;
   a = a + eps2d;
   d = d + eps2d;
@@ -255,6 +386,9 @@ constexpr int kKsGradFloats = 4;
 // gradient above) through mean_c = R m + t and cov_c = R Sigma R^T.  A literal nullptr compiles the block out.
 // v_K (nullable): also accumulates the intrinsics gradient above through means2d and the Jacobian J (which carries the
 // conic's and the compensation's cotangents).  A literal nullptr compiles the block out.
+// CM: the camera model of the project_fwd that filled st.  For kOrtho and kFisheye, v_K holds
+// v_fx = (v_m2x (m2x - cx) + sum_j vJ_0j J_0j) / fx (likewise v_fy), v_cx = v_m2x, v_cy = v_m2y.
+template <int CM = kPinhole>
 EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera& cam, float v_m2x, float v_m2y,
                         float v_depth, float v_ca, float v_cb, float v_cc, const ProjOut& o, float v_mean[3],
                         float v_quat[4], float v_scale[3], float v_comp = 0.f, float eps2d = 0.f,
@@ -278,15 +412,18 @@ EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera&
     V11 += vs * (om * q11 - eps2d * detc);
   }
   // cov2d = J Sc J^T ;  v_Sc = J^T V J ; v_J = 2 V J Sc
-  float J00 = st.J00, J02 = st.J02, J11 = st.J11, J12 = st.J12;
   const float* k = st.k;
+  float vx, vy, vz;
+  float vk00, vk01, vk02, vk10, vk11, vk12, vk20, vk21, vk22;
+  if constexpr (CM == kPinhole) {
+  float J00 = st.J00, J02 = st.J02, J11 = st.J11, J12 = st.J12;
   // VJ (2x3) = V * J
   float VJ00 = V00 * J00, VJ01 = V01 * J11, VJ02 = V00 * J02 + V01 * J12;
   float VJ10 = V01 * J00, VJ11 = V11 * J11, VJ12 = V01 * J02 + V11 * J12;
   // v_Sc (3x3 symmetric, full matrix gradient) = J^T (V J)
-  float vk00 = J00 * VJ00, vk01 = J00 * VJ01, vk02 = J00 * VJ02;
-  float vk10 = J11 * VJ10, vk11 = J11 * VJ11, vk12 = J11 * VJ12;
-  float vk20 = J02 * VJ00 + J12 * VJ10, vk21 = J02 * VJ01 + J12 * VJ11, vk22 = J02 * VJ02 + J12 * VJ12;
+  vk00 = J00 * VJ00; vk01 = J00 * VJ01; vk02 = J00 * VJ02;
+  vk10 = J11 * VJ10; vk11 = J11 * VJ11; vk12 = J11 * VJ12;
+  vk20 = J02 * VJ00 + J12 * VJ10; vk21 = J02 * VJ01 + J12 * VJ11; vk22 = J02 * VJ02 + J12 * VJ12;
   // v_J = 2 * (V J) Sc   (only the 4 structurally non-zero entries are needed)
   float vJ00 = 2.f * (VJ00 * k[0] + VJ01 * k[1] + VJ02 * k[2]);
   float vJ02 = 2.f * (VJ00 * k[2] + VJ01 * k[4] + VJ02 * k[5]);
@@ -307,9 +444,9 @@ EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera&
     v_K[3] += v_m2y;
   }
   // mean2d = (fx x rz + cx, fy y rz + cy); depth = z
-  float vx = fx * rz * v_m2x;
-  float vy = fy * rz * v_m2y;
-  float vz = -(fx * x * v_m2x + fy * y * v_m2y) * rz2 + v_depth;
+  vx = fx * rz * v_m2x;
+  vy = fy * rz * v_m2y;
+  vz = -(fx * x * v_m2x + fy * y * v_m2y) * rz2 + v_depth;
   // J00 = fx rz ; J11 = fy rz
   vz += -fx * rz2 * vJ00 - fy * rz2 * vJ11;
   // J02 = -fx tx rz^2 with tx = x (unclamped) or z*lim (clamped)
@@ -317,6 +454,64 @@ EGS_HD void project_bwd(const ProjState& st, const float scale[3], const Camera&
   else             { vz += fx * st.tx * rz3 * vJ02; }
   if (!st.clamp_y) { vy += -fy * rz2 * vJ12; vz += 2.f * fy * st.ty * rz3 * vJ12; }
   else             { vz += fy * st.ty * rz3 * vJ12; }
+  } else {
+    // full 2x3 J (kOrtho: only J00 = fx and J11 = fy, the zeros are literals and compile out)
+    const bool ortho = CM == kOrtho;
+    const float J00 = st.J00, J11 = st.J11;
+    const float J01 = ortho ? 0.f : st.J01, J02 = ortho ? 0.f : st.J02;
+    const float J10 = ortho ? 0.f : st.J10, J12 = ortho ? 0.f : st.J12;
+    const float VJ00 = V00 * J00 + V01 * J10, VJ01 = V00 * J01 + V01 * J11, VJ02 = V00 * J02 + V01 * J12;
+    const float VJ10 = V01 * J00 + V11 * J10, VJ11 = V01 * J01 + V11 * J11, VJ12 = V01 * J02 + V11 * J12;
+    vk00 = J00 * VJ00 + J10 * VJ10; vk01 = J00 * VJ01 + J10 * VJ11; vk02 = J00 * VJ02 + J10 * VJ12;
+    vk10 = J01 * VJ00 + J11 * VJ10; vk11 = J01 * VJ01 + J11 * VJ11; vk12 = J01 * VJ02 + J11 * VJ12;
+    vk20 = J02 * VJ00 + J12 * VJ10; vk21 = J02 * VJ01 + J12 * VJ11; vk22 = J02 * VJ02 + J12 * VJ12;
+    // v_J = 2 (V J) Sc, all six entries
+    const float vJ00 = 2.f * (VJ00 * k[0] + VJ01 * k[1] + VJ02 * k[2]);
+    const float vJ01 = 2.f * (VJ00 * k[1] + VJ01 * k[3] + VJ02 * k[4]);
+    const float vJ02 = 2.f * (VJ00 * k[2] + VJ01 * k[4] + VJ02 * k[5]);
+    const float vJ10 = 2.f * (VJ10 * k[0] + VJ11 * k[1] + VJ12 * k[2]);
+    const float vJ11 = 2.f * (VJ10 * k[1] + VJ11 * k[3] + VJ12 * k[4]);
+    const float vJ12 = 2.f * (VJ10 * k[2] + VJ11 * k[4] + VJ12 * k[5]);
+    const float fx = cam.fx, fy = cam.fy, x = st.x, y = st.y;
+    if constexpr (CM == kOrtho) {
+      // mean2d = (fx x + cx, fy y + cy), J constant in (x, y, z); depth = z
+      if (v_K != nullptr) {
+        v_K[0] += v_m2x * x + vJ00;
+        v_K[1] += v_m2y * y + vJ11;
+        v_K[2] += v_m2x;
+        v_K[3] += v_m2y;
+      }
+      vx = fx * v_m2x;
+      vy = fy * v_m2y;
+      vz = v_depth;
+    } else {
+      // J is the Jacobian of mean2d, so mean2d contributes J^T v_m2.  With s = theta / r, g = (1/r) ds/dr,
+      // q = 1 / (r^2 + z^2) and G = (1/r) dg/dr = (-2 z q^2 - 3 g) / r^2:  ds/d(x, y, z) = (x g, y g, -q),
+      // dg/d(x, y, z) = (x G, y G, 2 q^2), dq/d(x, y, z) = -2 q^2 (x, y, z).  sum_ij vJ_ij J_ij is
+      //   Phi = A0 (s + x^2 g) + A1 x y g + A2 (s + y^2 g) - (B0 x + B1 y) q
+      // with A0 = fx vJ00, A1 = fx vJ01 + fy vJ10, A2 = fy vJ11, B0 = fx vJ02, B1 = fy vJ12, and its gradient is
+      //   dPhi/dx = g ((3 A0 + A2) x + A1 y) + x Qf G - B0 q + 2 q^2 x L
+      //   dPhi/dy = g ((A0 + 3 A2) y + A1 x) + y Qf G - B1 q + 2 q^2 y L
+      //   dPhi/dz = -q (A0 + A2) + 2 q^2 Qf + 2 z q^2 L,    Qf = A0 x^2 + A1 x y + A2 y^2, L = B0 x + B1 y.
+      // Qf G is evaluated as (-2 z q^2 - 3 g) (Qf / r^2): Qf / r^2 is bounded, and the cancellation in the bracket
+      // is then scaled by |x| <= r, so no term loses precision as r -> 0 (r = 0: Qf / r^2 = 0).
+      const float s = st.fs, g = st.fg, q = st.fq, r2 = st.r2, z = st.z;
+      if (v_K != nullptr) {
+        v_K[0] += v_m2x * (x * s) + ((vJ00 * (s + (x * x) * g) + vJ01 * ((x * y) * g)) - vJ02 * (x * q));
+        v_K[1] += v_m2y * (y * s) + ((vJ10 * ((x * y) * g) + vJ11 * (s + (y * y) * g)) - vJ12 * (y * q));
+        v_K[2] += v_m2x;
+        v_K[3] += v_m2y;
+      }
+      const float A0 = fx * vJ00, A1 = fx * vJ01 + fy * vJ10, A2 = fy * vJ11, B0 = fx * vJ02, B1 = fy * vJ12;
+      const float Qf = A0 * (x * x) + A1 * (x * y) + A2 * (y * y);
+      const float L = B0 * x + B1 * y;
+      const float q2 = q * q;
+      const float QG = (-2.f * z * q2 - 3.f * g) * (r2 > 0.f ? Qf / r2 : 0.f);
+      vx = J00 * v_m2x + J10 * v_m2y + g * ((3.f * A0 + A2) * x + A1 * y) + x * QG - B0 * q + 2.f * q2 * x * L;
+      vy = J01 * v_m2x + J11 * v_m2y + g * ((A0 + 3.f * A2) * y + A1 * x) + y * QG - B1 * q + 2.f * q2 * y * L;
+      vz = J02 * v_m2x + J12 * v_m2y + v_depth - q * (A0 + A2) + 2.f * q2 * Qf + 2.f * z * q2 * L;
+    }
+  }
   // camera -> world
   const float* W = cam.r;
   v_mean[0] += W[0] * vx + W[3] * vy + W[6] * vz;

@@ -10,12 +10,18 @@
 // A third flag, kDepthGrad, passes the depth cotangent of gradient-record slot 11 (written by the depth blend) to
 // project_bwd; projection.cu includes the file again under egs::depth with it set.  The forms without it read 0, so
 // their registers and code are those of the kernels before the flag existed.
+// kCameraModel: see projection_kernels.cuh.  The ortho and fisheye forms are compiled with kDepthGrad only: slot 11 is 0
+// from every blend backward but the depth one, so one set of forms serves every render mode.
 // (No include guard on purpose.)
 
 // Camera-gradient floats per (camera, Gaussian) pair and per warp partial: 15 padded to 16 for the view matrices, with
 // the intrinsics 15 + 4 padded to 20.
 constexpr int kCamAccFloats = kKsGrad ? kCamGradFloats + kKsGradFloats : kCamGradFloats;
 constexpr int kCamPartialStride = kKsGrad ? kCamKsPartialFloats : kCamPartialFloats;
+// Near plane of the backward kernels' recomputation of the projection.  Visibility was decided by the forward pass, so
+// the recomputation must not cull a pair the forward kept: the ortho and fisheye forms cull nothing on z (near_plane
+// <= 0 lets z <= 0 through, fisheye theta up to pi).  The pinhole forms keep the 0 they have always been built with.
+constexpr float kBwdNearPlane = kCameraModel == kPinhole ? 0.f : -INFINITY;
 
 // One thread per Gaussian, looping over cameras: gradients summed over cameras stay in registers,
 // so there are no atomics for any C.  Every output element is written exactly once (zeros for culled
@@ -92,13 +98,13 @@ __global__ void __launch_bounds__(kProjBwdThreads) projection_bwd_kernel(const P
       }
       ProjState st;
       ProjOut o;
-      project_fwd(mean, quat, scale, *cam, p.width, p.height, p.eps2d, 0.f, INFINITY, -1.f, st, o);
+      project_fwd<kCameraModel>(mean, quat, scale, *cam, p.width, p.height, p.eps2d, kBwdNearPlane, INFINITY, -1.f, st, o);
       // (culling thresholds are irrelevant here: visibility was decided by the forward pass; the
       //  off-screen test cannot fire differently because it only depends on the same values.)
       float v_comp = 0.f, w_opac = 1.f;
       if (p.antialiased) { v_comp = g1.y * __ldg(p.opacities + n); w_opac = o.comp; }
       if (o.radius > 0)
-        project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, v_comp, p.eps2d,
+        project_bwd<kCameraModel>(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, v_comp, p.eps2d,
                     VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
       v_opac += g1.y * w_opac;
       v_rgb[0] = g1.z; v_rgb[1] = g1.w; v_rgb[2] = g2.x;
@@ -142,8 +148,9 @@ __global__ void __launch_bounds__(kProjBwdThreads) projection_bwd_kernel(const P
 // rows of the camera (zeros for rows it does not see) coalesced before moving on.
 // kKsGrad (VG forms only): the partials also carry v_fx, v_fy, v_cx, v_cy.
 // kDepthGrad: the per-camera form spills 16 bytes at 168 registers even without VG, so it runs 2 CTAs per SM as well.
+// kFisheye: the classic VG form spills 32 bytes at 168 registers (the fisheye Jacobian's VJP), so it runs 2 as well.
 template <bool AA, bool VG = false>
-__global__ void EGS_PB_BOUNDS(((kPerCameraSh || kKsGrad) && VG) || (kDepthGrad && kPerCameraSh)) projection_bwd_sh16_kernel(const ProjBwdParams p) {
+__global__ void EGS_PB_BOUNDS(((kPerCameraSh || kKsGrad || (kCameraModel == kFisheye && !AA)) && VG) || (kDepthGrad && kPerCameraSh)) projection_bwd_sh16_kernel(const ProjBwdParams p) {
   static_assert(VG || !kKsGrad, "intrinsics gradients are reduced with the view-matrix gradient partials");
   extern __shared__ __align__(16) float smem_pb[];
   __shared__ Camera cams[kMaxCamerasSmem];
@@ -267,17 +274,17 @@ __global__ void EGS_PB_BOUNDS(((kPerCameraSh || kKsGrad) && VG) || (kDepthGrad &
       {
         ProjState st;
         ProjOut o;
-        project_fwd(mean, quat, scale, *cam, p.width, p.height, p.eps2d, 0.f, INFINITY, -1.f, st, o);
+        project_fwd<kCameraModel>(mean, quat, scale, *cam, p.width, p.height, p.eps2d, kBwdNearPlane, INFINITY, -1.f, st, o);
         if constexpr (AA) {
           float op = __ldg(p.opacities + n);
           if (p.raw) op = act_sigmoid(op);
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, g1.y * op, p.eps2d,
+            project_bwd<kCameraModel>(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, g1.y * op, p.eps2d,
                         VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y * o.comp;
         } else {
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
+            project_bwd<kCameraModel>(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
                         VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y;
         }
@@ -478,16 +485,16 @@ __global__ void __launch_bounds__(kPB2Threads, kSh4BwdMinCtas) projection_bwd_sh
       {
         ProjState st;
         ProjOut o;
-        project_fwd(mean, quat, scale, *cam, p.width, p.height, p.eps2d, 0.f, INFINITY, -1.f, st, o);
+        project_fwd<kCameraModel>(mean, quat, scale, *cam, p.width, p.height, p.eps2d, kBwdNearPlane, INFINITY, -1.f, st, o);
         if constexpr (AA) {
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale,
+            project_bwd<kCameraModel>(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale,
                         g1.y * __ldg(p.opacities + n), p.eps2d, VG ? vcam : nullptr, mean,
                         kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y * o.comp;
         } else {
           if (o.radius > 0)
-            project_bwd(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
+            project_bwd<kCameraModel>(st, scale, *cam, v_m2x, v_m2y, kDepthGrad ? g2.w : 0.f, g0.z, g0.w, g1.x, o, v_mean, v_quat, v_scale, 0.f, 0.f,
                         VG ? vcam : nullptr, mean, kKsGrad ? vcam + kCamGradFloats : nullptr);
           v_opac += g1.y;
         }

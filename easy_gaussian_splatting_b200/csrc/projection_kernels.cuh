@@ -3,6 +3,8 @@
 // coefficients [N,K,3] shared by all cameras, or direct colours) and in egs::percam with kPerCameraSh = true (SH
 // coefficients [C,N,K,3], one row per (camera, Gaussian)).  The per-camera code is behind `if constexpr`, so the
 // shared-coefficient kernels keep their names and compile exactly as without it.
+// kCameraModel (egs_math.cuh kPinhole / kOrtho / kFisheye) is the camera model of project_fwd / project_bwd: kPinhole in
+// projection.cu; projection_ortho.cu and projection_fisheye.cu include this file in egs::ortho and egs::fisheye.
 // (No include guard on purpose.)
 
 template <bool VEC4>
@@ -28,7 +30,7 @@ __global__ void __launch_bounds__(kProjThreads) projection_fwd_kernel(const Proj
 
   ProjState st;
   ProjOut o;
-  const bool vis = project_fwd(mean, quat, scale, cam, p.width, p.height, p.eps2d, p.near_plane, p.far_plane,
+  const bool vis = project_fwd<kCameraModel>(mean, quat, scale, cam, p.width, p.height, p.eps2d, p.near_plane, p.far_plane,
                                p.radius_clip, st, o);
   int32_t ntiles = 0;
   int2 tight = make_int2(0, 0);
@@ -102,7 +104,7 @@ __global__ void __launch_bounds__(kPF2Threads) projection_fwd_sh16_kernel(const 
     scale[2] = __ldg(p.scales + 3 * (size_t)n + 2);
     if (p.raw) { scale[0] = act_exp(scale[0]); scale[1] = act_exp(scale[1]); scale[2] = act_exp(scale[2]); }
     ProjState st;
-    vis = project_fwd(mean, quat, scale, cam, p.width, p.height, p.eps2d, p.near_plane, p.far_plane, p.radius_clip, st, o);
+    vis = project_fwd<kCameraModel>(mean, quat, scale, cam, p.width, p.height, p.eps2d, p.near_plane, p.far_plane, p.radius_clip, st, o);
   }
   const uint32_t vis_mask = __ballot_sync(0xffffffffu, vis);
   const int nb = (p.sh_degree + 1) * (p.sh_degree + 1);
@@ -211,7 +213,7 @@ __global__ void __launch_bounds__(kPF2Threads) projection_fwd_sh4_kernel(const P
     scale[1] = __ldg(p.scales + 3 * (size_t)n + 1);
     scale[2] = __ldg(p.scales + 3 * (size_t)n + 2);
     ProjState st;
-    vis = project_fwd(mean, quat, scale, cam, p.width, p.height, p.eps2d, p.near_plane, p.far_plane, p.radius_clip, st, o);
+    vis = project_fwd<kCameraModel>(mean, quat, scale, cam, p.width, p.height, p.eps2d, p.near_plane, p.far_plane, p.radius_clip, st, o);
   }
   const uint32_t vis_mask = __ballot_sync(0xffffffffu, vis);
   if (vis_mask != 0)

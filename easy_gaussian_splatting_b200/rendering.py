@@ -23,7 +23,7 @@ from torch import Tensor
 
 from . import stages
 
-__all__ = ["rasterization", "rasterization_from_parameters"]
+__all__ = ["rasterization", "rasterization_camera_model", "rasterization_from_parameters"]
 
 
 class _LazyMeta(dict):
@@ -220,7 +220,8 @@ class _Rasterization(torch.autograd.Function):
         with stages.nvtx_range("egs.projection_fwd"):
             proj = stages.projection_fwd(means, quats, scales, opacities, rgb, viewmats, Ks, width, height, sh_degree,
                                          eps2d=cfg["eps2d"], near_plane=cfg["near_plane"], far_plane=cfg["far_plane"],
-                                         radius_clip=cfg["radius_clip"], antialiased=cfg["antialiased"])
+                                         radius_clip=cfg["radius_clip"], antialiased=cfg["antialiased"],
+                                         **_camera_model_keyword(cfg))
         cfg["compensations"] = proj.get("compensations")  # non-differentiable side output, like the thunk below
         tiles_per_gauss = proj["tiles_per_gauss"]
         blend_bg = backgrounds
@@ -296,7 +297,7 @@ class _Rasterization(torch.autograd.Function):
             out = stages.projection_bwd(means, quats, scales, colors, viewmats, Ks, width, height, cfg["sh_degree"],
                                         cfg["eps2d"], radii, colors_rgb, v_splats, v_means2d, want_absgrad=target is not None,
                                         antialiased_opacities=opacities if cfg["antialiased"] else None, opacities=opacities,
-                                        **want_cam)
+                                        **_camera_model_keyword(cfg), **want_cam)
         v_means, v_quats, v_scales, v_opac, v_cols = out[:5]
         if feat:
             v_cols = v_features
@@ -311,6 +312,12 @@ class _Rasterization(torch.autograd.Function):
             vc = v_colors[..., :backgrounds.shape[-1]] if depth else v_colors  # the colour channels only
             v_bg = ((1.0 - render_alphas) * vc).sum(dim=(1, 2))
         return v_means, v_quats, v_scales, v_opac, v_cols, v_viewmats, v_Ks, v_bg, None
+
+
+def _camera_model_keyword(cfg: dict) -> Dict[str, str]:
+    """The projection stages' camera_model keyword: passed only for a model other than the pinhole, so that pinhole
+    calls are exactly the ones rasterization() makes."""
+    return {} if cfg["camera_model"] == "pinhole" else {"camera_model": cfg["camera_model"]}
 
 
 def _camera_grad_keywords(want_viewmats: bool, want_Ks: bool) -> Dict[str, bool]:
@@ -479,7 +486,68 @@ def rasterization(
     ``render_alphas.clamp(min=1e-10)``.  "RGB+ED" returns [C,H,W,D+1] (the colours, then the expected depth), "ED"
     [C,H,W,1]; ``render_alphas`` and ``meta`` are those of "RGB".  Gradients of the depth reach the geometry,
     ``viewmats`` and absgrad; in "ED" ``colors`` and ``backgrounds`` get none, in "RGB+ED" ``backgrounds`` [C,D] get the
-    colour channels' gradient.  "D" and "RGB+D" raise ``NotImplementedError``."""
+    colour channels' gradient.  "D" and "RGB+D" raise ``NotImplementedError``.
+    The camera is a pinhole; ``rasterization_camera_model`` takes orthographic and fisheye cameras as well."""
+    return _rasterization(means, quats, scales, opacities, colors, viewmats, Ks, width, height, near_plane, far_plane,
+                          radius_clip, eps2d, sh_degree, packed, tile_size, backgrounds, render_mode, sparse_grad, absgrad,
+                          rasterize_mode, "pinhole")
+
+
+CAMERA_MODELS = ("pinhole", "ortho", "fisheye")
+
+
+def rasterization_camera_model(
+    means: Tensor,
+    quats: Tensor,
+    scales: Tensor,
+    opacities: Tensor,
+    colors: Tensor,
+    viewmats: Tensor,
+    Ks: Tensor,
+    width: int,
+    height: int,
+    near_plane: float = 0.01,
+    far_plane: float = 1e10,
+    radius_clip: float = 0.0,
+    eps2d: float = 0.3,
+    sh_degree: Optional[int] = None,
+    packed: bool = True,
+    tile_size: int = 16,
+    backgrounds: Optional[Tensor] = None,
+    render_mode: str = "RGB",
+    sparse_grad: bool = False,
+    absgrad: bool = False,
+    rasterize_mode: str = "classic",
+    channel_chunk: int = 32,
+    camera_model: str = "pinhole",
+) -> Tuple[Tensor, Tensor, Dict]:
+    """``rasterization()`` with a camera model, as later gsplat releases take it: ``camera_model`` "pinhole", "ortho" or
+    "fisheye"; every other argument, output and gradient (``viewmats`` and ``Ks`` included) as in ``rasterization()``,
+    which ``camera_model="pinhole"`` is exactly.  With (x, y, z) the camera-space mean and fx, fy, cx, cy from ``Ks``:
+
+    - "pinhole": means2d = (fx x / z + cx, fy y / z + cy), with gsplat's 1.3 x fov clamp in the Jacobian.
+    - "ortho": means2d = (fx x + cx, fy y + cy) (fx, fy in pixels per world unit), J = [[fx, 0, 0], [0, fy, 0]].
+    - "fisheye": equidistant, r = sqrt(x^2 + y^2), theta = atan2(r, z): means2d = (fx x theta / r + cx,
+      fy y theta / r + cy), J the exact Jacobian of means2d (gsplat's fisheye_proj).  theta / r is a polynomial that
+      is exact in fp32 to 2 ulp for theta in [0, pi) and equals 1 / z on the optical axis.
+
+    Neither "ortho" nor "fisheye" has an fov clamp, and both project z <= 0 as well: with ``near_plane <= 0``, Gaussians
+    behind the camera are rendered and differentiated (fisheye theta up to pi).  The near / far cull on z, the eps2d blur, the radius, the
+    off-screen test and the antialiased compensation are the same for all models, and ``meta["depths"]`` is the
+    camera-space z for all of them, so "ED" renders the expected z.  ``Ks`` gradients: v_cx, v_cy sum the means2d
+    cotangents and v_fx = (v_m2x (m2x - cx) + sum_j v_J0j J0j) / fx (likewise v_fy).  Any other ``camera_model`` raises
+    ``ValueError``."""
+    if camera_model not in CAMERA_MODELS:
+        raise ValueError(f"camera_model must be one of {CAMERA_MODELS}, got {camera_model!r}")
+    return _rasterization(means, quats, scales, opacities, colors, viewmats, Ks, width, height, near_plane, far_plane,
+                          radius_clip, eps2d, sh_degree, packed, tile_size, backgrounds, render_mode, sparse_grad, absgrad,
+                          rasterize_mode, camera_model)
+
+
+def _rasterization(means, quats, scales, opacities, colors, viewmats, Ks, width, height, near_plane, far_plane,
+                   radius_clip, eps2d, sh_degree, packed, tile_size, backgrounds, render_mode, sparse_grad, absgrad,
+                   rasterize_mode, camera_model):
+    """The one path of rasterization() and rasterization_camera_model()."""
     if render_mode not in ("RGB",) + DEPTH_MODES:
         raise NotImplementedError(f"render_mode={render_mode!r}: 'RGB', 'ED' and 'RGB+ED' are implemented")
     if rasterize_mode not in ("classic", "antialiased"):
@@ -496,7 +564,7 @@ def rasterization(
     cfg = dict(width=width, height=height, sh_degree=sh_degree, eps2d=float(eps2d), near_plane=float(near_plane),
                far_plane=float(far_plane), radius_clip=float(radius_clip), absgrad=bool(absgrad),
                antialiased=rasterize_mode == "antialiased", grad_enabled=torch.is_grad_enabled(),
-               features=sh_degree is None and colors.shape[-1] != 3, render_mode=render_mode)
+               features=sh_degree is None and colors.shape[-1] != 3, render_mode=render_mode, camera_model=camera_model)
     outs = _Rasterization.apply(means, quats, scales, opacities, colors, viewmats, Ks, backgrounds, cfg)
     meta_colors = None
     if cfg["features"]:  # gsplat: the colours as given, per (camera, Gaussian)

@@ -147,15 +147,27 @@ def level1_end_bit(C: int) -> int:
     return 32
 
 
+# camera_model codes of the ABI's camera-model entries (include/egs_raster.h); "pinhole" uses the other entries
+CAMERA_MODELS = {"pinhole": 0, "ortho": 1, "fisheye": 2}
+
+
+def _camera_model_code(camera_model: str) -> int:
+    if camera_model not in CAMERA_MODELS:
+        raise ValueError(f"camera_model must be one of {tuple(CAMERA_MODELS)}, got {camera_model!r}")
+    return CAMERA_MODELS[camera_model]
+
+
 def projection_fwd(means: Tensor, quats: Tensor, scales: Tensor, opacities: Tensor, colors: Tensor,
                    viewmats: Tensor, Ks: Tensor, width: int, height: int, sh_degree: Optional[int],
                    eps2d: float = 0.3, near_plane: float = 0.01, far_plane: float = 1e10,
                    radius_clip: float = 0.0, tile_size: int = TILE_SIZE,
-                   antialiased: bool = False) -> Dict[str, Tensor]:
+                   antialiased: bool = False, camera_model: str = "pinhole") -> Dict[str, Tensor]:
     """g1+g2+count(g3).  colors: [N,K,3] or per-camera [C,N,K,3] SH coefficients when sh_degree is not None, else
     [N,3]/[C,N,3].
     antialiased: gsplat's rasterize_mode="antialiased" — adds out["compensations"] [C,N]; the splat records then
-    carry opacity * compensation."""
+    carry opacity * compensation.
+    camera_model: "pinhole", "ortho" or "fisheye" (egs_projection_fwd_camera_model for the latter two)."""
+    cm = _camera_model_code(camera_model)
     lib = _lib.load()
     means, quats, scales = _f32c(means, "means"), _f32c(quats, "quats"), _f32c(scales, "scales")
     opacities, colors = _f32c(opacities, "opacities"), _f32c(colors, "colors")
@@ -185,6 +197,9 @@ def projection_fwd(means: Tensor, quats: Tensor, scales: Tensor, opacities: Tens
     with torch.cuda.device(dev):
         if antialiased:
             out["compensations"] = torch.empty(C, N, dtype=torch.float32, device=dev)
+        if cm:
+            rc = lib.egs_projection_fwd_camera_model(cm, *args, _ptr(out.get("compensations")), _stream(dev))
+        elif antialiased:
             rc = lib.egs_projection_fwd_antialiased(*args, _ptr(out["compensations"]), _stream(dev))
         else:
             rc = lib.egs_projection_fwd(*args, _stream(dev))
@@ -197,14 +212,17 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
                    colors_rgb: Tensor, v_splats: Tensor, v_means2d_extra: Optional[Tensor] = None,
                    want_absgrad: bool = False, antialiased_opacities: Optional[Tensor] = None,
                    opacities: Optional[Tensor] = None, want_viewmats_grad: bool = False, want_Ks_grad: bool = False,
-                   depth_grad: bool = False):
+                   depth_grad: bool = False, camera_model: str = "pinhole"):
     """g8+g9. -> v_means[N,3], v_quats[N,4], v_scales[N,3], v_opacities[N], v_colors (shape of colors)
     (+ absgrad[C,N,2] when want_absgrad) (+ v_viewmats[C,4,4] when want_viewmats_grad) (+ v_Ks[C,3,3] when
     want_Ks_grad, always last).
     antialiased_opacities: the opacities[N] of an antialiased forward; opacities: only consulted for a registered
     gradient buffer (register_grad_target).
     depth_grad: also take slot 11 of v_splats (v_depth, from rasterize_bwd_depth) as the gradient w.r.t. the
-    camera-space depths (egs_projection_bwd_depth); otherwise that slot is not read."""
+    camera-space depths (egs_projection_bwd_depth); otherwise that slot is not read.
+    camera_model: "pinhole", "ortho" or "fisheye"; the latter two always go through egs_projection_bwd_camera_model,
+    which always reads slot 11 (0 unless the blend was a depth one)."""
+    cm = _camera_model_code(camera_model)
     lib = _lib.load()
     dev = means.device
     means, quats, scales, colors, viewmats, Ks = dense_inputs(means, quats, scales, colors, viewmats, Ks)
@@ -230,16 +248,20 @@ def projection_bwd(means: Tensor, quats: Tensor, scales: Tensor, colors: Tensor,
     with torch.cuda.device(dev):
         if want_viewmats_grad:
             v_viewmats = torch.empty(C, 4, 4, dtype=torch.float32, device=dev)
-        if want_Ks_grad or want_viewmats_grad or depth_grad:
+        if want_Ks_grad or want_viewmats_grad or depth_grad or cm:
             aa = antialiased_opacities is not None
             aa_op = _f32c(antialiased_opacities, "opacities") if aa else None
             head = (C, N, _ptr(means), _ptr(quats), _ptr(scales), _ptr(aa_op), *tail[:-1], int(aa), _ptr(v_viewmats))
-        if depth_grad:
+        if depth_grad or cm:
             if want_Ks_grad:
                 v_Ks = torch.empty(C, 3, 3, dtype=torch.float32, device=dev)
             ws = (_intrinsics_workspace(lib, C, N, dev) if want_Ks_grad else _viewmats_workspace(lib, C, N, dev)
                   if want_viewmats_grad else None)
-            rc = lib.egs_projection_bwd_depth(*head, _ptr(v_Ks), _ptr(ws), 0 if ws is None else ws.numel(), tail[-1])
+            ws_args = (_ptr(v_Ks), _ptr(ws), 0 if ws is None else ws.numel(), tail[-1])
+            if cm:
+                rc = lib.egs_projection_bwd_camera_model(cm, *head, *ws_args)
+            else:
+                rc = lib.egs_projection_bwd_depth(*head, *ws_args)
         elif want_Ks_grad:  # one launch for both camera gradients
             v_Ks = torch.empty(C, 3, 3, dtype=torch.float32, device=dev)
             ws = _intrinsics_workspace(lib, C, N, dev)

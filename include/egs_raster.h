@@ -219,6 +219,34 @@ int egs_projection_bwd_depth(int32_t C, int32_t N, const float* means, const flo
                              int32_t antialiased, float* v_viewmats, float* v_Ks, void* workspace,
                              int64_t workspace_bytes, egs_stream_t stream);
 
+/* ---- orthographic and fisheye camera models ----------------------------------------------------------------------------
+ * The projection of the entries above for another camera model; pinhole calls keep the entries above.
+ *   camera_model = 1 (ortho):   means2d = (fx x + cx, fy y + cy), J = [[fx, 0, 0], [0, fy, 0]];
+ *   camera_model = 2 (fisheye): equidistant, r = sqrt(x^2 + y^2), theta = atan2(r, z),
+ *                               means2d = (fx x theta / r + cx, fy y theta / r + cy), J its exact Jacobian;
+ * (x, y, z) the camera-space mean.  Neither has the pinhole fov clamp; culling, the eps2d blur, radius, compensation and
+ * depths (camera-space z) are the pinhole ones.  Any other camera_model is rejected before any launch.
+ * egs_projection_fwd_camera_model: egs_projection_fwd, or egs_projection_fwd_antialiased when compensations is not NULL.
+ * egs_projection_bwd_camera_model: egs_projection_bwd_depth for the camera model (slot 11 of the gradient records is
+ *   always read; it is 0 from every blend backward but the depth one), same nullable v_viewmats / v_Ks and workspace.
+ *   v_Ks[c] = [[v_fx, 0, v_cx], [0, v_fy, v_cy], [0, 0, 0]] with v_fx = (v_m2x (m2x - cx) + sum_j v_J0j J0j) / fx. */
+int egs_projection_fwd_camera_model(int32_t camera_model, int32_t C, int32_t N, const float* means, const float* quats,
+                                    const float* scales, const float* opacities, const float* sh_coeffs, int32_t K,
+                                    int32_t sh_degree, int32_t colors_per_camera, const float* viewmats, const float* Ks,
+                                    int32_t width, int32_t height, float eps2d, float near_plane, float far_plane,
+                                    float radius_clip, int32_t tile_size, int32_t tile_width, int32_t tile_height,
+                                    int32_t* radii, float* means2d, float* depths, float* conics, float* colors,
+                                    int32_t* tiles_per_gauss, int32_t* tight_rects, float* splats, float* compensations,
+                                    egs_stream_t stream);
+int egs_projection_bwd_camera_model(int32_t camera_model, int32_t C, int32_t N, const float* means, const float* quats,
+                                    const float* scales, const float* opacities, const float* sh_coeffs, int32_t K,
+                                    int32_t sh_degree, int32_t colors_per_camera, const float* viewmats, const float* Ks,
+                                    int32_t width, int32_t height, float eps2d, const int32_t* radii, const float* colors,
+                                    const float* v_splats, const float* v_means2d_extra, float* v_means, float* v_quats,
+                                    float* v_scales, float* v_opacities, float* v_sh_coeffs, float* absgrad,
+                                    int32_t antialiased, float* v_viewmats, float* v_Ks, void* workspace,
+                                    int64_t workspace_bytes, egs_stream_t stream);
+
 /* ---- g3: exclusive scan of tiles_per_gauss, then key emission -------------------------------------
  * Replaces `torch.cumsum` + the second launch of gsplat `isect_tiles`.
  * egs_exclusive_scan: out[i] = sum_{j<i} in[j] (int64), *total = sum of all (device int64). */
